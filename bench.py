@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — headline benchmark: YOLOv3-416 (80 classes) frames/s at batch 64 per GPU, preprocess -> NMS.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--config NAME]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--config NAME] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 One "step" = one pass of the detection hot path over one batch of synthetic frames per GPU
@@ -31,6 +31,12 @@ JSON keys beyond the base contract:
                 Runtime's CPU EP, which is not installable here + the reference's Python pre/post restated),
                 timed on this box's host cores on a bounded sample of the same workload (rank 0, N=1 only)
 --impl reference times that same CPU path as its own arm.
+
+--dump-outputs DIR (b200 arm of headline / rsu / 608, rank 0) writes what the last timed step computed as
+DIR/<name>.npy: the detection records of every frame of the step, one float64 array per record field (det_<field>[frame,
+slot], frames in the step's order, slots past det_count zeroed), and the fp32 head tensors of a fixed seeded sample of
+those frames (head<i>[k] belongs to frame head_frames[k]).  Model and frames come from fixed seeds, so two builds run
+with the same arguments can be compared file for file.
 """
 from __future__ import annotations
 
@@ -247,8 +253,8 @@ def run_reference(args):
 
 def run_tiny_cpu(args):
     """BASELINE config 1: YOLOv3-tiny 416 (80 classes), batch 1, on the reference CPU path; dog.jpg (the reference's
-    testdata fixture, committed as tests/golden/ref_images.npz) and a dog-shaped synthetic frame; 20 warm-up + 200 timed
-    calls; p50 / p90 and the stage split."""
+    testdata fixture, committed as tests/golden/ref_images.npz) and a dog-shaped synthetic frame; 20 warm-up + --steps
+    timed calls (200 unless given); p50 / p90 and the stage split."""
     rank, _, _ = dist_env()
     if rank != 0:
         return 0
@@ -269,7 +275,7 @@ def run_tiny_cpu(args):
     Image.fromarray(modelgen.synthetic_frame(0, 416), "RGB").save(buf, format="JPEG", quality=90)
     payloads["synthetic q90"] = buf.getvalue()
     out = {}
-    calls = max(args.steps, 20) if args.steps != 100 else 200
+    calls = args.steps
     for name, data in payloads.items():
         lat, dec = [], []
         for i in range(20 + calls):
@@ -375,6 +381,43 @@ def parity_in_run(model, onnx_bytes, w, frames, n, sp):
     return out
 
 
+DUMP_HEAD_FRAMES = 4  # full head maps of 4 frames: 14.5 MB at 416 x 416, 31 MB at 608 x 608 (80 classes)
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def last_step_outputs(model, n, batches, run_batch, sp):
+    """--dump-outputs: the records fd_fetch returns for every frame of the last timed step, and the heads of a seeded
+    sample of those frames.  The model's buffers hold only the batch it ran last; the step's earlier batches (608: four
+    batches of 64 frames per GPU) are run again with run_batch(b) from the same inputs, which the deterministic path
+    turns into the same outputs."""
+    from fastdet_b200 import _native
+    frames = np.sort(np.random.default_rng(0).choice(n * batches, min(n * batches, DUMP_HEAD_FRAMES), replace=False))
+    got = {}
+    for b in [batches - 1] + list(range(batches - 1)):  # the last batch first, while it is still in the buffers
+        if b != batches - 1:
+            run_batch(b)
+        dets, counts, total = model.fetch(n, stream=sp)
+        mine = frames[(frames >= b * n) & (frames < (b + 1) * n)] - b * n
+        got[b] = (dets, counts, total, [h[mine] for h in model.heads(n)] if len(mine) else [])
+    dets, counts, total = (np.concatenate([got[b][k] for b in range(batches)]) for k in range(3))
+    valid = np.arange(dets.shape[1])[None, :] < counts[:, None]
+    out = {"det_count": counts.astype(np.float64), "det_total": total.astype(np.float64)}
+    for field in _native.DET_DTYPE.names:
+        out["det_" + field] = np.where(valid, dets[field], 0).astype(np.float64)
+    out["head_frames"] = frames.astype(np.float64)
+    for i in range(len(model.head_shapes)):
+        out[f"head{i}"] = np.concatenate([got[b][3][i] for b in range(batches) if got[b][3]])
+    size = sum(a.nbytes for a in out.values())
+    assert size <= DUMP_LIMIT_BYTES, f"--dump-outputs would write {size} bytes"
+    return out
+
+
+def write_outputs(path, arrays):
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), a)
+
+
 def run_b200(args):
     import torch
     from fastdet_b200 import _native, modelgen
@@ -425,18 +468,21 @@ def run_b200(args):
     sp = stream.cuda_stream
     assert sp != 0
 
+    def run_batch(i, b, ev=None):
+        d = dev_sets[(i * batches_per_step + b) % 4]
+        model.preprocess(d.data_ptr(), n, (size, size), on_device=True, stream=sp)
+        if ev:
+            ev[3 * b].record(stream)
+        model.forward(n, stream=sp)
+        if ev:
+            ev[3 * b + 1].record(stream)
+        model.postprocess(n, THRESHOLD, max_det=MAX_DET, stream=sp)
+        if ev:
+            ev[3 * b + 2].record(stream)
+
     def step_device(i, ev=None):
         for b in range(batches_per_step):
-            d = dev_sets[(i * batches_per_step + b) % 4]
-            model.preprocess(d.data_ptr(), n, (size, size), on_device=True, stream=sp)
-            if ev:
-                ev[3 * b].record(stream)
-            model.forward(n, stream=sp)
-            if ev:
-                ev[3 * b + 1].record(stream)
-            model.postprocess(n, THRESHOLD, max_det=MAX_DET, stream=sp)
-            if ev:
-                ev[3 * b + 2].record(stream)
+            run_batch(i, b, ev)
 
     def barrier():
         if use_dist:
@@ -465,6 +511,11 @@ def run_b200(args):
     elapsed_ms = e0.elapsed_time(e1)
     fwd_ms = float(np.mean([ev[3 * b].elapsed_time(ev[3 * b + 1]) for ev in step_events for b in range(batches_per_step)]))
     post_ms = float(np.mean([ev[3 * b + 1].elapsed_time(ev[3 * b + 2]) for ev in step_events for b in range(batches_per_step)]))
+    # read back before the regions below reuse the model's buffers
+    if args.dump_outputs and rank == 0:
+        dumped = last_step_outputs(model, n, batches_per_step, lambda b: run_batch(args.steps - 1, b), sp)
+    else:
+        dumped = None
 
     # ---- timed region 2: end to end through the synchronous C-ABI call with pinned host frames
     out = np.zeros((n, MAX_DET), _native.DET_DTYPE)
@@ -632,6 +683,8 @@ def run_b200(args):
                                   "what": "fd_detect, 1 pinned host frame in, records out (H2D + D2H included), 1000 calls, host wall clock; "
                                           "device_only = CUDA events around preprocess(device frame) + forward + postprocess, 200 calls"}
         line["e2e"]["from_jpeg"] = jpeg_arm(model, sets[0], n, args.steps)
+    if dumped is not None:
+        write_outputs(args.dump_outputs, dumped)
     if rank == 0:
         print(json.dumps(line))
     if use_dist:
@@ -643,7 +696,7 @@ def run_b200(args):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=100)
+    ap.add_argument("--steps", type=int, default=None, help="timed steps (default 100; 200 calls for --config tiny-cpu)")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--config", default="headline", choices=sorted(WORKLOADS) + ["serve", "tiny-cpu"])
@@ -651,7 +704,17 @@ def main():
     ap.add_argument("--quick", action="store_true", help="skip the CPU baseline and the bs1 latency loop (profiling runs)")
     ap.add_argument("--no-parity", action="store_true", help="skip the in-run oracle check (profiling runs)")
     ap.add_argument("--seconds", type=float, default=20.0, help="--config serve: length of the measured run")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the records of every frame of the last timed step and "
+                                                           "the heads of a seeded sample of them as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.config == "serve" and args.steps is not None:
+        ap.error("--config serve runs for --seconds, not a number of steps")
+    if args.steps is None:
+        args.steps = 200 if args.config == "tiny-cpu" else 100
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "b200" or args.config not in WORKLOADS):
+        ap.error("--dump-outputs applies to the b200 arm of " + " / ".join(WORKLOADS))
     if args.config == "tiny-cpu":
         return run_tiny_cpu(args)
     if args.config == "serve":

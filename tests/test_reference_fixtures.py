@@ -6,13 +6,17 @@
   CPU: the restatement (oracle/ref_jpeg.py) and the library's host half reproduce the pixels the reference's decode
   lines give.  GPU: device decode bit-exact, perform(bytes) through the library's JPEG route == the reference's route
   (PIL pixels), and the detections against the oracle's restatement of perform() on those pixels.
+* dropin/detector.py as server.py uses it: imported as `detector` from a server/-shaped directory by a fresh
+  interpreter, constructed and called with the arguments server.py passes, its answer packed as the response the
+  reference client receives (DummyDetector on the CPU, ONNXDetector on the GPU).
 * server/server.py + server/client.py, UNCHANGED, over loopback with this repo's `detector` module in place of the
-  reference's (the deployment INTEGRATION.md §1 describes).  Needs /root/reference (present in the build container,
-  absent on the GPU box): skipped where it is missing.
+  reference's (the deployment INTEGRATION.md §1 describes).  Those two files are the original project's, not this
+  one's: the tests run when FASTDET_REFERENCE names a checkout of it and are skipped otherwise.
 """
 import hashlib
 import importlib.util
 import io
+import json
 import os
 import shutil
 import socket
@@ -30,7 +34,9 @@ from oracle import ref_jpeg
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(HERE)
-REF = os.environ.get("FASTDET_REFERENCE", "/root/reference")
+REF = os.environ.get("FASTDET_REFERENCE", "")
+NEEDS_REF = pytest.mark.skipif(not (REF and os.path.exists(os.path.join(REF, "server", "server.py"))),
+                               reason="needs FASTDET_REFERENCE: a checkout of the original project (server/server.py, server/client.py)")
 NAMES = ("dog", "rsu1", "rsu2")
 
 
@@ -82,6 +88,62 @@ def test_reference_images_on_device():
     assert det.jpeg_device_frames == len(NAMES) and det.jpeg_host_frames == 0
     t32.check("reference images vs fp32 oracle", min_solid=3)
     t16.check("reference images vs bf16-operand oracle", min_solid=3)
+
+
+# ------------------------------------------------------------------------------------------ the drop-in module
+# The calls server.py makes on its `detector` module (INTEGRATION.md §1), run by a fresh interpreter in a directory laid out
+# like the reference's server/ with dropin/detector.py as its detector.py.
+_SERVER_CALLS = r"""
+import json, sys
+from detector import DummyDetector, ONNXDetector                                          # server.py:17
+data_path, spec, threshold, dbgout = sys.argv[1], sys.argv[2], int(sys.argv[3]), sys.argv[4] or None
+if spec:                                                                                  # "name:classes:path", :355-358
+    name, num_classes, path = spec.split(":")
+    detector = ONNXDetector(path, mode=None, num_classes=int(num_classes), dbgout=dbgout)
+else:                                                                                     # no model argument, :359-360
+    detector = DummyDetector(dbgout=dbgout)
+with open(data_path, "rb") as fp:
+    print(json.dumps(detector.perform(fp.read(), threshold=threshold * 0.01)))           # :232
+"""
+
+
+def _perform_through_dropin(tmp_path, payload, spec="", threshold_percent=10, dbgout=""):
+    srv = tmp_path / "server"
+    srv.mkdir()
+    shutil.copy(os.path.join(ROOT, "dropin", "detector.py"), srv / "detector.py")
+    (tmp_path / "payload.jpg").write_bytes(payload)
+    env = dict(os.environ, FASTDET_B200_HOME=ROOT)  # where the deployment finds the package (INTEGRATION.md §1)
+    r = subprocess.run([sys.executable, "-c", _SERVER_CALLS, str(tmp_path / "payload.jpg"), spec, str(threshold_percent), dbgout],
+                       cwd=str(srv), env=env, stdout=subprocess.PIPE, stderr=subprocess.PIPE, text=True, timeout=300)
+    assert r.returncode == 0, r.stderr[-3000:]
+    return [tuple(t) for t in json.loads(r.stdout.strip().splitlines()[-1])]
+
+
+def test_dropin_module_answers_server_calls_dummy(tmp_path):
+    """No model argument: DummyDetector from the drop-in answers with the reference's fixed box, packed as the response
+    the reference client receives, and dumps the payload to dbgout as the reference's -o does."""
+    from oracle import ref_wire
+    dog = fixtures()["dog"][0]
+    got = _perform_through_dropin(tmp_path, dog, dbgout=str(tmp_path / "dbgout"))
+    assert got == [(16, 1.0, 208.0, 208.0, 166.4, 166.4)]
+    assert _unpack(ref_wire.pack_results(got, 7, 0)) == (7, [(16, 255, 208, 208, 166, 166)])
+    assert (tmp_path / "dbgout").read_bytes() == dog
+
+
+@pytest.mark.gpu
+def test_dropin_module_answers_server_calls_onnx(tmp_path):
+    """`name:classes:model.onnx`: ONNXDetector from the drop-in, built and called as server.py does, returns what the
+    package's ONNXDetector.perform returns for the same payload, and packs to the same response."""
+    from fastdet_b200 import detector as fdet
+    from oracle import ref_wire
+    data = modelgen.build_onnx("tiny", 80, 416, 1)
+    onnx_path = tmp_path / "tiny.onnx"
+    onnx_path.write_bytes(data)
+    dog = fixtures()["dog"][0]
+    got = _perform_through_dropin(tmp_path, dog, spec=f"tiny:80:{onnx_path}")
+    want = fdet.ONNXDetector(data, num_classes=80).perform(dog, threshold=0.1)
+    assert want and got == want
+    assert ref_wire.pack_results(got, 7, 0) == ref_wire.pack_results(want, 7, 0)
 
 
 # ------------------------------------------------------------------------------------------ the unchanged caller
@@ -148,7 +210,7 @@ def _unpack(resp):
     return reqid, [struct.unpack(">BBhhhh", resp[16 + i:26 + i]) for i in range(0, length, 10)]
 
 
-@pytest.mark.skipif(not os.path.exists(os.path.join(REF, "server", "server.py")), reason="needs the reference checkout")
+@NEEDS_REF
 def test_unchanged_server_and_client_round_trip_dummy(tmp_path):
     """No model argument -> server.py builds DummyDetector from OUR detector module (server.py:17,360) and answers the
     reference client's request with the packed fixed box (detector.py:83-92 -> server.py:234-239)."""
@@ -159,7 +221,7 @@ def test_unchanged_server_and_client_round_trip_dummy(tmp_path):
 
 
 @pytest.mark.gpu
-@pytest.mark.skipif(not os.path.exists(os.path.join(REF, "server", "server.py")), reason="needs the reference checkout")
+@NEEDS_REF
 def test_unchanged_server_and_client_round_trip_onnx(tmp_path):
     """`server.py full:80:model.onnx` with our module: the response the reference client receives is the wire packing of
     ONNXDetector.perform on the same payload.  (Runs only where a GPU and the reference checkout are both present.)"""
