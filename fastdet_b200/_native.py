@@ -51,8 +51,8 @@ class FdLayerDesc(C.Structure):
 class FdLayerExec(C.Structure):
     _fields_ = [("kernel", C.c_int32), ("bucket", C.c_int32), ("block_n", C.c_int32), ("split_k", C.c_int32),
                 ("grid", C.c_int32), ("num_stages", C.c_int32), ("kb_per_stage", C.c_int32), ("b_resident", C.c_int32),
-                ("smem_bytes", C.c_int32), ("chunk_frames", C.c_int32), ("launches", C.c_int32), ("tile_linked", C.c_int32),
-                ("reserved", C.c_int32 * 4)]
+                ("smem_bytes", C.c_int32), ("chunk_frames", C.c_int32), ("launches", C.c_int32),
+                ("reserved", C.c_int32 * 5)]
 
 
 KERNEL_NAMES = {0: "conv0", 1: "tc_single", 2: "tc_pair", 3: "tc_pair_strip", 4: "tc_swapped", 5: "halo", 6: "maxpool",

@@ -55,38 +55,33 @@ int fail(int code, const char* fmt, ...) {
 const float kAnchors3[3][3][2] = {{{116, 90}, {156, 198}, {373, 326}}, {{30, 61}, {62, 45}, {59, 119}}, {{10, 13}, {16, 30}, {33, 23}}};
 const float kAnchors2[2][3][2] = {{{81, 82}, {135, 169}, {344, 319}}, {{10, 14}, {23, 27}, {37, 58}}};
 
-// A run of leading layers executed chunk by chunk: the first stages of the network move hundreds of MB per layer at
-// batch 64 (conv1 writes 709 MB that conv2 reads back), far more than the 126 MB L2 holds, and their kernels are bound by
-// DRAM latency x bytes in flight, not by arithmetic.  Running layers first..last over `chunk` frames at a time keeps a
-// chunk's activations in L2 from the kernel that writes them to the kernel that reads them; buffers that only live inside
-// the segment are chunk-sized and reused by every chunk, so most of their lines are overwritten in L2 and never reach HBM.
-struct Segment { int first = 0, last = 0, chunk = 0; };
+// Launch descriptors of layers [0, layers) for pieces of `frames` frames each (piece k starts at frame k * frames, in the
+// same buffers): the whole batch is one piece over every layer, fd_detect's copy-overlapped front four quarter-batch
+// pieces over the leading layers.
+struct LaunchSet {
+    int layers = 0, frames = 0;
+    std::vector<std::vector<ConvLaunch>> conv;  // [layer][piece]
+    std::vector<std::vector<HaloLaunch>> halo;  // [layer][piece], used where use_halo[layer]
+    std::vector<char> use_halo;                 // [layer]
+    std::vector<StemLaunch> stem;               // [piece]; empty: no fused stem
+    std::vector<BlockLaunch> block;             // [piece]; empty: no fused block
+    size_t ws_bytes = 0, counter_ints = 0;      // split-K workspace the conv launches need (0: none)
+};
 
 struct Exec {  // everything that depends on the batch size
     int n = 0;
     std::vector<void*> bufs;
-    std::vector<char> buf_internal;  // 1: chunk-sized, reused by every chunk of its segment
-    std::vector<Segment> segs;
-    std::vector<int> seg_of;         // layer -> index into segs, -1: runs on the whole batch
-    // per layer, per chunk (one entry for layers outside a segment)
-    std::vector<std::vector<ConvLaunch>> conv;
-    std::vector<std::vector<HaloLaunch>> halo;  // used where use_halo[layer]
-    std::vector<char> use_halo;
+    LaunchSet whole;  // the forward pass
     // Fused stem (conv_stem.cu): layer 0 (u8 frames -> first convolution) runs inside layer 1's kernel; layer 0 has no launch
     // and its output tensor is never written (its buffer is only allocated when a parity hook asks for that tensor)
     bool use_stem = false;
-    std::vector<StemLaunch> stem;  // per chunk of layer 1's segment (one entry outside segments)
     // Fused residual block (conv_block.cu): layer block_layer (1x1) runs inside layer block_layer + 1's kernel (3x3 + residual)
     int block_layer = -1;          // -1: none
-    std::vector<BlockLaunch> block;
     // per layer: 0 launches its own kernel, 1 computed inside the next layer's kernel (no launch, no output tensor), 2 launches a
     // fused kernel that also does the previous layer's work
     std::vector<char> fused_role;
     float* splitk_ws = nullptr;     // shared by the split-K launches of this batch size (they run one after another)
     int* splitk_counters = nullptr;
-    int* tile_flags = nullptr;      // per-M-tile completion counters of the layers linked by tile-level dependencies
-    size_t tile_flag_ints = 0;      // (zeroed at the start of every forward pass)
-    int linked_layers = 0;
     uint8_t* frames = nullptr;     // [n, net_h, net_w, 3]
     uint8_t* src = nullptr;        // staging for frames that need the letterbox
     size_t src_cap = 0;
@@ -103,13 +98,9 @@ struct Exec {  // everything that depends on the batch size
     cudaGraphExec_t graph = nullptr;
     bool graph_tried = false;
     // fd_detect's copy-overlapped front (see forward_overlapping_copy): the layers in front of the second down-sampling
-    // layer get a second set of launch descriptors for quarter batches (same buffers, frame offsets), the rest is graph_tail
-    int ov_layers = 0, ov_chunk = 0;  // 0: not built / not applicable (-1 in ov_layers)
-    std::vector<std::vector<ConvLaunch>> ov_conv;
-    std::vector<std::vector<HaloLaunch>> ov_halo;
-    std::vector<char> ov_use_halo;
-    std::vector<StemLaunch> ov_stem;
-    std::vector<BlockLaunch> ov_block;
+    // layer run from `front` quarter batch by quarter batch, the rest is graph_tail
+    int ov_layers = 0;  // layers in the front; 0: not built yet, -1: not applicable
+    LaunchSet front;
     cudaGraphExec_t graph_tail = nullptr;
     bool graph_tail_tried = false;
 };
@@ -177,7 +168,7 @@ size_t buf_bytes(const BufferPlan& b, int n) { return size_t(n) * b.h * b.w * b.
 
 void free_exec(Exec* e) {
     for (void* p : e->bufs) cudaFree(p);
-    cudaFree(e->splitk_ws); cudaFree(e->splitk_counters); cudaFree(e->tile_flags);
+    cudaFree(e->splitk_ws); cudaFree(e->splitk_counters);
     cudaFree(e->frames); cudaFree(e->src); cudaFree(e->cand); cudaFree(e->cand_count); cudaFree(e->scores);
     cudaFree(e->dets); cudaFree(e->det_count); cudaFree(e->scratch);
     if (e->h_dets) cudaFreeHost(e->h_dets);
@@ -186,10 +177,9 @@ void free_exec(Exec* e) {
     if (e->graph_tail) cudaGraphExecDestroy(e->graph_tail);
 }
 
-// first byte of tensor `t` for chunk `k` of a segment with `chunk` frames (k = 0, chunk = 0: the whole batch)
-void* loc_ptr(const Exec& e, const ModelPlan& P, const TensorLoc& t, bool fp32, int k = 0, int chunk = 0) {
-    char* base = static_cast<char*>(e.bufs[t.buf]);
-    if (k && !e.buf_internal[t.buf]) base += static_cast<size_t>(k) * chunk * (buf_bytes(P.buffers[t.buf], 1));
+// first byte of tensor `t` for frames [k * frames, (k + 1) * frames) (k = 0: the whole batch)
+void* loc_ptr(const Exec& e, const ModelPlan& P, const TensorLoc& t, bool fp32, int k = 0, int frames = 0) {
+    char* base = static_cast<char*>(e.bufs[t.buf]) + static_cast<size_t>(k) * frames * buf_bytes(P.buffers[t.buf], 1);
     return base + size_t(t.ch_off) * (fp32 ? 4 : 2);
 }
 
@@ -203,47 +193,6 @@ int bucket_of(int n) {
     int b = 1;
     while (b < n) b *= 2;
     return b;
-}
-
-// Chunked leading segments for batch n (see Segment).  Segment boundaries sit in front of the 2nd and the 3rd
-// down-sampling layer (YOLOv3: [conv1..conv4] at 416/208, [conv5..conv9] at 104; the 52x52 stage and everything after it
-// run on the whole batch: their tensors are small enough and their tiles too few to cut).  The chunk is the largest power
-// of two of frames whose biggest tensor stays under the option chunk_mb (default 44 MB for the first segment, half of
-// that for the second: it also has to hold the residual inputs), and must divide n.
-void plan_segments(const ModelPlan& P, int n, std::vector<Segment>* out) {
-    out->clear();
-    const Options& O = options();
-    if (O.chunk_frames < 0 || n < 2) return;
-    std::vector<int> downs;  // layers that halve the map
-    for (size_t i = 0; i < P.layers.size(); ++i) {
-        const LayerPlan& L = P.layers[i];
-        const bool down = (L.kind == LAYER_CONV && L.stride == 2) || (L.kind == LAYER_MAXPOOL && L.pool_s == 2) || L.pool2;
-        if (down) downs.push_back(static_cast<int>(i));
-    }
-    if (downs.size() < 3) return;
-    const int bounds[3] = {0, downs[1], downs[2]};
-    for (int sgi = 0; sgi < 2; ++sgi) {
-        Segment sg;
-        sg.first = bounds[sgi]; sg.last = bounds[sgi + 1] - 1;
-        if (sg.last < sg.first) continue;
-        size_t biggest = 1;
-        for (int i = sg.first; i <= sg.last; ++i) {
-            const LayerPlan& L = P.layers[i];
-            if (L.out_fp32 || L.upsample2x || L.kind == LAYER_COPY) return;  // heads / route layers this early: not a YOLO-shaped graph, leave it alone
-            biggest = std::max(biggest, static_cast<size_t>(L.out.h) * L.out.w * L.out.c * 2);
-        }
-        int chunk;
-        if (O.chunk_frames > 0) chunk = sgi == 0 ? O.chunk_frames : 2 * O.chunk_frames;
-        else {
-            const double budget = (sgi == 0 ? 1.0 : 0.5) * O.chunk_mb * 1e6;
-            chunk = 1;
-            while (static_cast<double>(biggest) * (2 * chunk) <= budget) chunk *= 2;
-        }
-        while (chunk > 1 && n % chunk) chunk /= 2;
-        if (chunk >= n) continue;  // the whole batch already fits
-        sg.chunk = chunk;
-        out->push_back(sg);
-    }
 }
 
 // The fused stem applies when layer 0 is the u8 first convolution, layer 1 a 3x3 stride-2 convolution that is the ONLY
@@ -276,11 +225,12 @@ StemDesc stem_desc(const fd_model* m, int frames) {
     return d;
 }
 
-int prepare_stem(fd_model* m, Exec* e, int frames, int k, int chunk, StemLaunch* sl) {
+// the fused stem on frames [k * frames, (k + 1) * frames)
+int prepare_stem(fd_model* m, Exec* e, int frames, int k, StemLaunch* sl) {
     const ModelPlan& P = m->plan;
     StemDesc d = stem_desc(m, frames);
-    d.frames = e->frames + static_cast<size_t>(k) * chunk * P.net_h * P.net_w * 3;
-    d.out = static_cast<__nv_bfloat16*>(loc_ptr(*e, P, P.layers[1].out, false, k, chunk));
+    d.frames = e->frames + static_cast<size_t>(k) * frames * P.net_h * P.net_w * 3;
+    d.out = static_cast<__nv_bfloat16*>(loc_ptr(*e, P, P.layers[1].out, false, k, frames));
     char err[256] = "";
     if (conv_stem_prepare(d, m->num_sms, sl, err, sizeof(err))) return fail(FD_ERR_CUDA, "stem (layers 0 + 1): %s", err);
     return FD_OK;
@@ -323,23 +273,24 @@ BlockDesc block_desc(const fd_model* m, int layer, int frames) {
     return d;
 }
 
-int prepare_block(fd_model* m, Exec* e, int layer, int frames, int k, int chunk, BlockLaunch* bl) {
+// the fused block on frames [k * frames, (k + 1) * frames)
+int prepare_block(fd_model* m, Exec* e, int layer, int frames, int k, BlockLaunch* bl) {
     const ModelPlan& P = m->plan;
     BlockDesc d = block_desc(m, layer, frames);
-    d.in = static_cast<const __nv_bfloat16*>(loc_ptr(*e, P, P.layers[layer].in, false, k, chunk));
-    d.out = static_cast<__nv_bfloat16*>(loc_ptr(*e, P, P.layers[layer + 1].out, false, k, chunk));
+    d.in = static_cast<const __nv_bfloat16*>(loc_ptr(*e, P, P.layers[layer].in, false, k, frames));
+    d.out = static_cast<__nv_bfloat16*>(loc_ptr(*e, P, P.layers[layer + 1].out, false, k, frames));
     char err[256] = "";
     if (conv_block_prepare(d, m->num_sms, bl, err, sizeof(err))) return fail(FD_ERR_CUDA, "residual block (layers %d + %d): %s", layer, layer + 1, err);
     return FD_OK;
 }
 
-// tensor maps + launch geometry of conv layer i for `frames` frames, chunk k of its segment (k = chunk = 0: whole batch)
-int prepare_conv_layer(fd_model* m, Exec* e, size_t i, int frames, int k, int chunk, ConvLaunch* cl, HaloLaunch* hl, char* use_halo) {
+// tensor maps + launch geometry of conv layer i on frames [k * frames, (k + 1) * frames)
+int prepare_conv_layer(fd_model* m, Exec* e, size_t i, int frames, int k, ConvLaunch* cl, HaloLaunch* hl, char* use_halo) {
     const ModelPlan& P = m->plan;
     const LayerPlan& L = P.layers[i];
-    const __nv_bfloat16* in = static_cast<const __nv_bfloat16*>(loc_ptr(*e, P, L.in, false, k, chunk));
-    const __nv_bfloat16* res = L.res.buf >= 0 ? static_cast<const __nv_bfloat16*>(loc_ptr(*e, P, L.res, false, k, chunk)) : nullptr;
-    void* out = loc_ptr(*e, P, L.out, L.out_fp32 != 0, k, chunk);
+    const __nv_bfloat16* in = static_cast<const __nv_bfloat16*>(loc_ptr(*e, P, L.in, false, k, frames));
+    const __nv_bfloat16* res = L.res.buf >= 0 ? static_cast<const __nv_bfloat16*>(loc_ptr(*e, P, L.res, false, k, frames)) : nullptr;
+    void* out = loc_ptr(*e, P, L.out, L.out_fp32 != 0, k, frames);
     {   // narrow 3x3 layers on large maps: halo-patch kernel (conv_halo.cu)
         HaloDesc h;
         memset(&h, 0, sizeof(h));
@@ -376,9 +327,41 @@ int ensure_fused_away_buffer(fd_model* m, Exec* e, int layer) {
     const int b = P.layers[layer].out.buf;
     if (e->bufs[b]) return FD_OK;
     DEVICE_SETUP_LOCK(m);
-    const int frames = e->buf_internal[b] ? e->segs[e->seg_of[layer]].chunk : e->n;
-    cudaError_t err = cudaMalloc(&e->bufs[b], buf_bytes(P.buffers[b], frames));
+    cudaError_t err = cudaMalloc(&e->bufs[b], buf_bytes(P.buffers[b], e->n));
     if (err != cudaSuccess) return fail(FD_ERR_CUDA, "cudaMalloc(output of layer %d, batch %d) failed: %s", layer, e->n, cudaGetErrorString(err));
+    return FD_OK;
+}
+
+// Launch descriptors of layers [0, layers) for `pieces` pieces of `frames` frames, following the Exec's fusion plan.
+int prepare_set(fd_model* m, Exec* e, int layers, int pieces, int frames, LaunchSet* ls) {
+    const ModelPlan& P = m->plan;
+    ls->layers = layers; ls->frames = frames;
+    ls->conv.assign(layers, {});
+    ls->halo.assign(layers, {});
+    ls->use_halo.assign(layers, 0);
+    for (int i = 0; i < layers; ++i) {
+        if (P.layers[i].kind != LAYER_CONV) continue;
+        ls->conv[i].resize(pieces);
+        ls->halo[i].resize(pieces);
+        if (e->fused_role[i]) continue;  // fused layers: a tensor of the pair does not exist, the pair has its own launch below
+        for (int k = 0; k < pieces; ++k) {
+            char uh = 0;
+            if (int rc = prepare_conv_layer(m, e, i, frames, k, &ls->conv[i][k], &ls->halo[i][k], &uh)) return rc;
+            ls->use_halo[i] = uh;
+            ls->ws_bytes = std::max(ls->ws_bytes, ls->conv[i][k].ws_bytes);
+            ls->counter_ints = std::max(ls->counter_ints, ls->conv[i][k].counter_ints);
+        }
+    }
+    if (e->use_stem) {
+        ls->stem.resize(pieces);
+        for (int k = 0; k < pieces; ++k)
+            if (int rc = prepare_stem(m, e, frames, k, &ls->stem[k])) return rc;
+    }
+    if (e->block_layer >= 0 && e->block_layer < layers) {
+        ls->block.resize(pieces);
+        for (int k = 0; k < pieces; ++k)
+            if (int rc = prepare_block(m, e, e->block_layer, frames, k, &ls->block[k])) return rc;
+    }
     return FD_OK;
 }
 
@@ -391,49 +374,21 @@ int get_exec(fd_model* m, int n_frames, Exec** out) {
     std::unique_ptr<Exec> e(new Exec());
     e->n = n;
     const ModelPlan& P = m->plan;
-    plan_segments(P, n, &e->segs);
-    e->seg_of.assign(P.layers.size(), -1);
-    for (size_t sgi = 0; sgi < e->segs.size(); ++sgi)
-        for (int i = e->segs[sgi].first; i <= e->segs[sgi].last; ++i) e->seg_of[i] = static_cast<int>(sgi);
-    // a buffer is internal to a segment when its producer and every reader (input or residual) lie inside that segment
-    e->buf_internal.assign(P.buffers.size(), 0);
-    {
-        std::vector<int> seg_of_buf(P.buffers.size(), -2);  // -2 unseen, -1 touched outside any segment / by two segments
-        auto touch = [&](const TensorLoc& t, int layer) {
-            if (t.buf < 0) return;
-            const int sgi = e->seg_of[layer];
-            if (seg_of_buf[t.buf] == -2) seg_of_buf[t.buf] = sgi;
-            else if (seg_of_buf[t.buf] != sgi) seg_of_buf[t.buf] = -1;
-        };
-        for (size_t i = 0; i < P.layers.size(); ++i) { touch(P.layers[i].in, static_cast<int>(i)); touch(P.layers[i].out, static_cast<int>(i)); touch(P.layers[i].res, static_cast<int>(i)); }
-        for (size_t b = 0; b < P.buffers.size(); ++b) e->buf_internal[b] = seg_of_buf[b] >= 0 ? 1 : 0;
-    }
     e->bufs.assign(P.buffers.size(), nullptr);
-    // fused stem: decided here, from the shapes, because layer 0's output buffer is then not allocated at all
-    bool want_stem = false;
-    if (options().stem && stem_candidate(P) && e->seg_of[0] == e->seg_of[1]) {
-        const int sgi = e->seg_of[1];
-        want_stem = conv_stem_supported(stem_desc(m, sgi >= 0 ? e->segs[sgi].chunk : n));
-    }
-    int want_block = -1;
-    if (options().block) {
-        const int bc = block_candidate(P);
-        if (bc >= 0 && e->seg_of[bc] == e->seg_of[bc + 1] && conv_block_supported(block_desc(m, bc, e->seg_of[bc] >= 0 ? e->segs[e->seg_of[bc]].chunk : n)))
-            want_block = bc;
-    }
+    // fused kernels: decided here, from the shapes, because the output buffer of a fused-away layer is then not allocated at all
+    int32_t stem = 0, block = -1;
+    if (int rc = fd_planned_fusions(m, n, &stem, &block)) return rc;
+    e->use_stem = stem != 0;
+    e->block_layer = block;
     e->fused_role.assign(P.layers.size(), 0);
-    if (want_stem) { e->fused_role[0] = 1; e->fused_role[1] = 2; }
-    if (want_block >= 0) { e->fused_role[want_block] = 1; e->fused_role[want_block + 1] = 2; }
+    if (e->use_stem) { e->fused_role[0] = 1; e->fused_role[1] = 2; }
+    if (e->block_layer >= 0) { e->fused_role[e->block_layer] = 1; e->fused_role[e->block_layer + 1] = 2; }
     for (size_t i = 0; i < P.buffers.size(); ++i) {
         bool skip = false;  // outputs of fused-away layers are never written: allocated on demand by the parity hook
         for (size_t li = 0; li < P.layers.size(); ++li)
             if (e->fused_role[li] == 1 && P.layers[li].out.buf == static_cast<int>(i)) skip = true;
         if (skip) continue;
-        int frames = n;
-        if (e->buf_internal[i])
-            for (size_t li = 0; li < P.layers.size(); ++li)
-                if (P.layers[li].out.buf == static_cast<int>(i)) frames = e->segs[e->seg_of[li]].chunk;
-        cudaError_t err = cudaMalloc(&e->bufs[i], buf_bytes(P.buffers[i], frames));
+        cudaError_t err = cudaMalloc(&e->bufs[i], buf_bytes(P.buffers[i], n));
         if (err != cudaSuccess) { free_exec(e.get()); return fail(FD_ERR_CUDA, "cudaMalloc(activation buffer %zu, batch %d) failed: %s", i, n, cudaGetErrorString(err)); }
     }
     const size_t frame_bytes = size_t(n) * P.net_h * P.net_w * 3;
@@ -448,176 +403,71 @@ int get_exec(fd_model* m, int n_frames, Exec** out) {
         free_exec(e.get());
         return fail(FD_ERR_CUDA, "cudaMalloc(per-batch state, batch %d) failed: %s", n, cudaGetErrorString(cudaGetLastError()));
     }
-    e->conv.resize(P.layers.size());
-    e->halo.resize(P.layers.size());
-    e->use_halo.assign(P.layers.size(), 0);
-    for (size_t i = 0; i < P.layers.size(); ++i) {
-        const LayerPlan& L = P.layers[i];
-        if (L.kind != LAYER_CONV) continue;
-        const int sgi = e->seg_of[i];
-        const int chunk = sgi >= 0 ? e->segs[sgi].chunk : 0, chunks = sgi >= 0 ? n / chunk : 1;
-        e->conv[i].resize(chunks);
-        e->halo[i].resize(chunks);
-        if (e->fused_role[i]) continue;  // fused layers: a tensor of the pair does not exist, the pair has its own launch below
-        for (int k = 0; k < chunks; ++k) {
-            char uh = 0;
-            if (int rc = prepare_conv_layer(m, e.get(), i, sgi >= 0 ? chunk : n, k, chunk, &e->conv[i][k], &e->halo[i][k], &uh)) { free_exec(e.get()); return rc; }
-            e->use_halo[i] = uh;
-        }
-    }
-    if (want_stem) {
-        const int sgi = e->seg_of[1];
-        const int chunk = sgi >= 0 ? e->segs[sgi].chunk : 0, chunks = sgi >= 0 ? n / chunk : 1;
-        e->stem.resize(chunks);
-        for (int k = 0; k < chunks; ++k)
-            if (int rc = prepare_stem(m, e.get(), sgi >= 0 ? chunk : n, k, chunk, &e->stem[k])) { free_exec(e.get()); return rc; }
-        e->use_stem = true;
-    }
-    if (want_block >= 0) {
-        const int sgi = e->seg_of[want_block];
-        const int chunk = sgi >= 0 ? e->segs[sgi].chunk : 0, chunks = sgi >= 0 ? n / chunk : 1;
-        e->block.resize(chunks);
-        for (int k = 0; k < chunks; ++k)
-            if (int rc = prepare_block(m, e.get(), want_block, sgi >= 0 ? chunk : n, k, chunk, &e->block[k])) { free_exec(e.get()); return rc; }
-        e->block_layer = want_block;
-    }
-    size_t ws_bytes = 0, counter_ints = 0;
-    for (const auto& v : e->conv)
-        for (const ConvLaunch& c : v) { ws_bytes = std::max(ws_bytes, c.ws_bytes); counter_ints = std::max(counter_ints, c.counter_ints); }
-    if (ws_bytes) {
-        if (cudaMalloc(&e->splitk_ws, ws_bytes) != cudaSuccess || cudaMalloc(&e->splitk_counters, counter_ints * sizeof(int)) != cudaSuccess ||
+    if (int rc = prepare_set(m, e.get(), static_cast<int>(P.layers.size()), 1, n, &e->whole)) { free_exec(e.get()); return rc; }
+    if (e->whole.ws_bytes) {
+        const size_t counter_ints = e->whole.counter_ints;
+        if (cudaMalloc(&e->splitk_ws, e->whole.ws_bytes) != cudaSuccess || cudaMalloc(&e->splitk_counters, counter_ints * sizeof(int)) != cudaSuccess ||
             cudaMemset(e->splitk_counters, 0, counter_ints * sizeof(int)) != cudaSuccess) {
             free_exec(e.get());
             return fail(FD_ERR_CUDA, "cudaMalloc(split-K workspace, batch %d) failed: %s", n, cudaGetErrorString(cudaGetLastError()));
         }
-        for (auto& v : e->conv)
+        for (auto& v : e->whole.conv)
             for (ConvLaunch& c : v)
                 if (c.ws_bytes) conv_tc_bind_workspace(&c, e->splitk_ws, e->splitk_counters);
-    }
-    // Tile-level dependencies between consecutive conv_tc layers (conv_tc_link_tiles): the consumer must read exactly the
-    // tensor its predecessor writes (a plain chain: no concat slice, no route, no up-sampling in between).
-    if (e->segs.empty() && options().tile_deps) {
-        std::vector<size_t> cand;
-        size_t ints = 0;
-        for (size_t i = 1; i < P.layers.size(); ++i) {
-            const LayerPlan& A = P.layers[i - 1];
-            const LayerPlan& B = P.layers[i];
-            if (A.kind != LAYER_CONV || B.kind != LAYER_CONV || e->use_halo[i - 1] || e->use_halo[i] || e->fused_role[i - 1] || e->fused_role[i]) continue;
-            if (A.out_fp32 || A.upsample2x || A.pool2 || A.out.pitch != A.out.c) continue;
-            if (B.in.buf != A.out.buf || B.in.ch_off != A.out.ch_off || B.in.c != A.out.c || B.in.pitch != A.out.pitch || B.stride != 1) continue;
-            cand.push_back(i);
-            ints += static_cast<size_t>(conv_tc_tile_counters(e->conv[i - 1][0]));
-        }
-        if (ints) {
-            if (cudaMalloc(&e->tile_flags, ints * sizeof(int)) != cudaSuccess || cudaMemset(e->tile_flags, 0, ints * sizeof(int)) != cudaSuccess) {
-                free_exec(e.get());
-                return fail(FD_ERR_CUDA, "cudaMalloc(tile flags, batch %d) failed: %s", n, cudaGetErrorString(cudaGetLastError()));
-            }
-            e->tile_flag_ints = ints;
-            size_t off = 0;
-            for (size_t i : cand) {
-                e->linked_layers += conv_tc_link_tiles(&e->conv[i - 1][0], &e->conv[i][0], e->tile_flags + off, m->num_sms);
-                off += static_cast<size_t>(conv_tc_tile_counters(e->conv[i - 1][0]));
-            }
-        }
     }
     *out = e.get();
     m->execs[n] = std::move(e);
     return FD_OK;
 }
 
-// layer i on frames [k * chunk, (k + 1) * chunk) (chunk = 0: the whole batch) with the given conv launch descriptors
-// The fused kernels' launches for these frames: stem = layers 0 + 1, block = layers block_layer + block_layer + 1 (null: the
-// layers launch their own kernels — the parity hook's way to materialise a fused-away tensor).
-struct FusedLaunch {
-    const StemLaunch* stem = nullptr;
-    const BlockLaunch* block = nullptr;
-    int block_layer = -1;
-};
-
-int launch_layer(fd_model* m, Exec* e, size_t i, int k, int chunk, bool halo, const ConvLaunch* cl, const HaloLaunch* hl, const FusedLaunch& fz, cudaStream_t s) {
+// layer i's own kernel on frames [k * frames, (k + 1) * frames), conv layers with the given launch descriptors
+int launch_own(fd_model* m, Exec* e, int i, int k, int frames, bool halo, const ConvLaunch* cl, const HaloLaunch* hl, cudaStream_t s) {
     const ModelPlan& P = m->plan;
     const LayerPlan& L = P.layers[i];
-    const int frames = chunk ? chunk : e->n;
     int rc = 0;
-    if (fz.stem && i == 0) return FD_OK;  // computed inside layer 1's kernel
-    if (fz.stem && i == 1) {
-        if (conv_stem_launch(*fz.stem, s)) return fail(FD_ERR_CUDA, "launch of the fused stem (layers 0 + 1) failed: %s", cudaGetErrorString(cudaGetLastError()));
-        return FD_OK;
-    }
-    if (fz.block && static_cast<int>(i) == fz.block_layer) return FD_OK;  // computed inside the next layer's kernel
-    if (fz.block && static_cast<int>(i) == fz.block_layer + 1) {
-        if (conv_block_launch(*fz.block, s)) return fail(FD_ERR_CUDA, "launch of the fused residual block (layers %zu + %zu) failed: %s", i - 1, i, cudaGetErrorString(cudaGetLastError()));
-        return FD_OK;
-    }
     switch (L.kind) {
         case LAYER_CONV0:
-            rc = launch_conv0_u8(e->frames + static_cast<size_t>(k) * chunk * P.net_h * P.net_w * 3, m->d_conv0 + L.w_off, m->d_bias + L.b_off,
-                                 static_cast<__nv_bfloat16*>(loc_ptr(*e, P, L.out, false, k, chunk)), frames, L.in.h, L.in.w, L.cout,
+            rc = launch_conv0_u8(e->frames + static_cast<size_t>(k) * frames * P.net_h * P.net_w * 3, m->d_conv0 + L.w_off, m->d_bias + L.b_off,
+                                 static_cast<__nv_bfloat16*>(loc_ptr(*e, P, L.out, false, k, frames)), frames, L.in.h, L.in.w, L.cout,
                                  L.out.pitch, L.act, L.alpha, L.pool2, s);
             break;
         case LAYER_CONV: rc = halo ? conv_halo_launch(*hl, s) : conv_tc_launch(*cl, s); break;
         case LAYER_MAXPOOL:
-            rc = launch_maxpool(static_cast<const __nv_bfloat16*>(loc_ptr(*e, P, L.in, false, k, chunk)), L.in.pitch,
-                                static_cast<__nv_bfloat16*>(loc_ptr(*e, P, L.out, false, k, chunk)), L.out.pitch, frames, L.in.h, L.in.w,
+            rc = launch_maxpool(static_cast<const __nv_bfloat16*>(loc_ptr(*e, P, L.in, false, k, frames)), L.in.pitch,
+                                static_cast<__nv_bfloat16*>(loc_ptr(*e, P, L.out, false, k, frames)), L.out.pitch, frames, L.in.h, L.in.w,
                                 L.in.c, L.pool_k, L.pool_s, L.pool_pad_lo, L.out.h, L.out.w, L.pad_value, s);
             break;
         case LAYER_COPY:
-            rc = launch_copy_slice(static_cast<const __nv_bfloat16*>(loc_ptr(*e, P, L.in, false, k, chunk)), L.in.pitch,
-                                   static_cast<__nv_bfloat16*>(loc_ptr(*e, P, L.out, false, k, chunk)), L.out.pitch, frames, L.in.h, L.in.w,
+            rc = launch_copy_slice(static_cast<const __nv_bfloat16*>(loc_ptr(*e, P, L.in, false, k, frames)), L.in.pitch,
+                                   static_cast<__nv_bfloat16*>(loc_ptr(*e, P, L.out, false, k, frames)), L.out.pitch, frames, L.in.h, L.in.w,
                                    L.in.c, L.upsample2x, s);
             break;
         default: rc = -1;
     }
-    if (rc) return fail(FD_ERR_CUDA, "launch of layer %zu (%s) failed: %s", i, L.name.c_str(), cudaGetErrorString(cudaGetLastError()));
+    if (rc) return fail(FD_ERR_CUDA, "launch of layer %d (%s) failed: %s", i, L.name.c_str(), cudaGetErrorString(cudaGetLastError()));
     return FD_OK;
 }
 
-// one layer on the whole batch (k = 0 outside segments) or on chunk k of its segment
-int launch_one(fd_model* m, Exec* e, size_t i, int k, cudaStream_t s) {
-    const int sgi = e->seg_of[i];
+// layer i, piece k of a launch set: a layer computed inside the next layer's kernel has no launch, the second layer of a
+// fused pair launches the fused kernel (stem = layers 0 + 1, block = layers block_layer + block_layer + 1)
+int launch_piece(fd_model* m, Exec* e, const LaunchSet& ls, int i, int k, cudaStream_t s) {
+    if (e->fused_role[i] == 1) return FD_OK;
+    if (e->fused_role[i] == 2 && e->use_stem && i == 1) {
+        if (conv_stem_launch(ls.stem[k], s)) return fail(FD_ERR_CUDA, "launch of the fused stem (layers 0 + 1) failed: %s", cudaGetErrorString(cudaGetLastError()));
+        return FD_OK;
+    }
+    if (e->fused_role[i] == 2) {
+        if (conv_block_launch(ls.block[k], s)) return fail(FD_ERR_CUDA, "launch of the fused residual block (layers %d + %d) failed: %s", i - 1, i, cudaGetErrorString(cudaGetLastError()));
+        return FD_OK;
+    }
     const bool conv = m->plan.layers[i].kind == LAYER_CONV;
-    FusedLaunch fz;
-    if (e->use_stem && i < 2) fz.stem = &e->stem[k];
-    if (e->block_layer >= 0 && (static_cast<int>(i) == e->block_layer || static_cast<int>(i) == e->block_layer + 1)) { fz.block = &e->block[k]; fz.block_layer = e->block_layer; }
-    return launch_layer(m, e, i, k, sgi >= 0 ? e->segs[sgi].chunk : 0, e->use_halo[i] != 0, conv ? &e->conv[i][k] : nullptr,
-                        conv ? &e->halo[i][k] : nullptr, fz, s);
+    return launch_own(m, e, i, k, ls.frames, ls.use_halo[i] != 0, conv ? &ls.conv[i][k] : nullptr, conv ? &ls.halo[i][k] : nullptr, s);
 }
 
-// The forward pass: chunked segments chunk by chunk (all layers of the segment per chunk), then the rest layer by layer.
+// The forward pass on the whole batch, from layer `from_layer` on.
 int launch_layers(fd_model* m, Exec* e, cudaStream_t s, int from_layer = 0) {
-    const ModelPlan& P = m->plan;
-    size_t i = static_cast<size_t>(from_layer);  // 0, or the first layer after a segment
-    if (from_layer == 0 && e->tile_flags)  // a new pass: no tile of any linked layer is done yet
-        if (cudaMemsetAsync(e->tile_flags, 0, e->tile_flag_ints * sizeof(int), s) != cudaSuccess) return fail(FD_ERR_CUDA, "tile-flag reset failed");
-    while (i < P.layers.size()) {
-        const int sgi = e->seg_of[i];
-        if (sgi < 0) {
-            if (int rc = launch_one(m, e, i, 0, s)) return rc;
-            ++i;
-            continue;
-        }
-        const Segment& sg = e->segs[sgi];
-        const Segment* nx = static_cast<size_t>(sgi) + 1 < e->segs.size() ? &e->segs[sgi + 1] : nullptr;
-        if (options().chunk_interleave && nx && nx->first == sg.last + 1 && nx->chunk % sg.chunk == 0) {
-            // the two segments interleaved: the second segment's chunk runs as soon as the first has produced its frames, so
-            // the tensor that crosses from one to the other is read back from L2 as well
-            const int ratio = nx->chunk / sg.chunk;
-            for (int kb = 0; kb < e->n / nx->chunk; ++kb) {
-                for (int k = kb * ratio; k < (kb + 1) * ratio; ++k)
-                    for (int j = sg.first; j <= sg.last; ++j)
-                        if (int rc = launch_one(m, e, j, k, s)) return rc;
-                for (int j = nx->first; j <= nx->last; ++j)
-                    if (int rc = launch_one(m, e, j, kb, s)) return rc;
-            }
-            i = nx->last + 1;
-            continue;
-        }
-        for (int k = 0; k < e->n / sg.chunk; ++k)
-            for (int j = sg.first; j <= sg.last; ++j)
-                if (int rc = launch_one(m, e, j, k, s)) return rc;
-        i = sg.last + 1;
-    }
+    for (int i = from_layer; i < e->whole.layers; ++i)
+        if (int rc = launch_piece(m, e, e->whole, i, 0, s)) return rc;
     return FD_OK;
 }
 
@@ -778,7 +628,7 @@ int fd_layer_info(const fd_model* m, int layer, fd_layer_desc* out) {
     out->flops = L.flops;
     if (L.kind == LAYER_CONV && !m->execs.empty()) {
         const Exec& e0 = *m->execs.begin()->second;
-        out->block_n = e0.use_halo[layer] ? -1 : e0.conv[layer][0].block_n;  // -1: halo-patch kernel
+        out->block_n = e0.whole.use_halo[layer] ? -1 : e0.whole.conv[layer][0].block_n;  // -1: halo-patch kernel
     }
     snprintf(out->name, sizeof(out->name), "%s", L.name.c_str());
     snprintf(out->out_name, sizeof(out->out_name), "%s", L.out_name.c_str());
@@ -787,8 +637,7 @@ int fd_layer_info(const fd_model* m, int layer, fd_layer_desc* out) {
 
 // Host logic only (works on a plan-only model): which layers the planner would hand to the fused kernels at batch n under the
 // current options — *stem = 1 when layers 0 + 1 run as conv_stem_kernel, *block_layer = the 1x1 layer of the pair that runs
-// as conv_block_kernel (or -1).  Chunked segments (option chunk_frames) can still keep a pair apart; fd_layer_exec_info
-// reports what an execution state really does.
+// as conv_block_kernel (or -1).  The execution state of batch n is built from this answer.
 int fd_planned_fusions(const fd_model* m, int n, int32_t* stem, int32_t* block_layer) {
     if (!m || !stem || !block_layer || n < 1) return fail(FD_ERR_ARG, "fd_planned_fusions: bad argument");
     const ModelPlan& P = m->plan;
@@ -810,18 +659,17 @@ int fd_layer_exec_info(fd_model* m, int layer, int n, fd_layer_exec* out) {
     const LayerPlan& L = m->plan.layers[layer];
     memset(out, 0, sizeof(*out));
     out->bucket = e->n;
-    out->chunk_frames = e->seg_of[layer] >= 0 ? e->segs[e->seg_of[layer]].chunk : e->n;
-    out->launches = e->n / out->chunk_frames;
+    out->chunk_frames = e->n;
+    out->launches = e->fused_role[layer] == 1 ? 0 : 1;
+    const LaunchSet& W = e->whole;
     if (e->use_stem && layer < 2) {
         out->kernel = layer == 0 ? FD_KERNEL_FUSED_NEXT : FD_KERNEL_STEM;
-        if (layer == 0) out->launches = 0;
-        else { out->grid = e->stem[0].grid; out->smem_bytes = static_cast<int32_t>(e->stem[0].smem_bytes); }
+        if (layer == 1) { out->grid = W.stem[0].grid; out->smem_bytes = static_cast<int32_t>(W.stem[0].smem_bytes); }
         return FD_OK;
     }
     if (e->block_layer >= 0 && (layer == e->block_layer || layer == e->block_layer + 1)) {
         out->kernel = layer == e->block_layer ? FD_KERNEL_FUSED_NEXT : FD_KERNEL_BLOCK;
-        if (layer == e->block_layer) out->launches = 0;
-        else { out->grid = e->block[0].grid; out->smem_bytes = static_cast<int32_t>(e->block[0].smem_bytes); }
+        if (layer != e->block_layer) { out->grid = W.block[0].grid; out->smem_bytes = static_cast<int32_t>(W.block[0].smem_bytes); }
         return FD_OK;
     }
     switch (L.kind) {
@@ -829,16 +677,15 @@ int fd_layer_exec_info(fd_model* m, int layer, int n, fd_layer_exec* out) {
         case LAYER_MAXPOOL: out->kernel = FD_KERNEL_MAXPOOL; break;
         case LAYER_COPY: out->kernel = FD_KERNEL_COPY; break;
         default:
-            if (e->use_halo[layer]) {
+            if (W.use_halo[layer]) {
                 out->kernel = FD_KERNEL_HALO;
-                out->grid = e->halo[layer][0].grid;
-                out->smem_bytes = static_cast<int32_t>(e->halo[layer][0].smem_bytes);
+                out->grid = W.halo[layer][0].grid;
+                out->smem_bytes = static_cast<int32_t>(W.halo[layer][0].smem_bytes);
             } else {
-                const ConvLaunch& c = e->conv[layer][0];
+                const ConvLaunch& c = W.conv[layer][0];
                 out->kernel = c.p.strip ? FD_KERNEL_TC_PAIR_STRIP : c.two_cta ? FD_KERNEL_TC_PAIR : c.p.swap ? FD_KERNEL_TC_SWAPPED : FD_KERNEL_TC_SINGLE;
                 out->block_n = c.block_n; out->split_k = c.p.split_k; out->grid = c.grid; out->num_stages = c.p.num_stages;
                 out->kb_per_stage = c.p.kb_per_stage; out->b_resident = c.p.b_resident;
-                out->tile_linked = c.p.dep != nullptr;
                 out->smem_bytes = static_cast<int32_t>(c.smem_bytes);
             }
     }
@@ -1021,7 +868,7 @@ int fd_fetch(fd_model* m, int n, fd_det* out, int32_t* counts, int32_t* total, v
 static int build_overlap_plan(fd_model* m, Exec* e) {
     const ModelPlan& P = m->plan;
     e->ov_layers = -1;
-    if (!e->segs.empty() || e->n < 16 || e->n % 4) return FD_OK;
+    if (e->n < 16 || e->n % 4) return FD_OK;
     int downs = 0, depth = 0;
     for (size_t i = 0; i < P.layers.size(); ++i) {
         const LayerPlan& L = P.layers[i];
@@ -1032,36 +879,14 @@ static int build_overlap_plan(fd_model* m, Exec* e) {
         depth = static_cast<int>(i) + 1;
     }
     if (downs < 2 || depth < 1 || P.layers[0].kind != LAYER_CONV0) return FD_OK;
-    const int chunk = e->n / 4;
-    e->ov_conv.assign(depth, {});
-    e->ov_halo.assign(depth, {});
-    e->ov_use_halo.assign(depth, 0);
-    for (int i = 0; i < depth; ++i) {
-        if (P.layers[i].kind != LAYER_CONV) continue;
-        e->ov_conv[i].resize(4);
-        e->ov_halo[i].resize(4);
-        if (e->fused_role[i]) continue;
-        for (int k = 0; k < 4; ++k) {
-            char uh = 0;
-            if (int rc = prepare_conv_layer(m, e, i, chunk, k, chunk, &e->ov_conv[i][k], &e->ov_halo[i][k], &uh)) return rc;
-            if (e->ov_conv[i][k].ws_bytes) return FD_OK;  // (a split-K layer this early would need its own workspace: leave the plain path)
-            e->ov_use_halo[i] = uh;
-        }
-    }
-    if (e->use_stem) {
-        if (depth < 2) return FD_OK;
-        e->ov_stem.resize(4);
-        if (!conv_stem_supported(stem_desc(m, chunk))) return FD_OK;  // (cannot happen for shapes the whole-batch stem took; leave the plain path)
-        for (int k = 0; k < 4; ++k)
-            if (int rc = prepare_stem(m, e, chunk, k, chunk, &e->ov_stem[k])) return rc;
-    }
-    if (e->block_layer >= 0 && e->block_layer < depth) {
-        if (e->block_layer + 1 >= depth || !conv_block_supported(block_desc(m, e->block_layer, chunk))) return FD_OK;  // (the pair must lie inside the front)
-        e->ov_block.resize(4);
-        for (int k = 0; k < 4; ++k)
-            if (int rc = prepare_block(m, e, e->block_layer, chunk, k, chunk, &e->ov_block[k])) return rc;
-    }
-    e->ov_chunk = chunk;
+    const int quarter = e->n / 4;
+    // a fused pair must lie inside the front or behind it, and take quarter batches (as it does for every shape the
+    // whole-batch plan fused); otherwise leave the plain path
+    if (e->use_stem && (depth < 2 || !conv_stem_supported(stem_desc(m, quarter)))) return FD_OK;
+    const int bl = e->block_layer;
+    if (bl >= 0 && bl < depth && (bl + 1 >= depth || !conv_block_supported(block_desc(m, bl, quarter)))) return FD_OK;
+    if (int rc = prepare_set(m, e, depth, 4, quarter, &e->front)) return rc;
+    if (e->front.ws_bytes) return FD_OK;  // (a split-K layer this early would need its own workspace: leave the plain path)
     e->ov_layers = depth;
     return FD_OK;
 }
@@ -1075,26 +900,19 @@ static int forward_overlapping_copy(fd_model* m, Exec* e, const uint8_t* frames,
         for (cudaEvent_t& ev : m->h2d_ev) CU(cudaEventCreateWithFlags(&ev, cudaEventDisableTiming));
     }
     const size_t frame_bytes = size_t(P.net_h) * P.net_w * 3;
-    const int chunk = e->ov_chunk;
+    const int quarter = e->front.frames;
     // everything queued on the compute stream so far (a previous pass that reads this input tensor) comes first
     CU(cudaEventRecord(m->idle_ev, s));
     CU(cudaStreamWaitEvent(m->copy_stream, m->idle_ev, 0));
     for (int p = 0; p < 4; ++p) {
-        const int f0 = p * chunk, f1 = std::min(n, f0 + chunk);
+        const int f0 = p * quarter, f1 = std::min(n, f0 + quarter);
         if (f1 > f0) CU(cudaMemcpyAsync(e->frames + f0 * frame_bytes, frames + f0 * frame_bytes, (f1 - f0) * frame_bytes, cudaMemcpyHostToDevice, m->copy_stream));
         CU(cudaEventRecord(m->h2d_ev[p], m->copy_stream));
     }
-    if (e->tile_flags) CU(cudaMemsetAsync(e->tile_flags, 0, e->tile_flag_ints * sizeof(int), s));  // (launch_layers does it for a whole pass)
     for (int k = 0; k < 4; ++k) {
         CU(cudaStreamWaitEvent(s, m->h2d_ev[k], 0));
-        for (int i = 0; i < e->ov_layers; ++i) {
-            const bool conv = P.layers[i].kind == LAYER_CONV;
-            FusedLaunch fz;
-            if (e->use_stem && i < 2) fz.stem = &e->ov_stem[k];
-            if (e->block_layer >= 0 && (i == e->block_layer || i == e->block_layer + 1)) { fz.block = &e->ov_block[k]; fz.block_layer = e->block_layer; }
-            if (int rc = launch_layer(m, e, i, k, chunk, e->ov_use_halo[i] != 0, conv ? &e->ov_conv[i][k] : nullptr, conv ? &e->ov_halo[i][k] : nullptr, fz, s))
-                return rc;
-        }
+        for (int i = 0; i < e->ov_layers; ++i)
+            if (int rc = launch_piece(m, e, e->front, i, k, s)) return rc;
     }
     if (m->use_graph && !e->graph_tail_tried) {
         e->graph_tail_tried = true;
@@ -1571,49 +1389,28 @@ int fd_pack_wire(const fd_det* dets, int count, uint32_t reqid, uint32_t msec, i
 }
 
 // ------------------------------------------------------------------ parity / profiling hooks
-// `layer`: the layer that produces `t`.  A buffer internal to a chunked segment only ever holds one chunk of frames, so
-// its value for the whole batch is gathered by replaying the segment chunk by chunk up to that layer (the same launches
-// the forward pass makes) and copying each chunk out.
+// `layer`: the layer that produces `t`.
 // The output of a layer that is computed inside the next layer's kernel never exists during a forward pass; the hook for
 // that tensor runs the layer's own kernel (the two-kernel path's, which the fused kernel is checked against) into a buffer
 // allocated on demand.
-static int launch_unfused(fd_model* m, Exec* e, int layer, int k, int chunk) {
+static int launch_unfused(fd_model* m, Exec* e, int layer) {
     const LayerPlan& L = m->plan.layers[layer];
-    if (L.kind == LAYER_CONV0) return launch_layer(m, e, layer, k, chunk, false, nullptr, nullptr, FusedLaunch(), m->stream);
+    if (L.kind == LAYER_CONV0) return launch_own(m, e, layer, 0, e->n, false, nullptr, nullptr, m->stream);
     ConvLaunch cl;
     HaloLaunch hl;
     char uh = 0;
-    if (int rc = prepare_conv_layer(m, e, layer, chunk ? chunk : e->n, k, chunk, &cl, &hl, &uh)) return rc;
+    if (int rc = prepare_conv_layer(m, e, layer, e->n, 0, &cl, &hl, &uh)) return rc;
     if (!uh && cl.ws_bytes) return fail(FD_ERR_ARG, "layer %d: its unfused form would need a split-K workspace", layer);
-    return launch_layer(m, e, layer, k, chunk, uh != 0, &cl, &hl, FusedLaunch(), m->stream);
+    return launch_own(m, e, layer, 0, e->n, uh != 0, &cl, &hl, m->stream);
 }
 
 static int tensor_to_host_nchw(fd_model* m, Exec* e, int layer, const TensorLoc& t, bool fp32, float* dst, int n) {
-    const size_t per_frame = size_t(t.c) * t.h * t.w;
-    const bool fused_away = e->fused_role[layer] == 1;
-    if (fused_away)
-        if (int rc = ensure_fused_away_buffer(m, e, layer)) return rc;
-    if (t.buf >= 0 && e->buf_internal[t.buf]) {
-        const Segment& sg = e->segs[e->seg_of[layer]];
-        if (int rc = ensure_scratch(e, per_frame * sg.chunk * 4)) return rc;
-        for (int k = 0; k * sg.chunk < n; ++k) {
-            // replay the segment up to the layer (a fused-away layer's input is whole or has just been produced by this replay)
-            for (int j = sg.first; j <= layer; ++j) {
-                if (j == layer && fused_away) { if (int rc = launch_unfused(m, e, layer, k, sg.chunk)) return rc; }
-                else if (int rc = launch_one(m, e, j, k, m->stream)) return rc;
-            }
-            const int frames = std::min(sg.chunk, n - k * sg.chunk);
-            if (launch_nhwc_to_nchw_f32(loc_ptr(*e, m->plan, t, fp32), t.pitch, fp32, e->scratch, frames, t.h, t.w, t.c, m->stream))
-                return fail(FD_ERR_CUDA, "layout kernel launch failed");
-            CU(cudaMemcpyAsync(dst + size_t(k) * sg.chunk * per_frame, e->scratch, per_frame * frames * 4, cudaMemcpyDeviceToHost, m->stream));
-            CU(cudaStreamSynchronize(m->stream));
-        }
-        return FD_OK;
-    }
-    const size_t elems = size_t(n) * per_frame;
+    const size_t elems = size_t(n) * t.c * t.h * t.w;
     if (int rc = ensure_scratch(e, elems * 4)) return rc;
-    if (fused_away)
-        if (int rc = launch_unfused(m, e, layer, 0, 0)) return rc;
+    if (e->fused_role[layer] == 1) {
+        if (int rc = ensure_fused_away_buffer(m, e, layer)) return rc;
+        if (int rc = launch_unfused(m, e, layer)) return rc;
+    }
     if (launch_nhwc_to_nchw_f32(loc_ptr(*e, m->plan, t, fp32), t.pitch, fp32, e->scratch, n, t.h, t.w, t.c, m->stream))
         return fail(FD_ERR_CUDA, "layout kernel launch failed");
     CU(cudaMemcpyAsync(dst, e->scratch, elems * 4, cudaMemcpyDeviceToHost, m->stream));
@@ -1703,52 +1500,22 @@ int fd_time_layers(fd_model* m, int n, int reps, float* ms) {
     CU(cudaSetDevice(m->device));
     Exec* e;
     if (int rc = get_exec(m, n, &e)) return rc;
-    const size_t nl = m->plan.layers.size();
+    const int nl = static_cast<int>(m->plan.layers.size());
     cudaEvent_t e0, e1;
     CU(cudaEventCreate(&e0));
     CU(cudaEventCreate(&e1));
     if (int rc = launch_layers(m, e, m->stream)) return rc;  // warm-up, also fills every buffer
     CU(cudaStreamSynchronize(m->stream));
-    for (size_t i = 0; i < nl; ++i) ms[i] = 0.f;
-    size_t i = 0;
-    while (i < nl) {
-        const int sgi = e->seg_of[i];
-        if (sgi < 0) {  // a layer on the whole batch, timed alone: reps back-to-back launches
-            if (int rc = launch_one(m, e, i, 0, m->stream)) return rc;
-            CU(cudaEventRecord(e0, m->stream));
-            for (int r = 0; r < reps; ++r)
-                if (int rc = launch_one(m, e, i, 0, m->stream)) return rc;
-            CU(cudaEventRecord(e1, m->stream));
-            CU(cudaStreamSynchronize(m->stream));
-            float t = 0.f;
-            CU(cudaEventElapsedTime(&t, e0, e1));
-            ms[i] = t / reps;
-            ++i;
-            continue;
-        }
-        // a chunked segment is timed as it runs (chunk by chunk, its activations L2-resident): one event after every launch,
-        // a layer's time = the sum of its chunks' intervals
-        const Segment& sg = e->segs[sgi];
-        const int chunks = e->n / sg.chunk, per = sg.last - sg.first + 1;
-        std::vector<cudaEvent_t> ev(static_cast<size_t>(chunks) * per + 1);
-        for (auto& x : ev) CU(cudaEventCreate(&x));
-        for (int r = 0; r < reps; ++r) {
-            CU(cudaEventRecord(ev[0], m->stream));
-            for (int k = 0; k < chunks; ++k)
-                for (int j = 0; j < per; ++j) {
-                    if (int rc = launch_one(m, e, sg.first + j, k, m->stream)) return rc;
-                    CU(cudaEventRecord(ev[static_cast<size_t>(k) * per + j + 1], m->stream));
-                }
-            CU(cudaStreamSynchronize(m->stream));
-            for (int k = 0; k < chunks; ++k)
-                for (int j = 0; j < per; ++j) {
-                    float t = 0.f;
-                    CU(cudaEventElapsedTime(&t, ev[static_cast<size_t>(k) * per + j], ev[static_cast<size_t>(k) * per + j + 1]));
-                    ms[sg.first + j] += t / reps;
-                }
-        }
-        for (auto& x : ev) cudaEventDestroy(x);
-        i = sg.last + 1;
+    for (int i = 0; i < nl; ++i) {  // each layer timed alone: reps back-to-back launches
+        if (int rc = launch_piece(m, e, e->whole, i, 0, m->stream)) return rc;
+        CU(cudaEventRecord(e0, m->stream));
+        for (int r = 0; r < reps; ++r)
+            if (int rc = launch_piece(m, e, e->whole, i, 0, m->stream)) return rc;
+        CU(cudaEventRecord(e1, m->stream));
+        CU(cudaStreamSynchronize(m->stream));
+        float t = 0.f;
+        CU(cudaEventElapsedTime(&t, e0, e1));
+        ms[i] = t / reps;
     }
     cudaEventDestroy(e0);
     cudaEventDestroy(e1);

@@ -679,37 +679,8 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
             for (int kb = 0; kb < nkb; ++kb)
                 ptx::tma_load_2d_addr(ptx::smem_u32(bres) + kb * b_bytes, mapB, bar, kb * block_k, 0);
         }
-        // weights above are constants; everything below reads the previous layer's output: either the whole previous grid has
-        // to be complete, or (tile-level dependencies) just the producer tiles that cover the rows of the tile at hand
-        const int* dep = p.dep;
-        if (!dep) ptx::grid_dep_wait();
-        const int gh = p.ho, gw = p.wo;  // the pixel grid (a linked consumer is stride 1: its input grid is its output grid)
-        // rows [pix_lo, pix_hi] of the input tensor are about to be loaded: wait for the producer tiles that hold them
-        auto wait_rows = [&](long long pix_lo, long long pix_hi) {
-            if (pix_hi >= p.M) pix_hi = p.M - 1;
-            if (pix_lo < 0) pix_lo = 0;
-            int t_lo, t_hi;
-            if (p.dep_strip) {  // producer tiles walk padded positions q = (img (H+1) + y + 1)(W+1) + x + 1 from dep_qfirst
-                auto pos = [&](long long pix) {
-                    const int img = static_cast<int>(pix / (gh * gw)), rem = static_cast<int>(pix - static_cast<long long>(img) * gh * gw);
-                    const int y = rem / gw, x = rem - y * gw;
-                    return (img * (gh + 1) + y + 1) * (gw + 1) + x + 1;
-                };
-                t_lo = (pos(pix_lo) - p.dep_qfirst) / p.dep_tile_m;
-                t_hi = (pos(pix_hi) - p.dep_qfirst) / p.dep_tile_m;
-            } else {
-                t_lo = static_cast<int>(pix_lo / p.dep_tile_m);
-                t_hi = static_cast<int>(pix_hi / p.dep_tile_m);
-            }
-            const long long t0 = clock64();
-            for (int t = t_lo + lane; t <= t_hi; t += 32)
-                while (ptx::ld_acquire_gpu(dep + t) < p.dep_full) {
-                    __nanosleep(64);
-                    if (clock64() - t0 > FD_MBAR_TIMEOUT_CYCLES) __trap();  // a protocol bug must not hang the GPU
-                }
-            __syncwarp();
-            ptx::fence_proxy_async_all();  // the acquired rows are read by the TMA engine (async proxy)
-        };
+        // weights above are constants; everything below reads the previous layer's output: its whole grid has to be complete
+        ptx::grid_dep_wait();
         const long long t_start = prof ? clock64() : 0;
         int sidx = 0;  // strips loaded so far (strip mode)
         const uint32_t strips_base = __shfl_sync(0xffffffffu, strips_base_v, 0), strip_bar = __shfl_sync(0xffffffffu, strip_bar_v, 0);
@@ -722,13 +693,6 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
                 const int wp = p.strip_wp, plane = p.strip_wp * p.strip_hp;
                 const int qs = p.strip_qfirst + m_tile * TILE_M + static_cast<int>(cta_rank) * BLOCK_M - wp - 1;  // first strip position
                 const int simg = qs / plane, srem = qs - simg * plane, syp = srem / wp, sxp = srem - syp * wp;
-                if (dep) {  // whole image rows, conservatively: from the row of the strip's first position to the row of its last
-                    const int qe = min(qs + p.strip_rows - 1, p.strip_total_q - 1);
-                    const int eimg = qe / plane, erem = qe - eimg * plane, eyp = erem / wp;
-                    const long long lo = (static_cast<long long>(simg) * gh + max(syp, 1) - 1) * gw;
-                    const long long hi = (static_cast<long long>(eimg) * gh + max(eyp, 1) - 1) * gw + gw - 1;
-                    wait_rows(lo, hi);
-                }
                 for (int cbi = 0; cbi < cin_blocks; ++cbi, ++sidx) {
                     const int sb = sidx & 1;
                     const uint32_t sfull = strip_bar + 8u * sb;
@@ -754,7 +718,6 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
             const int n0 = swap ? (tile - m_tile * n_tiles_n) * BLOCK_M
                                 : (tile - m_tile * n_tiles_n) * BLOCK_N + static_cast<int>(cta_rank) * B_ROWS * (TWO ? 1 : 0);
             const int m0 = swap ? m_tile * 256 : m_tile * TILE_M + static_cast<int>(cta_rank) * BLOCK_M;
-            if (dep) wait_rows(m0, m0 + (swap ? 256 : BLOCK_M) - 1);  // (a linked consumer of this form is a 1x1 layer: its rows are pixels)
             int img = 0, base_w = 0, base_h = 0;
             if (im2col) {
                 img = m0 / ho_wo;
@@ -937,23 +900,8 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
         int sbuf = 0;
         // the production configuration takes the copy of the epilogue that has its flags compiled in
         const bool fast_epi = !STRIP && !swap && p.epi_mode == 0 && p.store64 && p.split_k == 1 && p.act != 2 && !(kDev && p.debug);
-        // residual reads / output writes must not overtake the previous layer.  With tile-level dependencies the accumulator
-        // barrier below already implies it: the tile's MMAs ran on rows the producer warp waited for, and the residual rows
-        // of a tile are a subset of what its producer tiles had themselves waited for, one layer further up.
-        if (!p.dep) ptx::grid_dep_wait();
-        // this tile's rows are in memory: tell the next layer (one count per epilogue warp; TMA stores have to have
-        // COMPLETED, not just been read out of shared memory)
-        auto signal_tile = [&](int m_tile) {
-            if (!p.sig) return;
-            if (lane == 0) ptx::tma_store_wait<0>();
-            __threadfence();
-            ptx::fence_proxy_async_all();  // generic-proxy row stores -> visible to the consumer's TMA loads
-            __syncwarp();
-            if (lane == 0) {
-                __threadfence();
-                atomicAdd(p.sig + m_tile, 1);
-            }
-        };
+        // residual reads / output writes must not overtake the previous layer
+        ptx::grid_dep_wait();
         long long t_acc[8] = {0, 0, 0, 0, 0, 0, 0, 0}, t_start = prof ? clock64() : 0;
         for (int item = unit; item < num_items; item += units, ++it) {
             const int tile = tile_of(item), part = item - tile * split_k;
@@ -971,7 +919,6 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
                 else
                     epilogue_tile_swapped<false>(p, &tmOut, sbuf, taddr0, reinterpret_cast<float*>(stage), ch_warp, static_cast<long long>(m_tile) * 256,
                                                  lane, half, full_addr, aphase, empty_addr, prof ? t_acc : nullptr);
-                signal_tile(m_tile);
                 continue;
             }
             const int n0 = (tile - m_tile * n_tiles_n) * BLOCK_N;
@@ -994,7 +941,6 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
                 epilogue_tile<BLOCK_N>(p, &tmOut, taddr0, stage, sbuf, m_base, n0, lane, half, full_addr, aphase, empty_addr,
                                        prof ? t_acc : nullptr, tile, part, static_cast<int>(cta_rank) * 4 + quarter);
             }
-            signal_tile(m_tile);
         }
         if (lane == 0) ptx::tma_store_wait<0>();  // outstanding TMA stores read this CTA's shared memory
         if (prof && warp == 4 && lane == 0) {
@@ -1327,34 +1273,6 @@ int conv_tc_prepare(const ConvDesc& d, int num_sms, int block_n_hint, ConvLaunch
     L->smem_bytes = 1024 + SMEM_RING_OFF + (b_res ? bn * block_k * 2 * p.num_k_blocks : 0) + static_cast<size_t>(stages) * stage_bytes + strips_bytes;
     L->flops = 2.0 * double(M) * d.cout * K;
     return 0;
-}
-
-int conv_tc_tile_counters(const ConvLaunch& producer) { return producer.p.num_m_tiles; }
-
-int conv_tc_link_tiles(ConvLaunch* P, ConvLaunch* C, int* counters, int num_sms) {
-    const int mode = options().tile_deps;  // bit 0 on, bit 1 strip producers, bit 2 other producers, bit 3 only the 13x13-sized grids
-    if (!(mode & 1) || !counters) return 0;
-    const ConvParams& pp = P->p;
-    ConvParams& cp = C->p;
-    if (pp.strip ? !(mode & 2) : !(mode & 4)) return 0;
-    if ((mode & 8) && pp.M > options().tile_deps_max_m) return 0;
-    // producer: CTA-pair kernel (im2col / tiled / strip) or the swapped form, plain bf16 output, whole-K tiles
-    if (!(P->two_cta || pp.swap) || pp.split_k != 1 || pp.epi_mode != 0 || pp.out_fp32) return 0;
-    // consumer: a 1x1 layer on the pair kernel or the swapped form, or a strip 3x3 layer; whole-K tiles, stride 1
-    const bool c_1x1 = cp.ksize == 1 && !cp.a_im2col && (C->two_cta || cp.swap);
-    if (!(c_1x1 || cp.strip) || cp.split_k != 1 || cp.stride != 1) return 0;
-    if (cp.ho != pp.ho || cp.wo != pp.wo || cp.M != pp.M) return 0;
-    // both must occupy every SM: the consumer's CTAs then only start once the producer's have begun to exit, i.e. once
-    // its last wave is running (and every producer CTA is resident: no tile a consumer waits for can be left without an SM)
-    if (P->grid < num_sms - 1 || C->grid < num_sms - 1) return 0;
-    P->p.sig = counters;
-    cp.dep = counters;
-    // one count per epilogue warp (8 per CTA; both CTAs of a pair) and per N tile of the producer
-    cp.dep_full = (P->two_cta ? 16 : 8) * pp.num_n_tiles;
-    cp.dep_strip = pp.strip;
-    cp.dep_tile_m = 256;  // M tile of the pair kernel and pixel tile of the swapped form
-    cp.dep_qfirst = pp.strip_qfirst;
-    return 1;
 }
 
 void conv_tc_bind_workspace(ConvLaunch* L, float* ws, int* counters) {

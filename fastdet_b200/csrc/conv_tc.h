@@ -78,13 +78,6 @@ struct ConvParams {
     int store64;   // 1: the output map's box is 64 channels x 32 rows (SWIZZLE_128B), two chunks per TMA store
     int res_v8;    // 1: residual rows are 32-byte aligned -> 256-bit loads
     int epi_mode;  // 0 bf16 slice through a TMA store (+ residual), 1 fp32 head rows, 2 bf16 with x2 upsampling
-    // Tile-level dependencies (conv_tc_link_tiles): instead of waiting for the whole previous grid (griddepcontrol.wait), the
-    // TMA producer warp waits, tile by tile, until the producer layer's M tiles that cover the rows it is about to load have
-    // been stored (`dep` counters reach dep_full); this layer's epilogue warps bump `sig` when a tile's rows are in memory.
-    // SMs the previous layer leaves idle in its last, partial wave then start this layer's first tiles.
-    const int* dep;
-    int dep_full, dep_strip, dep_tile_m, dep_qfirst;  // dep_strip: the producer's M tiles walk padded strip positions
-    int* sig;
     // the layer's bias, read by the epilogue from the constant bank with a warp-uniform index (shared-memory and
     // L1 loads queue behind the operand traffic in this kernel; the constant cache does not)
     float bias_c[1024];
@@ -117,10 +110,5 @@ int encode_tiled_bf16(CUtensorMap* out, void* base, int rank, const unsigned lon
                       const unsigned long long* strides_bytes, const unsigned* box, int swizzle);
 // One-time per device: opt in to the large dynamic shared memory the kernels need.
 int conv_tc_init(char* err, size_t errlen);
-// Links two consecutive launches (the consumer reads exactly the tensor the producer writes, stride 1, same pixel grid)
-// by tile-level dependencies if both kernel forms support it.  `counters` must hold conv_tc_tile_counters(producer) ints,
-// zeroed before every forward pass.  Returns 1 if linked, 0 if the pair keeps the grid-wide wait.
-int conv_tc_tile_counters(const ConvLaunch& producer);
-int conv_tc_link_tiles(ConvLaunch* producer, ConvLaunch* consumer, int* counters, int num_sms);
 
 }  // namespace fd

@@ -17,9 +17,9 @@ int* option_slot(const char* name) {
     const Entry table[] = {
         {"strip", &o.strip}, {"strip_min_w", &o.strip_min_w}, {"swap", &o.swap}, {"two_cta", &o.two_cta},
         {"split_k", &o.split_k}, {"split_k_min_kb", &o.split_k_min_kb}, {"split_k_max", &o.split_k_max},
-        {"b_resident", &o.b_resident}, {"latency_bn", &o.latency_bn}, {"stem", &o.stem}, {"block", &o.block}, {"halo", &o.halo}, {"halo_skew", &o.halo_skew}, {"halo_slots", &o.halo_slots}, {"tile_deps", &o.tile_deps}, {"tile_deps_max_m", &o.tile_deps_max_m}, {"fuse_pool", &o.fuse_pool}, {"pdl", &o.pdl}, {"graph", &o.graph},
+        {"b_resident", &o.b_resident}, {"latency_bn", &o.latency_bn}, {"stem", &o.stem}, {"block", &o.block}, {"halo", &o.halo}, {"halo_skew", &o.halo_skew}, {"halo_slots", &o.halo_slots}, {"fuse_pool", &o.fuse_pool}, {"pdl", &o.pdl}, {"graph", &o.graph},
         {"exact_batch", &o.exact_batch}, {"nms_general", &o.nms_general}, {"jpeg_threads", &o.jpeg_threads},
-        {"chunk_frames", &o.chunk_frames}, {"chunk_mb", &o.chunk_mb}, {"chunk_interleave", &o.chunk_interleave}, {"detect_overlap", &o.detect_overlap}, {"server_inflight", &o.server_inflight},
+        {"detect_overlap", &o.detect_overlap}, {"server_inflight", &o.server_inflight},
     };
     for (const Entry& e : table)
         if (!strcmp(e.name, name)) return e.slot;

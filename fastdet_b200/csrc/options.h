@@ -23,21 +23,12 @@ struct Options {
     int halo = 1;             // halo-patch kernel for 16/32/64-channel 3x3 layers on large maps
     int halo_skew = 1;        // ... with chunk planes skewed against shared-memory bank conflicts
     int halo_slots = 0;       // ... patch ring depth cap (0: the kernel's maximum)
-    int tile_deps = 0;        // experiment kept as an option (measured 3-4 % SLOWER when on everywhere, no reliable gain when limited to
-                              // the 13x13 stage; DESIGN.md): consecutive conv_tc layers synchronise tile by tile instead of grid by grid;
-                              // bit 0 on, bit 1 strip producers, bit 2 other producers, bit 3 only grids of <= tile_deps_max_m pixels
-    int tile_deps_max_m = 12000;
     int fuse_pool = 1;        // MaxPool(2, 2) after the first convolution / a halo-patch layer runs in that kernel's epilogue
     int pdl = 1;              // programmatic dependent launch between layers
     int graph = 1;            // replay the forward pass as a captured CUDA graph
     int exact_batch = 0;      // one execution state per exact batch size instead of per bucket
     int nms_general = 0;      // force the general (global-memory) Soft-NMS loop
     int jpeg_threads = 0;     // host threads of the JPEG entropy decoder; 0 = all hardware threads (max 64)
-    int chunk_frames = -1;    // experiment kept as an option (measured SLOWER on B200, see DESIGN.md): the leading layers run in chunks
-                              // of this many frames (twice as many in the second segment) so a chunk's activations stay in L2;
-                              // 0 = sized from chunk_mb, -1 = no chunking (default)
-    int chunk_mb = 48;        // auto chunk size: largest tensor of a first-segment chunk at most this many MB (half of it in the second)
-    int chunk_interleave = 0; // run the second chunked segment's chunk right after the first-segment chunks that feed it
     int server_inflight = 2;  // fd_server: micro-batches in flight per lane (2: copy / compute overlap at saturation; 1: a closed loop
                               // of few streams per lane gathers larger batches, see DESIGN.md section 6)
     int detect_overlap = 1;   // synchronous fd_detect: the frame copy in four pieces, overlapped with the first layers

@@ -39,15 +39,6 @@ __device__ __forceinline__ U32x8 ld_nc_v8(const void* p) {
     return r;
 }
 
-// acquire load at GPU scope (tile-completion counters written by CTAs of a concurrently running kernel)
-__device__ __forceinline__ int ld_acquire_gpu(const int* p) {
-    int v;
-    asm volatile("ld.acquire.gpu.global.s32 %0, [%1];" : "=r"(v) : "l"(p) : "memory");
-    return v;
-}
-// generic-proxy <-> async-proxy ordering for every state space (global data that TMA reads / wrote)
-__device__ __forceinline__ void fence_proxy_async_all() { asm volatile("fence.proxy.async;" ::: "memory"); }
-
 // ---------------------------------------------------------------- programmatic dependent launch
 // wait: returns once every grid this launch depends on has completed and its writes are visible (no-op for a
 // launch without the programmatic-serialisation attribute).  launch_dependents: lets the next kernel in the

@@ -103,10 +103,9 @@ typedef struct fd_layer_exec {
     int32_t bucket;       /* batch-size bucket whose execution state answered (n rounded up) */
     int32_t block_n, split_k, grid, num_stages, kb_per_stage, b_resident;
     int32_t smem_bytes;
-    int32_t chunk_frames; /* frames per launch of this layer (< bucket: the layer belongs to an L2-resident chunked segment) */
-    int32_t launches;     /* launches of this layer per forward pass */
-    int32_t tile_linked;  /* 1: waits for its predecessor tile by tile (per-M-tile completion counters) instead of grid-wide */
-    int32_t reserved[4];
+    int32_t chunk_frames; /* frames per launch of this layer (the bucket) */
+    int32_t launches;     /* launches of this layer per forward pass (0: FD_KERNEL_FUSED_NEXT, else 1) */
+    int32_t reserved[5];
 } fd_layer_exec;
 
 const char* fd_last_error(void);
@@ -279,8 +278,8 @@ int fd_layer_output_fp32(fd_model* m, int layer, float* dst_nchw, int n);
 int fd_normalise_f32(fd_model* m, const uint8_t* frames, int n, float* dst_nchw);
 /* Device letterbox of host frames [n, src_h, src_w, 3] to [n, net_h, net_w, 3]. */
 int fd_letterbox_u8(fd_model* m, const uint8_t* frames, int n, int src_w, int src_h, uint8_t* dst);
-/* Per-layer device time (ms, mean over reps) of the forward pass at batch n: layers that run on the whole batch are timed
- * alone (reps back-to-back launches), layers of an L2-resident chunked segment as the segment runs (sum over its chunks). */
+/* Per-layer device time (ms, mean over reps) of the forward pass at batch n: every layer timed alone (reps back-to-back
+ * launches; 0 for a layer computed inside the next layer's kernel). */
 int fd_time_layers(fd_model* m, int n, int reps, float* ms_per_layer);
 /* Device time (ms, mean over reps back-to-back runs) of fd_forward at batch n: the captured graph as serving runs it. */
 int fd_time_forward(fd_model* m, int n, int reps, float* ms);

@@ -8,7 +8,6 @@ These tests put exactly those forms under the CPU oracle:
   * the strip form forced at a small batch (option strip=2), per layer, for the 416 and the 608 grids
     (strip widths W+1 = 53 / 27 / 14 and 77 / 39 / 20);
   * the default plan at batch 8 per layer (52x52 strips by the library's own choice);
-  * the optional L2-resident chunked execution of the leading layers (option chunk_frames; off by default) at batch 16;
   * the production batch 64 (rsu-416-9, BASELINE config 3): heads and detections of 8 of the 64 frames;
   * full-608 at a batch whose 76x76 layers take strips by default (BASELINE config 4's per-GPU shard, reduced);
   * the stand-alone kernel checker (csrc/dev/test_conv.cu: every kernel form against a float64 CPU loop).
@@ -68,29 +67,6 @@ def test_default_plan_batch8_per_layer():
     m.close()
 
 
-def test_chunked_segments_batch16_per_layer():
-    """Option chunk_frames=0 (auto-sized L2-resident chunks; off by default because it measured slower), batch 16: both
-    leading segments are chunked (conv1..conv4: 4 chunks of 4 frames; conv5..conv9: 2 chunks of 8) — the layer outputs of
-    the chunked region (the parity hook replays the segment's launches chunk by chunk) and the heads against the oracle,
-    and the same heads bit for bit as the default plan (a chunk runs the same kernels on the same frames)."""
-    data = modelgen.build_onnx("full", 80, 416, seed=2)
-    frames = frames_for(16, 416, first_seed=170)
-    with _native.option("chunk_frames", 0):
-        m = _native.Model(data, 80, (416, 416), device=0)
-        info = m.exec_info(16)
-        assert [e["chunk_frames"] for e in info[:10]] == [4, 4, 4, 4, 8, 8, 8, 8, 8, 16]
-        assert [e["launches"] for e in info[:10]] == [0, 4, 0, 4, 2, 2, 2, 2, 2, 1]  # (conv1 / conv3 are computed inside conv2's / conv4's kernel)
-        got, _ = _check_heads(data, m, frames, per_layer=True, layers=range(10))
-        m.close()
-    m2 = _native.Model(data, 80, (416, 416), device=0)
-    assert all(e["launches"] == (0 if e["kernel_name"] == "fused_next" else 1) for e in m2.exec_info(16))
-    m2.preprocess(frames, 16, (416, 416))
-    m2.forward(16)
-    for a, b in zip(got, m2.heads(16)):
-        assert np.array_equal(a, b)
-    m2.close()
-
-
 def test_production_batch64_against_oracle():
     """BASELINE config 3 (rsu-416-9, batch 64) — the configuration bench.py times: all 29 strip layers in strip form by
     the library's own choice; heads of 8 of the 64 frames against the fp32 oracle (2e-2 * max|ref|) and their
@@ -144,39 +120,6 @@ def test_full_608_batch_with_strips_against_oracle():
     assert len(s76) == 11 and all(f[i] == "tc_pair_strip" for i in s76), [(i, f[i]) for i in s76]
     _check_heads(data, m, frames_for(4, 608, first_seed=1000))
     m.close()
-
-
-def test_tile_level_dependencies_change_nothing():
-    """Option tile_deps (off by default: it measured slower): at batch 64 most consecutive conv_tc layers then synchronise
-    tile by tile (the consumer's TMA warp waits for the producer tiles that cover its rows; SMs the producer leaves idle in
-    its last wave start the consumer early) instead of grid by grid.  A missed dependency would show as a race: the heads
-    must be bit-identical over repeated passes, on two different input sets, and identical to the default plan's."""
-    import hashlib
-    data = modelgen.build_onnx("rsu", 9, 416, seed=3)
-    sets = [frames_for(64, 416, first_seed=100), frames_for(64, 416, first_seed=300)]
-    with _native.option("tile_deps", 7):
-        m = _native.Model(data, 9, (416, 416), device=0)
-        info = m.exec_info(64)
-    linked = [i for i, e in enumerate(info) if e["tile_linked"]]
-    assert len(linked) >= 40, linked
-    L = m.layers()
-    assert all(L[i]["kind"] == 1 and L[i]["stride"] == 1 for i in linked)
-
-    def digest(model, frames):
-        model.preprocess(frames, 64, (416, 416))
-        model.forward(64)
-        return [hashlib.sha256(h.tobytes()).hexdigest() for h in model.heads(64)]
-
-    want = [digest(m, f) for f in sets]
-    for rep in range(6):
-        for f, w in zip(sets, want):
-            assert digest(m, f) == w, rep
-    m.close()
-    m2 = _native.Model(data, 9, (416, 416), device=0)
-    assert not any(e["tile_linked"] for e in m2.exec_info(64))
-    for f, w in zip(sets, want):
-        assert digest(m2, f) == w
-    m2.close()
 
 
 def test_fused_maxpool_equals_the_pool_kernel():
