@@ -24,6 +24,10 @@ activation (the value after LeakyRelu, and after a residual Add) is rounded to b
 It separates the two sources of difference from the fp32 oracle: what the prescribed operand precision costs
 (bf16 oracle vs fp32 oracle, a CPU-only comparison: tests/test_oracle_graph.py::test_bf16_operand_floor) and what
 the CUDA kernels add on top (GPU vs bf16 oracle: fp32 summation order only).
+
+``GraphExecutor.run_forced`` is the teacher-forced form of the bf16 mode: it evaluates every fused layer in float64 from an
+implementation's own values of the layer's inputs, so that each layer of the CUDA path can be held to a rounding bound of
+its own (tests/compare.py::layer_bound, tests/test_gpu_layers_exact.py).
 """
 from __future__ import annotations
 
@@ -218,113 +222,16 @@ class GraphExecutor:
     # -- graph walk ----------------------------------------------------------
     def run(self, x: np.ndarray, keep: Optional[List[str]] = None, all_values: bool = False):
         """x: [N,3,H,W] float array.  Returns the graph outputs as float32 numpy arrays (graph order),
-        or a dict name->array when `keep`/`all_values` is given."""
+        or a dict name->array when `keep`/`all_values` is given.  bf16 mode with accumulate=float64 keeps the sum, bias,
+        activation and residual add in float64 and rounds once where an activation is stored."""
         vals: Dict[str, torch.Tensor] = dict(self.consts)
         vals["input"] = torch.from_numpy(np.ascontiguousarray(x)).to(self.dtype)
         vals[""] = None
+        acc64 = self.bf16 and self.accumulate == torch.float64
         with torch.no_grad():
             for n in self.graph.nodes:
                 ins = [vals.get(i) if i else None for i in n.inputs]
-                op = n.op
-                if op == "Conv" and self.bf16:
-                    w16, bias = self.folded[n.outputs[0]]
-                    xin = ins[0] if id(n) in self.tail else _bf16(ins[0])
-                    if self.accumulate == torch.float64:
-                        out = self._conv(n, xin.double(), w16.double(), bias.double()).to(torch.float32)
-                    else:
-                        out = self._conv(n, xin, w16, bias)
-                elif op == "Conv":
-                    out = self._conv(n, *ins)
-                elif op == "BatchNormalization" and id(n) in self.bn_identity:
-                    out = ins[0]
-                elif op == "BatchNormalization":
-                    xx, sc, bb, mean, var = ins
-                    eps = n.attrs.get("epsilon", 1e-5)
-                    shp = (1, -1, 1, 1)
-                    out = sc.view(shp) * (xx - mean.view(shp)) / torch.sqrt(var.view(shp) + eps) + bb.view(shp)
-                elif op == "LeakyRelu":
-                    out = F.leaky_relu(ins[0], n.attrs.get("alpha", 0.01))
-                elif op == "Relu":
-                    out = F.relu(ins[0])
-                elif op == "Add":
-                    out = ins[0] + ins[1]
-                elif op == "Sub":
-                    out = ins[0] - ins[1]
-                elif op == "Mul":
-                    out = ins[0] * ins[1]
-                elif op == "Div":
-                    if not ins[0].is_floating_point() and not ins[1].is_floating_point():
-                        out = torch.div(ins[0], ins[1], rounding_mode="trunc")
-                    else:
-                        out = ins[0] / ins[1]
-                elif op == "Floor":
-                    out = torch.floor(ins[0])
-                elif op == "MaxPool":
-                    out = self._maxpool(n, ins[0])
-                elif op in ("Resize", "Upsample"):
-                    out = self._resize(n, ins[0], ins)
-                elif op == "Concat":
-                    axis = n.attrs.get("axis", 1)
-                    out = torch.cat([i for i in ins], dim=axis)
-                elif op == "Pad":
-                    out = self._pad(n, ins)
-                elif op == "Constant":
-                    v = n.attrs["value"]
-                    out = torch.from_numpy(np.ascontiguousarray(v))
-                    if out.is_floating_point():
-                        out = out.to(self.dtype)
-                elif op == "Identity":
-                    out = ins[0]
-                elif op == "Shape":
-                    out = torch.tensor(list(ins[0].shape), dtype=torch.int64)
-                elif op == "Gather":
-                    axis = n.attrs.get("axis", 0)
-                    idx = ins[1].to(torch.int64)
-                    out = torch.index_select(ins[0], axis, idx.reshape(-1)).reshape(
-                        list(ins[0].shape[:axis]) + list(idx.shape) + list(ins[0].shape[axis + 1:]))
-                elif op == "Cast":
-                    to = n.attrs["to"]
-                    out = ins[0].to({1: self.dtype, 6: torch.int32, 7: torch.int64, 11: torch.float64}[to])
-                elif op == "Slice":
-                    if len(ins) > 1:
-                        starts, ends = [int(v) for v in ins[1]], [int(v) for v in ins[2]]
-                        axes = [int(v) for v in ins[3]] if len(ins) > 3 and ins[3] is not None else list(range(len(starts)))
-                        steps = [int(v) for v in ins[4]] if len(ins) > 4 and ins[4] is not None else [1] * len(starts)
-                    else:
-                        starts, ends = n.attrs["starts"], n.attrs["ends"]
-                        axes = n.attrs.get("axes", list(range(len(starts))))
-                        steps = [1] * len(starts)
-                    arr = ins[0].numpy()
-                    index = [slice(None)] * arr.ndim
-                    for s, e, ax, st in zip(starts, ends, axes, steps):
-                        # numpy slicing clamps exactly like the ONNX Slice specification (INT64 extremes included)
-                        index[ax] = slice(int(np.clip(s, -2**62, 2**62)), int(np.clip(e, -2**62, 2**62)), st)
-                        if st < 0 and e < -arr.shape[ax]:
-                            index[ax] = slice(int(np.clip(s, -2**62, 2**62)), None, st)
-                    out = torch.from_numpy(np.ascontiguousarray(arr[tuple(index)]))
-                elif op == "Unsqueeze":
-                    axes = n.attrs.get("axes") or [int(v) for v in ins[1]]
-                    out = ins[0]
-                    for ax in sorted(axes):
-                        out = out.unsqueeze(ax)
-                elif op == "Squeeze":
-                    axes = n.attrs.get("axes") or ([int(v) for v in ins[1]] if len(ins) > 1 else None)
-                    out = ins[0]
-                    if axes is None:
-                        out = out.squeeze()
-                    else:
-                        for ax in sorted(axes, reverse=True):
-                            out = out.squeeze(ax)
-                elif op == "ConstantOfShape":
-                    v = n.attrs.get("value")
-                    fill = torch.from_numpy(np.ascontiguousarray(v)).reshape(-1)[0] if v is not None else torch.tensor(0.0)
-                    out = torch.full([int(d) for d in ins[0]], fill.item(), dtype=fill.dtype)
-                elif op == "Reshape":
-                    out = ins[0].reshape([int(d) for d in ins[1]])
-                elif op == "Transpose":
-                    out = ins[0].permute(n.attrs["perm"])
-                else:
-                    raise NotImplementedError(f"oracle: ONNX op {op}")
+                out = self._node(n, ins, acc64)
                 if n.outputs[0] in self.round_after:
                     out = _bf16(out)
                 vals[n.outputs[0]] = out
@@ -332,6 +239,182 @@ class GraphExecutor:
             names = keep if keep is not None else [k for k in vals if k and k not in self.consts]
             return {k: vals[k].to(torch.float32).numpy() for k in names if isinstance(vals.get(k), torch.Tensor)}
         return [vals[o].to(torch.float32).numpy() for o in self.graph.outputs]
+
+    def run_forced(self, x: np.ndarray, overrides: Dict[str, np.ndarray], on_value=None):
+        """Teacher-forced bf16 evaluation: predicts each fused layer of an implementation from that implementation's OWN
+        inputs, so that a layer is judged by its own arithmetic and not by the rounding noise of every layer before it.
+
+        x: [N,3,H,W] network input.  overrides: {value name: array} — the implementation's values of graph tensors (the
+        library's fd_layer_desc.out_name of every layer: the value after all ops fused into that layer).  Every Conv uses the
+        bf16 semantics of this executor (the folded bf16 weights of `self.folded`, bf16-rounded inputs); the sum, bias,
+        activation and residual Add are evaluated in float64 and nothing is rounded to bf16 in between.  When a value named
+        in `overrides` has been computed, its record is produced and the value is REPLACED by the override before any later
+        node reads it, so Concat / Resize / MaxPool and the next convolutions see exactly the tensors the implementation's
+        consumers read.  Record of a value (float64 tensors of the value's shape):
+          r       the unrounded value;
+          S       magnitude of the sums behind each element: conv(|x|, |w|) + |b| at the Conv (fp32), carried through the
+                  activation, + |residual| at an Add, max-pooled / repeated by MaxPool / Resize; None for a value computed
+                  exactly from overridden inputs (stand-alone MaxPool, Concat);
+          K       cin * kh * kw of the convolution behind it (0 when S is None);
+          m       magnitude for the rounding step: |r|, or for a MaxPool output the window maximum of |input|;
+          pool    True for a MaxPool output;
+          branch, S_branch   (residual Add only) the value after the activation, before the Add, and its S.
+        Values not in `overrides` are carried unrounded (a convolution still rounds its input to bf16).
+        on_value(name, record) is called for every overridden value; without it the records are returned as a dict."""
+        if not self.bf16 or self.tail:
+            raise ValueError("run_forced needs dtype='bf16' and fp32_tail=0")
+        vals: Dict[str, torch.Tensor] = dict(self.consts)
+        vals["input"] = torch.from_numpy(np.ascontiguousarray(x)).to(torch.float32)
+        vals[""] = None
+        mag: Dict[str, torch.Tensor] = {}   # computed (not overridden) values -> S
+        ksz: Dict[str, int] = {}
+        recs = {}
+
+        def absval(i):
+            return mag[i] if i in mag else vals[i].abs().double()
+
+        with torch.no_grad():
+            for n in self.graph.nodes:
+                name, op = n.outputs[0], n.op
+                ins = [vals.get(i) if i else None for i in n.inputs]
+                out = self._node(n, ins, True)
+                computed = [i for i in n.inputs if i in mag]
+                if op == "Conv":
+                    w16, bias = self.folded[name]
+                    mag[name] = self._conv(n, _bf16(ins[0].float()).abs(), w16.abs(), bias.abs()).double()
+                    ksz[name] = int(w16[0].numel())
+                elif computed and op == "BatchNormalization" and id(n) not in self.bn_identity:
+                    raise NotImplementedError("run_forced: BatchNormalization that is not folded into a Conv")
+                elif computed and op in ("BatchNormalization", "LeakyRelu", "Relu", "Identity"):
+                    mag[name], ksz[name] = mag[computed[0]], ksz[computed[0]]
+                elif computed and op == "Add":
+                    mag[name] = absval(n.inputs[0]) + absval(n.inputs[1])
+                    ksz[name] = max(ksz[i] for i in computed)
+                elif computed and op in ("MaxPool", "Resize", "Upsample", "Pad", "Concat"):
+                    data = range(len(ins)) if op == "Concat" else [0]
+                    m_ins = list(ins)
+                    for j in data:
+                        m_ins[j] = absval(n.inputs[j])
+                    mag[name] = self._node(n, m_ins, True)
+                    ksz[name] = max(ksz[i] for i in computed)
+                if name in overrides:
+                    rec = {"r": out.double(), "S": mag.get(name), "K": ksz.get(name, 0), "pool": op == "MaxPool"}
+                    rec["m"] = self._maxpool(n, ins[0].double().abs()) if op == "MaxPool" else out.double().abs()
+                    if op == "Add" and len(computed) == 1:
+                        rec["branch"], rec["S_branch"] = vals[computed[0]].double(), mag[computed[0]]
+                    if on_value is not None:
+                        on_value(name, rec)
+                    else:
+                        recs[name] = rec
+                    out = torch.as_tensor(np.ascontiguousarray(overrides[name]), dtype=torch.float32)
+                    mag.pop(name, None)
+                    ksz.pop(name, None)
+                vals[name] = out
+        return recs
+
+    def _node(self, n, ins, acc64: bool):
+        """One node's value.  acc64 (bf16 mode): the convolution sums its bf16 products in float64 and keeps float64."""
+        op = n.op
+        if op == "Conv" and self.bf16:
+            w16, bias = self.folded[n.outputs[0]]
+            xin = ins[0] if id(n) in self.tail else _bf16(ins[0])
+            if acc64:
+                out = self._conv(n, xin.double(), w16.double(), bias.double())
+            else:
+                out = self._conv(n, xin, w16, bias)
+        elif op == "Conv":
+            out = self._conv(n, *ins)
+        elif op == "BatchNormalization" and id(n) in self.bn_identity:
+            out = ins[0]
+        elif op == "BatchNormalization":
+            xx, sc, bb, mean, var = ins
+            eps = n.attrs.get("epsilon", 1e-5)
+            shp = (1, -1, 1, 1)
+            out = sc.view(shp) * (xx - mean.view(shp)) / torch.sqrt(var.view(shp) + eps) + bb.view(shp)
+        elif op == "LeakyRelu":
+            out = F.leaky_relu(ins[0], float(np.float32(n.attrs.get("alpha", 0.01))))  # the kernels' fp32 alpha
+        elif op == "Relu":
+            out = F.relu(ins[0])
+        elif op == "Add":
+            out = ins[0] + ins[1]
+        elif op == "Sub":
+            out = ins[0] - ins[1]
+        elif op == "Mul":
+            out = ins[0] * ins[1]
+        elif op == "Div":
+            if not ins[0].is_floating_point() and not ins[1].is_floating_point():
+                out = torch.div(ins[0], ins[1], rounding_mode="trunc")
+            else:
+                out = ins[0] / ins[1]
+        elif op == "Floor":
+            out = torch.floor(ins[0])
+        elif op == "MaxPool":
+            out = self._maxpool(n, ins[0])
+        elif op in ("Resize", "Upsample"):
+            out = self._resize(n, ins[0], ins)
+        elif op == "Concat":
+            axis = n.attrs.get("axis", 1)
+            out = torch.cat([i for i in ins], dim=axis)
+        elif op == "Pad":
+            out = self._pad(n, ins)
+        elif op == "Constant":
+            v = n.attrs["value"]
+            out = torch.from_numpy(np.ascontiguousarray(v))
+            if out.is_floating_point():
+                out = out.to(self.dtype)
+        elif op == "Identity":
+            out = ins[0]
+        elif op == "Shape":
+            out = torch.tensor(list(ins[0].shape), dtype=torch.int64)
+        elif op == "Gather":
+            axis = n.attrs.get("axis", 0)
+            idx = ins[1].to(torch.int64)
+            out = torch.index_select(ins[0], axis, idx.reshape(-1)).reshape(
+                list(ins[0].shape[:axis]) + list(idx.shape) + list(ins[0].shape[axis + 1:]))
+        elif op == "Cast":
+            to = n.attrs["to"]
+            out = ins[0].to({1: self.dtype, 6: torch.int32, 7: torch.int64, 11: torch.float64}[to])
+        elif op == "Slice":
+            if len(ins) > 1:
+                starts, ends = [int(v) for v in ins[1]], [int(v) for v in ins[2]]
+                axes = [int(v) for v in ins[3]] if len(ins) > 3 and ins[3] is not None else list(range(len(starts)))
+                steps = [int(v) for v in ins[4]] if len(ins) > 4 and ins[4] is not None else [1] * len(starts)
+            else:
+                starts, ends = n.attrs["starts"], n.attrs["ends"]
+                axes = n.attrs.get("axes", list(range(len(starts))))
+                steps = [1] * len(starts)
+            arr = ins[0].numpy()
+            index = [slice(None)] * arr.ndim
+            for s, e, ax, st in zip(starts, ends, axes, steps):
+                # numpy slicing clamps exactly like the ONNX Slice specification (INT64 extremes included)
+                index[ax] = slice(int(np.clip(s, -2**62, 2**62)), int(np.clip(e, -2**62, 2**62)), st)
+                if st < 0 and e < -arr.shape[ax]:
+                    index[ax] = slice(int(np.clip(s, -2**62, 2**62)), None, st)
+            out = torch.from_numpy(np.ascontiguousarray(arr[tuple(index)]))
+        elif op == "Unsqueeze":
+            axes = n.attrs.get("axes") or [int(v) for v in ins[1]]
+            out = ins[0]
+            for ax in sorted(axes):
+                out = out.unsqueeze(ax)
+        elif op == "Squeeze":
+            axes = n.attrs.get("axes") or ([int(v) for v in ins[1]] if len(ins) > 1 else None)
+            out = ins[0]
+            if axes is None:
+                out = out.squeeze()
+            else:
+                for ax in sorted(axes, reverse=True):
+                    out = out.squeeze(ax)
+        elif op == "ConstantOfShape":
+            v = n.attrs.get("value")
+            fill = torch.from_numpy(np.ascontiguousarray(v)).reshape(-1)[0] if v is not None else torch.tensor(0.0)
+            out = torch.full([int(d) for d in ins[0]], fill.item(), dtype=fill.dtype)
+        elif op == "Reshape":
+            out = ins[0].reshape([int(d) for d in ins[1]])
+        elif op == "Transpose":
+            out = ins[0].permute(n.attrs["perm"])
+        else:
+            raise NotImplementedError(f"oracle: ONNX op {op}")
+        return out
 
 
 class OrtSubstituteSession:

@@ -10,8 +10,12 @@ These tests put exactly those forms under the CPU oracle:
   * the default plan at batch 8 per layer (52x52 strips by the library's own choice);
   * the production batch 64 (rsu-416-9, BASELINE config 3): heads and detections of 8 of the 64 frames;
   * full-608 at a batch whose 76x76 layers take strips by default (BASELINE config 4's per-GPU shard, reduced);
-  * the stand-alone kernel checker (csrc/dev/test_conv.cu: every kernel form against a float64 CPU loop).
+  * the stand-alone kernel checker (csrc/dev/test_conv.cu: every kernel form, the production split-K shapes included,
+    against a float64 CPU loop under the rounding model of tests/compare.py).
 Every test first asserts, through fd_layer_exec_info, that the layers really took the form it means to check.
+The per-layer checks here are RMS-relative against the fp32 oracle's own chain (drift from fp32); the element-wise check of
+every layer against a float64 prediction from the layer's own GPU inputs, at every batch bucket, is
+tests/test_gpu_layers_exact.py.
 """
 import os
 import subprocess
@@ -209,8 +213,9 @@ def test_stem_checker():
 
 
 def test_kernel_checker_all_forms():
-    """csrc/dev/test_conv: every conv kernel form (single CTA, CTA pair, swapped, split-K, strips incl. the 608 widths,
-    halo-patch) against a float64 CPU loop on small shapes."""
+    """csrc/dev/test_conv: every conv kernel form (single CTA, CTA pair, swapped, split-K incl. the production 13x13 / 26x26
+    shapes, strips incl. the 608 widths, halo-patch) against a float64 CPU loop, each element held to the rounding model of
+    tests/compare.py (half a bf16 step + 2^-23 (K + 4) S)."""
     exe = os.path.join(ROOT, "build", "test_conv")
     if not os.path.exists(exe):
         from fastdet_b200 import build
@@ -219,3 +224,7 @@ def test_kernel_checker_all_forms():
     tail = "\n".join(r.stdout.splitlines()[-60:])
     assert r.returncode == 0 and "check: 0 failing case(s)" in r.stdout, tail
     assert "x2 strip" in r.stdout  # the strip cases really took the strip form
+    # the split-K cases really split (which also runs the check that a relaunch finds its counters back at zero)
+    split_cases = [l for l in r.stdout.splitlines() if l.startswith("[splitK")]
+    assert len(split_cases) == 4 and all(" splitK " in l for l in split_cases), "\n".join(split_cases)
+    assert all("x2 splitK" in l for l in split_cases if l.startswith("[splitK 2cta")), "\n".join(split_cases)  # the CTA pair
