@@ -98,6 +98,7 @@ _PROTOS = {
     "fd_preprocess": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p]),
     "fd_forward": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p]),
     "fd_postprocess": (C.c_int, [C.c_void_p, C.c_int, C.c_double, C.c_int, C.c_void_p]),
+    "fd_postprocess_thresholds": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p, C.c_int, C.c_void_p]),
     "fd_fetch": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     "fd_detect": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_double, C.c_int,
                             C.c_void_p, C.c_void_p]),
@@ -117,6 +118,8 @@ _PROTOS = {
     "fd_server_destroy": (None, [C.c_void_p]),
     "fd_server_perform": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_int, C.c_int, C.c_double, C.c_void_p, C.c_int,
                                     C.POINTER(C.c_int32)]),
+    "fd_server_perform_jpeg": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_size_t, C.c_double, C.c_void_p, C.c_int,
+                                         C.POINTER(C.c_int32), C.POINTER(C.c_int32)]),
     "fd_server_warm": (C.c_int, [C.c_void_p, C.c_int]),
     "fd_server_lane_stats": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.POINTER(C.c_int64), C.POINTER(C.c_int64)]),
     "fd_server_closed_loop": (C.c_int, [C.c_void_p, C.c_int, C.POINTER(C.c_int32), C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_double,
@@ -245,6 +248,12 @@ class Model:
 
     def postprocess(self, n: int, threshold: float, max_det: int = 2048, stream=0):
         _check(lib().fd_postprocess(self._h, n, float(threshold), max_det, C.c_void_p(stream)))
+        self._max_det = max_det
+
+    def postprocess_thresholds(self, thresholds, max_det: int = 2048, stream=0):
+        """postprocess with one threshold per frame: frame f at thresholds[f] (n = len(thresholds))."""
+        thr = np.ascontiguousarray(thresholds, np.float64)
+        _check(lib().fd_postprocess_thresholds(self._h, thr.size, _ptr(thr), max_det, C.c_void_p(stream)))
         self._max_det = max_det
 
     def fetch(self, n: int, stream=0):

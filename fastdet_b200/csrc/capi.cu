@@ -90,6 +90,7 @@ struct Exec {  // everything that depends on the batch size
     double* scores = nullptr;
     Detection* dets = nullptr;
     int* det_count = nullptr;  // [2n]: truncated counts then totals
+    double* thr = nullptr;     // per-frame thresholds of the batch being post-processed: thr[b], then float obj_cut[b] (b frames)
     int max_det = 0;
     Detection* h_dets = nullptr;  // pinned
     int* h_count = nullptr;       // pinned [2n]
@@ -116,6 +117,10 @@ struct Slot {  // one in-flight fd_submit: staged input + pinned results + the e
     size_t h_count_cap = 0;
     char* h_stage = nullptr;      // pinned: JPEG frame descriptors + quantised coefficients of one batch
     size_t h_stage_cap = 0;
+    char* h_thr = nullptr;        // pinned: the batch's thresholds as the Exec's thr array takes them (stage_thresholds)
+    size_t h_thr_cap = 0;
+    int thr_n = 0;                // frames h_thr holds
+    cudaEvent_t thr_copied = nullptr;  // the last copy out of h_thr has run
     cudaEvent_t staged = nullptr, stage_free = nullptr, done = nullptr;
     int n = 0, max_det = 0;
     bool busy = false;
@@ -125,7 +130,7 @@ struct fd_model {
     int device = 0;
     int num_sms = 148;
     cudaStream_t copy_stream = nullptr;
-    Slot slots[FD_MAX_SLOTS + 1];  // the last one serves the synchronous JPEG calls
+    Slot slots[FD_MAX_SLOTS + 1];  // the last one serves the synchronous JPEG calls and fd_postprocess
     std::unique_ptr<JpegPool> jpeg_pool;
     std::vector<JpegInfo> jpeg_info;
     uint8_t* jpeg_planes = nullptr;  // decoded component planes of the batch being converted (compute stream only)
@@ -170,7 +175,7 @@ void free_exec(Exec* e) {
     for (void* p : e->bufs) cudaFree(p);
     cudaFree(e->splitk_ws); cudaFree(e->splitk_counters);
     cudaFree(e->frames); cudaFree(e->src); cudaFree(e->cand); cudaFree(e->cand_count); cudaFree(e->scores);
-    cudaFree(e->dets); cudaFree(e->det_count); cudaFree(e->scratch);
+    cudaFree(e->dets); cudaFree(e->det_count); cudaFree(e->thr); cudaFree(e->scratch);
     if (e->h_dets) cudaFreeHost(e->h_dets);
     if (e->h_count) cudaFreeHost(e->h_count);
     if (e->graph) cudaGraphExecDestroy(e->graph);
@@ -398,6 +403,7 @@ int get_exec(fd_model* m, int n_frames, Exec** out) {
         cudaMalloc(&e->cand_count, sizeof(int) * n) != cudaSuccess ||
         cudaMalloc(&e->scores, sizeof(double) * size_t(n) * bpf) != cudaSuccess ||
         cudaMalloc(&e->det_count, sizeof(int) * 2 * n) != cudaSuccess ||
+        cudaMalloc(&e->thr, (sizeof(double) + sizeof(float)) * n) != cudaSuccess ||
         cudaMallocHost(&e->h_count, sizeof(int) * 2 * n) != cudaSuccess ||
         cudaMemset(e->frames, 0, frame_bytes) != cudaSuccess) {
         free_exec(e.get());
@@ -603,6 +609,8 @@ void fd_model_destroy(fd_model* m) {
         if (S.h_stage) cudaFreeHost(S.h_stage);
         if (S.h_dets) cudaFreeHost(S.h_dets);
         if (S.h_count) cudaFreeHost(S.h_count);
+        if (S.h_thr) cudaFreeHost(S.h_thr);
+        if (S.thr_copied) cudaEventDestroy(S.thr_copied);
         if (S.staged) { cudaEventDestroy(S.staged); cudaEventDestroy(S.stage_free); cudaEventDestroy(S.done); }
     }
     cudaFree(m->jpeg_planes);
@@ -792,10 +800,42 @@ int fd_forward(fd_model* m, int n, void* stream) {
     return launch_layers(m, e, s);
 }
 
-// decode + Soft-NMS on the head tensors, then the records to pinned host memory (h_dets / h_count) on stream s
-static int postprocess_on(fd_model* m, Exec* e, int n, double threshold, int max_det, cudaStream_t s, Detection* h_dets,
+// The batch's thresholds thr[n] (host) and their objectness cuts, through slot T's pinned area into the Exec's thr array on
+// stream s (ahead of decode).  Pinned contents an earlier copy may still be reading are rewritten only after that copy has run;
+// a repeat at the same thresholds (fd_postprocess in a loop) rewrites nothing and never waits.
+static int stage_thresholds(fd_model* m, Exec* e, Slot& T, int n, const double* thr, cudaStream_t s) {
+    const size_t bytes = (sizeof(double) + sizeof(float)) * size_t(n);
+    if (!T.thr_copied) {
+        DEVICE_SETUP_LOCK(m);
+        CU(cudaEventCreateWithFlags(&T.thr_copied, cudaEventDisableTiming));
+    }
+    if (T.thr_n != n || memcmp(T.h_thr, thr, sizeof(double) * size_t(n)) != 0) {
+        CU(cudaEventSynchronize(T.thr_copied));
+        if (T.h_thr_cap < bytes) {
+            DEVICE_SETUP_LOCK(m);
+            if (T.h_thr) cudaFreeHost(T.h_thr);
+            T.h_thr = nullptr; T.h_thr_cap = 0; T.thr_n = 0;
+            CU(cudaMallocHost(&T.h_thr, bytes));
+            T.h_thr_cap = bytes;
+        }
+        double* h = reinterpret_cast<double*>(T.h_thr);
+        float* cut = reinterpret_cast<float*>(h + n);
+        for (int f = 0; f < n; ++f) { h[f] = thr[f]; cut[f] = obj_cut_for(thr[f]); }
+        T.thr_n = n;
+    }
+    CU(cudaMemcpyAsync(e->thr, T.h_thr, bytes, cudaMemcpyHostToDevice, s));
+    CU(cudaEventRecord(T.thr_copied, s));
+    return FD_OK;
+}
+
+// decode + Soft-NMS on the head tensors, frame f at threshold thr[f] (host array, staged through slot T), then the records to
+// pinned host memory (h_dets / h_count) on stream s
+static int postprocess_on(fd_model* m, Exec* e, Slot& T, int n, const double* thr, int max_det, cudaStream_t s, Detection* h_dets,
                           int* h_count) {
     const fd_info& I = m->info;
+    if (int rc = stage_thresholds(m, e, T, n, thr, s)) return rc;
+    const double* d_thr = e->thr;
+    const float* d_cut = reinterpret_cast<const float*>(e->thr + n);
     HeadDesc heads[FD_MAX_HEADS];
     int first = 0;
     for (int h = 0; h < I.n_heads; ++h) {
@@ -806,9 +846,9 @@ static int postprocess_on(fd_model* m, Exec* e, int n, double threshold, int max
         first += 3 * L.out.h * L.out.w;
         for (int k = 0; k < 3; ++k) { heads[h].anchor_w[k] = I.anchors[h][k][0]; heads[h].anchor_h[k] = I.anchors[h][k][1]; }
     }
-    if (launch_decode(heads, I.n_heads, I.num_classes, n, I.net_w, I.net_h, threshold, e->cand, e->cand_count, I.boxes_per_frame, s))
+    if (launch_decode(heads, I.n_heads, I.num_classes, n, I.net_w, I.net_h, d_thr, d_cut, e->cand, e->cand_count, I.boxes_per_frame, s))
         return fail(FD_ERR_CUDA, "decode launch failed: %s", cudaGetErrorString(cudaGetLastError()));
-    if (launch_soft_nms(e->cand, e->cand_count, e->scores, I.boxes_per_frame, n, I.net_w, I.net_h, threshold, e->dets,
+    if (launch_soft_nms(e->cand, e->cand_count, e->scores, I.boxes_per_frame, n, I.net_w, I.net_h, d_thr, e->dets,
                         e->det_count, e->det_count + n, max_det, s))
         return fail(FD_ERR_CUDA, "soft-nms launch failed: %s", cudaGetErrorString(cudaGetLastError()));
     CU(cudaMemcpyAsync(h_count, e->det_count, sizeof(int) * 2 * n, cudaMemcpyDeviceToHost, s));
@@ -818,6 +858,13 @@ static int postprocess_on(fd_model* m, Exec* e, int n, double threshold, int max
 
 int fd_postprocess(fd_model* m, int n, double threshold, int max_det, void* stream) {
     if (!m) return fail(FD_ERR_ARG, "fd_postprocess: null model");
+    if (n < 1) return fail(FD_ERR_ARG, "batch size must be positive (got %d)", n);
+    const std::vector<double> thr(n, threshold);
+    return fd_postprocess_thresholds(m, n, thr.data(), max_det, stream);
+}
+
+int fd_postprocess_thresholds(fd_model* m, int n, const double* thresholds, int max_det, void* stream) {
+    if (!m || !thresholds) return fail(FD_ERR_ARG, "fd_postprocess: null argument");
     const fd_info& I = m->info;
     if (I.n_heads != 2 && I.n_heads != 3) return fail(FD_ERR_HEADS, "%d", I.n_heads);  // KeyError(len(outputs)) in the reference
     if (max_det < 1) return fail(FD_ERR_ARG, "max_det must be >= 1");
@@ -836,7 +883,7 @@ int fd_postprocess(fd_model* m, int n, double threshold, int max_det, void* stre
         e->max_det = max_det;
     }
     // results to pinned host memory on the same stream; fd_fetch synchronises
-    if (int rc = postprocess_on(m, e, n, threshold, max_det, s, e->h_dets, e->h_count)) return rc;
+    if (int rc = postprocess_on(m, e, m->slots[FD_MAX_SLOTS], n, thresholds, max_det, s, e->h_dets, e->h_count)) return rc;
     m->last_n = n;
     m->last_max_det = max_det;
     return FD_OK;
@@ -1030,11 +1077,12 @@ int slot_stage_reserve(fd_model* m, Slot& S, size_t bytes) {
     return FD_OK;
 }
 
-// common tail: the conv stack, decode + Soft-NMS, results into the slot's pinned buffers, the `done` event
-int slot_finish(fd_model* m, Exec* e, Slot& S, int n, double threshold, int max_det) {
+// common tail: the conv stack, decode + Soft-NMS (frame f at threshold thr[f]), results into the slot's pinned buffers, the
+// `done` event
+int slot_finish(fd_model* m, Exec* e, Slot& S, int n, const double* thr, int max_det) {
     cudaStream_t s = m->stream;
     if (int rc = fd_forward(m, n, nullptr)) return rc;
-    if (int rc = postprocess_on(m, e, n, threshold, max_det, s, S.h_dets, S.h_count)) return rc;
+    if (int rc = postprocess_on(m, e, S, n, thr, max_det, s, S.h_dets, S.h_count)) return rc;
     CU(cudaEventRecord(S.done, s));
     S.n = n; S.max_det = max_det; S.busy = true;
     return FD_OK;
@@ -1095,7 +1143,7 @@ int jpeg_host_stage(fd_model* m, Slot& S, const uint8_t* const* data, const size
         if (only_size) return fail(FD_ERR_SIZE, "invalid image size");  // reference detector.py:132
         return fail(FD_ERR_JPEG, "frame %d: %s (status %d)", bad, why[bad].c_str(), st[bad]);
     }
-    const size_t head = (sizeof(JpegFrameDev) * size_t(n) + 255) / 256 * 256;
+    const size_t head = jpeg_head_bytes(n);
     std::vector<size_t> off(n + 1);
     off[0] = head;
     int max_blocks = 0;
@@ -1124,33 +1172,22 @@ int jpeg_host_stage(fd_model* m, Slot& S, const uint8_t* const* data, const size
     for (int i = 0; i < n; ++i)
         if (st[i] != JPEG_OK) return fail(FD_ERR_JPEG, "frame %d: %s (status %d)", i, why[i].c_str(), st[i]);
     JpegFrameDev* fr = reinterpret_cast<JpegFrameDev*>(base);
-    for (int i = 0; i < n; ++i) {
-        const JpegInfo& J = info[i];
-        JpegFrameDev& F = fr[i];
-        memset(&F, 0, sizeof(F));
-        memcpy(F.q, J.q, sizeof(F.q));
-        size_t co = (off[i] - head) / sizeof(int16_t), po = 0;
-        for (int c = 0; c < 3; ++c) {
-            F.coef_off[c] = static_cast<uint32_t>(co);
-            F.plane_off[c] = static_cast<uint32_t>(po);
-            F.bw[c] = static_cast<uint16_t>(J.bw[c]);
-            F.bh[c] = static_cast<uint16_t>(J.bh[c]);
-            co += size_t(J.bw[c]) * J.bh[c] * 64;
-            po += size_t(J.bw[c]) * J.bh[c] * 64;
-        }
-        F.hs = static_cast<uint16_t>(J.hs);
-        F.vs = static_cast<uint16_t>(J.vs);
-    }
+    for (int i = 0; i < n; ++i) jpeg_frame_desc(info[i], (off[i] - head) / sizeof(int16_t), &fr[i]);
     *bytes_out = off[n];
     *max_blocks_out = max_blocks;
     return FD_OK;
 }
 
-// Device half: pinned -> device staging on the copy stream, then IDCT and colour conversion on the compute stream,
-// ending with RGB u8 frames in the Exec's input tensor (where fd_preprocess would have put them).
-int jpeg_device_stage(fd_model* m, Exec* e, Slot& S, int n, size_t bytes, int max_blocks, int src_w, int src_h) {
+// byte ranges [first, second) of a pinned JPEG batch that hold descriptors or coefficients
+using ByteRuns = std::vector<std::pair<size_t, size_t>>;
+
+// Device half: the byte ranges `runs` of the pinned batch `src` -> the same offsets of the slot's device staging on the copy
+// stream, then IDCT and colour conversion on the compute stream, ending with RGB u8 frames in the Exec's input tensor (where
+// fd_preprocess would have put them).  The batch is [JpegFrameDev x n] from offset 0, coefficients from offset `head`.
+int jpeg_device_stage(fd_model* m, Exec* e, Slot& S, const char* src, size_t head, const ByteRuns& runs, int n, int max_blocks,
+                      int src_w, int src_h) {
     const ModelPlan& P = m->plan;
-    if (int rc = slot_stage_reserve(m, S, bytes)) return rc;
+    if (int rc = slot_stage_reserve(m, S, runs.back().second)) return rc;
     const bool same = src_w == P.net_w && src_h == P.net_h;
     const size_t plane_stride = size_t(3) * ((src_w + 15) / 16 * 16) * ((src_h + 15) / 16 * 16);
     uint8_t* rgb = e->frames;
@@ -1174,10 +1211,9 @@ int jpeg_device_stage(fd_model* m, Exec* e, Slot& S, int n, size_t bytes, int ma
     }
     cudaStream_t cs = m->copy_stream, s = m->stream;
     CU(cudaStreamWaitEvent(cs, S.stage_free, 0));
-    CU(cudaMemcpyAsync(S.stage, S.h_stage, bytes, cudaMemcpyHostToDevice, cs));
+    for (const auto& r : runs) CU(cudaMemcpyAsync(S.stage + r.first, src + r.first, r.second - r.first, cudaMemcpyHostToDevice, cs));
     CU(cudaEventRecord(S.staged, cs));
     CU(cudaStreamWaitEvent(s, S.staged, 0));
-    const size_t head = (sizeof(JpegFrameDev) * size_t(n) + 255) / 256 * 256;
     const JpegFrameDev* fr = reinterpret_cast<const JpegFrameDev*>(S.stage);
     const int16_t* coefs = reinterpret_cast<const int16_t*>(S.stage + head);
     if (launch_jpeg_idct(coefs, fr, m->jpeg_planes, plane_stride, n, max_blocks, s))
@@ -1223,7 +1259,8 @@ int fd_submit(fd_model* m, int slot, const uint8_t* frames, int n, int src_w, in
         return fail(FD_ERR_CUDA, "letterbox launch failed: %s", cudaGetErrorString(cudaGetLastError()));
     }
     CU(cudaEventRecord(S.stage_free, s));
-    if (int rc = slot_finish(m, e, S, n, threshold, max_det)) return quiesce_after_failure(m, rc);
+    const std::vector<double> thr(n, threshold);
+    if (int rc = slot_finish(m, e, S, n, thr.data(), max_det)) return quiesce_after_failure(m, rc);
     return FD_OK;
 }
 
@@ -1235,6 +1272,38 @@ int fd_collect(fd_model* m, int slot, fd_det* out, int32_t* counts, int32_t* tot
     if (!S.busy) return fail(FD_ERR_ARG, "fd_collect: nothing was submitted to slot %d", slot);
     return slot_collect(m, S, out, counts, total);
 }
+
+}  // extern "C"
+
+// library-internal (csrc/server.cc): submit a JPEG batch that the callers of fd_server_perform_jpeg have entropy-decoded
+// into pinned memory, with frame f at threshold thresholds[f].  Layout: [JpegFrameDev x cap] from offset 0, frame i's
+// coefficients from byte jpeg_head_bytes(cap) + i * stride.  Only the bytes the n frames use are copied.
+int fd_internal_submit_jpeg(fd_model* m, int slot, const uint8_t* pinned, int n, int cap, size_t stride, const double* thresholds,
+                            int max_det) {
+    if (!m || !pinned || !thresholds || n < 1 || n > cap) return fail(FD_ERR_ARG, "fd_internal_submit_jpeg: bad argument");
+    if (slot < 0 || slot >= FD_MAX_SLOTS) return fail(FD_ERR_ARG, "fd_internal_submit_jpeg: slot %d out of range [0, %d)", slot, FD_MAX_SLOTS);
+    const size_t head = jpeg_head_bytes(cap);
+    const JpegFrameDev* fr = reinterpret_cast<const JpegFrameDev*>(pinned);
+    ByteRuns runs{{0, sizeof(JpegFrameDev) * size_t(n)}};
+    int max_blocks = 0;
+    for (int i = 0; i < n; ++i) {
+        int blocks = 0;
+        for (int c = 0; c < 3; ++c) blocks += fr[i].bw[c] * fr[i].bh[c];
+        max_blocks = std::max(max_blocks, blocks);
+        const size_t o = head + stride * i, end = o + size_t(blocks) * 64 * sizeof(int16_t);
+        if (runs.back().second == o) runs.back().second = end;
+        else runs.push_back({o, end});
+    }
+    Exec* e;
+    Slot* sp;
+    if (int rc = slot_begin(m, slot, n, max_det, &e, &sp)) return rc;
+    if (int rc = jpeg_device_stage(m, e, *sp, reinterpret_cast<const char*>(pinned), head, runs, n, max_blocks, m->plan.net_w, m->plan.net_h))
+        return quiesce_after_failure(m, rc);
+    if (int rc = slot_finish(m, e, *sp, n, thresholds, max_det)) return quiesce_after_failure(m, rc);
+    return FD_OK;
+}
+
+extern "C" {
 
 // ------------------------------------------------------------------ JPEG in: reference detector.py:128-133
 int fd_jpeg_probe(const uint8_t* data, size_t len, fd_jpeg_info* out) {
@@ -1287,7 +1356,7 @@ int fd_decode_jpeg(fd_model* m, const uint8_t* const* data, const size_t* lens, 
     size_t bytes = 0;
     int max_blocks = 0, sw = 0, sh = 0;
     if (int rc = jpeg_host_stage(m, S, data, lens, n, allow_resize, status, &bytes, &max_blocks, &sw, &sh)) return rc;
-    if (int rc = jpeg_device_stage(m, e, S, n, bytes, max_blocks, sw, sh)) return rc;
+    if (int rc = jpeg_device_stage(m, e, S, S.h_stage, jpeg_head_bytes(n), ByteRuns{{0, bytes}}, n, max_blocks, sw, sh)) return rc;
     if (rgb_out) CU(cudaMemcpyAsync(rgb_out, e->frames, size_t(n) * m->plan.net_w * m->plan.net_h * 3, cudaMemcpyDeviceToHost, m->stream));
     CU(cudaStreamSynchronize(m->stream));
     return FD_OK;
@@ -1303,8 +1372,9 @@ int fd_submit_jpeg(fd_model* m, int slot, const uint8_t* const* data, const size
     size_t bytes = 0;
     int max_blocks = 0, sw = 0, sh = 0;
     if (int rc = jpeg_host_stage(m, *sp, data, lens, n, allow_resize, status, &bytes, &max_blocks, &sw, &sh)) return rc;  // nothing queued yet
-    if (int rc = jpeg_device_stage(m, e, *sp, n, bytes, max_blocks, sw, sh)) return quiesce_after_failure(m, rc);
-    if (int rc = slot_finish(m, e, *sp, n, threshold, max_det)) return quiesce_after_failure(m, rc);
+    if (int rc = jpeg_device_stage(m, e, *sp, sp->h_stage, jpeg_head_bytes(n), ByteRuns{{0, bytes}}, n, max_blocks, sw, sh)) return quiesce_after_failure(m, rc);
+    const std::vector<double> thr(n, threshold);
+    if (int rc = slot_finish(m, e, *sp, n, thr.data(), max_det)) return quiesce_after_failure(m, rc);
     return FD_OK;
 }
 
@@ -1317,8 +1387,9 @@ int fd_detect_jpeg(fd_model* m, const uint8_t* const* data, const size_t* lens, 
     size_t bytes = 0;
     int max_blocks = 0, sw = 0, sh = 0;
     if (int rc = jpeg_host_stage(m, *sp, data, lens, n, allow_resize, status, &bytes, &max_blocks, &sw, &sh)) return rc;  // nothing queued yet
-    if (int rc = jpeg_device_stage(m, e, *sp, n, bytes, max_blocks, sw, sh)) return quiesce_after_failure(m, rc);
-    if (int rc = slot_finish(m, e, *sp, n, threshold, max_det)) return quiesce_after_failure(m, rc);
+    if (int rc = jpeg_device_stage(m, e, *sp, sp->h_stage, jpeg_head_bytes(n), ByteRuns{{0, bytes}}, n, max_blocks, sw, sh)) return quiesce_after_failure(m, rc);
+    const std::vector<double> thr(n, threshold);
+    if (int rc = slot_finish(m, e, *sp, n, thr.data(), max_det)) return quiesce_after_failure(m, rc);
     return slot_collect(m, *sp, out, counts, nullptr);
 }
 

@@ -222,6 +222,27 @@ size_t jpeg_coef_count(const JpegInfo& J) {
     return blocks * 64;
 }
 
+size_t jpeg_frame_stride(int width, int height) {
+    // 4:4:4 on a 16-pixel grid: at least the coefficients of 4:2:2 and 4:2:0, whose planes are padded to 16-pixel MCUs
+    return size_t((width + 15) / 16) * ((height + 15) / 16) * 4 * 3 * 64 * sizeof(int16_t);
+}
+
+void jpeg_frame_desc(const JpegInfo& J, size_t coef_index, JpegFrameDev* F) {
+    memset(F, 0, sizeof(*F));
+    memcpy(F->q, J.q, sizeof(F->q));
+    size_t co = coef_index, po = 0;
+    for (int c = 0; c < 3; ++c) {
+        F->coef_off[c] = static_cast<uint32_t>(co);
+        F->plane_off[c] = static_cast<uint32_t>(po);
+        F->bw[c] = static_cast<uint16_t>(J.bw[c]);
+        F->bh[c] = static_cast<uint16_t>(J.bh[c]);
+        co += size_t(J.bw[c]) * J.bh[c] * 64;
+        po += size_t(J.bw[c]) * J.bh[c] * 64;
+    }
+    F->hs = static_cast<uint16_t>(J.hs);
+    F->vs = static_cast<uint16_t>(J.vs);
+}
+
 // ------------------------------------------------------------------------------------------- host: entropy decode
 namespace {
 

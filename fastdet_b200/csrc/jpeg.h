@@ -64,6 +64,13 @@ struct alignas(16) JpegFrameDev {
     uint16_t hs, vs;
 };
 
+// the descriptor of a frame whose coefficients start at int16 index coef_index of the batch coefficient buffer
+void jpeg_frame_desc(const JpegInfo& info, size_t coef_index, JpegFrameDev* out);
+// bytes in front of a JPEG batch's coefficients: the descriptors of `frames` frames, rounded up to 256
+inline size_t jpeg_head_bytes(int frames) { return (sizeof(JpegFrameDev) * size_t(frames) + 255) / 256 * 256; }
+// bytes that hold the coefficients of any frame of this size the device path takes (4:4:4 / 4:2:2 / 4:2:0); a multiple of 512
+size_t jpeg_frame_stride(int width, int height);
+
 // coefficients -> u8 component planes [frame][plane_stride]
 int launch_jpeg_idct(const int16_t* coefs, const JpegFrameDev* frames, uint8_t* planes, size_t plane_stride, int n,
                      int max_blocks, cudaStream_t s);

@@ -53,13 +53,18 @@ struct Detection {     // mirrors include/fastdet_b200.h: fd_det
     int32_t klass, box;
     double conf, x, y, w, h;
 };
+// Thresholds are per frame: thr[n] (the reference's `threshold`, a Python float) and obj_cut[n] = obj_cut_for(thr[f]),
+// both device arrays, so frames of one batch may carry different thresholds.
+// host: the objectness pre-test cut of decode for one threshold (-inf for thresholds outside (0, 1): no pre-test)
+float obj_cut_for(double threshold);
 // decode + two-stage threshold + compaction: fills cand[frame][*] (capacity boxes_per_frame) and counts.
 int launch_decode(const HeadDesc* heads, int n_heads, int num_classes, int n, int net_w, int net_h,
-                  double threshold, Candidate* cand, int* cand_count, int boxes_per_frame, cudaStream_t s);
-// class-agnostic Gaussian Soft-NMS per frame (reference detector.py:45-59); writes up to max_det detections
-// per frame in selection order (pixels, top-left + size) and the per-frame count (untruncated count in total).
+                  const double* thr, const float* obj_cut, Candidate* cand, int* cand_count, int boxes_per_frame, cudaStream_t s);
+// class-agnostic Gaussian Soft-NMS per frame (reference detector.py:45-59), frame f at threshold thr[f]; writes up to
+// max_det detections per frame in selection order (pixels, top-left + size) and the per-frame count (untruncated count
+// in total).
 int launch_soft_nms(Candidate* cand, const int* cand_count, double* score_scratch, int boxes_per_frame, int n,
-                    int net_w, int net_h, double threshold, Detection* out, int* out_count, int* total_count,
+                    int net_w, int net_h, const double* thr, Detection* out, int* out_count, int* total_count,
                     int max_det, cudaStream_t s);
 
 }  // namespace fd

@@ -25,9 +25,13 @@ struct DecodeParams {
     HeadDesc heads[4];
     int cell_start[5];  // prefix sum of h*w per head
     int n_heads, num_classes, n, net_w, net_h, boxes_per_frame;
-    double threshold;
-    float obj_cut;  // logits below this cannot reach the threshold (logit(threshold) minus a safety margin); -inf: no pre-test
+    const double* thr;     // [n] the frame's threshold
+    const float* obj_cut;  // [n] objectness logits below this cannot reach the frame's threshold (obj_cut_for)
 };
+
+float obj_cut_for(double threshold) {  // logit(threshold) minus a safety margin; -inf: no pre-test
+    return (threshold > 0.0 && threshold < 1.0) ? static_cast<float>(log(threshold / (1.0 - threshold)) - 1e-3) : -INFINITY;
+}
 
 __device__ __forceinline__ double logistic(float v) { return 1.0 / (1.0 + exp(-static_cast<double>(v))); }
 
@@ -54,16 +58,17 @@ decode_kernel(const DecodeParams p, Candidate* __restrict__ cand, int* __restric
         return H.data + (1LL * frame * H.h * H.w + cell) * H.pitch + k * span;
     };
 
-    double obj = 0.0;
+    double obj = 0.0, threshold = 0.0;
     bool pass = false;
     if (live) {
         int hi, cell, k;
         const float t4 = __ldg(locate(f, b, hi, cell, k) + 4);
+        threshold = __ldg(p.thr + f);
         // float pre-test (sigmoid is monotonic, the margin dwarfs any rounding): ~99 % of the boxes end here; the decision
         // itself is taken in float64 exactly as the reference does
-        if (!(t4 < p.obj_cut)) {
+        if (!(t4 < __ldg(p.obj_cut + f))) {
             obj = logistic(t4);
-            pass = !(obj < p.threshold);  // reference: `if conf < threshold: continue`
+            pass = !(obj < threshold);  // reference: `if conf < threshold: continue`
         }
     }
     unsigned mask = __ballot_sync(0xffffffffu, pass);
@@ -87,9 +92,9 @@ decode_kernel(const DecodeParams p, Candidate* __restrict__ cand, int* __restric
             const int oi = __shfl_xor_sync(0xffffffffu, best_i, o);
             if (oi != INT_MAX && (best_i == INT_MAX || ov > best || (ov == best && oi < best_i))) { best = ov; best_i = oi; }
         }
-        if (lane == src) {
+        if (lane == src) {  // (the owning lane: its f is bf, its threshold the frame's)
             const double conf = obj * logistic(best);
-            if (!(conf < p.threshold)) {
+            if (!(conf < threshold)) {
                 const HeadDesc& H = p.heads[hi];
                 const int gy = cell / H.w, gx = cell - gy * H.w;
                 const double x = (gx + logistic(__ldg(box + 0))) / H.w;
@@ -112,7 +117,7 @@ decode_kernel(const DecodeParams p, Candidate* __restrict__ cand, int* __restric
 }
 
 int launch_decode(const HeadDesc* heads, int n_heads, int num_classes, int n, int net_w, int net_h,
-                  double threshold, Candidate* cand, int* cand_count, int boxes_per_frame, cudaStream_t s) {
+                  const double* thr, const float* obj_cut, Candidate* cand, int* cand_count, int boxes_per_frame, cudaStream_t s) {
     if (n_heads < 1 || n_heads > 4) return -1;
     DecodeParams p;
     p.cell_start[0] = 0;
@@ -121,8 +126,7 @@ int launch_decode(const HeadDesc* heads, int n_heads, int num_classes, int n, in
         p.cell_start[i + 1] = p.cell_start[i] + heads[i].h * heads[i].w;
     }
     p.n_heads = n_heads; p.num_classes = num_classes; p.n = n; p.net_w = net_w; p.net_h = net_h;
-    p.boxes_per_frame = boxes_per_frame; p.threshold = threshold;
-    p.obj_cut = (threshold > 0.0 && threshold < 1.0) ? static_cast<float>(log(threshold / (1.0 - threshold)) - 1e-3) : -INFINITY;
+    p.boxes_per_frame = boxes_per_frame; p.thr = thr; p.obj_cut = obj_cut;
     if (cudaMemsetAsync(cand_count, 0, sizeof(int) * n, s) != cudaSuccess) return -1;
     if (boxes_per_frame != 3 * p.cell_start[n_heads]) return -1;
     const long long boxes = 1LL * n * boxes_per_frame;
@@ -212,9 +216,10 @@ __device__ __forceinline__ void soft_nms_in_registers(const Candidate* __restric
 
 __global__ void __launch_bounds__(NMS_THREADS)
 soft_nms_kernel(const Candidate* __restrict__ cand_all, const int* __restrict__ cand_count, double* __restrict__ score_all,
-                int cap, int net_w, int net_h, double threshold, Detection* __restrict__ out, int* __restrict__ out_count,
+                int cap, int net_w, int net_h, const double* __restrict__ thr, Detection* __restrict__ out, int* __restrict__ out_count,
                 int* __restrict__ total_count, int max_det, int allow_fast) {
     const int f = blockIdx.x;
+    const double threshold = thr[f];
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     const int C = min(cand_count[f], cap);
     const Candidate* cand = cand_all + 1LL * f * cap;
@@ -300,10 +305,10 @@ soft_nms_kernel(const Candidate* __restrict__ cand_all, const int* __restrict__ 
 }
 
 int launch_soft_nms(Candidate* cand, const int* cand_count, double* score_scratch, int boxes_per_frame, int n,
-                    int net_w, int net_h, double threshold, Detection* out, int* out_count, int* total_count,
+                    int net_w, int net_h, const double* thr, Detection* out, int* out_count, int* total_count,
                     int max_det, cudaStream_t s) {
     const int allow_fast = options().nms_general ? 0 : 1;  // option nms_general: force the general loop (tests run both)
-    soft_nms_kernel<<<n, NMS_THREADS, 0, s>>>(cand, cand_count, score_scratch, boxes_per_frame, net_w, net_h, threshold,
+    soft_nms_kernel<<<n, NMS_THREADS, 0, s>>>(cand, cand_count, score_scratch, boxes_per_frame, net_w, net_h, thr,
                                               out, out_count, total_count, max_det, allow_fast);
     return cudaPeekAtLastError() == cudaSuccess ? 0 : -1;  // (peek: the caller reports the reason)
 }

@@ -12,6 +12,10 @@
 // host->device copy and the entropy of forming the next batch overlap the conv stack of the previous one, and — like
 // fastdet_b200/service.py — never waits for more requests while the device has work: whatever has arrived when a slot
 // frees up is the next batch.
+// JPEG payloads (fd_server_perform_jpeg, the reference's own request) ride JPEG batches: each caller parses its payload and
+// entropy-decodes it straight into its place in the batch's pinned buffer, again in parallel in the callers' threads; the
+// worker submits the batch to the device half of fd_submit_jpeg (IDCT + colour on the device, then the forward pass).  The
+// threshold is per frame in a JPEG batch, so requests with different thresholds share it; an RGB batch keeps one threshold.
 #include <string.h>
 
 #include <algorithm>
@@ -28,10 +32,13 @@
 #include <cuda_runtime.h>
 
 #include "../../include/fastdet_b200.h"
+#include "jpeg.h"
 #include "options.h"
 
 void* fd_internal_pinned_alloc(int device, size_t bytes);  // capi.cu
 void fd_internal_pinned_free(int device, void* p);
+int fd_internal_submit_jpeg(fd_model* m, int slot, const uint8_t* pinned, int n, int cap, size_t stride, const double* thresholds,
+                            int max_det);
 
 namespace {
 
@@ -43,6 +50,8 @@ struct Backend {  // what a lane drives: the two-slot submit / collect pair of o
     int w = 0, h = 0, device = 0;
     virtual ~Backend() {}
     virtual int submit(int slot, const uint8_t* frames, int n, double thr, int max_det) = 0;
+    // a JPEG batch laid out as fd_internal_submit_jpeg takes it; frame f at threshold thr[f]
+    virtual int submit_jpeg(int slot, const uint8_t* pinned, int n, int cap, size_t stride, const double* thr, int max_det) = 0;
     virtual int collect(int slot, fd_det* out, int32_t* counts) = 0;
     virtual uint8_t* alloc_pinned(size_t bytes) = 0;
     virtual void free_pinned(uint8_t* p) = 0;
@@ -54,6 +63,9 @@ struct ModelBackend : Backend {
     int submit(int slot, const uint8_t* frames, int n, double thr, int max_det) override {
         return fd_submit(m, slot, frames, n, w, h, 0, 0, thr, max_det);
     }
+    int submit_jpeg(int slot, const uint8_t* pinned, int n, int cap, size_t stride, const double* thr, int max_det) override {
+        return fd_internal_submit_jpeg(m, slot, pinned, n, cap, stride, thr, max_det);
+    }
     int collect(int slot, fd_det* out, int32_t* counts) override { return fd_collect(m, slot, out, counts, nullptr); }
     // (under the device's set-up lock: a pinned allocation must not run into another lane's graph capture, capi.cu)
     uint8_t* alloc_pinned(size_t bytes) override { return static_cast<uint8_t*>(fd_internal_pinned_alloc(device, bytes)); }
@@ -62,13 +74,24 @@ struct ModelBackend : Backend {
 
 // Host-only stand-in (tests of the routing / batching logic on machines without a GPU): "detects" one box per frame
 // that records where and how the frame was served: klass = first byte of the frame, box = batch size it rode in,
-// conf = device, x = model index, y = slot.
+// conf = device, x = model index, y = slot.  JPEG frames (decoded by the real host half): klass = the first quantised
+// luma DC coefficient, w = the frame's threshold.
 struct FakeBackend : Backend {
     int model = 0, latency_us = 0;
-    struct Held { std::vector<uint8_t> first; int n = 0, slot = 0; } held[FD_MAX_SLOTS];
+    struct Held { std::vector<int> first; std::vector<double> thr; int n = 0, slot = 0; } held[FD_MAX_SLOTS];
     int submit(int slot, const uint8_t* frames, int n, double, int) override {
         held[slot].first.resize(n);
+        held[slot].thr.assign(n, 0.0);
         for (int i = 0; i < n; ++i) held[slot].first[i] = frames[static_cast<size_t>(i) * w * h * 3];
+        held[slot].n = n;
+        held[slot].slot = slot;
+        return FD_OK;
+    }
+    int submit_jpeg(int slot, const uint8_t* pinned, int n, int cap, size_t stride, const double* thr, int) override {
+        held[slot].first.resize(n);
+        held[slot].thr.assign(thr, thr + n);
+        for (int i = 0; i < n; ++i)
+            held[slot].first[i] = *reinterpret_cast<const int16_t*>(pinned + fd::jpeg_head_bytes(cap) + static_cast<size_t>(i) * stride);
         held[slot].n = n;
         held[slot].slot = slot;
         return FD_OK;
@@ -79,7 +102,7 @@ struct FakeBackend : Backend {
             counts[i] = 1;
             fd_det& d = out[static_cast<size_t>(i) * max_det];
             memset(&d, 0, sizeof(d));
-            d.klass = held[slot].first[i]; d.box = held[slot].n; d.conf = device; d.x = model; d.y = slot;
+            d.klass = held[slot].first[i]; d.box = held[slot].n; d.conf = device; d.x = model; d.y = slot; d.w = held[slot].thr[i];
         }
         return FD_OK;
     }
@@ -89,11 +112,13 @@ struct FakeBackend : Backend {
 };
 
 struct Batch {
-    uint8_t* pinned = nullptr;
+    enum Kind { RGB, JPEG } kind = RGB;
+    uint8_t* pinned = nullptr;  // RGB: frames [cap][h][w][3]; JPEG: [JpegFrameDev x cap], then coefficients at Lane::jpeg_stride
     int cap = 0;                // frames the pinned buffer holds
     int n = 0;                  // frames claimed by callers
-    std::atomic<int> ready{0};  // frames copied in
-    double threshold = 0.0;
+    std::atomic<int> ready{0};  // frames copied (RGB) or entropy-decoded (JPEG) in
+    double threshold = 0.0;     // RGB: the batch's threshold
+    std::vector<double> thr;    // JPEG: [cap] each frame's threshold
     Clock::time_point t_first;
     std::vector<fd_det> dets;
     std::vector<int32_t> counts;
@@ -109,6 +134,7 @@ struct Lane {
     int max_batch = 64, max_det = 256;
     double max_delay_s = 0.0;
     size_t frame_bytes = 0;
+    size_t jpeg_stride = 0;  // coefficient bytes per frame of a JPEG batch (a network-sized 4:4:4 frame)
     std::mutex mu;
     std::condition_variable cv_work, cv_done;
     Batch* open = nullptr;
@@ -121,10 +147,14 @@ struct Lane {
     std::thread worker;
     int64_t batches = 0, frames = 0;
 
-    Batch* fresh() {  // mu held; nullptr when pinned memory cannot be had
+    size_t pinned_bytes(Batch::Kind kind, int cap) const {
+        return kind == Batch::RGB ? frame_bytes * cap : fd::jpeg_head_bytes(cap) + jpeg_stride * cap;
+    }
+
+    Batch* fresh(Batch::Kind kind) {  // mu held; nullptr when pinned memory cannot be had
         Batch* b = nullptr;
         for (size_t i = 0; i < pool.size(); ++i)
-            if (pool[i]->cap >= cur_cap) { b = pool[i]; pool.erase(pool.begin() + i); break; }
+            if (pool[i]->kind == kind && pool[i]->cap >= cur_cap) { b = pool[i]; pool.erase(pool.begin() + i); break; }
         if (!b) {
             if (!pool.empty()) {  // recycle an object whose buffer has become too small
                 b = pool.back(); pool.pop_back();
@@ -134,11 +164,13 @@ struct Lane {
                 b = new Batch();
                 all.push_back(b);
             }
-            b->pinned = be->alloc_pinned(frame_bytes * cur_cap);
+            b->kind = kind;
+            b->pinned = be->alloc_pinned(pinned_bytes(kind, cur_cap));
             if (!b->pinned) { pool.push_back(b); return nullptr; }
             b->cap = cur_cap;
             b->dets.resize(static_cast<size_t>(b->cap) * max_det);
             b->counts.resize(b->cap);
+            b->thr.resize(b->cap);
         }
         b->n = 0; b->ready.store(0); b->rc = FD_OK; b->err.clear(); b->done = false; b->waiting = 0; b->slot = -1;
         return b;
@@ -170,8 +202,13 @@ struct Lane {
                     b->slot = slot;
                     const int n = b->n;
                     lk.unlock();
-                    while (b->ready.load(std::memory_order_acquire) < n) std::this_thread::yield();  // a caller is still copying its frame in
-                    const int rc = be->submit(slot, b->pinned, n, b->threshold, max_det);
+                    // a caller is still copying its frame in (RGB: microseconds) or entropy-decoding it (JPEG: a millisecond or more)
+                    while (b->ready.load(std::memory_order_acquire) < n) {
+                        if (b->kind == Batch::JPEG) std::this_thread::sleep_for(std::chrono::microseconds(20));
+                        else std::this_thread::yield();
+                    }
+                    const int rc = b->kind == Batch::JPEG ? be->submit_jpeg(slot, b->pinned, n, b->cap, jpeg_stride, b->thr.data(), max_det)
+                                                          : be->submit(slot, b->pinned, n, b->threshold, max_det);
                     std::string err = rc ? fd_last_error() : "";
                     lk.lock();
                     ++batches; frames += n;
@@ -200,6 +237,50 @@ struct Lane {
             if (stop) return;
             cv_work.wait(lk);
         }
+    }
+
+    // A caller's place in the open batch of `kind`: the open batch is closed first when it is full or of the other kind, or
+    // (RGB, whose batches hold one threshold) has another threshold.  Returns nullptr when pinned memory cannot be had.
+    Batch* claim(Batch::Kind kind, double threshold, int* idx) {
+        std::unique_lock<std::mutex> lk(mu);
+        if (open && (open->n >= open->cap || open->kind != kind || (kind == Batch::RGB && open->threshold != threshold))) {
+            closed.push_back(open);
+            open = nullptr;
+        }
+        if (!open) {
+            open = fresh(kind);
+            if (!open) return nullptr;
+            open->threshold = threshold;
+            open->t_first = Clock::now();
+        }
+        Batch* b = open;
+        *idx = b->n++;
+        ++b->waiting;
+        b->thr[*idx] = threshold;
+        if (b->n >= b->cap) {  // full: it goes as it is, and the next batches get more room
+            if (b->cap < max_batch) cur_cap = std::min(max_batch, 2 * b->cap);
+            closed.push_back(b);
+            open = nullptr;
+        }
+        lk.unlock();
+        cv_work.notify_one();
+        return b;
+    }
+
+    // Sleeps until the batch is back, then copies frame idx's records out (none when out is null) and lets go of the batch.
+    int await(Batch* b, int idx, fd_det* out, int out_max, int32_t* count) {
+        std::unique_lock<std::mutex> lk(mu);
+        cv_done.wait(lk, [&] { return b->done; });
+        const int rc = b->rc;
+        if (rc == FD_OK && out) {
+            const int c = std::min<int>(b->counts[idx], out_max);
+            *count = c;
+            memcpy(out, b->dets.data() + static_cast<size_t>(idx) * max_det, sizeof(fd_det) * static_cast<size_t>(c));
+        } else if (rc != FD_OK) {
+            snprintf(g_serr, sizeof(g_serr), "%s", b->err.c_str());
+        }
+        if (--b->waiting == 0) pool.push_back(b);
+        return rc;
     }
 };
 
@@ -250,6 +331,7 @@ int fd_server_create(const fd_server_model* models, int n_models, const int32_t*
             l->max_batch = max_batch; l->max_det = max_det; l->max_delay_s = max_delay_ms * 1e-3; l->cur_cap = std::min(8, max_batch);
             l->max_inflight = std::max(1, std::min<int>(FD_MAX_SLOTS, fd::options().server_inflight));
             l->frame_bytes = static_cast<size_t>(be->w) * be->h * 3;
+            l->jpeg_stride = fd::jpeg_frame_stride(be->w, be->h);
             l->be = std::move(be);
             s->lanes.push_back(std::move(l));
         }
@@ -272,6 +354,7 @@ int fd_server_create_fake(int n_models, int n_devices, int net_w, int net_h, int
             l->max_batch = max_batch; l->max_det = 1; l->max_delay_s = max_delay_ms * 1e-3; l->cur_cap = std::min(8, max_batch);
             l->max_inflight = std::max(1, std::min<int>(FD_MAX_SLOTS, fd::options().server_inflight));
             l->frame_bytes = static_cast<size_t>(net_w) * net_h * 3;
+            l->jpeg_stride = fd::jpeg_frame_stride(net_w, net_h);
             l->be = std::move(be);
             s->lanes.push_back(std::move(l));
         }
@@ -303,45 +386,53 @@ int fd_server_perform(fd_server* s, int stream_id, int model, const uint8_t* fra
     if (src_w != s->net_w[model] || src_h != s->net_h[model]) return sfail(FD_ERR_SIZE, "invalid image size");  // reference detector.py:132
     if (s->closing.load()) return sfail(FD_ERR_ARG, "fd_server_perform: server is shutting down");
     Lane& L = s->lane(stream_id % s->n_devices, model);
-    Batch* b;
     int idx;
-    {
-        std::unique_lock<std::mutex> lk(L.mu);
-        if (L.open && (L.open->n >= L.open->cap || L.open->threshold != threshold)) {  // one threshold per batch (it is a kernel argument)
-            L.closed.push_back(L.open);
-            L.open = nullptr;
-        }
-        if (!L.open) {
-            L.open = L.fresh();
-            if (!L.open) return sfail(FD_ERR_CUDA, "fd_server_perform: pinned host memory for a micro-batch could not be allocated");
-            L.open->threshold = threshold;
-            L.open->t_first = Clock::now();
-        }
-        b = L.open;
-        idx = b->n++;
-        ++b->waiting;
-        if (b->n >= b->cap) {  // full: it goes as it is, and the next batches get more room
-            if (b->cap < L.max_batch) L.cur_cap = std::min(L.max_batch, 2 * b->cap);
-            L.closed.push_back(b);
-            L.open = nullptr;
-        }
-    }
-    L.cv_work.notify_one();
+    Batch* b = L.claim(Batch::RGB, threshold, &idx);
+    if (!b) return sfail(FD_ERR_CUDA, "fd_server_perform: pinned host memory for a micro-batch could not be allocated");
     memcpy(b->pinned + static_cast<size_t>(idx) * L.frame_bytes, frame, L.frame_bytes);  // in the caller's thread: concurrent callers copy in parallel
     b->ready.fetch_add(1, std::memory_order_release);
-    int rc;
-    {
-        std::unique_lock<std::mutex> lk(L.mu);
-        L.cv_done.wait(lk, [&] { return b->done; });
-        rc = b->rc;
-        if (rc == FD_OK) {
-            const int c = std::min<int>(b->counts[idx], max_det);
-            *count = c;
-            memcpy(out, b->dets.data() + static_cast<size_t>(idx) * L.max_det, sizeof(fd_det) * static_cast<size_t>(c));
-        } else {
-            snprintf(g_serr, sizeof(g_serr), "%s", b->err.c_str());
-        }
-        if (--b->waiting == 0) L.pool.push_back(b);
+    return L.await(b, idx, out, max_det, count);
+}
+
+int fd_server_perform_jpeg(fd_server* s, int stream_id, int model, const uint8_t* data, size_t len, double threshold, fd_det* out,
+                           int max_det, int32_t* count, int32_t* status) {
+    int32_t st_local = 0;
+    int32_t& st = status ? *status : st_local;
+    st = FD_JPEG_OK;
+    if (!s || !data || !out || !count || stream_id < 0 || model < 0 || model >= s->n_models || max_det < 1)
+        return sfail(FD_ERR_ARG, "fd_server_perform_jpeg: bad argument");
+    std::unique_ptr<fd::JpegInfo> J(new fd::JpegInfo());
+    char why[160] = "";
+    st = fd::jpeg_parse(data, len, J.get(), why, sizeof(why));
+    if (st != fd::JPEG_OK) {
+        snprintf(g_serr, sizeof(g_serr), "%s (status %d)", why, st);
+        return FD_ERR_JPEG;
+    }
+    if (J->width != s->net_w[model] || J->height != s->net_h[model]) {  // reference detector.py:132
+        st = FD_JPEG_SIZE;
+        return sfail(FD_ERR_SIZE, "invalid image size");
+    }
+    if (s->closing.load()) return sfail(FD_ERR_ARG, "fd_server_perform_jpeg: server is shutting down");
+    Lane& L = s->lane(stream_id % s->n_devices, model);
+    if (fd::jpeg_coef_count(*J) * sizeof(int16_t) > L.jpeg_stride) {  // (the sampling factors jpeg_parse takes always fit)
+        st = FD_JPEG_UNSUPPORTED;
+        return sfail(FD_ERR_JPEG, "fd_server_perform_jpeg: coefficients exceed the batch's per-frame stride");
+    }
+    int idx;
+    Batch* b = L.claim(Batch::JPEG, threshold, &idx);
+    if (!b) return sfail(FD_ERR_CUDA, "fd_server_perform_jpeg: pinned host memory for a micro-batch could not be allocated");
+    // in the caller's thread: concurrent callers entropy-decode in parallel.  The descriptor comes from the header alone, so a
+    // frame whose entropy data is damaged still rides the batch (its caller gets no records)
+    const size_t off = static_cast<size_t>(idx) * L.jpeg_stride;
+    const int dst = fd::jpeg_decode_coefficients(data, len, *J, reinterpret_cast<int16_t*>(b->pinned + fd::jpeg_head_bytes(b->cap) + off),
+                                                 why, sizeof(why));
+    fd::jpeg_frame_desc(*J, off / sizeof(int16_t), reinterpret_cast<fd::JpegFrameDev*>(b->pinned) + idx);
+    b->ready.fetch_add(1, std::memory_order_release);
+    const int rc = L.await(b, idx, dst == fd::JPEG_OK ? out : nullptr, max_det, count);
+    if (rc == FD_OK && dst != fd::JPEG_OK) {
+        st = dst;
+        snprintf(g_serr, sizeof(g_serr), "%s (status %d)", why, dst);
+        return FD_ERR_JPEG;
     }
     return rc;
 }

@@ -12,6 +12,11 @@ include/fastdet_b200.h); this class owns the handle and converts records to the 
     srv = DetectServer({"full": (full_onnx_bytes, 80), "rsu": (rsu_onnx_bytes, 9)}, devices=range(8))
     results = srv.perform("full", stream_id, frame_u8_hwc, threshold=0.1)     # [(klass, conf, x, y, w, h), ...]
     srv.detector("full", stream_id).perform(jpeg_bytes, threshold)           # drop-in object for server.py's dict
+
+JPEG payloads (``perform_jpeg_records`` and the drop-in object) take the device decode path of ``fd_detect_jpeg``: each
+caller entropy-decodes its payload in its own thread straight into the lane's open micro-batch, and requests with
+different thresholds share that batch.  Payloads the device decoder refuses (PNG, progressive, greyscale, damaged
+entropy data) are decoded with PIL by the drop-in object, as the reference does.
 """
 import ctypes as C
 import io
@@ -93,6 +98,22 @@ class DetectServer:
                                                     _native._ptr(out), self.max_det, C.byref(count)))
         return out[:count.value]
 
+    def perform_jpeg_records(self, model, stream_id, data, threshold=0.1):
+        """data: one JPEG payload (bytes).  Returns the frame's fd_det records (structured array).  Raises
+        _native.JpegRefused (with the FD_JPEG_* status) for a payload the device decoder does not take or whose entropy data
+        is damaged, and ValueError('invalid image size') for a frame that is not the model's size."""
+        data = bytes(data)
+        out = np.zeros(self.max_det, _native.DET_DTYPE)
+        count, status = C.c_int32(), C.c_int32()
+        m = model if isinstance(model, int) else self.names.index(model)
+        rc = _native.lib().fd_server_perform_jpeg(self._h, int(stream_id), m, data, len(data), float(threshold), _native._ptr(out),
+                                                  self.max_det, C.byref(count), C.byref(status))
+        if rc == _native.FD_ERR_JPEG:
+            msg = (_native.lib().fd_server_last_error() or b"").decode("utf-8", "replace")
+            raise _native.JpegRefused(msg, np.array([status.value], np.int32))
+        self._check(rc)
+        return out[:count.value]
+
     def perform(self, model, stream_id, frame, threshold=0.1):
         """The reference's result list for one decoded frame: [(klass, conf, x, y, w, h), ...] (detector.py:142-144)."""
         return self.perform_records(model, stream_id, frame, threshold)[["klass", "conf", "x", "y", "w", "h"]].tolist()
@@ -143,7 +164,13 @@ class _BoundDetector:
         return f"<DetectServer.detector model={self.model}, stream={self.stream_id}, devices={self.server.devices}>"
 
     def perform(self, data, threshold=0.1):
-        """Encoded payload in, like the reference (detector.py:126-146); decode in the caller's thread."""
+        """Encoded payload in, like the reference (detector.py:126-146).  A JPEG the device decoder takes rides the lane's JPEG
+        micro-batch; anything else is decoded with PIL in the caller's thread, so it gives the reference's result or exception."""
+        try:
+            recs = self.server.perform_jpeg_records(self.model, self.stream_id, data, threshold)
+            return recs[["klass", "conf", "x", "y", "w", "h"]].tolist()
+        except _native.JpegRefused:
+            pass
         from PIL import Image
         img = Image.open(io.BytesIO(data))
         if img.size != self.image_size:

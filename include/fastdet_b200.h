@@ -140,6 +140,9 @@ int fd_forward(fd_model* m, int n, void* stream);
 /* Decode + Soft-NMS on the head tensors of the last fd_forward.  Results land in device/pinned buffers owned by
  * the model; fd_fetch copies them out.  threshold is the reference's `threshold` (a Python float). */
 int fd_postprocess(fd_model* m, int n, double threshold, int max_det, void* stream);
+/* fd_postprocess with one threshold per frame (thresholds[n], host memory; read before the call returns).  Frame f's
+ * records are bit for bit those of fd_postprocess at thresholds[f]. */
+int fd_postprocess_thresholds(fd_model* m, int n, const double* thresholds, int max_det, void* stream);
 /* Synchronise `stream` and copy the results of the last fd_postprocess: counts[n] and out[n][max_det]
  * (max_det as given to fd_postprocess).  total[n] (optional) receives the untruncated kept count. */
 int fd_fetch(fd_model* m, int n, fd_det* out, int32_t* counts, int32_t* total, void* stream);
@@ -218,7 +221,8 @@ int fd_pack_wire(const fd_det* dets, int count, uint32_t reqid, uint32_t msec, i
  * streams + a worker thread + a queue of micro-batches (two in flight through fd_submit / fd_collect).  A stream is
  * pinned to device slot (stream_id mod n_devices).  fd_server_perform has the call shape of perform() — one decoded RGB
  * frame in, that frame's records out, blocking — and may be called from any number of threads at once; concurrent calls
- * for the same (device, model) ride in one batch.  Results are those of fd_detect on the same frame (to the batch-size
+ * for the same (device, model) ride in one batch.  fd_server_perform_jpeg takes the payload perform() gets, JPEG bytes with
+ * the request's own threshold, and decodes it on the device path of fd_detect_jpeg.  Results are those of fd_detect on the same frame (to the batch-size
  * dependence documented for split-K).  No collective, no cross-device traffic: frames are independent. */
 #define FD_SERVER_MAX_MODELS 8
 #define FD_SERVER_MAX_DEVICES 16
@@ -248,9 +252,19 @@ int fd_server_create(const fd_server_model* models, int n_models, const int32_t*
                      int max_det, double max_delay_ms, fd_server** out);
 void fd_server_destroy(fd_server* s);
 /* Blocking, thread-safe.  frame: host RGB u8 [src_h, src_w, 3] (copied before the call sleeps); src size must be the
- * model's (FD_ERR_SIZE otherwise, reference detector.py:132).  out[max_det], *count: the frame's records. */
+ * model's (FD_ERR_SIZE otherwise, reference detector.py:132).  out[max_det], *count: the frame's records.  A micro-batch
+ * of RGB frames holds one threshold: a caller with another threshold starts a new batch. */
 int fd_server_perform(fd_server* s, int stream_id, int model, const uint8_t* frame, int src_w, int src_h, double threshold,
                       fd_det* out, int max_det, int32_t* count);
+/* fd_server_perform for one encoded payload: blocking, thread-safe.  A payload the device decoder does not take returns
+ * FD_ERR_JPEG with *status (FD_JPEG_*) and never enters a batch; a decodable frame of another size returns FD_ERR_SIZE.
+ * The caller's thread parses the payload and entropy-decodes it straight into the open JPEG micro-batch of its lane; the
+ * IDCT, colour conversion, forward pass and post-processing of the batch run on the device.  Callers with different
+ * thresholds share a JPEG batch (the thresholds are per frame).  A payload whose entropy data turns out damaged behind a
+ * valid header still rides its batch, but its caller gets FD_ERR_JPEG / FD_JPEG_CORRUPT and no records; the other
+ * frames of the batch are not affected.  status may be NULL. */
+int fd_server_perform_jpeg(fd_server* s, int stream_id, int model, const uint8_t* data, size_t len, double threshold,
+                           fd_det* out, int max_det, int32_t* count, int32_t* status);
 /* Build every lane's execution state for the batch-size buckets up to `up_to` frames now (in parallel over the lanes), so
  * that no request pays for buffer allocation and graph capture later.  Call before serving. */
 int fd_server_warm(fd_server* s, int up_to);
@@ -262,7 +276,8 @@ int fd_server_closed_loop(fd_server* s, int n_streams, const int32_t* stream_mod
                           int src_w, int src_h, double threshold, double warmup_seconds, double seconds, fd_serve_stats* out);
 /* Host-only stand-in backend (tests of routing / batching without a GPU): every frame "detects" one record that says where
  * it was served: klass = the frame's first byte, box = size of the batch it rode in, conf = device slot, x = model, y = ring
- * slot; collect sleeps latency_us. */
+ * slot; collect sleeps latency_us.  JPEG payloads go through the real host half (parse, entropy decode into the batch);
+ * their record has klass = the frame's first quantised luma DC coefficient and w = the frame's threshold. */
 int fd_server_create_fake(int n_models, int n_devices, int net_w, int net_h, int max_batch, double max_delay_ms, int latency_us,
                           fd_server** out);
 const char* fd_server_last_error(void);
