@@ -10,7 +10,10 @@ partial tile, wrong pad read or doubled split-K part exceeds.
 
 The matrix runs each batch-size bucket (power of two, execution state is built per bucket) and the paths that only some
 buckets take; test_matrix_covers_every_kernel_form asserts, through fd_layer_exec_info, that the rows together still run every
-kernel form, so a planner change that moves a form out of the matrix fails there.  Each row prints one line per layer:
+kernel form, so a planner change that moves a form out of the matrix fails there.  Rows on non-square nets (416x256 and its
+transpose, 640x384, 320x192, 96x160) catch what a square map hides — a swapped height and width, a row pitch or a tile count
+taken from the wrong axis — and test_nonsquare_rows_cover_every_kernel_form asserts that they alone run every form.  Each row
+prints one line per layer:
 index, name, kernel form, block_n, split_k, K, the worst ratio of |g - r| to the bound, the share of elements that differ from
 r rounded to the output type, and the worst fp32 accumulation error in units of U*S (the model allows K + 4)."""
 import numpy as np
@@ -26,22 +29,31 @@ pytestmark = pytest.mark.gpu
 
 THR = 0.1
 
-# id: (arch, classes, size, options, batch, path, checked frames (None: all))
+# id: (arch, classes, net (w, h), options, batch, path, checked frames (None: all))
 ROWS = {
-    "full416-n1": ("full", 80, 416, {}, 1, "forward", None),     # 64-wide latency tiles; split-K on 13x13 (+ residual) and 26x26
-    "full416-n2": ("full", 80, 416, {}, 2, "forward", None),     # split-K into 3 parts
-    "full416-n3": ("full", 80, 416, {}, 3, "forward", None),     # bucket 4 with a stale frame
-    "full416-n8": ("full", 80, 416, {}, 8, "forward", [0, 1, 4, 7]),      # 128-wide latency tiles; 52x52 strips
-    "full416-n13": ("full", 80, 416, {}, 13, "forward", [0, 1, 7, 12]),   # bucket 16: the CTA pair in im2col form on 13x13 3x3
-    "full416-n20": ("full", 80, 416, {}, 20, "detect", [0, 7, 8, 16, 19]),  # bucket 32: copy-overlapped quarter front
-    "full416-n64": ("full", 80, 416, {}, 64, "forward", [0, 1, 32, 63]),  # the benchmarked configuration
-    "full416-strip-n2": ("full", 80, 416, {"strip": 2}, 2, "forward", None),  # strips at widths 27 / 14
-    "full608-n1": ("full", 80, 608, {}, 1, "forward", None),
-    "full608-n4": ("full", 80, 608, {}, 4, "forward", [0, 3]),   # 76x76 strips
-    "full608-n32": ("full", 80, 608, {}, 32, "forward", [0, 31]),  # a per-GPU shard of the 2-GPU 608 configuration
-    "rsu416-n64": ("rsu", 9, 416, {}, 64, "forward", [0, 63]),   # 42-channel heads in 44-wide rows
-    "tiny416-n1": ("tiny", 80, 416, {}, 1, "forward", None),     # conv0_ws and halo with fused pool, stand-alone maxpool
-    "tiny416-n5": ("tiny", 80, 416, {}, 5, "forward", [0, 4]),
+    "full416-n1": ("full", 80, (416, 416), {}, 1, "forward", None),     # 64-wide latency tiles; split-K on 13x13 (+ residual) and 26x26
+    "full416-n2": ("full", 80, (416, 416), {}, 2, "forward", None),     # split-K into 3 parts
+    "full416-n3": ("full", 80, (416, 416), {}, 3, "forward", None),     # bucket 4 with a stale frame
+    "full416-n8": ("full", 80, (416, 416), {}, 8, "forward", [0, 1, 4, 7]),      # 128-wide latency tiles; 52x52 strips
+    "full416-n13": ("full", 80, (416, 416), {}, 13, "forward", [0, 1, 7, 12]),   # bucket 16: the CTA pair in im2col form on 13x13 3x3
+    "full416-n20": ("full", 80, (416, 416), {}, 20, "detect", [0, 7, 8, 16, 19]),  # bucket 32: copy-overlapped quarter front
+    "full416-n64": ("full", 80, (416, 416), {}, 64, "forward", [0, 1, 32, 63]),  # the benchmarked configuration
+    "full416-strip-n2": ("full", 80, (416, 416), {"strip": 2}, 2, "forward", None),  # strips at widths 27 / 14
+    "full608-n1": ("full", 80, (608, 608), {}, 1, "forward", None),
+    "full608-n4": ("full", 80, (608, 608), {}, 4, "forward", [0, 3]),   # 76x76 strips
+    "full608-n32": ("full", 80, (608, 608), {}, 32, "forward", [0, 31]),  # a per-GPU shard of the 2-GPU 608 configuration
+    "rsu416-n64": ("rsu", 9, (416, 416), {}, 64, "forward", [0, 63]),   # 42-channel heads in 44-wide rows
+    "tiny416-n1": ("tiny", 80, (416, 416), {}, 1, "forward", None),     # conv0_ws and halo with fused pool, stand-alone maxpool
+    "tiny416-n5": ("tiny", 80, (416, 416), {}, 5, "forward", [0, 4]),
+    # Non-square and off-grid nets: on a square map a kernel that swaps height and width, takes a row pitch or a tile count
+    # from the wrong axis, or decomposes a pixel index in the wrong order still gives the right answer.
+    "full416x256-n1": ("full", 80, (416, 256), {}, 1, "forward", None),   # split-K on 13x8 and 26x16, latency tiles, stem/block on 208x128
+    "full256x416-n3": ("full", 80, (256, 416), {}, 3, "forward", [0, 2]),  # the same net transposed: an axis swap fails one of the two
+    "full640x384-n8": ("full", 80, (640, 384), {}, 8, "forward", [0, 7]),  # 80x48 maps in the strip form, 20x12 heads
+    "full416x256-n20": ("full", 80, (416, 256), {}, 20, "detect", [0, 8, 16, 19]),  # quarter-batch front and copy pieces, non-square
+    "rsu320x192-n64": ("rsu", 9, (320, 192), {}, 64, "forward", [0, 63]),  # the batch-64 plan on a 6x10 grid; 42-channel heads
+    "tiny416x256-n5": ("tiny", 80, (416, 256), {}, 5, "forward", [0, 4]),  # conv0_ws / halo with fused pool, stride-1 maxpool on 8x13
+    "full96x160-n2": ("full", 80, (96, 160), {}, 2, "forward", None),     # too small for the stem: conv0 on the full graph, heads 3 wide and 5 tall
 }
 SEED = {"full": 2, "rsu": 3, "tiny": 1}
 
@@ -57,13 +69,14 @@ def _release_models():
     _models.clear()
 
 
-def _model(arch, nc, size, opts):
-    """One Model per (graph, options); options apply to execution state built while they are set, so every use of a model
-    with options runs inside the same option block."""
-    key = (arch, nc, size, tuple(sorted(opts.items())))
+def _model(arch, nc, wh, opts):
+    """One Model per (graph, net, options); options apply to execution state built while they are set, so every use of a
+    model with options runs inside the same option block.  A non-square net runs the graph generated at 416 (the planner
+    builds every layer from the net's (w, h), whatever input shape the graph declares)."""
+    key = (arch, nc, wh, tuple(sorted(opts.items())))
     if key not in _models:
-        data = modelgen.build_onnx(arch, nc, size, SEED[arch])
-        _models[key] = (data, _native.Model(data, nc, (size, size), device=0))
+        data = modelgen.build_onnx(arch, nc, wh[0] if wh[0] == wh[1] else 416, SEED[arch])
+        _models[key] = (data, _native.Model(data, nc, wh, device=0))
     return _models[key]
 
 
@@ -111,16 +124,16 @@ def _front_layers(L, pooled, net_h):
 
 def _run_path(m, frames, path):
     """Runs the batch through `path`; returns the detection records of the "detect" path (None for "forward")."""
-    n, size = frames.shape[0], frames.shape[1]
+    n, wh = frames.shape[0], (frames.shape[2], frames.shape[1])
     if path == "forward":
-        m.preprocess(frames, n, (size, size))
+        m.preprocess(frames, n, wh)
         m.forward(n)
         return None
     # "detect": the synchronous call (frame copy in pieces overlapped with the first layers, quarter batch by quarter batch).
     # The bucket's buffers first hold a pass over OTHER frames, so a quarter, a piece of the copy or a partial last quarter
     # that the call leaves unwritten shows up as a wrong layer instead of as the right value left behind
-    other = frames_for(n, size, first_seed=900)
-    m.preprocess(other, n, (size, size))
+    other = frames_for(n, wh, first_seed=900)
+    m.preprocess(other, n, wh)
     m.forward(n)
     dets, counts = m.detect(frames, THR, max_det=512)
     return [dets[f, :counts[f]].copy() for f in range(n)]
@@ -189,16 +202,16 @@ def check_layers_exact(data, m, frames, picks, label, front=frozenset()):
 
 @pytest.mark.parametrize("row", list(ROWS))
 def test_layers_exact(row):
-    arch, nc, size, opts, n, path, picks = ROWS[row]
+    arch, nc, wh, opts, n, path, picks = ROWS[row]
     picks = list(range(n)) if picks is None else picks
-    frames = frames_for(n, size, first_seed=700)
+    frames = frames_for(n, wh, first_seed=700)
     with _options(opts):
-        data, m = _model(arch, nc, size, opts)
+        data, m = _model(arch, nc, wh, opts)
         records = _run_path(m, frames, path)
-        front = _front_layers(m.layers(), _pooled(data), size) if path == "detect" else frozenset()
+        front = _front_layers(m.layers(), _pooled(data), wh[1]) if path == "detect" else frozenset()
         check_layers_exact(data, m, frames, picks, row, front)
         if records is not None:  # the staged path on the same frames returns the very same records
-            m.preprocess(frames, n, (size, size))
+            m.preprocess(frames, n, wh)
             m.forward(n)
             staged = _records(m, n)
             for f in range(n):
@@ -208,15 +221,12 @@ def test_layers_exact(row):
 REQUIRED_FORMS = {"fused_next", "stem", "block", "halo", "halo+pool", "conv0+pool", "maxpool", "tc_pair", "tc_pair_strip", "tc_swapped"}
 
 
-def test_matrix_covers_every_kernel_form():
-    """The rows of ROWS together run every kernel form: the fused stem and block, halo with and without a fused pool, conv0
-    (YOLOv3-tiny's, with its fused pool; YOLOv3's first layer runs inside the stem), the stand-alone maxpool, conv_tc
-    single-CTA with block_n 64 and 128, the CTA pair in im2col and strip form, the swapped form, and split-K on a layer with a
-    residual and on one without."""
+def _forms(rows):
+    """Kernel forms the rows run: (forms, block_n of the single-CTA launches, whether each split-K layer has a residual)."""
     seen, single_bn, split = set(), set(), set()
-    for row, (arch, nc, size, opts, n, path, picks) in ROWS.items():
+    for row, (arch, nc, wh, opts, n, path, picks) in rows.items():
         with _options(opts):
-            data, m = _model(arch, nc, size, opts)
+            data, m = _model(arch, nc, wh, opts)
             L, pooled = m.layers(), _pooled(data)
             for i, e in enumerate(m.exec_info(n)):
                 name = e["kernel_name"]
@@ -225,6 +235,24 @@ def test_matrix_covers_every_kernel_form():
                     single_bn.add(e["block_n"])
                 if e["split_k"] > 1:
                     split.add(bool(L[i]["has_residual"]))
+    return seen, single_bn, split
+
+
+def test_matrix_covers_every_kernel_form():
+    """The rows of ROWS together run every kernel form: the fused stem and block, halo with and without a fused pool, conv0
+    (YOLOv3-tiny's, with its fused pool; YOLOv3's first layer runs inside the stem), the stand-alone maxpool, conv_tc
+    single-CTA with block_n 64 and 128, the CTA pair in im2col and strip form, the swapped form, and split-K on a layer with a
+    residual and on one without."""
+    seen, single_bn, split = _forms(ROWS)
+    assert REQUIRED_FORMS <= seen, sorted(REQUIRED_FORMS - seen)
+    assert {64, 128} <= single_bn, single_bn
+    assert split == {True, False}, split
+
+
+def test_nonsquare_rows_cover_every_kernel_form():
+    """The rows whose net has w != h on their own run every kernel form, so each form meets a map where a swapped height
+    and width would show."""
+    seen, single_bn, split = _forms({k: r for k, r in ROWS.items() if r[2][0] != r[2][1]})
     assert REQUIRED_FORMS <= seen, sorted(REQUIRED_FORMS - seen)
     assert {64, 128} <= single_bn, single_bn
     assert split == {True, False}, split

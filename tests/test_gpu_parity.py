@@ -7,6 +7,7 @@ Tolerances (BASELINE.json north_star): raw head tensors  max|gpu-ref| <= 2e-2 * 
 Integer / byte work (normalisation LUT, letterbox, box indices, classes, ordering) is bit-exact; the float64
 decode / Soft-NMS arithmetic is compared at 1e-12 relative (device exp() may differ from glibc in the last bit).
 """
+import contextlib
 import glob
 import io
 import os
@@ -40,20 +41,30 @@ def _golden_heads(z):
 _models = {}
 
 
+def net_wh(size):
+    """A network size given as an int (square) or as (w, h)."""
+    return (size, size) if isinstance(size, int) else tuple(size)
+
+
 def get_model(arch, nc, size, seed, opts_key=None):
+    """size: int or (w, h).  A non-square net runs the graph generated at 416: the graph's weights do not depend on the
+    size it declares, and the planner builds every layer from the net's own (w, h)."""
     key = (arch, nc, size, seed, opts_key)
     if key not in _models:
         opts = None
         if opts_key == "alt":
             opts = modelgen.ExportOptions(fold_bn=False, upsample_op="Upsample", pool_pad="pad_node",
                                           const_as="constant_node", raw_data=False, packed_attrs=False, batch=1)
-        data = modelgen.build_onnx(arch, nc, size, seed, opts)
-        _models[key] = (data, _native.Model(data, nc, (size, size), device=0))
+        w, h = net_wh(size)
+        data = modelgen.build_onnx(arch, nc, w if w == h else 416, seed, opts)
+        _models[key] = (data, _native.Model(data, nc, (w, h), device=0))
     return _models[key]
 
 
 def frames_for(n, size, first_seed=100):
-    return np.stack([modelgen.synthetic_frame(first_seed + i, size) for i in range(n)])
+    """n synthetic frames [n, h, w, 3]; a non-square size crops the square frame of its longer side."""
+    w, h = net_wh(size)
+    return np.stack([modelgen.synthetic_frame(first_seed + i, max(w, h))[:h, :w] for i in range(n)])
 
 
 def iou(a, b):
@@ -87,24 +98,38 @@ def test_normalise_bit_exact(golden_dir):
     assert np.array_equal(got[0, :, ::52, ::52], z["input_probe"])
 
 
-@pytest.mark.parametrize("shape", [(480, 640), (640, 480), (416, 416), (97, 1031), (1080, 1920)])
-def test_letterbox_bit_exact(shape):
-    _, m = get_model("tiny", 80, 416, 1)
+@pytest.mark.parametrize("net", [416, (416, 256), (256, 416)])
+@pytest.mark.parametrize("shape", [(480, 640), (640, 480), (416, 416), (97, 1031), (1080, 1920), (37, 100), (500, 13), (7, 6)])
+def test_letterbox_bit_exact(shape, net):
+    """shape: the source's (h, w).  Down-scales, the identity, up-scales (37x100, 7x6) and a picture a few pixels wide
+    (500x13), into nets where the width or the height limits the scale."""
+    _, m = get_model("tiny", 80, net, 1)
     rng = np.random.default_rng(shape[0])
     src = rng.integers(0, 256, size=(2,) + shape + (3,), dtype=np.uint8)
     got = m.letterbox(src)
     for i in range(2):
-        want, _ = ref_post.letterbox_u8(src[i], 416, 416)
+        want, _ = ref_post.letterbox_u8(src[i], m.net_w, m.net_h)
         assert np.array_equal(got[i], want)
 
 
 # ------------------------------------------------------------------ postprocess on exact inputs
-def _check_post(m, heads, nc, thr, size=416):
+def _nms(mode):
+    """Soft-NMS path: "auto" keeps frames of at most 512 candidates in registers and runs larger ones on the general loop;
+    "general" runs every frame on the general loop."""
+    return _native.option("nms_general", 1) if mode == "general" else contextlib.nullcontext()
+
+
+def _check_post(m, heads, nc, thr):
+    """Post-processing of `heads` on the model's net (net_w, net_h) against the oracle: the same boxes in Soft-NMS order,
+    values at 1e-12.  Returns (dets, counts, candidates per frame in the oracle)."""
     n = m.set_heads(heads)
     m.postprocess(n, thr, max_det=m.info.boxes_per_frame)
     dets, counts, total = m.fetch(n)
+    cands = []
     for f in range(n):
-        want, want_idx, _ = ref_post.detect_from_heads(heads, f, nc, (size, size), thr)
+        left = {}
+        want, want_idx, _ = ref_post.detect_from_heads(heads, f, nc, (m.net_w, m.net_h), thr, leftovers=left)
+        cands.append(len(want_idx) + len(left))
         assert counts[f] == total[f] == len(want)
         d = dets[f, :counts[f]]
         assert [int(k) for k in d["klass"]] == [r[0] for r in want]      # classes, in Soft-NMS order
@@ -113,7 +138,7 @@ def _check_post(m, heads, nc, thr, size=416):
             got = np.stack([d["conf"], d["x"], d["y"], d["w"], d["h"]], axis=1)
             ref = np.array([r[1:] for r in want], np.float64)
             np.testing.assert_allclose(got, ref, rtol=1e-12, atol=1e-12)
-    return dets, counts
+    return dets, counts, cands
 
 
 @pytest.mark.parametrize("path", POST, ids=[os.path.basename(p)[:-4] for p in POST])
@@ -126,7 +151,7 @@ def test_post_matches_reference_golden(path):
     if key in shapes:
         arch, nc_, size = shapes[key]
         _, m = get_model(arch, nc_, size, {"tiny": 1, "rsu": 3}[arch])
-        dets, counts = _check_post(m, heads, nc, thr)
+        dets, counts, _ = _check_post(m, heads, nc, thr)
         ref = z["results"]
         assert counts[0] == len(ref)  # and against the reference module's own output
         if len(ref):
@@ -143,40 +168,128 @@ def test_post_matches_reference_golden(path):
         # the fixture's reference output assumes the reference's hard-wired 416x416 image_size, which no real net
         # has together with this grid; the head tensors are still a good input, checked against the oracle
         # (itself pinned to the reference on the 416 fixtures) evaluated at this net's size
-        _check_post(m, heads, nc, thr, size=size)
+        _check_post(m, heads, nc, thr)
         m.close()
 
 
 def test_post_dense_random_batch():
-    """Thousands of candidates per frame, several frames: exercises compaction order-independence and ties."""
-    _, m = get_model("rsu", 9, 416, 3)
-    rng = np.random.default_rng(5)
-    n = 3
-    heads = []
-    for (c, h, w) in m.head_shapes:
-        a = rng.normal(0.0, 1.5, size=(n, c, h, w)).astype(np.float32)
-        a[:, 4::14] -= 2.0
-        a[:, 2::14] *= 0.3
-        a[:, 3::14] *= 0.3
-        heads.append(np.round(a * 8) / 8)  # coarse grid of values -> many exact ties in the scores
-    heads = [h.astype(np.float32) for h in heads]
-    dets, counts = _check_post(m, heads, 9, 0.25)
+    """Hundreds to thousands of candidates per frame, several frames: exercises compaction order-independence and ties.
+    The non-square heads (8x13 / 16x26 / 32x52 and 6x10 / 12x20) tell a decode or a result scaling that swaps the axes
+    from a correct one.  Every case runs on both Soft-NMS paths."""
+    for arch, nc, size, seed, n in [("rsu", 9, 416, 3, 3), ("full", 80, (416, 256), 2, 2), ("tiny", 80, (320, 192), 1, 3)]:
+        _, m = get_model(arch, nc, size, seed)
+        rng = np.random.default_rng(5)
+        span = 5 + nc
+        heads = []
+        for (c, h, w) in m.head_shapes:
+            a = rng.normal(0.0, 1.5, size=(n, c, h, w)).astype(np.float32)
+            a[:, 4::span] -= 2.0
+            a[:, 2::span] *= 0.3
+            a[:, 3::span] *= 0.3
+            heads.append(np.round(a * 8) / 8)  # coarse grid of values -> many exact ties in the scores
+        heads = [h.astype(np.float32) for h in heads]
+        for nms in ("auto", "general"):
+            with _nms(nms):
+                dets, counts, _ = _check_post(m, heads, nc, 0.25)
+            assert counts.min() > 50, (arch, size, nms, counts)
+
+
+def _built_heads(m, n, seed, picks):
+    """Random heads [n, C, H, W] per head whose only possible candidates are the boxes of picks[f] (indices in insertion
+    order): every other box's objectness logit is -20.  Returns the heads and, per frame, each picked box's
+    (head, anchor, row, column)."""
+    rng = np.random.default_rng(seed)
+    span = (m.head_shapes[0][0]) // 3
+    heads = [rng.normal(0.0, 1.5, size=(n,) + s).astype(np.float32) for s in m.head_shapes]
+    for a in heads:
+        a[:, 4::span] = -20.0
+    where = []
+    for f in range(n):
+        at = []
+        for box in picks[f]:
+            for hi, (c, h, w) in enumerate(m.head_shapes):
+                if box < 3 * h * w:
+                    cell, k = divmod(int(box), 3)
+                    at.append((hi, k, cell // w, cell % w))
+                    break
+                box -= 3 * h * w
+        where.append(at)
+    return heads, where, span
+
+
+@pytest.mark.parametrize("nms", ["auto", "general"])
+def test_post_at_the_register_path_limit(nms):
+    """Frames with exactly 512 and 513 candidates on a 416x256 net: one on each side of the switch from the register path
+    (one candidate per thread of the 512-thread block) to the general loop; with nms="general" both take the loop."""
+    _, m = get_model("full", 80, (416, 256), 2)
+    nb = m.info.boxes_per_frame
+    rng = np.random.default_rng(11)
+    picks = [rng.choice(nb, 512, replace=False), rng.choice(nb, 513, replace=False)]
+    heads, where, span = _built_heads(m, 2, 12, picks)
+    for f, at in enumerate(where):
+        for hi, k, y, x in at:
+            heads[hi][f, k * span + 4, y, x] = rng.uniform(1.0, 3.0)   # objectness 0.73 .. 0.95
+            heads[hi][f, k * span + 5 + rng.integers(0, 80), y, x] = 4.0  # best class 0.98: every picked box clears 0.25
+    with _nms(nms):
+        _, counts, cands = _check_post(m, heads, 80, 0.25)
+    assert cands == [512, 513], cands
     assert counts.min() > 50
+
+
+@pytest.mark.parametrize("nms", ["auto", "general"])
+def test_post_threshold_zero_keeps_every_box(nms):
+    """Threshold 0: the objectness pre-test is off (cut -inf), every box of the 320x192 tiny net is a candidate (900: the
+    general loop on both paths) and Soft-NMS, which stops only below the threshold, selects all of them."""
+    _, m = get_model("tiny", 80, (320, 192), 1)
+    rng = np.random.default_rng(13)
+    heads = [rng.normal(0.0, 1.5, size=(2,) + s).astype(np.float32) for s in m.head_shapes]
+    with _nms(nms):
+        _, counts, cands = _check_post(m, heads, 80, 0.0)
+    assert m.info.boxes_per_frame == 900 and cands == [900, 900] and counts.tolist() == [900, 900]
+
+
+@pytest.mark.parametrize("nms", ["auto", "general"])
+def test_post_threshold_one_keeps_certain_boxes(nms):
+    """Threshold 1.0: only boxes whose float64 conf is exactly 1.0 survive.  Objectness and class logits >= 40 give
+    logistic() == 1.0 exactly (exp(-40) is below half an ulp of 1); decoys with one of the two at 30 (1 - 9e-14) do not.
+    The kept boxes are a few hundredths of a pixel wide in distinct cells, so none decays another, and with every score
+    at 1.0 they come out in insertion order."""
+    _, m = get_model("tiny", 80, (320, 192), 1)
+    nb = m.info.boxes_per_frame
+    rng = np.random.default_rng(17)
+    cells = [rng.choice(nb // 3, 10, replace=False) for _ in range(2)]
+    picks = [3 * c + rng.integers(0, 3, size=c.size) for c in cells]
+    heads, where, span = _built_heads(m, 2, 18, picks)
+    logits = [(40.0, 40.0)] * 3 + [(45.0, 52.0)] * 3 + [(30.0, 45.0), (45.0, 30.0)] * 2  # (objectness, best class): 6 sure, 4 decoys
+    for f, at in enumerate(where):
+        for (hi, k, y, x), (obj, cls) in zip(at, logits):
+            heads[hi][f, k * span + 2:k * span + 4, y, x] = -8.0
+            heads[hi][f, k * span + 4, y, x] = obj
+            heads[hi][f, k * span + 5 + rng.integers(0, 80), y, x] = cls
+    with _nms(nms):
+        dets, counts, cands = _check_post(m, heads, 80, 1.0)
+    assert counts.tolist() == [6, 6]
+    for f in range(2):
+        assert [int(b) for b in dets[f, :6]["box"]] == sorted(int(b) for b in picks[f][:6])
+        assert (dets[f, :6]["conf"] == 1.0).all()
 
 
 def test_post_truncation_and_empty():
     _, m = get_model("tiny", 80, 416, 1)
     z = np.load(os.path.join(HERE, "golden", "post_tiny80.npz"))
     heads = _golden_heads(z)
-    m.set_heads(heads)
-    m.postprocess(1, 0.1, max_det=5)
-    dets, counts, total = m.fetch(1)
-    assert counts[0] == 5 and total[0] == len(z["results"])
-    np.testing.assert_allclose(dets[0, :5]["conf"], z["results"][:5, 1], rtol=1e-12)
-    m.set_heads([np.full_like(h, -20.0) for h in heads])
-    m.postprocess(1, 0.1, max_det=16)
-    _, counts, total = m.fetch(1)
-    assert counts[0] == 0 and total[0] == 0
+    for nms in ("auto", "general"):
+        m.set_heads(heads)
+        with _nms(nms):
+            m.postprocess(1, 0.1, max_det=5)
+        dets, counts, total = m.fetch(1)
+        assert counts[0] == 5 and total[0] == len(z["results"]), nms
+        np.testing.assert_allclose(dets[0, :5]["conf"], z["results"][:5, 1], rtol=1e-12)
+        m.set_heads([np.full_like(h, -20.0) for h in heads])
+        with _nms(nms):
+            m.postprocess(1, 0.1, max_det=16)
+        _, counts, total = m.fetch(1)
+        assert counts[0] == 0 and total[0] == 0, nms
 
 
 # ------------------------------------------------------------------ conv stack vs the fp32 oracle

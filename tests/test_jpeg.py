@@ -273,11 +273,11 @@ def test_service_routes_jpeg_bytes_to_the_library_and_other_formats_to_pil(fake)
 _model = {}
 
 
-def gpu_model():
-    if 'm' not in _model:
+def gpu_model(wh=(416, 416)):
+    if wh not in _model:
         data = modelgen.build_onnx('tiny', 80, 416, 1)
-        _model['m'] = (data, _native.Model(data, 80, (416, 416), device=0))
-    return _model['m']
+        _model[wh] = (data, _native.Model(data, 80, wh, device=0))
+    return _model[wh]
 
 
 @pytest.mark.gpu
@@ -301,6 +301,13 @@ def test_device_decode_bit_exact_against_pillow():
         for sub in (0, 2):
             d = encode(a, quality=90, subsampling=sub)
             assert np.array_equal(m.decode_jpeg([d])[0], ref_jpeg.decode_reference(d))
+    # a 416x256 net decoding 416x256 JPEGs (no letterbox): the chroma rows, the MCU grid (26x16 4:2:0 MCUs) and the output
+    # rows follow the frame's own width and height
+    _, m = gpu_model((416, 256))
+    datas = [encode(modelgen.synthetic_frame(230 + sub, 416)[:256], quality=80, subsampling=sub) for sub in (0, 1, 2)]
+    got = m.decode_jpeg(datas)
+    for i, d in enumerate(datas):
+        assert np.array_equal(got[i], ref_jpeg.decode_reference(d)), i
 
 
 @pytest.mark.gpu
@@ -345,7 +352,9 @@ def test_jpeg_of_another_size_is_letterboxed_like_decoded_frames():
     from fastdet_b200 import detector as fdet
     onnx, m = gpu_model()
     rng = np.random.default_rng(9)
-    for (h, w, sub) in [(480, 640, 2), (360, 202, 1), (833, 417, 0)]:
+    # odd sizes with subsampled chroma: the last pixel pair of a row has no second pixel, the last chroma column takes the
+    # edge rule, and the bottom 4:2:0 output row's context row lies past the picture; 7x6 has 3 chroma columns
+    for (h, w, sub) in [(480, 640, 2), (360, 202, 1), (481, 641, 2), (417, 833, 2), (361, 203, 1), (7, 6, 2), (833, 417, 0)]:
         frames = [np.clip(np.kron(rng.integers(0, 255, (h // 8 + 1, w // 8 + 1, 3)), np.ones((8, 8, 1)))[:h, :w] +
                           rng.normal(0, 6, (h, w, 3)), 0, 255).astype(np.uint8) for _ in range(3)]
         datas = [encode(f, quality=85, subsampling=sub) for f in frames]

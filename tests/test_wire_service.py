@@ -174,18 +174,19 @@ def test_letterbox_geometry_and_unmapping():
     the caller's pixels.  Restated here: scale = min(net/src) with the long side filling the network, centred."""
     import numpy as np
     from fastdet_b200 import _native
-    for (sw, sh) in [(640, 480), (480, 640), (416, 416), (1920, 1080), (97, 1031), (1, 1), (832, 416)]:
-        nw, nh, ox, oy = _native.letterbox_geometry((sw, sh), (416, 416))
-        if sw * 416 >= sh * 416:
-            want = (416, max(1, (sh * 416 + sw // 2) // sw))
-        else:
-            want = (max(1, (sw * 416 + sh // 2) // sh), 416)
-        assert (nw, nh) == want and (ox, oy) == ((416 - nw) // 2, (416 - nh) // 2)
-        d = np.zeros(3, _native.DET_DTYPE)
-        d['x'], d['y'], d['w'], d['h'] = [ox, ox + nw / 2, 10.0], [oy, oy + nh / 2, 20.0], [nw, 5.0, 1.0], [nh, 7.0, 2.0]
-        d['klass'], d['conf'] = [1, 2, 3], [0.9, 0.8, 0.7]
-        u = _native.unmap_letterbox(d, (sw, sh), (416, 416))
-        assert np.allclose(u['x'], (d['x'] - ox) * sw / nw, rtol=0, atol=1e-9) and np.allclose(u['w'], d['w'] * sw / nw, rtol=0, atol=1e-9)
-        assert np.allclose(u['y'], (d['y'] - oy) * sh / nh, rtol=0, atol=1e-9) and np.allclose(u['h'], d['h'] * sh / nh, rtol=0, atol=1e-9)
-        assert u['x'][0] == 0 and u['y'][0] == 0 and abs(u['w'][0] - sw) < 1e-9 and abs(u['h'][0] - sh) < 1e-9  # the whole picture
-        assert np.array_equal(u['klass'], d['klass']) and np.array_equal(u['conf'], d['conf'])
+    for (NW, NH) in [(416, 416), (416, 256), (256, 416)]:  # on the non-square nets either side can limit a source
+        for (sw, sh) in [(640, 480), (480, 640), (416, 416), (1920, 1080), (97, 1031), (1, 1), (832, 416), (416, 256), (13, 500)]:
+            nw, nh, ox, oy = _native.letterbox_geometry((sw, sh), (NW, NH))
+            if sw * NH >= sh * NW:
+                want = (NW, max(1, (sh * NW + sw // 2) // sw))
+            else:
+                want = (max(1, (sw * NH + sh // 2) // sh), NH)
+            assert (nw, nh) == want and (ox, oy) == ((NW - nw) // 2, (NH - nh) // 2), ((sw, sh), (NW, NH))
+            d = np.zeros(3, _native.DET_DTYPE)
+            d['x'], d['y'], d['w'], d['h'] = [ox, ox + nw / 2, 10.0], [oy, oy + nh / 2, 20.0], [nw, 5.0, 1.0], [nh, 7.0, 2.0]
+            d['klass'], d['conf'] = [1, 2, 3], [0.9, 0.8, 0.7]
+            u = _native.unmap_letterbox(d, (sw, sh), (NW, NH))
+            assert np.allclose(u['x'], (d['x'] - ox) * sw / nw, rtol=0, atol=1e-9) and np.allclose(u['w'], d['w'] * sw / nw, rtol=0, atol=1e-9)
+            assert np.allclose(u['y'], (d['y'] - oy) * sh / nh, rtol=0, atol=1e-9) and np.allclose(u['h'], d['h'] * sh / nh, rtol=0, atol=1e-9)
+            assert u['x'][0] == 0 and u['y'][0] == 0 and abs(u['w'][0] - sw) < 1e-9 and abs(u['h'][0] - sh) < 1e-9  # the whole picture
+            assert np.array_equal(u['klass'], d['klass']) and np.array_equal(u['conf'], d['conf'])
