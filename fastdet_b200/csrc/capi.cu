@@ -146,7 +146,6 @@ struct fd_model {
     fd_info info;
     int last_n = 0;
     int last_max_det = 0;
-    bool use_graph = true;
 };
 
 namespace {
@@ -193,7 +192,6 @@ void* loc_ptr(const Exec& e, const ModelPlan& P, const TensorLoc& t, bool fp32, 
 // and tens of GB.  n <= 64 rounds up to a power of two, larger batches to a multiple of 64; the conv stack runs on the
 // bucket's frame count (frames past n hold stale pixels and are never decoded or copied out), everything else on n.
 int bucket_of(int n) {
-    if (options().exact_batch) return n;  // option exact_batch: one Exec per exact size
     if (n > 64) return (n + 63) / 64 * 64;
     int b = 1;
     while (b < n) b *= 2;
@@ -531,7 +529,7 @@ int fd_model_create(const void* onnx_bytes, size_t len, int num_classes, int net
     struct Cleanup { void operator()(fd_model* p) const { fd_model_destroy(p); } };  // frees whatever a failed create had already allocated
     std::unique_ptr<fd_model, Cleanup> m(new fd_model());
     m->device = -1;  // until a device is attached: destroy then only frees host state
-    if (!build_plan(g, net_w, net_h, num_classes, options().fuse_pool && options().halo, &m->plan, &err)) return fail(FD_ERR_MODEL, "unsupported ONNX graph: %s", err.c_str());
+    if (!build_plan(g, net_w, net_h, num_classes, options().fuse_pool, &m->plan, &err)) return fail(FD_ERR_MODEL, "unsupported ONNX graph: %s", err.c_str());
     ModelPlan& P = m->plan;
     if (P.head_layers.size() > FD_MAX_HEADS) return fail(FD_ERR_MODEL, "graph has %zu outputs (max %d)", P.head_layers.size(), FD_MAX_HEADS);
 
@@ -591,7 +589,6 @@ int fd_model_create(const void* onnx_bytes, size_t len, int num_classes, int net
     CU(cudaMemcpy(m->d_conv0, P.conv0_w.data(), P.conv0_w.size() * 4, cudaMemcpyHostToDevice));
     // host copies are no longer needed
     std::vector<uint16_t>().swap(P.weights_bf16);
-    m->use_graph = options().graph != 0;
     *out = m.release();
     return FD_OK;
 }
@@ -789,7 +786,7 @@ int fd_forward(fd_model* m, int n, void* stream) {
     if (int rc = get_exec(m, n, &e)) return rc;
     cudaStream_t s = pick(m, stream);
     m->last_n = n;
-    if (m->use_graph && !e->graph_tried) {
+    if (!e->graph_tried) {
         e->graph_tried = true;
         e->graph = capture_layers(m, e, 0);
     }
@@ -961,7 +958,7 @@ static int forward_overlapping_copy(fd_model* m, Exec* e, const uint8_t* frames,
         for (int i = 0; i < e->ov_layers; ++i)
             if (int rc = launch_piece(m, e, e->front, i, k, s)) return rc;
     }
-    if (m->use_graph && !e->graph_tail_tried) {
+    if (!e->graph_tail_tried) {
         e->graph_tail_tried = true;
         e->graph_tail = capture_layers(m, e, e->ov_layers);
     }
@@ -975,7 +972,7 @@ static int forward_overlapping_copy(fd_model* m, Exec* e, const uint8_t* frames,
 
 int fd_detect(fd_model* m, const uint8_t* frames, int n, int src_w, int src_h, int on_device, int allow_resize,
               double threshold, int max_det, fd_det* out, int32_t* counts) {
-    if (m && frames && m->device >= 0 && !on_device && src_w == m->plan.net_w && src_h == m->plan.net_h && options().detect_overlap) {
+    if (m && frames && m->device >= 0 && !on_device && src_w == m->plan.net_w && src_h == m->plan.net_h) {
         CU(cudaSetDevice(m->device));
         Exec* e;
         if (int rc = get_exec(m, n, &e)) return rc;

@@ -25,7 +25,6 @@
 #include <string.h>
 
 #include "conv_tc.h"
-#include "options.h"
 #include "ptx.cuh"
 
 namespace fd {
@@ -374,7 +373,6 @@ conv_block_kernel(const __grid_constant__ CUtensorMap tm_out, const __grid_const
 }  // namespace
 
 bool conv_block_supported(const BlockDesc& d) {
-    if (!options().block) return false;
     if (d.cin != CIN || d.cmid != CMID || d.cout != COUT) return false;
     if (d.act_a && !(d.alpha_a >= 0.f && d.alpha_a <= 1.f)) return false;
     if (d.act_b && !(d.alpha_b >= 0.f && d.alpha_b <= 1.f)) return false;
@@ -427,7 +425,7 @@ int conv_block_launch(const BlockLaunch& L, cudaStream_t stream) {
     attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
     attr[0].val.programmaticStreamSerializationAllowed = 1;
     cfg.attrs = attr;
-    cfg.numAttrs = options().pdl ? 1 : 0;
+    cfg.numAttrs = 1;
     return cudaLaunchKernelEx(&cfg, conv_block_kernel, L.tm_out, L.p) == cudaSuccess ? 0 : -1;
 }
 

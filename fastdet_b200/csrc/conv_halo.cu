@@ -27,7 +27,6 @@
 #include <string.h>
 
 #include "conv_tc.h"
-#include "options.h"
 #include "ptx.cuh"
 
 namespace fd {
@@ -91,17 +90,16 @@ __global__ void __launch_bounds__(THREADS, 1)
 conv_halo_kernel(const __grid_constant__ CUtensorMap tm_out, const __grid_constant__ HaloParams p) {
     using G = Geo<STRIDE>;
     constexpr int NCH = CIN / 8;                    // 16-byte channel chunks per pixel
-    const int PLANE_BYTES = p.plane_bytes;          // Plane<CIN, STRIDE>::BYTES, or the unskewed stride (option halo_skew)
-    const int PATCH_BYTES = NCH * PLANE_BYTES;
+    constexpr int PLANE_BYTES = Plane<CIN, STRIDE>::BYTES;
+    constexpr int PATCH_BYTES = NCH * PLANE_BYTES;
     constexpr int KSTEPS = CIN / 16;                // MMAs per filter tap
-    const int SLOTS = p.slots;                      // patch ring depth (<= Ring<CIN, STRIDE>::SLOTS)
+    constexpr int SLOTS = Ring<CIN, STRIDE>::SLOTS;
     extern __shared__ uint8_t smem_raw[];
     uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
     // [0, 1024) barriers | staging 8 warps x 4 KB | weights 9*NCH*cout*16 | patch ring SLOTS x PATCH_BYTES
-    constexpr int MAX_SLOTS = Ring<CIN, STRIDE>::SLOTS;
     uint64_t* patch_full = reinterpret_cast<uint64_t*>(smem);
-    uint64_t* patch_empty = patch_full + MAX_SLOTS;
-    uint64_t* acc_full = patch_empty + MAX_SLOTS;
+    uint64_t* patch_empty = patch_full + SLOTS;
+    uint64_t* acc_full = patch_empty + SLOTS;
     uint64_t* acc_empty = acc_full + ACCS;
     uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(acc_empty + ACCS);
     uint8_t* s_stage = smem + 1024;
@@ -181,7 +179,7 @@ conv_halo_kernel(const __grid_constant__ CUtensorMap tm_out, const __grid_consta
         const bool issuer = ptx::elect_one();
         for (int it = 0; it < my_tiles; ++it) {
             const uint32_t slot = it % SLOTS, phase = (it / SLOTS) & 1, as = it & 3, aphase = (it >> 2) & 1;
-            ptx::mbar_wait_addr(bar0 + 8u * (2 * MAX_SLOTS + ACCS + as), aphase ^ 1);  // acc_empty
+            ptx::mbar_wait_addr(bar0 + 8u * (2 * SLOTS + ACCS + as), aphase ^ 1);  // acc_empty
             ptx::mbar_wait_addr(bar0 + 8u * slot, phase);                          // patch_full
             ptx::fence_proxy_async();  // the builders' cp.async writes (generic proxy), acquired through the barrier -> tensor core
             ptx::tc_fence_after();
@@ -198,8 +196,8 @@ conv_halo_kernel(const __grid_constant__ CUtensorMap tm_out, const __grid_consta
                         ptx::umma_bf16(d, ad + start + j * (2 * PLANE_BYTES / 16), b0 + (t * KSTEPS + j) * b_step, idesc,
                                        (t | j) ? 1u : 0u);
                 }
-                ptx::umma_commit_addr(bar0 + 8u * (MAX_SLOTS + slot));    // patch_empty
-                ptx::umma_commit_addr(bar0 + 8u * (2 * MAX_SLOTS + as));  // acc_full
+                ptx::umma_commit_addr(bar0 + 8u * (SLOTS + slot));    // patch_empty
+                ptx::umma_commit_addr(bar0 + 8u * (2 * SLOTS + as));  // acc_full
             }
             __syncwarp();
         }
@@ -343,18 +341,14 @@ conv_halo_kernel(const __grid_constant__ CUtensorMap tm_out, const __grid_consta
 }
 
 template <int CIN, int STRIDE>
-size_t smem_bytes(int cout, int* plane_bytes, int* slots) {
-    const Options& O = options();
-    *plane_bytes = O.halo_skew ? Plane<CIN, STRIDE>::BYTES : Geo<STRIDE>::PLANE_BASE;
-    *slots = Ring<CIN, STRIDE>::SLOTS;
-    if (O.halo_slots > 0 && O.halo_slots < *slots) *slots = O.halo_slots;
-    return 1024 + 1024 + EPI_WARPS * 4096 + ((9 * (CIN / 8) * cout * 16 + 1023) & ~1023) + static_cast<size_t>(*slots) * (CIN / 8) * *plane_bytes;
+size_t smem_bytes(int cout) {
+    return 1024 + 1024 + EPI_WARPS * 4096 + ((9 * (CIN / 8) * cout * 16 + 1023) & ~1023) +
+           static_cast<size_t>(Ring<CIN, STRIDE>::SLOTS) * (CIN / 8) * Plane<CIN, STRIDE>::BYTES;
 }
 
 }  // namespace
 
 bool conv_halo_supported(const HaloDesc& d) {
-    if (!options().halo) return false;
     if (!(d.cin == 64 || d.cin == 32 || d.cin == 16) || d.ksize != 3 || d.pad_lo != 1 || d.pad_hi > 1 || !(d.stride == 1 || d.stride == 2)) return false;
     if (!(d.cout == 32 || d.cout == 64 || d.cout == 128) || d.out_fp32 || d.upsample2x) return false;
     if (d.pool2 && (d.stride != 1 || d.residual || d.hi % 2 || d.wi % 2 || d.pad_hi != 1)) return false;
@@ -401,9 +395,9 @@ int conv_halo_prepare(const HaloDesc& d, int num_sms, HaloLaunch* L, char* err, 
     if (encode_tiled_bf16(&L->tm_out, d.out, 4, dims, strides, box, 2)) { if (err && errlen) snprintf(err, errlen, "conv_halo: output tensor map encode failed"); return -1; }
     L->stride = d.stride;
     L->cin = d.cin;
-    L->smem_bytes = d.cin == 64 ? smem_bytes<64, 1>(d.cout, &p.plane_bytes, &p.slots)
-                    : d.cin == 32 ? (d.stride == 1 ? smem_bytes<32, 1>(d.cout, &p.plane_bytes, &p.slots) : smem_bytes<32, 2>(d.cout, &p.plane_bytes, &p.slots))
-                                  : (d.stride == 1 ? smem_bytes<16, 1>(d.cout, &p.plane_bytes, &p.slots) : smem_bytes<16, 2>(d.cout, &p.plane_bytes, &p.slots));
+    L->smem_bytes = d.cin == 64 ? smem_bytes<64, 1>(d.cout)
+                    : d.cin == 32 ? (d.stride == 1 ? smem_bytes<32, 1>(d.cout) : smem_bytes<32, 2>(d.cout))
+                                  : (d.stride == 1 ? smem_bytes<16, 1>(d.cout) : smem_bytes<16, 2>(d.cout));
     if (L->smem_bytes > static_cast<size_t>(SMEM_LIMIT)) { if (err && errlen) snprintf(err, errlen, "conv_halo: %zu bytes of shared memory", L->smem_bytes); return -1; }
     L->grid = p.total < num_sms ? p.total : num_sms;
     L->flops = 2.0 * d.n * p.ho * p.wo * d.cout * 9.0 * d.cin;
@@ -423,7 +417,6 @@ int conv_halo_init() {
 }
 
 int conv_halo_launch(const HaloLaunch& L, cudaStream_t stream) {
-    const bool no_pdl = !options().pdl;
     cudaLaunchConfig_t cfg = {};
     cfg.gridDim = dim3(L.grid);
     cfg.blockDim = dim3(THREADS);
@@ -433,7 +426,7 @@ int conv_halo_launch(const HaloLaunch& L, cudaStream_t stream) {
     attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
     attr[0].val.programmaticStreamSerializationAllowed = 1;
     cfg.attrs = attr;
-    cfg.numAttrs = no_pdl ? 0 : 1;
+    cfg.numAttrs = 1;
     cudaError_t e;
     if (L.cin == 64) e = cudaLaunchKernelEx(&cfg, conv_halo_kernel<64, 1>, L.tm_out, L.p);
     else if (L.cin == 32) e = L.stride == 1 ? cudaLaunchKernelEx(&cfg, conv_halo_kernel<32, 1>, L.tm_out, L.p) : cudaLaunchKernelEx(&cfg, conv_halo_kernel<32, 2>, L.tm_out, L.p);

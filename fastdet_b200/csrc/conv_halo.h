@@ -34,7 +34,6 @@ struct HaloParams {
     long long res_pitch;
     int tiles_x, tiles_y, per_frame, total;
     int pool2;
-    int plane_bytes, slots;  // chunk-plane stride and patch ring depth (conv_halo.cu: Plane / Ring)
     unsigned long long m_per_frame, m_tiles_x;  // ceil(2^40 / d): x / d == (x * m) >> 40 for the ranges checked on the host
     float bias_c[128];
 };

@@ -36,7 +36,6 @@
 #include <string.h>
 
 #include "conv_tc.h"
-#include "options.h"
 #include "ptx.cuh"
 
 namespace fd {
@@ -483,7 +482,6 @@ conv_stem_kernel(const __grid_constant__ CUtensorMap tm_out, const __grid_consta
 }  // namespace
 
 bool conv_stem_supported(const StemDesc& d) {
-    if (!options().stem) return false;
     if (d.c1 != C1 || d.c2 != C2 || d.pad_hi2 < 0 || d.pad_hi2 > 1) return false;
     if (d.act1 && !(d.alpha1 >= 0.f && d.alpha1 <= 1.f)) return false;
     if (d.act2 && !(d.alpha2 >= 0.f && d.alpha2 <= 1.f)) return false;

@@ -1064,19 +1064,18 @@ int conv_tc_prepare(const ConvDesc& d, int num_sms, int block_n_hint, ConvLaunch
     // swapped mode for narrow layers: channels on the MMA's M side (128-row tiles), 256 pixels on its N side
     // (only where Cout fills the 128 lanes: with fewer channels most epilogue warps idle and the normal mode wins)
     const Options& O = options();
-    int swap = (d.cout > 64 && d.cout <= 128 && !d.out_fp32 && M >= 256 && O.swap) ? 1 : 0;
+    int swap = (d.cout > 64 && d.cout <= 128 && !d.out_fp32 && M >= 256) ? 1 : 0;
     if (block_n_hint == 1024) { swap = 1; block_n_hint = 0; }
     else if (block_n_hint) swap = 0;
-    // Small batches (option latency_bn: 1 = choose, 64 / 128 = forced, 0 = off): a layer whose 256-wide tiles would occupy
-    // less than a quarter of the SMs is cut into 128 x 64 (or 128 x 128) single-CTA tiles instead — up to eight times as
-    // many CTAs, each with a proportionally shorter main loop.  A launch is as long as ONE CTA's work, and at batch 1 that
-    // is what a layer costs: full-416 batch 1 0.90 -> 0.64 ms.  64-wide tiles where they still fit the GPU in one wave,
-    // 128-wide otherwise (measured: 64 everywhere makes batch 4 slower than the 256-wide default, 128 faster).
-    if (O.latency_bn && !block_n_hint && !d.out_fp32 && O.strip != 2) {  // (strip = 2 forces the CTA-pair strip form wherever it is legal)
+    // Small batches: a layer whose 256-wide tiles would occupy less than a quarter of the SMs is cut into 128 x 64 (or
+    // 128 x 128) single-CTA tiles instead — up to eight times as many CTAs, each with a proportionally shorter main loop.
+    // A launch is as long as ONE CTA's work, and at batch 1 that is what a layer costs: full-416 batch 1 0.90 -> 0.64 ms.
+    // 64-wide tiles where they still fit the GPU in one wave, 128-wide otherwise (measured: 64 everywhere makes batch 4
+    // slower than the 256-wide default, 128 faster).
+    if (!block_n_hint && !d.out_fp32 && O.strip != 2) {  // (strip = 2 forces the CTA-pair strip form wherever it is legal)
         const long long tiles256 = ((M + 255) / 256) * ((d.cout + 255) / 256);
         if (tiles256 * 4 <= num_sms) {
-            int lb = O.latency_bn;
-            if (lb == 1) lb = ((M + BLOCK_M - 1) / BLOCK_M) * ((d.cout + 63) / 64) <= num_sms ? 64 : 128;
+            const int lb = ((M + BLOCK_M - 1) / BLOCK_M) * ((d.cout + 63) / 64) <= num_sms ? 64 : 128;
             if (d.cout > lb) { swap = 0; block_n_hint = lb; }
         }
     }
@@ -1087,7 +1086,7 @@ int conv_tc_prepare(const ConvDesc& d, int num_sms, int block_n_hint, ConvLaunch
     int bn = block_n_hint ? block_n_hint : choose_block_n(d.cout, m_tiles, num_sms);
     if (!(bn == 32 || bn == 64 || bn == 128 || bn == 256)) { set_err(err, errlen, "conv_tc: bad block_n %lld", bn); return -1; }
 
-    if (two < 0) two = (bn == 256 && block_k == 64 && m_tiles >= 2 && O.two_cta) ? 1 : 0;
+    if (two < 0) two = (bn == 256 && block_k == 64 && m_tiles >= 2) ? 1 : 0;
     if (two && (bn != 256 || block_k != 64)) { set_err(err, errlen, "conv_tc: the CTA-pair kernel needs Cout > 128 and Cin %% 64 == 0"); return -1; }
     if (two) m_tiles = (M + 2 * BLOCK_M - 1) / (2 * BLOCK_M);
     // (clusters of two pairs sharing the filter tile through TMA multicast were built and measured in round 1: 812 instead
@@ -1104,7 +1103,8 @@ int conv_tc_prepare(const ConvDesc& d, int num_sms, int block_n_hint, ConvLaunch
         const bool plain_act = !d.act || (d.alpha >= 0.f && d.alpha <= 1.f);  // the strip kernel compiles the max(x, alpha x) form only
         const bool legal = two && plain_act && k == 3 && d.stride == 1 && d.pad_lo == 1 && d.pad_hi == 1 && block_k == 64 && !d.out_fp32 &&
                            !d.upsample2x && rows <= 400 && static_cast<long long>(d.n) * wp * hp < (1LL << 30);  // 400 rows: two strip buffers + a 5-stage B ring still fit
-        const bool pays = d.wi >= O.strip_min_w;  // (W+1)(H+1)/(WH) extra rows: 1.04 at 52x52, 1.08 at 26x26, 1.16 at 13x13
+        constexpr int STRIP_MIN_W = 12;  // (W+1)(H+1)/(WH) extra rows: 1.04 at 52x52, 1.08 at 26x26, 1.16 at 13x13
+        const bool pays = d.wi >= STRIP_MIN_W;
         // small batches keep the im2col form: it can split K over idle CTA pairs, the strip form cannot
         const long long strip_tiles = (static_cast<long long>(d.n) * wp * hp - (wp + 1) + 2 * BLOCK_M - 1) / (2 * BLOCK_M) * ((d.cout + bn - 1) / bn);
         const bool fills = strip_tiles >= num_sms / 2;
@@ -1219,17 +1219,16 @@ int conv_tc_prepare(const ConvDesc& d, int num_sms, int block_n_hint, ConvLaunch
     }
     L->block_n = bn;
     L->two_cta = two;
-    L->pdl = 1;
     // split-K for launches that cannot fill the GPU with whole tiles (small batches): parts of >= 4 K blocks
     p.split_k = 1;
     {
         const long long whole = m_tiles * p.num_n_tiles;
         const long long units_max = two ? num_sms / 2 : num_sms;
         // (a split costs ~8-10 us of fences, counter traffic and partial-sum reads, so it only pays on long K loops)
-        const int min_kb = O.split_k_min_kb, max_s = O.split_k_max;
-        if (d.allow_split_k && O.split_k && !swap && !p.strip && bn >= 64 && whole * 2 <= units_max && p.num_k_blocks >= min_kb) {
+        constexpr int SPLIT_K_MIN_KB = 32, SPLIT_K_MAX = 4;
+        if (d.allow_split_k && !swap && !p.strip && bn >= 64 && whole * 2 <= units_max && p.num_k_blocks >= SPLIT_K_MIN_KB) {
             long long sk = units_max / whole;
-            if (sk > max_s) sk = max_s;
+            if (sk > SPLIT_K_MAX) sk = SPLIT_K_MAX;
             if (sk > p.num_k_blocks / 4) sk = p.num_k_blocks / 4;
             if (sk >= 2) p.split_k = static_cast<int>(sk);
         }
@@ -1247,7 +1246,7 @@ int conv_tc_prepare(const ConvDesc& d, int num_sms, int block_n_hint, ConvLaunch
     // full barrier round trip (~450 cycles of wait/fence/commit in the issuing warp), so narrow layers put several
     // K blocks into one stage; then as many stages as fit (bytes in flight hide the ~1.5 us L2->SM fill latency).
     const int b_total = bn * K * 2;  // the whole filter bank of one N tile
-    const int b_res = (!two && !swap && p.num_n_tiles == 1 && b_total <= 65536 && O.b_resident) ? 1 : 0;
+    const int b_res = (!two && !swap && p.num_n_tiles == 1 && b_total <= 65536) ? 1 : 0;
     p.b_resident = b_res;
     const int sub_bytes = ((p.strip ? 0 : BLOCK_M) + (b_res ? 0 : (two ? bn / 2 : bn))) * block_k * 2;
     const int strips_bytes = p.strip ? 2 * ((p.strip_rows * 128 + 1023) / 1024 * 1024) : 0;
@@ -1282,7 +1281,6 @@ void conv_tc_bind_workspace(ConvLaunch* L, float* ws, int* counters) {
 
 int conv_tc_launch(const ConvLaunch& L, cudaStream_t stream) {
     if (L.p.split_k > 1 && (!L.p.ws || !L.p.counters)) return -1;  // conv_tc_bind_workspace was not called
-    const bool no_pdl = !options().pdl;
     cudaLaunchConfig_t cfg = {};
     cfg.gridDim = dim3(L.grid);
     cfg.blockDim = dim3(NUM_THREADS);
@@ -1297,12 +1295,10 @@ int conv_tc_launch(const ConvLaunch& L, cudaStream_t stream) {
         attr[na].val.clusterDim.z = 1;
         ++na;
     }
-    if (L.pdl && !no_pdl) {
-        // programmatic dependent launch: this kernel may start while its predecessor in the stream drains
-        attr[na].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-        attr[na].val.programmaticStreamSerializationAllowed = 1;
-        ++na;
-    }
+    // programmatic dependent launch: this kernel may start while its predecessor in the stream drains
+    attr[na].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+    attr[na].val.programmaticStreamSerializationAllowed = 1;
+    ++na;
     cfg.attrs = attr;
     cfg.numAttrs = na;
     cudaError_t e;

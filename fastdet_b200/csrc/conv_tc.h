@@ -89,7 +89,6 @@ struct ConvLaunch {
     int block_n;
     int two_cta;  // 1: CTA-pair kernel (cta_group::2, 256 x 256 tiles)
     int grid;
-    int pdl;      // 1: launched with programmatic stream serialisation (overlaps the previous kernel's drain)
     size_t smem_bytes;
     size_t ws_bytes;      // split-K workspace this launch needs (0: none)
     size_t counter_ints;  // zero-initialised ints it needs

@@ -172,3 +172,22 @@ def test_planned_fusions_host_logic():
         m = _native.Model(modelgen.build_onnx(arch, nc, size, seed=2), nc, (size, size), device=-1)
         assert m.planned_fusions(8) == want, (arch, size, m.planned_fusions(8))
         m.close()
+
+
+def test_option_names():
+    """Every plan-time option round-trips through fd_set_option / fd_get_option; the retired A/B switches are unknown
+    names, refused by both calls with FD_ERR_ARG."""
+    for name in ("strip", "stem", "block", "fuse_pool", "nms_general", "jpeg_threads", "server_inflight"):
+        old = _native.get_option(name)
+        try:
+            _native.set_option(name, old + 3)
+            assert _native.get_option(name) == old + 3, name
+        finally:
+            _native.set_option(name, old)
+        assert _native.get_option(name) == old, name
+    for name in ("strip_min_w", "swap", "two_cta", "split_k", "split_k_min_kb", "split_k_max", "latency_bn", "b_resident",
+                 "halo", "halo_skew", "halo_slots", "pdl", "graph", "exact_batch", "detect_overlap"):
+        for call in (lambda: _native.set_option(name, 1), lambda: _native.get_option(name)):
+            with pytest.raises(_native.NativeError) as e:
+                call()
+            assert e.value.code == _native.FD_ERR_ARG, name
