@@ -433,7 +433,7 @@ int launch_own(fd_model* m, Exec* e, int i, int k, int frames, bool halo, const 
         case LAYER_CONV0:
             rc = launch_conv0_u8(e->frames + static_cast<size_t>(k) * frames * P.net_h * P.net_w * 3, m->d_conv0 + L.w_off, m->d_bias + L.b_off,
                                  static_cast<__nv_bfloat16*>(loc_ptr(*e, P, L.out, false, k, frames)), frames, L.in.h, L.in.w, L.cout,
-                                 L.out.pitch, L.act, L.alpha, L.pool2, s);
+                                 L.stride, L.out.pitch, L.act, L.alpha, L.pool2, s);
             break;
         case LAYER_CONV: rc = halo ? conv_halo_launch(*hl, s) : conv_tc_launch(*cl, s); break;
         case LAYER_MAXPOOL:
@@ -916,7 +916,7 @@ static int build_overlap_plan(fd_model* m, Exec* e) {
     int downs = 0, depth = 0;
     for (size_t i = 0; i < P.layers.size(); ++i) {
         const LayerPlan& L = P.layers[i];
-        const bool down = (L.kind == LAYER_CONV && L.stride == 2) || (L.kind == LAYER_MAXPOOL && L.pool_s == 2) || L.pool2;
+        const bool down = ((L.kind == LAYER_CONV || L.kind == LAYER_CONV0) && L.stride == 2) || (L.kind == LAYER_MAXPOOL && L.pool_s == 2) || L.pool2;
         if (down && ++downs == 2) break;
         if (L.out_fp32 || L.upsample2x || L.kind == LAYER_COPY) return FD_OK;
         // every tensor these layers touch must be written inside the front (or be the input frames): nothing may reach back

@@ -86,7 +86,7 @@ static int prepare_two(const Net& N, int sms, HaloLaunch* hl) {
     return 0;
 }
 static int launch_two(const Net& N, const HaloLaunch& hl) {
-    if (launch_conv0_u8(N.d_frames, N.d_w1, N.d_b1, N.d_mid, N.n, N.h, N.w, 32, 32, 1, N.alpha, 0, 0)) return -1;
+    if (launch_conv0_u8(N.d_frames, N.d_w1, N.d_b1, N.d_mid, N.n, N.h, N.w, 32, 1, 32, 1, N.alpha, 0, 0)) return -1;
     return conv_halo_launch(hl, 0);
 }
 static int prepare_stem(const Net& N, int sms, StemLaunch* sl) {

@@ -18,11 +18,12 @@ int launch_normalise_f32_nchw(const uint8_t* frames, float* out, int n, int h, i
 // (extension: the reference server rejects non-net-sized frames, detector.py:131-132).
 int launch_letterbox_u8(const uint8_t* src, uint8_t* dst, int n, int sh, int sw, int h, int w, int fill,
                         cudaStream_t s);
-// first convolution fused with the normalisation: u8 [n,h,w,3] -> bf16 NHWC slice, 3x3 s1 p1, Cout <= 64,
+// first convolution fused with the normalisation: u8 [n,h,w,3] -> bf16 NHWC slice, 3x3 p1, Cout <= 64,
 // fp32 weights [3][3][3][cout] (BatchNorm folded), LeakyReLU(alpha) if act.
-// pool2: MaxPool(2, stride 2) of the activation in the epilogue; `out` is then the (h/2, wd/2) map (Cout 16 / 32 only).
+// stride 2 (h, w even; `out` the (h/2, w/2) map): tensor cores only, Cout 16 / 32 with out_pitch == cout.
+// pool2: MaxPool(2, stride 2) of the activation in the epilogue; `out` is then the (h/2, wd/2) map (stride 1, Cout 16 / 32 only).
 int launch_conv0_u8(const uint8_t* frames, const float* w, const float* bias, __nv_bfloat16* out, int n, int h,
-                    int wd, int cout, int out_pitch, int act, float alpha, int pool2, cudaStream_t s);
+                    int wd, int cout, int stride, int out_pitch, int act, float alpha, int pool2, cudaStream_t s);
 
 // ---- pool.cu ------------------------------------------------------------------------------------
 // max-pool over bf16 NHWC slices; cells outside the input take `pad_value` (-inf = ONNX MaxPool padding).

@@ -19,7 +19,7 @@ uint16_t f32_to_bf16_rn(float f) {
 
 namespace {
 
-enum AKind { A_INPUT, A_CONV, A_BN, A_LEAKY, A_ADD, A_MAXPOOL, A_PAD, A_RESIZE, A_CONCAT };
+enum AKind { A_INPUT, A_CONV, A_BN, A_LEAKY, A_ADD, A_MAXPOOL, A_PAD, A_RESIZE, A_CONCAT, A_VIEW };
 
 struct ANode {
     AKind kind;
@@ -34,11 +34,14 @@ struct ANode {
     float alpha = 0.f;                                   // leaky
     float pad_value = 0.f;                               // pad
     int pads[4] = {0, 0, 0, 0};                          // pad node: t,l,b,r
+    int view_start = 0;                                  // view: first channel inside the source (Slice / Split on axis 1)
     int value = -1;                                      // Value id this anode's result lives in
 };
 
 struct Value {
     TensorLoc loc;
+    int view_of = -1;  // a channel view: the Value it reads, view_start channels in (resolved after buffer assignment)
+    int view_start = 0;
     bool placed = false;
     bool is_input = false;
     bool fp32 = false;
@@ -361,6 +364,79 @@ struct Builder {
         return true;
     }
 
+    // Slice / Split of an activation on the channel axis: a view of the source's channels [start, start + len), no layer.
+    // Views of views compose; the alignment rule is checked where the view is read (an unread Split output may be anything).
+    bool add_view(const OnnxNode& n, int x, int64_t start, int64_t len, const std::string& out) {
+        if (an[x].kind == A_INPUT) return fail(n.name + ": channel slice of the network input is not supported");
+        if (len <= 0 || start < 0 || start + len > an[x].c) return fail(n.name + ": empty or out-of-range channel slice");
+        int src = x;
+        int64_t off = start;
+        if (an[x].kind == A_VIEW) { off += an[x].view_start; src = an[x].in[0]; }
+        const int id = add_anode(A_VIEW, static_cast<int>(&n - g.nodes.data()), {src}, static_cast<int>(len), an[x].h, an[x].w, out);
+        an[id].view_start = static_cast<int>(off);
+        return true;
+    }
+    bool channel_axis(const OnnxNode& n, int64_t axis) {
+        if (axis != 1 && axis != -3) return fail(n.name + ": " + n.op + " on axis " + std::to_string(axis) + " (only channel slices, axis 1, are supported)");
+        return true;
+    }
+    bool slice_view(const OnnxNode& n, int x) {
+        std::vector<int64_t> starts, ends, axes, steps;
+        if (n.inputs.size() >= 3) {  // opset >= 10: inputs, constant or folded from the shape chain
+            const OnnxTensor* s = cst(n.inputs[1]);
+            const OnnxTensor* e = cst(n.inputs[2]);
+            const OnnxTensor* a = n.inputs.size() > 3 && !n.inputs[3].empty() ? cst(n.inputs[3]) : nullptr;
+            const OnnxTensor* st = n.inputs.size() > 4 && !n.inputs[4].empty() ? cst(n.inputs[4]) : nullptr;
+            if (!s || !e || (n.inputs.size() > 3 && !n.inputs[3].empty() && !a) || (n.inputs.size() > 4 && !n.inputs[4].empty() && !st))
+                return fail(n.name + ": Slice starts / ends / axes / steps must be constant");
+            starts = s->i; ends = e->i;
+            if (a) axes = a->i;
+            if (st) steps = st->i;
+        } else {
+            const auto* ss = n.attr_ints("starts");
+            const auto* ee = n.attr_ints("ends");
+            if (!ss || !ee) return fail(n.name + ": Slice without starts / ends");
+            starts = *ss; ends = *ee;
+            if (const auto* ax = n.attr_ints("axes")) axes = *ax;
+        }
+        if (axes.empty()) for (size_t k = 0; k < starts.size(); ++k) axes.push_back(static_cast<int64_t>(k));
+        if (steps.empty()) steps.assign(starts.size(), 1);
+        if (starts.size() != 1 || ends.size() != 1 || axes.size() != 1 || steps.size() != 1)
+            return fail(n.name + ": Slice must touch the channel axis only (it slices N, H or W)");
+        if (!channel_axis(n, axes[0])) return false;
+        if (steps[0] != 1) return fail(n.name + ": Slice step " + std::to_string(steps[0]) + " (only step 1 is supported)");
+        // ONNX clamping: negative values count from the end, anything past the ends (INT64_MAX) clamps to them
+        const int64_t c = an[x].c;
+        int64_t s0 = starts[0], e0 = ends[0];
+        if (s0 < 0) s0 += c;
+        if (e0 < 0) e0 += c;
+        s0 = std::min(std::max<int64_t>(s0, 0), c);
+        e0 = std::min(std::max<int64_t>(e0, 0), c);
+        return add_view(n, x, s0, e0 - s0, n.outputs[0]);
+    }
+    bool split_views(const OnnxNode& n, int x) {
+        if (!channel_axis(n, n.attr_i("axis", 0))) return false;
+        std::vector<int64_t> sizes;
+        if (const auto* sp = n.attr_ints("split")) sizes = *sp;
+        else if (n.inputs.size() > 1 && !n.inputs[1].empty()) {
+            const OnnxTensor* t = cst(n.inputs[1]);
+            if (!t) return fail(n.name + ": Split sizes must be constant");
+            sizes = t->i;
+        } else {
+            const int64_t parts = static_cast<int64_t>(n.outputs.size());
+            if (an[x].c % parts) return fail(n.name + ": Split into equal parts of a channel count they do not divide");
+            sizes.assign(static_cast<size_t>(parts), an[x].c / parts);
+        }
+        if (sizes.size() != n.outputs.size()) return fail(n.name + ": Split has " + std::to_string(sizes.size()) + " sizes for " + std::to_string(n.outputs.size()) + " outputs");
+        int64_t off = 0;
+        for (size_t k = 0; k < sizes.size(); ++k) {
+            if (!n.outputs[k].empty() && !add_view(n, x, off, sizes[k], n.outputs[k])) return false;
+            off += sizes[k];
+        }
+        if (off != an[x].c) return fail(n.name + ": Split sizes do not add up to the channel count");
+        return true;
+    }
+
     bool walk() {
         for (const auto& kv : g.initializers) consts[kv.first] = kv.second;
         // graph input: the reference feeds {'input': a} (server/detector.py:135)
@@ -505,6 +581,10 @@ bool build_plan(const OnnxGraph& g, int net_w, int net_h, int num_classes, bool 
             if (ins.empty()) return B.fail(n.name + ": empty Concat");
             const int h = B.an[ins[0]].h, w = B.an[ins[0]].w;
             B.add_anode(A_CONCAT, static_cast<int>(ni), ins, c, h, w, out);
+        } else if (n.op == "Slice") {
+            if (!B.slice_view(n, x)) return false;
+        } else if (n.op == "Split") {
+            if (!B.split_views(n, x)) return false;
         } else {
             return B.fail("unsupported ONNX operator '" + n.op + "' (node '" + n.name + "')");
         }
@@ -513,6 +593,7 @@ bool build_plan(const OnnxGraph& g, int net_w, int net_h, int num_classes, bool 
     for (const auto& o : g.outputs) {
         const int a = B.act(o.name);
         if (a < 0) return B.fail("graph output '" + o.name + "' is not produced by a supported operator");
+        if (B.an[a].kind == A_VIEW) return B.fail("graph output '" + o.name + "' is a channel slice (node '" + g.nodes[B.an[a].node].name + "'): a head must be a convolution's own output");
         B.an[a].is_output = true;
         out_anodes.push_back(a);
     }
@@ -526,7 +607,7 @@ bool build_plan(const OnnxGraph& g, int net_w, int net_h, int num_classes, bool 
         return (!an[a].is_output && an[a].consumers.size() == 1) ? an[a].consumers[0] : -1;
     };
     for (int a = 0; a < static_cast<int>(an.size()); ++a) {
-        if (owner[a] >= 0 || an[a].kind == A_INPUT || an[a].kind == A_CONCAT) continue;
+        if (owner[a] >= 0 || an[a].kind == A_INPUT || an[a].kind == A_CONCAT || an[a].kind == A_VIEW) continue;
         Fused f;
         const int id = static_cast<int>(ops.size());
         if (an[a].kind == A_CONV) {
@@ -591,6 +672,18 @@ bool build_plan(const OnnxGraph& g, int net_w, int net_h, int num_classes, bool 
     }
     for (auto& f : ops) new_value(f.final_anode);
     for (int a = 0; a < static_cast<int>(an.size()); ++a) if (an[a].kind == A_CONCAT) new_value(a);
+    for (int a = 0; a < static_cast<int>(an.size()); ++a) {
+        if (an[a].kind != A_VIEW) continue;
+        const int src = an[an[a].in[0]].value;
+        if (src < 0) return B.fail("internal: the source of channel slice '" + an[a].out_name + "' has no value");
+        const int v = new_value(a);
+        vals[v].view_of = src;
+        vals[v].view_start = an[a].view_start;
+        // 16-byte alignment of every read through the view (TMA bases, cp.async)
+        if (!an[a].consumers.empty() && (an[a].view_start % 8 || an[a].c % 8))
+            return B.fail(g.nodes[an[a].node].name + ": channel slice [" + std::to_string(an[a].view_start) + ", " +
+                          std::to_string(an[a].view_start + an[a].c) + ") must start and end on multiples of 8 channels");
+    }
     // every consumed anode must carry a value (i.e. nobody reads the inside of a fused chain)
     for (int a = 0; a < static_cast<int>(an.size()); ++a) {
         if (an[a].value >= 0) continue;
@@ -625,7 +718,7 @@ bool build_plan(const OnnxGraph& g, int net_w, int net_h, int num_classes, bool 
             if (vi < 0) return B.fail("Concat input '" + an[in].out_name + "' has no materialised value");
             Value& v = vals[vi];
             if (off % 8 || v.loc.c % 8) return B.fail("Concat '" + an[a].out_name + "': slices must start on multiples of 8 channels");
-            if (!v.placed && !v.fp32) {
+            if (!v.placed && !v.fp32 && v.view_of < 0) {  // (a view's channels are written by its source's producer)
                 v.loc.buf = buf; v.loc.pitch = total; v.loc.ch_off = off; v.placed = true;
             } else {
                 Fused f;
@@ -637,11 +730,17 @@ bool build_plan(const OnnxGraph& g, int net_w, int net_h, int num_classes, bool 
         }
     }
     for (auto& v : vals) {
-        if (v.placed) continue;
+        if (v.placed || v.view_of >= 0) continue;
         const int pitch = v.fp32 ? (v.loc.c + 3) / 4 * 4 : v.loc.c;
         if (!v.fp32 && pitch % 8) return B.fail("activation channel counts must be multiples of 8");
         v.loc.buf = new_buffer(pitch, v.loc.h, v.loc.w, v.fp32 ? 1 : 0);
         v.loc.pitch = pitch; v.loc.ch_off = 0; v.placed = true;
+    }
+    // views last: the source may itself live in a concat buffer.  A view of a view was composed at creation.
+    for (auto& v : vals) {
+        if (v.view_of < 0) continue;
+        const TensorLoc& src = vals[v.view_of].loc;
+        v.loc.buf = src.buf; v.loc.pitch = src.pitch; v.loc.ch_off = src.ch_off + v.view_start; v.placed = true;
     }
     std::stable_sort(ops.begin(), ops.end(), [](const Fused& x, const Fused& y) { return x.anchor < y.anchor; });
 
@@ -718,8 +817,14 @@ bool build_plan(const OnnxGraph& g, int net_w, int net_h, int num_classes, bool 
             plan->bias_f32.resize(L.b_off + (L.cout + 255) / 256 * 256, 0.f);
             memcpy(plan->bias_f32.data() + L.b_off, shift.data(), sizeof(float) * L.cout);
             if (f.kind == LAYER_CONV0) {
-                if (L.cin != 3 || k != 3 || L.stride != 1 || L.pad_lo != 1 || L.pad_hi != 1 || L.cout % 8 || L.cout > 64 || L.upsample2x || L.res.buf != -1 || L.out_fp32)  // (pool2 only with Cout 16 / 32, checked where it is set)
-                    return B.fail(L.name + ": the first convolution must be 3x3 stride 1 pad 1 over 3 channels with Cout in {8..64}");
+                if (L.stride == 2) {  // only the tensor-core form (conv0_ws_kernel) takes stride 2: dense Cout 16 / 32 rows
+                    if (L.cin != 3 || k != 3 || L.pad_lo != 1 || L.pad_hi != 1 || !(L.cout == 16 || L.cout == 32) || L.out.pitch != L.cout ||
+                        L.in.h % 2 || L.in.w % 2 || L.upsample2x || L.res.buf != -1 || L.out_fp32)
+                        return B.fail(L.name + ": a stride-2 first convolution must be 3x3 pad 1 over 3 channels with Cout 16 or 32, "
+                                      "on an even-sized input, into a tensor of its own");
+                } else if (L.cin != 3 || k != 3 || L.stride != 1 || L.pad_lo != 1 || L.pad_hi != 1 || L.cout % 8 || L.cout > 64 || L.upsample2x || L.res.buf != -1 || L.out_fp32) {  // (pool2 only with Cout 16 / 32, checked where it is set)
+                    return B.fail(L.name + ": the first convolution must be 3x3 stride 1 pad 1 over 3 channels with Cout in {8..64}, or 3x3 stride 2 with Cout 16 or 32");
+                }
                 L.w_off = plan->conv0_w.size();
                 plan->conv0_w.resize(L.w_off + static_cast<size_t>(K) * L.cout);
                 for (int co = 0; co < L.cout; ++co)

@@ -3,8 +3,8 @@
 // The optimisation half of `ort.InferenceSession(...)` (reference server/detector.py:118), rebuilt for this
 // path: Conv -> [BatchNormalization] -> [LeakyRelu] -> [Add] -> [Resize x2] chains collapse into one fused
 // convolution each (BatchNorm folded into fp32 weights/bias before the bf16 rounding), Concat becomes a shared
-// buffer its producers write channel slices of, Pad+MaxPool merge, and every activation gets a bf16 NHWC
-// location.  No device code here; capi.cu turns the plan into buffers, tensor maps and launches.
+// buffer its producers write channel slices of, a channel Slice / Split becomes a view (a location inside its source's
+// buffer, no layer), Pad+MaxPool merge, and every activation gets a bf16 NHWC location.  No device code here; capi.cu turns the plan into buffers, tensor maps and launches.
 #pragma once
 #include <stdint.h>
 

@@ -236,9 +236,24 @@ conv0_u8_kernel(const uint8_t* __restrict__ frames, const float* __restrict__ wg
 //     per tile, ~45 cycles each (dev/mma_rate.cu), against the 64 B/pixel the layer has to write to HBM.
 //   * Epilogue: each warp drains its TMEM lane quarter (lane = pixel), bias + LeakyReLU in registers, bf16 rows staged
 //     in shared memory and written by one TMA store per warp (box = Cout x 8 pixels x 4 rows).
+//
+// Stride 2 (YOLOv4-tiny: 416 -> 208) keeps the same trick with PAIR units: a 16-byte unit holds the RGB of input columns
+// (2u, 2u+1) and two zero slots.  Output column x reads columns 2x-1 (tap 0: unit x-1's second half) and 2x, 2x+1
+// (taps 1, 2: unit x), so K chunk 0 of filter row r is unit x-1 and chunk 1 unit x: LBO = 16 B again, 8 consecutive
+// output pixels are 8 consecutive units, and SBO = TWO patch rows walks down the output rows.  K = 16 per filter row:
+// 3 MMAs per 128 outputs; the patch of a 16 x 8 output tile is 33 rows x 9 units, no slack needed.
 static constexpr int C0D_TW = 8, C0D_TH = 16;
-static constexpr int C0D_PW = C0D_TW + 2, C0D_PH = C0D_TH + 2;   // halo patch, pixels
-static constexpr int C0D_PATCH_BYTES = (C0D_PH * C0D_PW + 8) * 16;  // + slack: tap 3 of the last pixels reads past the end
+template <int S> struct C0Geom;
+template <> struct C0Geom<1> {
+    static constexpr int PW = C0D_TW + 2, PH = C0D_TH + 2;     // halo patch, pixels
+    static constexpr int PATCH_BYTES = (PH * PW + 8) * 16;     // + slack: tap 3 of the last pixels reads past the end
+    static constexpr int MMAS = 6;                             // per tile: 3 filter rows x 2 K steps (taps 0-1, 2-3)
+};
+template <> struct C0Geom<2> {
+    static constexpr int PW = C0D_TW + 1, PH = 2 * C0D_TH + 1;  // halo patch, pair units
+    static constexpr int PATCH_BYTES = PH * PW * 16;
+    static constexpr int MMAS = 3;                              // per tile: one per filter row
+};
 
 // Warp-specialised: a lock-step version (build -> sync -> MMA -> wait -> drain per tile) spent most of a tile's ~5000
 // cycles waiting at its barriers (ncu: barrier + load-use stalls), so the three stages run decoupled over rings:
@@ -255,12 +270,16 @@ static constexpr int C0W_THREADS = (C0W_EPI_WARPS + 1 + C0W_BUILD_WARPS) * 32, C
 // publish -> MMA -> drain -> release round trip is ~3000 cycles, so 4 slots capped the kernel at ~800 cycles per tile
 // q = x / d for 0 <= x < 2^24 and d < 2^12 as one 64-bit multiply: m = ceil(2^40 / d)
 __device__ __forceinline__ int div_magic(int x, unsigned long long m) { return static_cast<int>((static_cast<unsigned long long>(x) * m) >> 40); }
-static constexpr int C0W_PPL = (C0D_PH * C0D_PW + 31) / 32;  // patch pixels per builder lane
 
+// h, wd: the input frame; the output map is (h / S, wd / S) (stride 2: h and wd even)
+template <int S>
 __global__ void __launch_bounds__(C0W_THREADS)
 conv0_ws_kernel(const uint8_t* __restrict__ frames, const float* __restrict__ wgt, const float* __restrict__ bias,
                 const __grid_constant__ CUtensorMap tm_out, int n, int h, int wd, int cout, int act, float alpha,
                 unsigned long long m_per_frame, unsigned long long m_tiles_x, int pool2) {
+    using G = C0Geom<S>;
+    constexpr int C0D_PATCH_BYTES = G::PATCH_BYTES;
+    constexpr int C0W_PPL = (G::PH * G::PW + 31) / 32;  // patch units per builder lane
     extern __shared__ __align__(1024) uint8_t c0w_dyn[];        // patch ring
     uint8_t (*s_patch)[C0D_PATCH_BYTES] = reinterpret_cast<uint8_t (*)[C0D_PATCH_BYTES]>(c0w_dyn);
     __shared__ __align__(1024) uint8_t s_w[12 * 32 * 16];       // B: [K chunk 0..11][32 filters][16 B]
@@ -274,14 +293,30 @@ conv0_ws_kernel(const uint8_t* __restrict__ frames, const float* __restrict__ wg
         const __nv_bfloat16 v = __float2bfloat16(norm_u8(i));
         lut[i] = *reinterpret_cast<const uint16_t*>(&v);
     }
-    for (int i = tid; i < 12 * 32; i += C0W_THREADS) {
-        const int c = i >> 5, f = i & 31, r = c >> 2, sx = c & 3;
-        float w0 = 0.f, w1 = 0.f, w2 = 0.f;
-        if (sx < 3 && f < cout) {
-            const float* wp = wgt + ((r * 3 + sx) * 3) * cout + f;
-            w0 = __ldg(wp); w1 = __ldg(wp + cout); w2 = __ldg(wp + 2 * cout);
+    if constexpr (S == 1) {
+        for (int i = tid; i < 12 * 32; i += C0W_THREADS) {
+            const int c = i >> 5, f = i & 31, r = c >> 2, sx = c & 3;
+            float w0 = 0.f, w1 = 0.f, w2 = 0.f;
+            if (sx < 3 && f < cout) {
+                const float* wp = wgt + ((r * 3 + sx) * 3) * cout + f;
+                w0 = __ldg(wp); w1 = __ldg(wp + cout); w2 = __ldg(wp + 2 * cout);
+            }
+            *reinterpret_cast<uint4*>(s_w + i * 16) = make_uint4(c0_pack(w0, w1), c0_pack(w2, 0.f), 0u, 0u);
         }
-        *reinterpret_cast<uint4*>(s_w + i * 16) = make_uint4(c0_pack(w0, w1), c0_pack(w2, 0.f), 0u, 0u);
+    } else {
+        // chunk 2r: slots 3..5 = tap (r, 0) (the second pixel of unit x-1); chunk 2r+1: slots 0..2 = tap (r, 1), 3..5 = tap (r, 2)
+        for (int i = tid; i < 6 * 32; i += C0W_THREADS) {
+            const int c = i >> 5, f = i & 31, r = c >> 1;
+            float w[6] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f};
+            if (f < cout) {
+#pragma unroll
+                for (int j = 0; j < 6; ++j) {
+                    const int sx = (c & 1) ? 1 + j / 3 : 0;
+                    if ((c & 1) || j >= 3) w[j] = __ldg(wgt + ((r * 3 + sx) * 3 + j % 3) * cout + f);
+                }
+            }
+            *reinterpret_cast<uint4*>(s_w + i * 16) = make_uint4(c0_pack(w[0], w[1]), c0_pack(w[2], w[3]), c0_pack(w[4], w[5]), 0u);
+        }
     }
     for (int i = tid; i < C0W_PATCHES * C0D_PATCH_BYTES / 16; i += C0W_THREADS) reinterpret_cast<uint4*>(c0w_dyn)[i] = make_uint4(0u, 0u, 0u, 0u);
     if (tid == 0) {
@@ -301,7 +336,7 @@ conv0_ws_kernel(const uint8_t* __restrict__ frames, const float* __restrict__ wg
     const uint32_t tmem = tmem_slot;
     ptx::grid_dep_launch();  // the next layer may start its set-up on SMs as they drain (it waits before reading)
 
-    const int tiles_x = (wd + C0D_TW - 1) / C0D_TW, tiles_y = (h + C0D_TH - 1) / C0D_TH;
+    const int tiles_x = (wd / S + C0D_TW - 1) / C0D_TW, tiles_y = (h / S + C0D_TH - 1) / C0D_TH;
     const int per_frame = tiles_x * tiles_y;
     const int total = n * per_frame;  // < 2^31 by far
     const int my_tiles = (total > static_cast<int>(blockIdx.x)) ? (total - 1 - static_cast<int>(blockIdx.x)) / static_cast<int>(gridDim.x) + 1 : 0;
@@ -311,15 +346,16 @@ conv0_ws_kernel(const uint8_t* __restrict__ frames, const float* __restrict__ wg
         // warp s of this role owns patch slot s and every 8th tile; a lane handles 6 fixed patch pixels, whose
         // offsets inside a tile are computed once (one warp's dependent-instruction latency per tile is what bounds
         // this role, so the per-tile work is kept to the loads, the LUT and the stores)
+        // (stride 2: a unit is 2 pixels = 6 bytes at an even offset, loaded as 3 u16; the frames are 2-byte aligned)
         const int slot = warp - C0W_MMA_WARP - 1;
         int pq[C0W_PPL], ppy[C0W_PPL], ppx[C0W_PPL], poff[C0W_PPL];
 #pragma unroll
         for (int k = 0; k < C0W_PPL; ++k) {
-            const int q = lane + 32 * k;  // patch pixel
-            pq[k] = q < C0D_PH * C0D_PW ? q : -1;
-            ppy[k] = q / C0D_PW;
-            ppx[k] = q - ppy[k] * C0D_PW;
-            poff[k] = (ppy[k] * wd + ppx[k]) * 3;
+            const int q = lane + 32 * k;  // patch unit
+            pq[k] = q < G::PH * G::PW ? q : -1;
+            ppy[k] = q / G::PW;
+            ppx[k] = q - ppy[k] * G::PW;
+            poff[k] = (ppy[k] * wd + S * ppx[k]) * 3;
         }
         // two register sets: the bytes of this warp's next TWO tiles are in flight while it converts the current one
         // (the loads come from DRAM: one tile of look-ahead left the warp waiting on them)
@@ -331,18 +367,25 @@ conv0_ws_kernel(const uint8_t* __restrict__ frames, const float* __restrict__ wg
             const int f = div_magic(tile, m_per_frame);
             const int rem = tile - f * per_frame;
             const int ty = div_magic(rem, m_tiles_x), tx = rem - ty * tiles_x;
-            const int y0 = ty * C0D_TH - 1, x0 = tx * C0D_TW - 1;
-            const uint8_t* origin = frames + (1LL * f * h * wd + 1LL * y0 * wd + x0) * 3;  // may point before the frame: only used when inside
+            const int y0 = ty * C0D_TH * S - 1, x0 = tx * C0D_TW - 1;  // first patch row (input) and unit (input pixel or pair)
+            const uint8_t* origin = frames + (1LL * f * h * wd + 1LL * y0 * wd + S * x0) * 3;  // may point before the frame: only used when inside
             inside = 0;
 #pragma unroll
             for (int k = 0; k < C0W_PPL; ++k) {
                 const int gy = y0 + ppy[k], gx = x0 + ppx[k];
-                if (pq[k] >= 0 && gy >= 0 && gy < h && gx >= 0 && gx < wd) {  // outside: zero padding of the normalised input
+                if (pq[k] >= 0 && gy >= 0 && gy < h && gx >= 0 && gx < wd / S) {  // outside: zero padding of the normalised input
                     const uint8_t* sp = origin + poff[k];
                     inside |= 1u << k;
-                    raw[3 * k] = __ldg(sp);
-                    raw[3 * k + 1] = __ldg(sp + 1);
-                    raw[3 * k + 2] = __ldg(sp + 2);
+                    if constexpr (S == 1) {
+                        raw[3 * k] = __ldg(sp);
+                        raw[3 * k + 1] = __ldg(sp + 1);
+                        raw[3 * k + 2] = __ldg(sp + 2);
+                    } else {
+                        const uint16_t* sp16 = reinterpret_cast<const uint16_t*>(sp);
+                        raw[3 * k] = __ldg(sp16);
+                        raw[3 * k + 1] = __ldg(sp16 + 1);
+                        raw[3 * k + 2] = __ldg(sp16 + 2);
+                    }
                 }
             }
         };
@@ -353,8 +396,14 @@ conv0_ws_kernel(const uint8_t* __restrict__ frames, const float* __restrict__ wg
                 if (pq[k] >= 0) {
                     uint4 v = make_uint4(0u, 0u, 0u, 0u);
                     if (inside & (1u << k)) {
-                        v.x = static_cast<uint32_t>(lut[raw[3 * k]]) | (static_cast<uint32_t>(lut[raw[3 * k + 1]]) << 16);
-                        v.y = static_cast<uint32_t>(lut[raw[3 * k + 2]]);
+                        if constexpr (S == 1) {
+                            v.x = static_cast<uint32_t>(lut[raw[3 * k]]) | (static_cast<uint32_t>(lut[raw[3 * k + 1]]) << 16);
+                            v.y = static_cast<uint32_t>(lut[raw[3 * k + 2]]);
+                        } else {  // (R0 G0) (B0 R1) (G1 B1): byte pairs in memory order
+                            v.x = static_cast<uint32_t>(lut[raw[3 * k] & 255]) | (static_cast<uint32_t>(lut[raw[3 * k] >> 8]) << 16);
+                            v.y = static_cast<uint32_t>(lut[raw[3 * k + 1] & 255]) | (static_cast<uint32_t>(lut[raw[3 * k + 1] >> 8]) << 16);
+                            v.z = static_cast<uint32_t>(lut[raw[3 * k + 2] & 255]) | (static_cast<uint32_t>(lut[raw[3 * k + 2] >> 8]) << 16);
+                        }
                     }
                     *reinterpret_cast<uint4*>(&s_patch[slot][pq[k] * 16]) = v;
                 }
@@ -367,17 +416,27 @@ conv0_ws_kernel(const uint8_t* __restrict__ frames, const float* __restrict__ wg
         };
         uint32_t phase = 0;
         if (slot < my_tiles) fetch(slot, raw_a, inside_a);
-        if (slot + C0W_PATCHES < my_tiles) fetch(slot + C0W_PATCHES, raw_b, inside_b);
-        for (int it = slot; it < my_tiles; it += 2 * C0W_PATCHES) {
-            publish(raw_a, inside_a, phase);
-            if (it + 2 * C0W_PATCHES < my_tiles) fetch(it + 2 * C0W_PATCHES, raw_a, inside_a);
-            signal();
-            phase ^= 1;
-            if (it + C0W_PATCHES >= my_tiles) break;
-            publish(raw_b, inside_b, phase);
-            if (it + 3 * C0W_PATCHES < my_tiles) fetch(it + 3 * C0W_PATCHES, raw_b, inside_b);
-            signal();
-            phase ^= 1;
+        if constexpr (S == 2) {
+            // one register set: 10 units per lane (30 loads in flight) leave no room for a second one in 80 registers
+            for (int it = slot; it < my_tiles; it += C0W_PATCHES) {
+                publish(raw_a, inside_a, phase);
+                if (it + C0W_PATCHES < my_tiles) fetch(it + C0W_PATCHES, raw_a, inside_a);
+                signal();
+                phase ^= 1;
+            }
+        } else {
+            if (slot + C0W_PATCHES < my_tiles) fetch(slot + C0W_PATCHES, raw_b, inside_b);
+            for (int it = slot; it < my_tiles; it += 2 * C0W_PATCHES) {
+                publish(raw_a, inside_a, phase);
+                if (it + 2 * C0W_PATCHES < my_tiles) fetch(it + 2 * C0W_PATCHES, raw_a, inside_a);
+                signal();
+                phase ^= 1;
+                if (it + C0W_PATCHES >= my_tiles) break;
+                publish(raw_b, inside_b, phase);
+                if (it + 3 * C0W_PATCHES < my_tiles) fetch(it + 3 * C0W_PATCHES, raw_b, inside_b);
+                signal();
+                phase ^= 1;
+            }
         }
     } else if (warp == C0W_MMA_WARP) {
         // ---------------------------------------------------------------- MMA issuer
@@ -397,13 +456,18 @@ conv0_ws_kernel(const uint8_t* __restrict__ frames, const float* __restrict__ wg
         const uint32_t bar_af = __shfl_sync(0xffffffffu, ptx::smem_u32(&acc_full[0]), 0);
         const uint32_t bar_ae = __shfl_sync(0xffffffffu, ptx::smem_u32(&acc_empty[0]), 0);
         const uint32_t tmem_u = __shfl_sync(0xffffffffu, tmem, 0);
-        const uint64_t a0 = desc(p_addr0, 16, C0D_PW * 16);
-        uint64_t bd[6], aoff[6];
+        const uint64_t a0 = desc(p_addr0, 16, S * G::PW * 16);
+        uint64_t bd[G::MMAS], aoff[G::MMAS];
 #pragma unroll
-        for (int j = 0; j < 6; ++j) {
-            const int r = j >> 1, s0 = (j & 1) * 2;  // filter row, first of the two taps of this K step
-            bd[j] = desc(w_addr + (r * 4 + s0) * 512, 512, 128);
-            aoff[j] = static_cast<uint64_t>(r * C0D_PW + s0);  // 16-byte units
+        for (int j = 0; j < G::MMAS; ++j) {
+            if constexpr (S == 1) {
+                const int r = j >> 1, s0 = (j & 1) * 2;  // filter row, first of the two taps of this K step
+                bd[j] = desc(w_addr + (r * 4 + s0) * 512, 512, 128);
+                aoff[j] = static_cast<uint64_t>(r * G::PW + s0);  // 16-byte units
+            } else {
+                bd[j] = desc(w_addr + 2 * j * 512, 512, 128);  // filter row j: chunks 2j, 2j + 1
+                aoff[j] = static_cast<uint64_t>(j * G::PW);    // patch row j, unit 0 (= output column -1 of the tile)
+            }
         }
         const bool issuer = ptx::elect_one();
         uint32_t slot = 0, phase = 0;
@@ -415,7 +479,7 @@ conv0_ws_kernel(const uint8_t* __restrict__ frames, const float* __restrict__ wg
             const uint32_t d = tmem_u + slot * 32;
             if (issuer) {
 #pragma unroll
-                for (int j = 0; j < 6; ++j) ptx::umma_bf16(d, ad + aoff[j], bd[j], idesc, j ? 1u : 0u);
+                for (int j = 0; j < G::MMAS; ++j) ptx::umma_bf16(d, ad + aoff[j], bd[j], idesc, j ? 1u : 0u);
                 ptx::umma_commit_addr(bar_pe + 8u * slot);
                 ptx::umma_commit_addr(bar_af + 8u * slot);
             }
@@ -525,22 +589,27 @@ conv0_ws_kernel(const uint8_t* __restrict__ frames, const float* __restrict__ wg
 
 int kernels_init() {
     return (cudaFuncSetAttribute(conv0_u8_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 100 * 1024) == cudaSuccess &&
-            cudaFuncSetAttribute(conv0_ws_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, C0W_PATCHES * C0D_PATCH_BYTES) == cudaSuccess)
+            cudaFuncSetAttribute(conv0_ws_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, C0W_PATCHES * C0Geom<1>::PATCH_BYTES) == cudaSuccess &&
+            cudaFuncSetAttribute(conv0_ws_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, C0W_PATCHES * C0Geom<2>::PATCH_BYTES) == cudaSuccess)
                ? 0
                : -1;
 }
 
 int launch_conv0_u8(const uint8_t* frames, const float* w, const float* bias, __nv_bfloat16* out, int n, int h,
-                    int wd, int cout, int out_pitch, int act, float alpha, int pool2, cudaStream_t s) {
+                    int wd, int cout, int stride, int out_pitch, int act, float alpha, int pool2, cudaStream_t s) {
     const int act_mode = act ? ((alpha >= 0.f && alpha <= 1.f) ? 1 : 2) : 0;
-    const long long tiles = 1LL * n * ((wd + C0D_TW - 1) / C0D_TW) * ((h + C0D_TH - 1) / C0D_TH);
-    const int tx = (wd + C0D_TW - 1) / C0D_TW, per_frame = tx * ((h + C0D_TH - 1) / C0D_TH);
+    if (stride != 1 && stride != 2) return -1;
+    // stride 2: tensor cores only (even input, dense Cout 16 / 32 rows, 2-byte aligned frames for the pair loads)
+    if (stride == 2 && (((h | wd) & 1) || pool2 || (reinterpret_cast<uintptr_t>(frames) & 1))) return -1;
+    const int sh = h / stride, sw = wd / stride;  // the convolution's output map
+    const long long tiles = 1LL * n * ((sw + C0D_TW - 1) / C0D_TW) * ((sh + C0D_TH - 1) / C0D_TH);
+    const int tx = (sw + C0D_TW - 1) / C0D_TW, per_frame = tx * ((sh + C0D_TH - 1) / C0D_TH);
     if ((cout == 16 || cout == 32) && out_pitch == cout && (reinterpret_cast<uintptr_t>(out) & 15) == 0 &&
         tiles < (1LL << 24) && per_frame < 65536) {  // (ranges of the multiply-shift division)
         // dense NHWC output: an image row is one run of W*C elements; TMA store box = 8 pixels x 4 rows
         CUtensorMap tm;
         // (pooled: the output map is (h/2, wd/2) and a warp's box its 2 x 4 surviving pixels)
-        const int oh = pool2 ? h / 2 : h, ow = pool2 ? wd / 2 : wd;
+        const int oh = pool2 ? h / 2 : sh, ow = pool2 ? wd / 2 : sw;
         if (pool2 && ((h | wd) & 1)) return -1;
         const unsigned long long dims[3] = {static_cast<unsigned long long>(cout) * ow, static_cast<unsigned long long>(oh),
                                             static_cast<unsigned long long>(n)};
@@ -549,12 +618,15 @@ int launch_conv0_u8(const uint8_t* frames, const float* w, const float* bias, __
         if (encode_tiled_bf16(&tm, out, 3, dims, strides, box, 0)) return -1;
         const int blocks = static_cast<int>(tiles < 148LL ? tiles : 148LL);
         const unsigned long long one40 = 1ULL << 40;
-        conv0_ws_kernel<<<blocks, C0W_THREADS, C0W_PATCHES * C0D_PATCH_BYTES, s>>>(frames, w, bias, tm, n, h, wd, cout, act_mode, alpha,
-                                                                                  (one40 + per_frame - 1) / per_frame, (one40 + tx - 1) / tx, pool2);
+        const unsigned long long mf = (one40 + per_frame - 1) / per_frame, mx = (one40 + tx - 1) / tx;
+        if (stride == 2)
+            conv0_ws_kernel<2><<<blocks, C0W_THREADS, C0W_PATCHES * C0Geom<2>::PATCH_BYTES, s>>>(frames, w, bias, tm, n, h, wd, cout, act_mode, alpha, mf, mx, 0);
+        else
+            conv0_ws_kernel<1><<<blocks, C0W_THREADS, C0W_PATCHES * C0Geom<1>::PATCH_BYTES, s>>>(frames, w, bias, tm, n, h, wd, cout, act_mode, alpha, mf, mx, pool2);
         return cudaPeekAtLastError() == cudaSuccess ? 0 : -1;  // (peek: the caller reports the reason)
     }
-    // any other first layer (Cout up to 64, any pitch): CUDA cores
-    if (pool2) return -1;  // (the planner fuses the pool only for shapes the kernel above takes)
+    // any other stride-1 first layer (Cout up to 64, any pitch): CUDA cores
+    if (pool2 || stride != 1) return -1;  // (the planner fuses the pool, and takes stride 2, only for shapes the kernel above takes)
     const size_t smem = (256 + (C0_TH + 2) * (C0_TW + 2) * 3 + 4 + 27 * cout + cout) * sizeof(float) +
                         static_cast<size_t>(C0_TH) * C0_TW * cout * 2;
     dim3 grid((wd + C0_TW - 1) / C0_TW, (h + C0_TH - 1) / C0_TH, n);

@@ -1,15 +1,15 @@
-"""modelgen.py — synthetic YOLOv3 / YOLOv3-tiny ONNX files with random-init weights.
+"""modelgen.py — synthetic YOLOv3 / YOLOv3-tiny / YOLOv4-tiny ONNX files with random-init weights.
 
 The reference ships no model files (``*.onnx`` is git-ignored, reference .gitignore:5; README.md:38-48
 names ``yolov3-full.onnx`` / ``yolov3-rsu.onnx`` / ``yolov3-tiny.onnx``), so tests and benchmarks
-generate them.  The topologies are the public Darknet ``yolov3.cfg`` / ``yolov3-tiny.cfg``; the graph
+generate them.  The topologies are the public Darknet ``yolov3.cfg`` / ``yolov3-tiny.cfg`` / ``yolov4-tiny.cfg``; the graph
 contract is what reference server/detector.py:135-140 requires: one input named ``input`` (f32 NCHW,
 range [0,1]) and 2 or 3 raw head maps ``[N, 3*(5+nc), S/32*k, S/32*k]``, coarsest first.
 
 The file is written with a small hand protobuf encoder (the ``onnx`` package is not installed); the
 exporter variants (BN folded or not, Resize vs Upsample, Pad+MaxPool vs padded MaxPool, initializers
-vs Constant nodes, raw vs typed tensor data) exist so the native loader is exercised on the forms
-real exporters emit.
+vs Constant nodes, raw vs typed tensor data, Slice vs Split for YOLOv4-tiny's channel groups) exist so the native
+loader is exercised on the forms real exporters emit.
 """
 from __future__ import annotations
 
@@ -162,6 +162,8 @@ class Layer:
     leaky: bool = True
     frm: Tuple[int, ...] = ()  # shortcut: (from,), route: layer indices (darknet-style, may be negative)
     res_tail: bool = False  # conv that closes a residual branch (its output feeds a shortcut)
+    groups: int = 1  # route: keep channel group `group_id` of `groups` equal groups (CSP "route groups")
+    group_id: int = 0
 
 
 def yolov3_layers(num_classes: int) -> List[Layer]:
@@ -234,7 +236,38 @@ def yolov3_tiny_layers(num_classes: int) -> List[Layer]:
     return L
 
 
-ARCHS = {"full": yolov3_layers, "rsu": yolov3_layers, "tiny": yolov3_tiny_layers}
+def yolov4_tiny_layers(num_classes: int) -> List[Layer]:
+    """Darknet yolov4-tiny.cfg: 21 convs (the first two stride 2), 3 CSP stages whose route groups take the second
+    half of a tensor's channels, 3 maxpools, 1 upsample, 2 heads (coarsest first)."""
+    L: List[Layer] = []
+    head_c = 3 * (5 + num_classes)
+    L.append(Layer("conv", 32, 3, 2))
+    L.append(Layer("conv", 64, 3, 2))
+    for c in (64, 128, 256):  # layers 2-9, 10-17, 18-25
+        L.append(Layer("conv", c, 3, 1))
+        L.append(Layer("route", frm=(-1,), groups=2, group_id=1))
+        L.append(Layer("conv", c // 2, 3, 1))
+        L.append(Layer("conv", c // 2, 3, 1))
+        L.append(Layer("route", frm=(-1, -2)))
+        L.append(Layer("conv", c, 1, 1))
+        L.append(Layer("route", frm=(-6, -1)))
+        L.append(Layer("maxpool", size=2, stride=2))
+    L.append(Layer("conv", 512, 3, 1))
+    L.append(Layer("conv", 256, 1, 1))  # 27: branch point
+    L.append(Layer("conv", 512, 3, 1))
+    L.append(Layer("conv", head_c, 1, 1, bn=False, leaky=False))
+    L.append(Layer("yolo"))
+    L.append(Layer("route", frm=(-4,)))
+    L.append(Layer("conv", 128, 1, 1))
+    L.append(Layer("upsample", stride=2))
+    L.append(Layer("route", frm=(-1, 23)))
+    L.append(Layer("conv", 256, 3, 1))
+    L.append(Layer("conv", head_c, 1, 1, bn=False, leaky=False))
+    L.append(Layer("yolo"))
+    return L
+
+
+ARCHS = {"full": yolov3_layers, "rsu": yolov3_layers, "tiny": yolov3_tiny_layers, "tiny4": yolov4_tiny_layers}
 
 
 def conv_gflops(arch: str, num_classes: int, size: int) -> float:
@@ -254,7 +287,7 @@ def conv_gflops(arch: str, num_classes: int, size: int) -> float:
             s = s * 2
         elif l.kind == "route":
             idx = [j if j >= 0 else i + j for j in l.frm]
-            c = sum(shapes[j][0] for j in idx)
+            c = sum(shapes[j][0] for j in idx) // l.groups
             s = shapes[idx[0]][1]
         elif l.kind == "shortcut":
             pass
@@ -280,6 +313,8 @@ class ExportOptions:
     obj_spread: float = 1.5  # standard deviation of the objectness logits over positions
     head_gain: float = 1.0  # RMS of the head logits (calibrated)
     opset: int = 11
+    split_op: str = "Slice"  # route groups: "Slice" (constant starts / ends inputs) | "Split" (sizes as the `split`
+    # attribute below opset 13, as an input from 13 on)
 
 
 def _he_sigma(fan_in: int) -> float:
@@ -293,7 +328,7 @@ def _leaky(x):
 
 def build_onnx(arch: str, num_classes: int, size: int = 416, seed: int = 0,
                opts: Optional[ExportOptions] = None) -> bytes:
-    """Serialized ModelProto for `arch` in {"tiny", "full", "rsu"} with seeded random weights.
+    """Serialized ModelProto for `arch` in {"tiny", "full", "rsu", "tiny4"} with seeded random weights.
 
     Weights are the SURVEY §8d recipe — He-normal convs, BatchNorm gamma~U(.8,1.2), beta~N(0,.1),
     mean~N(0,.1), var~U(.8,1.2) — followed by one scalar per layer, fitted on two synthetic frames: each
@@ -410,7 +445,29 @@ def build_onnx(arch: str, num_classes: int, size: int = 416, seed: int = 0,
                 cur, x = out, x + acts[j]
             elif l.kind == "route":
                 idx = [j if j >= 0 else i + j for j in l.frm]
-                if len(idx) == 1:
+                if l.groups > 1:  # one channel group of one tensor: Slice or Split on axis 1
+                    src, cs = names[idx[0]], chans[idx[0]]
+                    gc = cs // l.groups
+                    out = f"route{i}_out"
+                    if opts.split_op == "Slice":
+                        add_const(f"route{i}_starts", np.array([gc * l.group_id], np.int64))
+                        add_const(f"route{i}_ends", np.array([gc * (l.group_id + 1) if l.group_id + 1 < l.groups else 2**63 - 1], np.int64))
+                        add_const(f"route{i}_axes", np.array([1], np.int64))
+                        nodes.append(node_proto("Slice", [src, f"route{i}_starts", f"route{i}_ends", f"route{i}_axes"], [out],
+                                                name=f"route{i}"))
+                    elif opts.split_op == "Split":
+                        outs = [out if g == l.group_id else f"route{i}_part{g}" for g in range(l.groups)]
+                        if opts.opset >= 13:
+                            add_const(f"route{i}_split", np.full(l.groups, gc, np.int64))
+                            nodes.append(node_proto("Split", [src, f"route{i}_split"], outs, name=f"route{i}", axis=1))
+                        else:
+                            nodes.append(node_proto("Split", [src], outs, name=f"route{i}", packed=opts.packed_attrs, axis=1,
+                                                    split=[gc] * l.groups))
+                    else:
+                        raise ValueError(opts.split_op)
+                    cur, c, s = out, gc, spatial[idx[0]]
+                    x = acts[idx[0]][:, gc * l.group_id:gc * (l.group_id + 1)]
+                elif len(idx) == 1:
                     cur, c, s, x = names[idx[0]], chans[idx[0]], spatial[idx[0]], acts[idx[0]]
                 else:
                     out = f"concat{i}_out"
@@ -463,7 +520,7 @@ def build_onnx(arch: str, num_classes: int, size: int = 416, seed: int = 0,
             acts.append(x)
 
     graph = b"".join(_f_bytes(1, n) for n in nodes)
-    graph += _f_str(2, f"yolov3-{arch}")
+    graph += _f_str(2, "yolov4-tiny" if arch == "tiny4" else f"yolov3-{arch}")
     graph += b"".join(_f_bytes(5, t) for t in inits)
     graph += _f_bytes(11, value_info("input", (opts.batch, 3, size, size)))
     for name, shape in outputs:
