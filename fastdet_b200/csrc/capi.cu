@@ -88,12 +88,10 @@ struct Exec {  // everything that depends on the batch size
     Candidate* cand = nullptr;
     int* cand_count = nullptr;
     double* scores = nullptr;
-    Detection* dets = nullptr;
+    Detection* dets = nullptr;  // [n][max_det] of the batch being post-processed
+    size_t dets_cap = 0;
     int* det_count = nullptr;  // [2n]: truncated counts then totals
     double* thr = nullptr;     // per-frame thresholds of the batch being post-processed: thr[b], then float obj_cut[b] (b frames)
-    int max_det = 0;
-    Detection* h_dets = nullptr;  // pinned
-    int* h_count = nullptr;       // pinned [2n]
     float* scratch = nullptr;     // parity hooks
     size_t scratch_cap = 0;
     cudaGraphExec_t graph = nullptr;
@@ -108,7 +106,7 @@ struct Exec {  // everything that depends on the batch size
 
 }  // namespace
 
-struct Slot {  // one in-flight fd_submit: staged input + pinned results + the events that order them
+struct Slot {  // one batch's staged input + pinned results + the events that order them
     uint8_t* stage = nullptr;   // device staging for the H2D copy (copy stream)
     size_t stage_cap = 0;
     Detection* h_dets = nullptr;  // pinned
@@ -121,8 +119,8 @@ struct Slot {  // one in-flight fd_submit: staged input + pinned results + the e
     size_t h_thr_cap = 0;
     int thr_n = 0;                // frames h_thr holds
     cudaEvent_t thr_copied = nullptr;  // the last copy out of h_thr has run
-    cudaEvent_t staged = nullptr, stage_free = nullptr, done = nullptr;
-    int n = 0, max_det = 0;
+    cudaEvent_t staged = nullptr, stage_free = nullptr, done = nullptr;  // done: the last copy into h_dets / h_count has run
+    int n = 0, max_det = 0;  // of the results in h_dets / h_count (n = 0: none)
     bool busy = false;
 };
 
@@ -130,7 +128,7 @@ struct fd_model {
     int device = 0;
     int num_sms = 148;
     cudaStream_t copy_stream = nullptr;
-    Slot slots[FD_MAX_SLOTS + 1];  // the last one serves the synchronous JPEG calls and fd_postprocess
+    Slot slots[FD_MAX_SLOTS + 1];  // the last one serves the synchronous calls: fd_postprocess / fd_fetch and the JPEG calls
     std::unique_ptr<JpegPool> jpeg_pool;
     std::vector<JpegInfo> jpeg_info;
     uint8_t* jpeg_planes = nullptr;  // decoded component planes of the batch being converted (compute stream only)
@@ -144,8 +142,6 @@ struct fd_model {
     cudaEvent_t h2d_ev[8] = {nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr};  // fd_detect: pieces of the frame copy
     cudaEvent_t idle_ev = nullptr;  // end of the last forward pass on the compute stream (its input tensor may be overwritten)
     fd_info info;
-    int last_n = 0;
-    int last_max_det = 0;
 };
 
 namespace {
@@ -168,6 +164,45 @@ int sync_model_streams(fd_model* m) {
     return FD_OK;
 }
 
+// Grows *p to at least `bytes`: device memory, or (pinned != null) pinned host memory of that slot.  Growth is rare, so it runs
+// under the device's set-up lock, and before the old buffer is freed everything that may still use it drains: the model's two
+// streams and, for a slot's pinned buffer, the slot's `done` event (fd_postprocess copies into them on the caller's stream).
+template <class T>
+int grow(fd_model* m, T** p, size_t* cap, size_t bytes, const char* what, const Slot* pinned = nullptr) {
+    if (*cap >= bytes) return FD_OK;
+    DEVICE_SETUP_LOCK(m);
+    if (int rc = sync_model_streams(m)) return rc;
+    if (pinned) {
+        CU(cudaEventSynchronize(pinned->done));
+        cudaFreeHost(*p);
+    } else {
+        cudaFree(*p);
+    }
+    *p = nullptr;
+    *cap = 0;
+    void* q = nullptr;
+    const cudaError_t err = pinned ? cudaMallocHost(&q, bytes) : cudaMalloc(&q, bytes);
+    if (err != cudaSuccess)
+        return fail(FD_ERR_CUDA, "%s(%s, %zu bytes) failed: %s", pinned ? "cudaMallocHost" : "cudaMalloc", what, bytes, cudaGetErrorString(err));
+    *p = static_cast<T*>(q);
+    *cap = bytes;
+    return FD_OK;
+}
+
+// The copy stream and slot S's events, created on first use.
+int slot_setup(fd_model* m, Slot& S) {
+    if (m->copy_stream && S.staged) return FD_OK;
+    DEVICE_SETUP_LOCK(m);
+    if (!m->copy_stream) CU(cudaStreamCreateWithFlags(&m->copy_stream, cudaStreamNonBlocking));
+    if (!S.staged) {
+        CU(cudaEventCreateWithFlags(&S.staged, cudaEventDisableTiming));
+        CU(cudaEventCreateWithFlags(&S.stage_free, cudaEventDisableTiming));
+        CU(cudaEventCreateWithFlags(&S.done, cudaEventDisableTiming));
+        CU(cudaEventCreateWithFlags(&S.thr_copied, cudaEventDisableTiming));
+    }
+    return FD_OK;
+}
+
 size_t buf_bytes(const BufferPlan& b, int n) { return size_t(n) * b.h * b.w * b.pitch * (b.fp32 ? 4 : 2); }
 
 void free_exec(Exec* e) {
@@ -175,8 +210,6 @@ void free_exec(Exec* e) {
     cudaFree(e->splitk_ws); cudaFree(e->splitk_counters);
     cudaFree(e->frames); cudaFree(e->src); cudaFree(e->cand); cudaFree(e->cand_count); cudaFree(e->scores);
     cudaFree(e->dets); cudaFree(e->det_count); cudaFree(e->thr); cudaFree(e->scratch);
-    if (e->h_dets) cudaFreeHost(e->h_dets);
-    if (e->h_count) cudaFreeHost(e->h_count);
     if (e->graph) cudaGraphExecDestroy(e->graph);
     if (e->graph_tail) cudaGraphExecDestroy(e->graph_tail);
 }
@@ -402,7 +435,6 @@ int get_exec(fd_model* m, int n_frames, Exec** out) {
         cudaMalloc(&e->scores, sizeof(double) * size_t(n) * bpf) != cudaSuccess ||
         cudaMalloc(&e->det_count, sizeof(int) * 2 * n) != cudaSuccess ||
         cudaMalloc(&e->thr, (sizeof(double) + sizeof(float)) * n) != cudaSuccess ||
-        cudaMallocHost(&e->h_count, sizeof(int) * 2 * n) != cudaSuccess ||
         cudaMemset(e->frames, 0, frame_bytes) != cudaSuccess) {
         free_exec(e.get());
         return fail(FD_ERR_CUDA, "cudaMalloc(per-batch state, batch %d) failed: %s", n, cudaGetErrorString(cudaGetLastError()));
@@ -482,16 +514,55 @@ int launch_layers(fd_model* m, Exec* e, cudaStream_t s, int from_layer = 0) {
 
 cudaStream_t pick(fd_model* m, void* stream) { return stream ? static_cast<cudaStream_t>(stream) : m->stream; }
 
-int ensure_scratch(Exec* e, size_t bytes) {
-    if (e->scratch_cap >= bytes) return FD_OK;
-    int dev = 0;
-    cudaGetDevice(&dev);
-    std::lock_guard<std::recursive_mutex> lk(device_setup_mutex(dev));
-    cudaFree(e->scratch);
-    e->scratch = nullptr; e->scratch_cap = 0;
-    CU(cudaMalloc(&e->scratch, bytes));
-    e->scratch_cap = bytes;
+// frames of src_w x src_h: the network's size, or any size with allow_resize (the extension; the reference refuses them)
+int check_frame_size(const fd_model* m, int src_w, int src_h, int allow_resize) {
+    const bool same = src_w == m->plan.net_w && src_h == m->plan.net_h;
+    if (!same && !allow_resize) return fail(FD_ERR_SIZE, "invalid image size");  // reference detector.py:132
+    if (src_w < 1 || src_h < 1) return fail(FD_ERR_SIZE, "invalid image size");
     return FD_OK;
+}
+
+// u8 frames on the device at src_w x src_h -> the Exec's input tensor on stream s: copied when they are the network's size,
+// letterboxed otherwise
+int load_frames(fd_model* m, Exec* e, const uint8_t* src, int n, int src_w, int src_h, cudaStream_t s) {
+    const ModelPlan& P = m->plan;
+    if (src_w == P.net_w && src_h == P.net_h) {
+        CU(cudaMemcpyAsync(e->frames, src, size_t(n) * src_w * src_h * 3, cudaMemcpyDeviceToDevice, s));
+    } else if (launch_letterbox_u8(src, e->frames, n, src_h, src_w, P.net_h, P.net_w, 128, s)) {
+        return fail(FD_ERR_CUDA, "letterbox launch failed: %s", cudaGetErrorString(cudaGetLastError()));
+    }
+    return FD_OK;
+}
+
+// common front of everything that post-processes into a slot (fd_postprocess, fd_submit, the JPEG calls): argument
+// checks, the Exec of this batch size, the slot's events and its result buffers, grown for n frames of max_det records
+int slot_begin(fd_model* m, int slot, int n, int max_det, Exec** e_out, Slot** s_out) {
+    const fd_info& I = m->info;
+    if (I.n_heads != 2 && I.n_heads != 3) return fail(FD_ERR_HEADS, "%d", I.n_heads);  // KeyError(len(outputs)) in the reference
+    if (max_det < 1) return fail(FD_ERR_ARG, "max_det must be >= 1");
+    NEED_DEVICE(m);
+    CU(cudaSetDevice(m->device));
+    Slot& S = m->slots[slot];
+    if (S.busy) return fail(FD_ERR_ARG, "slot %d still holds uncollected results", slot);
+    S.n = 0;  // its results are about to be overwritten
+    Exec* e;
+    if (int rc = get_exec(m, n, &e)) return rc;
+    if (int rc = slot_setup(m, S)) return rc;
+    if (int rc = grow(m, &S.h_dets, &S.h_dets_cap, sizeof(Detection) * size_t(n) * max_det, "pinned records", &S)) return rc;
+    if (int rc = grow(m, &S.h_count, &S.h_count_cap, sizeof(int) * 2 * size_t(n), "pinned record counts", &S)) return rc;
+    if (int rc = grow(m, &e->dets, &e->dets_cap, sizeof(Detection) * size_t(e->n) * max_det, "records")) return rc;
+    *e_out = e;
+    *s_out = &S;
+    return FD_OK;
+}
+
+// the slot's results as fd_fetch / fd_collect return them: counts[n], out[n][max_det] and (total != null) total[n]
+void copy_records(const Slot& S, fd_det* out, int32_t* counts, int32_t* total) {
+    for (int f = 0; f < S.n; ++f) {
+        counts[f] = S.h_count[f];
+        if (total) total[f] = S.h_count[S.n + f];
+        memcpy(out + size_t(f) * S.max_det, S.h_dets + size_t(f) * S.max_det, sizeof(fd_det) * size_t(S.h_count[f]));
+    }
 }
 
 }  // namespace
@@ -607,8 +678,8 @@ void fd_model_destroy(fd_model* m) {
         if (S.h_dets) cudaFreeHost(S.h_dets);
         if (S.h_count) cudaFreeHost(S.h_count);
         if (S.h_thr) cudaFreeHost(S.h_thr);
-        if (S.thr_copied) cudaEventDestroy(S.thr_copied);
-        if (S.staged) { cudaEventDestroy(S.staged); cudaEventDestroy(S.stage_free); cudaEventDestroy(S.done); }
+        for (cudaEvent_t ev : {S.staged, S.stage_free, S.done, S.thr_copied})
+            if (ev) cudaEventDestroy(ev);
     }
     cudaFree(m->jpeg_planes);
     if (m->idle_ev) { cudaEventDestroy(m->idle_ev); for (cudaEvent_t ev : m->h2d_ev) cudaEventDestroy(ev); }
@@ -729,36 +800,21 @@ int fd_get_option(const char* name, int* value) {
 
 int fd_preprocess(fd_model* m, const uint8_t* frames, int n, int src_w, int src_h, int on_device, int allow_resize, void* stream) {
     if (!m || !frames) return fail(FD_ERR_ARG, "fd_preprocess: null argument");
-    const ModelPlan& P = m->plan;
-    const bool same = src_w == P.net_w && src_h == P.net_h;
-    if (!same && !allow_resize) return fail(FD_ERR_SIZE, "invalid image size");  // reference detector.py:132
-    if (src_w < 1 || src_h < 1) return fail(FD_ERR_SIZE, "invalid image size");
+    if (int rc = check_frame_size(m, src_w, src_h, allow_resize)) return rc;
     NEED_DEVICE(m);
     CU(cudaSetDevice(m->device));
     Exec* e;
     if (int rc = get_exec(m, n, &e)) return rc;
     cudaStream_t s = pick(m, stream);
+    if (on_device) return load_frames(m, e, frames, n, src_w, src_h, s);
     const size_t bytes = size_t(n) * src_w * src_h * 3;
-    const cudaMemcpyKind kind = on_device ? cudaMemcpyDeviceToDevice : cudaMemcpyHostToDevice;
-    if (same) {
-        CU(cudaMemcpyAsync(e->frames, frames, bytes, kind, s));
-    } else {
-        const uint8_t* src = frames;
-        if (!on_device) {
-            if (e->src_cap < bytes) {
-                DEVICE_SETUP_LOCK(m);
-                if (int rc = sync_model_streams(m)) return rc;
-                cudaFree(e->src); e->src = nullptr; e->src_cap = 0;
-                CU(cudaMalloc(&e->src, bytes));
-                e->src_cap = bytes;
-            }
-            CU(cudaMemcpyAsync(e->src, frames, bytes, cudaMemcpyHostToDevice, s));
-            src = e->src;
-        }
-        if (launch_letterbox_u8(src, e->frames, n, src_h, src_w, P.net_h, P.net_w, 128, s))
-            return fail(FD_ERR_CUDA, "letterbox launch failed: %s", cudaGetErrorString(cudaGetLastError()));
+    if (src_w == m->plan.net_w && src_h == m->plan.net_h) {  // straight into the input tensor
+        CU(cudaMemcpyAsync(e->frames, frames, bytes, cudaMemcpyHostToDevice, s));
+        return FD_OK;
     }
-    return FD_OK;
+    if (int rc = grow(m, &e->src, &e->src_cap, bytes, "letterbox source")) return rc;
+    CU(cudaMemcpyAsync(e->src, frames, bytes, cudaMemcpyHostToDevice, s));
+    return load_frames(m, e, e->src, n, src_w, src_h, s);
 }
 
 // the layers from `from_layer` on as an instantiated CUDA graph (nullptr if capture is not possible: callers then launch directly)
@@ -785,7 +841,6 @@ int fd_forward(fd_model* m, int n, void* stream) {
     Exec* e;
     if (int rc = get_exec(m, n, &e)) return rc;
     cudaStream_t s = pick(m, stream);
-    m->last_n = n;
     if (!e->graph_tried) {
         e->graph_tried = true;
         e->graph = capture_layers(m, e, 0);
@@ -802,19 +857,10 @@ int fd_forward(fd_model* m, int n, void* stream) {
 // a repeat at the same thresholds (fd_postprocess in a loop) rewrites nothing and never waits.
 static int stage_thresholds(fd_model* m, Exec* e, Slot& T, int n, const double* thr, cudaStream_t s) {
     const size_t bytes = (sizeof(double) + sizeof(float)) * size_t(n);
-    if (!T.thr_copied) {
-        DEVICE_SETUP_LOCK(m);
-        CU(cudaEventCreateWithFlags(&T.thr_copied, cudaEventDisableTiming));
-    }
     if (T.thr_n != n || memcmp(T.h_thr, thr, sizeof(double) * size_t(n)) != 0) {
         CU(cudaEventSynchronize(T.thr_copied));
-        if (T.h_thr_cap < bytes) {
-            DEVICE_SETUP_LOCK(m);
-            if (T.h_thr) cudaFreeHost(T.h_thr);
-            T.h_thr = nullptr; T.h_thr_cap = 0; T.thr_n = 0;
-            CU(cudaMallocHost(&T.h_thr, bytes));
-            T.h_thr_cap = bytes;
-        }
+        T.thr_n = 0;
+        if (int rc = grow(m, &T.h_thr, &T.h_thr_cap, bytes, "pinned thresholds", &T)) return rc;
         double* h = reinterpret_cast<double*>(T.h_thr);
         float* cut = reinterpret_cast<float*>(h + n);
         for (int f = 0; f < n; ++f) { h[f] = thr[f]; cut[f] = obj_cut_for(thr[f]); }
@@ -825,12 +871,11 @@ static int stage_thresholds(fd_model* m, Exec* e, Slot& T, int n, const double* 
     return FD_OK;
 }
 
-// decode + Soft-NMS on the head tensors, frame f at threshold thr[f] (host array, staged through slot T), then the records to
-// pinned host memory (h_dets / h_count) on stream s
-static int postprocess_on(fd_model* m, Exec* e, Slot& T, int n, const double* thr, int max_det, cudaStream_t s, Detection* h_dets,
-                          int* h_count) {
+// decode + Soft-NMS on the head tensors, frame f at threshold thr[f] (host array, staged through slot S), then the records to
+// S's pinned buffers and S's `done` event on stream s
+static int postprocess_on(fd_model* m, Exec* e, Slot& S, int n, const double* thr, int max_det, cudaStream_t s) {
     const fd_info& I = m->info;
-    if (int rc = stage_thresholds(m, e, T, n, thr, s)) return rc;
+    if (int rc = stage_thresholds(m, e, S, n, thr, s)) return rc;
     const double* d_thr = e->thr;
     const float* d_cut = reinterpret_cast<const float*>(e->thr + n);
     HeadDesc heads[FD_MAX_HEADS];
@@ -848,8 +893,11 @@ static int postprocess_on(fd_model* m, Exec* e, Slot& T, int n, const double* th
     if (launch_soft_nms(e->cand, e->cand_count, e->scores, I.boxes_per_frame, n, I.net_w, I.net_h, d_thr, e->dets,
                         e->det_count, e->det_count + n, max_det, s))
         return fail(FD_ERR_CUDA, "soft-nms launch failed: %s", cudaGetErrorString(cudaGetLastError()));
-    CU(cudaMemcpyAsync(h_count, e->det_count, sizeof(int) * 2 * n, cudaMemcpyDeviceToHost, s));
-    CU(cudaMemcpyAsync(h_dets, e->dets, sizeof(Detection) * size_t(n) * max_det, cudaMemcpyDeviceToHost, s));
+    CU(cudaMemcpyAsync(S.h_count, e->det_count, sizeof(int) * 2 * n, cudaMemcpyDeviceToHost, s));
+    CU(cudaMemcpyAsync(S.h_dets, e->dets, sizeof(Detection) * size_t(n) * max_det, cudaMemcpyDeviceToHost, s));
+    CU(cudaEventRecord(S.done, s));
+    S.n = n;
+    S.max_det = max_det;
     return FD_OK;
 }
 
@@ -862,45 +910,22 @@ int fd_postprocess(fd_model* m, int n, double threshold, int max_det, void* stre
 
 int fd_postprocess_thresholds(fd_model* m, int n, const double* thresholds, int max_det, void* stream) {
     if (!m || !thresholds) return fail(FD_ERR_ARG, "fd_postprocess: null argument");
-    const fd_info& I = m->info;
-    if (I.n_heads != 2 && I.n_heads != 3) return fail(FD_ERR_HEADS, "%d", I.n_heads);  // KeyError(len(outputs)) in the reference
-    if (max_det < 1) return fail(FD_ERR_ARG, "max_det must be >= 1");
-    NEED_DEVICE(m);
-    CU(cudaSetDevice(m->device));
     Exec* e;
-    if (int rc = get_exec(m, n, &e)) return rc;
-    cudaStream_t s = pick(m, stream);
-    if (e->max_det != max_det || !e->h_dets) {
-        DEVICE_SETUP_LOCK(m);
-        if (int rc = sync_model_streams(m)) return rc;  // (rare) the record buffers may be in use on the compute or the copy stream
-        cudaFree(e->dets); e->dets = nullptr;
-        if (e->h_dets) { cudaFreeHost(e->h_dets); e->h_dets = nullptr; }
-        CU(cudaMalloc(&e->dets, sizeof(Detection) * size_t(e->n) * max_det));
-        CU(cudaMallocHost(&e->h_dets, sizeof(Detection) * size_t(e->n) * max_det));
-        e->max_det = max_det;
-    }
-    // results to pinned host memory on the same stream; fd_fetch synchronises
-    if (int rc = postprocess_on(m, e, m->slots[FD_MAX_SLOTS], n, thresholds, max_det, s, e->h_dets, e->h_count)) return rc;
-    m->last_n = n;
-    m->last_max_det = max_det;
-    return FD_OK;
+    Slot* sp;
+    if (int rc = slot_begin(m, FD_MAX_SLOTS, n, max_det, &e, &sp)) return rc;
+    // results to the synchronous slot's pinned buffers on the caller's stream; fd_fetch synchronises it.  The slot is not
+    // marked busy: a caller may post-process batch after batch and fetch only the last.
+    return postprocess_on(m, e, *sp, n, thresholds, max_det, pick(m, stream));
 }
 
 int fd_fetch(fd_model* m, int n, fd_det* out, int32_t* counts, int32_t* total, void* stream) {
     if (!m || !out || !counts) return fail(FD_ERR_ARG, "fd_fetch: null argument");
-    auto it = m->execs.find(bucket_of(n));
-    if (n < 1 || it == m->execs.end() || !it->second->h_dets)
-        return fail(FD_ERR_ARG, "fd_fetch: no postprocess results for batch %d", n);
-    Exec* e = it->second.get();
+    const Slot& S = m->slots[FD_MAX_SLOTS];
+    if (n < 1 || n != S.n) return fail(FD_ERR_ARG, "fd_fetch: no postprocess results for batch %d (the last post-process had %d frames)", n, S.n);
     NEED_DEVICE(m);
     CU(cudaSetDevice(m->device));
     CU(cudaStreamSynchronize(pick(m, stream)));
-    const int md = m->last_max_det;
-    for (int f = 0; f < n; ++f) {
-        counts[f] = e->h_count[f];
-        if (total) total[f] = e->h_count[n + f];
-        memcpy(out + size_t(f) * md, e->h_dets + size_t(f) * md, sizeof(fd_det) * size_t(e->h_count[f]));
-    }
+    copy_records(S, out, counts, total);
     return FD_OK;
 }
 
@@ -938,7 +963,7 @@ static int build_overlap_plan(fd_model* m, Exec* e) {
 static int forward_overlapping_copy(fd_model* m, Exec* e, const uint8_t* frames, int n) {
     const ModelPlan& P = m->plan;
     cudaStream_t s = m->stream;
-    if (!m->copy_stream) CU(cudaStreamCreateWithFlags(&m->copy_stream, cudaStreamNonBlocking));
+    if (int rc = slot_setup(m, m->slots[FD_MAX_SLOTS])) return rc;  // the copy stream (fd_detect's records then land in that slot)
     if (!m->idle_ev) {
         CU(cudaEventCreateWithFlags(&m->idle_ev, cudaEventDisableTiming));
         for (cudaEvent_t& ev : m->h2d_ev) CU(cudaEventCreateWithFlags(&ev, cudaEventDisableTiming));
@@ -962,7 +987,6 @@ static int forward_overlapping_copy(fd_model* m, Exec* e, const uint8_t* frames,
         e->graph_tail_tried = true;
         e->graph_tail = capture_layers(m, e, e->ov_layers);
     }
-    m->last_n = n;
     if (e->graph_tail) {
         CU(cudaGraphLaunch(e->graph_tail, s));
         return FD_OK;
@@ -1005,83 +1029,11 @@ int quiesce_after_failure(fd_model* m, int rc) {
     return rc;
 }
 
-int slot_begin_resize(fd_model* m, Exec* e, Slot& S, int n, int max_det, Exec** e_out, Slot** s_out);
-
-// common front of fd_submit / fd_submit_jpeg: argument checks, the Exec of this batch size, the slot's events and
-// pinned result buffers
-int slot_begin(fd_model* m, int slot, int n, int max_det, Exec** e_out, Slot** s_out) {
-    const fd_info& I = m->info;
-    if (I.n_heads != 2 && I.n_heads != 3) return fail(FD_ERR_HEADS, "%d", I.n_heads);
-    if (max_det < 1) return fail(FD_ERR_ARG, "max_det must be >= 1");
-    NEED_DEVICE(m);
-    CU(cudaSetDevice(m->device));
-    Slot& S = m->slots[slot];
-    if (S.busy) return fail(FD_ERR_ARG, "slot %d still holds uncollected results", slot);
-    Exec* e;
-    if (int rc = get_exec(m, n, &e)) return rc;
-    if (!m->copy_stream || !S.staged) {
-        DEVICE_SETUP_LOCK(m);
-        if (!m->copy_stream) CU(cudaStreamCreateWithFlags(&m->copy_stream, cudaStreamNonBlocking));
-        if (!S.staged) {
-            CU(cudaEventCreateWithFlags(&S.staged, cudaEventDisableTiming));
-            CU(cudaEventCreateWithFlags(&S.stage_free, cudaEventDisableTiming));
-            CU(cudaEventCreateWithFlags(&S.done, cudaEventDisableTiming));
-        }
-    }
-    if (S.h_dets_cap < sizeof(Detection) * size_t(n) * max_det || S.h_count_cap < sizeof(int) * 2 * size_t(n) || e->max_det != max_det) {
-        DEVICE_SETUP_LOCK(m);
-        return slot_begin_resize(m, e, S, n, max_det, e_out, s_out);
-    }
-    *e_out = e;
-    *s_out = &S;
-    return FD_OK;
-}
-
-// (rare) the slot's pinned result buffers or the Exec's record buffer have to grow: under the device's set-up lock
-int slot_begin_resize(fd_model* m, Exec* e, Slot& S, int n, int max_det, Exec** e_out, Slot** s_out) {
-    const size_t det_bytes = sizeof(Detection) * size_t(n) * max_det, cnt_bytes = sizeof(int) * 2 * size_t(n);
-    if (S.h_dets_cap < det_bytes) {
-        if (S.h_dets) cudaFreeHost(S.h_dets);
-        S.h_dets = nullptr; S.h_dets_cap = 0;
-        CU(cudaMallocHost(&S.h_dets, det_bytes));
-        S.h_dets_cap = det_bytes;
-    }
-    if (S.h_count_cap < cnt_bytes) {
-        if (S.h_count) cudaFreeHost(S.h_count);
-        S.h_count = nullptr; S.h_count_cap = 0;
-        CU(cudaMallocHost(&S.h_count, cnt_bytes));
-        S.h_count_cap = cnt_bytes;
-    }
-    if (e->max_det != max_det) {
-        if (int rc = sync_model_streams(m)) return rc;  // the record buffers may be in use on the compute or the copy stream
-        cudaFree(e->dets); e->dets = nullptr;
-        if (e->h_dets) { cudaFreeHost(e->h_dets); e->h_dets = nullptr; }
-        CU(cudaMalloc(&e->dets, sizeof(Detection) * size_t(e->n) * max_det));
-        e->max_det = max_det;
-    }
-    *e_out = e;
-    *s_out = &S;
-    return FD_OK;
-}
-
-int slot_stage_reserve(fd_model* m, Slot& S, size_t bytes) {
-    if (S.stage_cap >= bytes) return FD_OK;
-    DEVICE_SETUP_LOCK(m);
-    if (int rc = sync_model_streams(m)) return rc;
-    cudaFree(S.stage); S.stage = nullptr; S.stage_cap = 0;
-    CU(cudaMalloc(&S.stage, bytes));
-    S.stage_cap = bytes;
-    return FD_OK;
-}
-
-// common tail: the conv stack, decode + Soft-NMS (frame f at threshold thr[f]), results into the slot's pinned buffers, the
-// `done` event
+// common tail: the conv stack, decode + Soft-NMS (frame f at threshold thr[f]), results into the slot's pinned buffers
 int slot_finish(fd_model* m, Exec* e, Slot& S, int n, const double* thr, int max_det) {
-    cudaStream_t s = m->stream;
     if (int rc = fd_forward(m, n, nullptr)) return rc;
-    if (int rc = postprocess_on(m, e, S, n, thr, max_det, s, S.h_dets, S.h_count)) return rc;
-    CU(cudaEventRecord(S.done, s));
-    S.n = n; S.max_det = max_det; S.busy = true;
+    if (int rc = postprocess_on(m, e, S, n, thr, max_det, m->stream)) return rc;
+    S.busy = true;
     return FD_OK;
 }
 
@@ -1089,11 +1041,7 @@ int slot_collect(fd_model* m, Slot& S, fd_det* out, int32_t* counts, int32_t* to
     CU(cudaSetDevice(m->device));
     S.busy = false;
     CU(cudaEventSynchronize(S.done));
-    for (int f = 0; f < S.n; ++f) {
-        counts[f] = S.h_count[f];
-        if (total) total[f] = S.h_count[S.n + f];
-        memcpy(out + size_t(f) * S.max_det, S.h_dets + size_t(f) * S.max_det, sizeof(fd_det) * size_t(S.h_count[f]));
-    }
+    copy_records(S, out, counts, total);
     return FD_OK;
 }
 
@@ -1150,16 +1098,8 @@ int jpeg_host_stage(fd_model* m, Slot& S, const uint8_t* const* data, const size
         max_blocks = std::max(max_blocks, static_cast<int>(count / 64));
     }
     if (off[n] > 0xffffffffull * 2) return fail(FD_ERR_ARG, "JPEG batch too large");
-    if (S.h_stage_cap < off[n]) {
-        DEVICE_SETUP_LOCK(m);
-        if (S.h_stage) {
-            CU(cudaStreamSynchronize(m->copy_stream));
-            cudaFreeHost(S.h_stage);
-        }
-        S.h_stage = nullptr; S.h_stage_cap = 0;
-        CU(cudaMallocHost(&S.h_stage, off[n] + off[n] / 4));
-        S.h_stage_cap = off[n] + off[n] / 4;
-    }
+    if (S.h_stage_cap < off[n])  // with a quarter to spare: batches of similar JPEGs then do not regrow it one by one
+        if (int rc = grow(m, &S.h_stage, &S.h_stage_cap, off[n] + off[n] / 4, "pinned JPEG staging", &S)) return rc;
     char* base = S.h_stage;
     m->jpeg_pool->run(n, [&](int i) {
         char buf[160] = "";
@@ -1184,28 +1124,14 @@ using ByteRuns = std::vector<std::pair<size_t, size_t>>;
 int jpeg_device_stage(fd_model* m, Exec* e, Slot& S, const char* src, size_t head, const ByteRuns& runs, int n, int max_blocks,
                       int src_w, int src_h) {
     const ModelPlan& P = m->plan;
-    if (int rc = slot_stage_reserve(m, S, runs.back().second)) return rc;
+    if (int rc = grow(m, &S.stage, &S.stage_cap, runs.back().second, "JPEG staging")) return rc;
     const bool same = src_w == P.net_w && src_h == P.net_h;
     const size_t plane_stride = size_t(3) * ((src_w + 15) / 16 * 16) * ((src_h + 15) / 16 * 16);
-    uint8_t* rgb = e->frames;
-    if (!same) {  // decode at the source size, then the letterbox of fd_preprocess
-        const size_t src_bytes = size_t(n) * src_w * src_h * 3;
-        if (e->src_cap < src_bytes) {
-            DEVICE_SETUP_LOCK(m);
-            if (int rc = sync_model_streams(m)) return rc;
-            cudaFree(e->src); e->src = nullptr; e->src_cap = 0;
-            CU(cudaMalloc(&e->src, src_bytes));
-            e->src_cap = src_bytes;
-        }
-        rgb = e->src;
-    }
-    if (m->jpeg_planes_cap < plane_stride * n) {
-        DEVICE_SETUP_LOCK(m);
-        if (int rc = sync_model_streams(m)) return rc;
-        cudaFree(m->jpeg_planes); m->jpeg_planes = nullptr; m->jpeg_planes_cap = 0;
-        CU(cudaMalloc(&m->jpeg_planes, plane_stride * n));
-        m->jpeg_planes_cap = plane_stride * n;
-    }
+    // frames of another size are decoded at the source size, then letterboxed
+    if (!same)
+        if (int rc = grow(m, &e->src, &e->src_cap, size_t(n) * src_w * src_h * 3, "letterbox source")) return rc;
+    uint8_t* rgb = same ? e->frames : e->src;
+    if (int rc = grow(m, &m->jpeg_planes, &m->jpeg_planes_cap, plane_stride * n, "JPEG planes")) return rc;
     cudaStream_t cs = m->copy_stream, s = m->stream;
     CU(cudaStreamWaitEvent(cs, S.stage_free, 0));
     for (const auto& r : runs) CU(cudaMemcpyAsync(S.stage + r.first, src + r.first, r.second - r.first, cudaMemcpyHostToDevice, cs));
@@ -1217,8 +1143,8 @@ int jpeg_device_stage(fd_model* m, Exec* e, Slot& S, const char* src, size_t hea
         return fail(FD_ERR_CUDA, "JPEG kernel launch failed: %s", cudaGetErrorString(cudaGetLastError()));
     if (launch_jpeg_rgb(m->jpeg_planes, plane_stride, fr, rgb, n, src_h, src_w, s))
         return fail(FD_ERR_CUDA, "JPEG kernel launch failed: %s", cudaGetErrorString(cudaGetLastError()));
-    if (!same && launch_letterbox_u8(rgb, e->frames, n, src_h, src_w, P.net_h, P.net_w, 128, s))
-        return fail(FD_ERR_CUDA, "letterbox launch failed: %s", cudaGetErrorString(cudaGetLastError()));
+    if (!same)  // (frames of the network's size were decoded straight into the input tensor: no copy)
+        if (int rc = load_frames(m, e, rgb, n, src_w, src_h, s)) return rc;
     CU(cudaEventRecord(S.stage_free, s));
     return FD_OK;
 }
@@ -1233,16 +1159,13 @@ int fd_submit(fd_model* m, int slot, const uint8_t* frames, int n, int src_w, in
               double threshold, int max_det) {
     if (!m || !frames) return fail(FD_ERR_ARG, "fd_submit: null argument");
     if (slot < 0 || slot >= FD_MAX_SLOTS) return fail(FD_ERR_ARG, "fd_submit: slot %d out of range [0, %d)", slot, FD_MAX_SLOTS);
-    const ModelPlan& P = m->plan;
-    const bool same = src_w == P.net_w && src_h == P.net_h;
-    if (!same && !allow_resize) return fail(FD_ERR_SIZE, "invalid image size");  // reference detector.py:132
-    if (src_w < 1 || src_h < 1) return fail(FD_ERR_SIZE, "invalid image size");
+    if (int rc = check_frame_size(m, src_w, src_h, allow_resize)) return rc;
     Exec* e;
     Slot* sp;
     if (int rc = slot_begin(m, slot, n, max_det, &e, &sp)) return rc;
     Slot& S = *sp;
     const size_t bytes = size_t(n) * src_w * src_h * 3;
-    if (int rc = slot_stage_reserve(m, S, bytes)) return rc;
+    if (int rc = grow(m, &S.stage, &S.stage_cap, bytes, "frame staging")) return rc;
     cudaStream_t cs = m->copy_stream, s = m->stream;
     // copy stream: wait until the compute stream has consumed this slot's previous contents, then stage the frames
     CU(cudaStreamWaitEvent(cs, S.stage_free, 0));
@@ -1250,11 +1173,7 @@ int fd_submit(fd_model* m, int slot, const uint8_t* frames, int n, int src_w, in
     CU(cudaEventRecord(S.staged, cs));
     // compute stream: staged frames -> the Exec's input tensor (33 MB device copy at bs64, ~10 us), then the batch
     CU(cudaStreamWaitEvent(s, S.staged, 0));
-    if (same) {
-        CU(cudaMemcpyAsync(e->frames, S.stage, bytes, cudaMemcpyDeviceToDevice, s));
-    } else if (launch_letterbox_u8(S.stage, e->frames, n, src_h, src_w, P.net_h, P.net_w, 128, s)) {
-        return fail(FD_ERR_CUDA, "letterbox launch failed: %s", cudaGetErrorString(cudaGetLastError()));
-    }
+    if (int rc = load_frames(m, e, S.stage, n, src_w, src_h, s)) return rc;
     CU(cudaEventRecord(S.stage_free, s));
     const std::vector<double> thr(n, threshold);
     if (int rc = slot_finish(m, e, S, n, thr.data(), max_det)) return quiesce_after_failure(m, rc);
@@ -1344,12 +1263,7 @@ int fd_decode_jpeg(fd_model* m, const uint8_t* const* data, const size_t* lens, 
     Slot& S = m->slots[FD_MAX_SLOTS];
     Exec* e;
     if (int rc = get_exec(m, n, &e)) return rc;
-    if (!m->copy_stream) CU(cudaStreamCreateWithFlags(&m->copy_stream, cudaStreamNonBlocking));
-    if (!S.staged) {
-        CU(cudaEventCreateWithFlags(&S.staged, cudaEventDisableTiming));
-        CU(cudaEventCreateWithFlags(&S.stage_free, cudaEventDisableTiming));
-        CU(cudaEventCreateWithFlags(&S.done, cudaEventDisableTiming));
-    }
+    if (int rc = slot_setup(m, S)) return rc;
     size_t bytes = 0;
     int max_blocks = 0, sw = 0, sh = 0;
     if (int rc = jpeg_host_stage(m, S, data, lens, n, allow_resize, status, &bytes, &max_blocks, &sw, &sh)) return rc;
@@ -1387,7 +1301,9 @@ int fd_detect_jpeg(fd_model* m, const uint8_t* const* data, const size_t* lens, 
     if (int rc = jpeg_device_stage(m, e, *sp, sp->h_stage, jpeg_head_bytes(n), ByteRuns{{0, bytes}}, n, max_blocks, sw, sh)) return quiesce_after_failure(m, rc);
     const std::vector<double> thr(n, threshold);
     if (int rc = slot_finish(m, e, *sp, n, thr.data(), max_det)) return quiesce_after_failure(m, rc);
-    return slot_collect(m, *sp, out, counts, nullptr);
+    const int rc = slot_collect(m, *sp, out, counts, nullptr);
+    sp->n = 0;  // these records replaced the last fd_postprocess's but are not fd_fetch's to return
+    return rc;
 }
 
 // ------------------------------------------------------------------ letterbox geometry (extension, SURVEY 8f rank 4)
@@ -1474,7 +1390,7 @@ static int launch_unfused(fd_model* m, Exec* e, int layer) {
 
 static int tensor_to_host_nchw(fd_model* m, Exec* e, int layer, const TensorLoc& t, bool fp32, float* dst, int n) {
     const size_t elems = size_t(n) * t.c * t.h * t.w;
-    if (int rc = ensure_scratch(e, elems * 4)) return rc;
+    if (int rc = grow(m, &e->scratch, &e->scratch_cap, elems * 4, "parity scratch")) return rc;
     if (e->fused_role[layer] == 1) {
         if (int rc = ensure_fused_away_buffer(m, e, layer)) return rc;
         if (int rc = launch_unfused(m, e, layer)) return rc;
@@ -1504,7 +1420,7 @@ int fd_set_heads_fp32(fd_model* m, int head, const float* src, int n) {
     if (int rc = get_exec(m, n, &e)) return rc;
     const TensorLoc& t = m->plan.layers[m->plan.head_layers[head]].out;
     const size_t elems = size_t(n) * t.c * t.h * t.w;
-    if (int rc = ensure_scratch(e, elems * 4)) return rc;
+    if (int rc = grow(m, &e->scratch, &e->scratch_cap, elems * 4, "parity scratch")) return rc;
     CU(cudaDeviceSynchronize());
     // same stream as the layout kernel: a plain cudaMemcpy from pageable memory may return before its DMA lands
     CU(cudaMemcpyAsync(e->scratch, src, elems * 4, cudaMemcpyHostToDevice, m->stream));

@@ -137,14 +137,17 @@ int fd_preprocess(fd_model* m, const uint8_t* frames, int n, int src_w, int src_
                   void* stream);
 /* Run the conv stack on the staged frames (captured CUDA graph per batch size). */
 int fd_forward(fd_model* m, int n, void* stream);
-/* Decode + Soft-NMS on the head tensors of the last fd_forward.  Results land in device/pinned buffers owned by
- * the model; fd_fetch copies them out.  threshold is the reference's `threshold` (a Python float). */
+/* Decode + Soft-NMS on the head tensors of the last fd_forward.  Results land in the pinned buffers of the model's
+ * synchronous slot, replacing the previous post-process's; fd_fetch copies them out.  threshold is the reference's
+ * `threshold` (a Python float). */
 int fd_postprocess(fd_model* m, int n, double threshold, int max_det, void* stream);
 /* fd_postprocess with one threshold per frame (thresholds[n], host memory; read before the call returns).  Frame f's
  * records are bit for bit those of fd_postprocess at thresholds[f]. */
 int fd_postprocess_thresholds(fd_model* m, int n, const double* thresholds, int max_det, void* stream);
 /* Synchronise `stream` and copy the results of the last fd_postprocess: counts[n] and out[n][max_det]
- * (max_det as given to fd_postprocess).  total[n] (optional) receives the untruncated kept count. */
+ * (max_det as given to fd_postprocess).  total[n] (optional) receives the untruncated kept count.  n must be the n
+ * of that fd_postprocess, and no fd_detect_jpeg may have run since (its records replace the post-process's in the
+ * synchronous slot); FD_ERR_ARG otherwise. */
 int fd_fetch(fd_model* m, int n, fd_det* out, int32_t* counts, int32_t* total, void* stream);
 /* preprocess -> forward -> postprocess -> fetch; synchronous; frames in host (or device) memory. */
 int fd_detect(fd_model* m, const uint8_t* frames, int n, int src_w, int src_h, int on_device, int allow_resize,

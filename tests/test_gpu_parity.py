@@ -290,6 +290,27 @@ def test_post_truncation_and_empty():
             m.postprocess(1, 0.1, max_det=16)
         _, counts, total = m.fetch(1)
         assert counts[0] == 0 and total[0] == 0, nms
+    # fetch returns the records of the last post-process only: a smaller batch post-processed before it (at another
+    # max_det) is refused, not read at the last batch's record stride
+    m.set_heads([np.repeat(h, 2, axis=0) for h in heads])
+    m.postprocess(2, 0.1, max_det=5)
+    m.set_heads([np.repeat(h, 8, axis=0) for h in heads])
+    m.postprocess(8, 0.1, max_det=16)
+    with pytest.raises(_native.NativeError) as err:
+        m.fetch(2)
+    assert err.value.code == _native.FD_ERR_ARG
+    dets, counts, total = m.fetch(8)
+    assert (counts == min(16, len(z["results"]))).all() and (total == len(z["results"])).all()
+    np.testing.assert_allclose(dets[:, :5]["conf"], np.tile(z["results"][:5, 1], (8, 1)), rtol=1e-12)
+    # the synchronous JPEG call writes its own records (at its own max_det) into the same pinned buffers: fetch, which
+    # returns only a post-process's records, then refuses even at the same n
+    from PIL import Image
+    buf = io.BytesIO()
+    Image.fromarray(modelgen.synthetic_frame(200, 416), "RGB").save(buf, format="JPEG", quality=80)
+    m.detect_jpeg([buf.getvalue()] * 8, 0.1)
+    with pytest.raises(_native.NativeError) as err:
+        m.fetch(8)
+    assert err.value.code == _native.FD_ERR_ARG
 
 
 # ------------------------------------------------------------------ conv stack vs the fp32 oracle
