@@ -56,7 +56,7 @@ class FdLayerExec(C.Structure):
 
 
 KERNEL_NAMES = {0: "conv0", 1: "tc_single", 2: "tc_pair", 3: "tc_pair_strip", 4: "tc_swapped", 5: "halo", 6: "maxpool",
-                7: "copy", 8: "stem", 9: "fused_next", 10: "block"}
+                7: "copy", 8: "stem", 9: "fused_next", 10: "block", 11: "spp"}
 
 
 FD_SERVER_MAX_MODELS, FD_SERVER_MAX_DEVICES = 8, 16

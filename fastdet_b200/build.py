@@ -17,7 +17,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libfastdet_b200.so")
 SOURCES = ["capi.cu", "conv_tc.cu", "conv_halo.cu", "conv_stem.cu", "conv_block.cu", "jpeg.cu", "pre.cu", "pool.cu", "post.cu", "plan.cc", "onnx_reader.cc", "options.cc", "server.cc"]
-HEADERS = ["conv_tc.h", "conv_halo.h", "conv_stem.h", "conv_block.h", "kernels.h", "jpeg.h", "plan.h", "onnx_reader.h", "options.h", "ptx.cuh", os.path.join("..", "..", "include", "fastdet_b200.h")]
+HEADERS = ["conv_tc.h", "conv_halo.h", "conv_stem.h", "conv_block.h", "kernels.h", "jpeg.h", "plan.h", "onnx_reader.h", "options.h", "ptx.cuh", "act.cuh", os.path.join("..", "..", "include", "fastdet_b200.h")]
 ARCH = ["-gencode", "arch=compute_100a,code=sm_100a"]
 
 

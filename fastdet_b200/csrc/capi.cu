@@ -469,6 +469,20 @@ int launch_own(fd_model* m, Exec* e, int i, int k, int frames, bool halo, const 
             break;
         case LAYER_CONV: rc = halo ? conv_halo_launch(*hl, s) : conv_tc_launch(*cl, s); break;
         case LAYER_MAXPOOL:
+            if (L.spp == 1) break;  // computed by its SPP group's launch, at the group's last layer
+            if (L.spp == 2) {
+                int ks[SPP_MAX_POOLS];
+                __nv_bfloat16* outs[SPP_MAX_POOLS];
+                const int np = static_cast<int>(L.spp_members.size());
+                for (int j = 0; j < np; ++j) {
+                    const LayerPlan& M = P.layers[L.spp_members[j]];
+                    ks[j] = M.pool_k;
+                    outs[j] = static_cast<__nv_bfloat16*>(loc_ptr(*e, P, M.out, false, k, frames));
+                }
+                rc = launch_spp(static_cast<const __nv_bfloat16*>(loc_ptr(*e, P, L.in, false, k, frames)), L.in.pitch, frames, L.in.h, L.in.w,
+                                L.in.c, np, ks, outs, L.out.pitch, s);
+                break;
+            }
             rc = launch_maxpool(static_cast<const __nv_bfloat16*>(loc_ptr(*e, P, L.in, false, k, frames)), L.in.pitch,
                                 static_cast<__nv_bfloat16*>(loc_ptr(*e, P, L.out, false, k, frames)), L.out.pitch, frames, L.in.h, L.in.w,
                                 L.in.c, L.pool_k, L.pool_s, L.pool_pad_lo, L.out.h, L.out.w, L.pad_value, s);
@@ -623,6 +637,7 @@ int fd_model_create(const void* onnx_bytes, size_t len, int num_classes, int net
     I.n_layers = static_cast<int>(P.layers.size());
     for (const auto& L : P.layers) I.n_conv += (L.kind == LAYER_CONV || L.kind == LAYER_CONV0);
     I.launches_per_detect = I.n_layers + 2;
+    for (const auto& L : P.layers) I.launches_per_detect -= L.spp == 1;
     I.conv_flops_per_frame = P.conv_flops_per_frame;
     I.num_params = P.num_params;
     I.weight_bytes = P.weights_bf16.size() * 2 + P.bias_f32.size() * 4 + P.conv0_w.size() * 4;
@@ -648,6 +663,7 @@ int fd_model_create(const void* onnx_bytes, size_t len, int num_classes, int net
     char cerr[256] = "";
     if (conv_tc_init(cerr, sizeof(cerr))) return fail(FD_ERR_CUDA, "conv_tc_init: %s", cerr);
     if (kernels_init()) return fail(FD_ERR_CUDA, "kernels_init failed: %s", cudaGetErrorString(cudaGetLastError()));
+    if (spp_init()) return fail(FD_ERR_CUDA, "spp_init failed: %s", cudaGetErrorString(cudaGetLastError()));
     if (conv_halo_init()) return fail(FD_ERR_CUDA, "conv_halo_init failed: %s", cudaGetErrorString(cudaGetLastError()));
     if (conv_stem_init()) return fail(FD_ERR_CUDA, "conv_stem_init failed: %s", cudaGetErrorString(cudaGetLastError()));
     if (conv_block_init()) return fail(FD_ERR_CUDA, "conv_block_init failed: %s", cudaGetErrorString(cudaGetLastError()));
@@ -736,7 +752,7 @@ int fd_layer_exec_info(fd_model* m, int layer, int n, fd_layer_exec* out) {
     memset(out, 0, sizeof(*out));
     out->bucket = e->n;
     out->chunk_frames = e->n;
-    out->launches = e->fused_role[layer] == 1 ? 0 : 1;
+    out->launches = (e->fused_role[layer] == 1 || L.spp == 1) ? 0 : 1;
     const LaunchSet& W = e->whole;
     if (e->use_stem && layer < 2) {
         out->kernel = layer == 0 ? FD_KERNEL_FUSED_NEXT : FD_KERNEL_STEM;
@@ -750,7 +766,7 @@ int fd_layer_exec_info(fd_model* m, int layer, int n, fd_layer_exec* out) {
     }
     switch (L.kind) {
         case LAYER_CONV0: out->kernel = FD_KERNEL_CONV0; break;
-        case LAYER_MAXPOOL: out->kernel = FD_KERNEL_MAXPOOL; break;
+        case LAYER_MAXPOOL: out->kernel = L.spp == 1 ? FD_KERNEL_FUSED_NEXT : L.spp == 2 ? FD_KERNEL_SPP : FD_KERNEL_MAXPOOL; break;
         case LAYER_COPY: out->kernel = FD_KERNEL_COPY; break;
         default:
             if (W.use_halo[layer]) {

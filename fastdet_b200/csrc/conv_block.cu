@@ -374,6 +374,7 @@ conv_block_kernel(const __grid_constant__ CUtensorMap tm_out, const __grid_const
 
 bool conv_block_supported(const BlockDesc& d) {
     if (d.cin != CIN || d.cmid != CMID || d.cout != COUT) return false;
+    if (d.act_a > 1 || d.act_b > 1) return false;  // LeakyReLU only (act 2, Mish, runs unfused)
     if (d.act_a && !(d.alpha_a >= 0.f && d.alpha_a <= 1.f)) return false;
     if (d.act_b && !(d.alpha_b >= 0.f && d.alpha_b <= 1.f)) return false;
     if (d.in_pitch % 8 || d.out_pitch % 8 || (reinterpret_cast<uintptr_t>(d.in) & 15) || (reinterpret_cast<uintptr_t>(d.out) & 15) ||

@@ -26,6 +26,7 @@
 #include <stdlib.h>
 #include <string.h>
 
+#include "act.cuh"
 #include "conv_tc.h"
 #include "ptx.cuh"
 
@@ -85,7 +86,9 @@ __device__ __forceinline__ uint64_t desc_kmajor(uint32_t addr, uint32_t lbo, uin
            (static_cast<uint64_t>((sbo >> 4) & 0x3FFF) << 32) | (static_cast<uint64_t>(1) << 46);
 }
 
-template <int CIN, int STRIDE>
+// MISH: the activation is Mish (act.cuh), and a residual is added to it in fp32 before the one bf16 rounding; a separate
+// instantiation, so the LeakyReLU kernels (bf16x2 residual add) are unchanged.
+template <int CIN, int STRIDE, bool MISH = false>
 __global__ void __launch_bounds__(THREADS, 1)
 conv_halo_kernel(const __grid_constant__ CUtensorMap tm_out, const __grid_constant__ HaloParams p) {
     using G = Geo<STRIDE>;
@@ -269,6 +272,15 @@ conv_halo_kernel(const __grid_constant__ CUtensorMap tm_out, const __grid_consta
                 uint32_t pk[16];
 #pragma unroll
                 for (int g = 0; g < 16; ++g) {
+                    if constexpr (MISH) {
+                        float2 x = bias_mish2(acc[2 * g], acc[2 * g + 1], bias[2 * g], bias[2 * g + 1]);
+                        if (has_res) {
+                            const uint32_t r = rcur[g >> 3].v[g & 7];
+                            x = __fadd2_rn(x, make_float2(__uint_as_float(r << 16), __uint_as_float(r & 0xFFFF0000u)));
+                        }
+                        pk[g] = pack2(x.x, x.y);
+                        continue;
+                    }
                     float2 x = __fadd2_rn(make_float2(__uint_as_float(acc[2 * g]), __uint_as_float(acc[2 * g + 1])),
                                           make_float2(bias[2 * g], bias[2 * g + 1]));
                     if (!generic_act) {
@@ -281,7 +293,7 @@ conv_halo_kernel(const __grid_constant__ CUtensorMap tm_out, const __grid_consta
                     }
                     pk[g] = pack2(x.x, x.y);
                 }
-                if (has_res) {  // (bf16x2 add: the fp32 form used by conv_tc.cu costs this kernel 20 % on its three residual layers, conv4 / conv7 / conv9)
+                if (!MISH && has_res) {  // (bf16x2 add: the fp32 form used by conv_tc.cu costs this kernel 20 % on its three residual layers, conv4 / conv7 / conv9)
 #pragma unroll
                     for (int g = 0; g < 16; ++g) pk[g] = add_bf16x2(pk[g], rcur[g >> 3].v[g & 7]);
                 }
@@ -373,7 +385,7 @@ int conv_halo_prepare(const HaloDesc& d, int num_sms, HaloLaunch* L, char* err, 
     p.ho = (d.hi + d.pad_lo + d.pad_hi - 3) / d.stride + 1;
     p.wo = (d.wi + d.pad_lo + d.pad_hi - 3) / d.stride + 1;
     p.w = d.w; p.cin = d.cin; p.cout = d.cout;
-    p.act = d.act ? ((d.alpha >= 0.f && d.alpha <= 1.f) ? 1 : 2) : 0;
+    p.act = d.act == 2 ? 3 : d.act ? ((d.alpha >= 0.f && d.alpha <= 1.f) ? 1 : 2) : 0;  // 3: Mish (the MISH instantiations)
     p.alpha = d.alpha;
     p.residual = d.residual; p.res_pitch = d.res_pitch;
     p.pool2 = d.pool2;
@@ -406,14 +418,22 @@ int conv_halo_prepare(const HaloDesc& d, int num_sms, HaloLaunch* L, char* err, 
 
 // One-time per DEVICE (the attribute belongs to the device's context: a process that drives several GPUs must set it on
 // each — a once-per-process guard here made every halo launch on the second and later GPUs of fd_server fail).
-int conv_halo_init() {
-    return (cudaFuncSetAttribute(conv_halo_kernel<32, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_LIMIT) == cudaSuccess &&
-            cudaFuncSetAttribute(conv_halo_kernel<32, 2>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_LIMIT) == cudaSuccess &&
-            cudaFuncSetAttribute(conv_halo_kernel<64, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_LIMIT) == cudaSuccess &&
-            cudaFuncSetAttribute(conv_halo_kernel<16, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_LIMIT) == cudaSuccess &&
-            cudaFuncSetAttribute(conv_halo_kernel<16, 2>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_LIMIT) == cudaSuccess)
-               ? 0
-               : -1;
+template <bool MISH>
+static bool set_smem_attrs() {
+    return cudaFuncSetAttribute(conv_halo_kernel<32, 1, MISH>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_LIMIT) == cudaSuccess &&
+           cudaFuncSetAttribute(conv_halo_kernel<32, 2, MISH>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_LIMIT) == cudaSuccess &&
+           cudaFuncSetAttribute(conv_halo_kernel<64, 1, MISH>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_LIMIT) == cudaSuccess &&
+           cudaFuncSetAttribute(conv_halo_kernel<16, 1, MISH>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_LIMIT) == cudaSuccess &&
+           cudaFuncSetAttribute(conv_halo_kernel<16, 2, MISH>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_LIMIT) == cudaSuccess;
+}
+
+int conv_halo_init() { return set_smem_attrs<false>() && set_smem_attrs<true>() ? 0 : -1; }
+
+template <bool MISH>
+static cudaError_t launch_form(const HaloLaunch& L, const cudaLaunchConfig_t& cfg) {
+    if (L.cin == 64) return cudaLaunchKernelEx(&cfg, conv_halo_kernel<64, 1, MISH>, L.tm_out, L.p);
+    if (L.cin == 32) return L.stride == 1 ? cudaLaunchKernelEx(&cfg, conv_halo_kernel<32, 1, MISH>, L.tm_out, L.p) : cudaLaunchKernelEx(&cfg, conv_halo_kernel<32, 2, MISH>, L.tm_out, L.p);
+    return L.stride == 1 ? cudaLaunchKernelEx(&cfg, conv_halo_kernel<16, 1, MISH>, L.tm_out, L.p) : cudaLaunchKernelEx(&cfg, conv_halo_kernel<16, 2, MISH>, L.tm_out, L.p);
 }
 
 int conv_halo_launch(const HaloLaunch& L, cudaStream_t stream) {
@@ -427,10 +447,7 @@ int conv_halo_launch(const HaloLaunch& L, cudaStream_t stream) {
     attr[0].val.programmaticStreamSerializationAllowed = 1;
     cfg.attrs = attr;
     cfg.numAttrs = 1;
-    cudaError_t e;
-    if (L.cin == 64) e = cudaLaunchKernelEx(&cfg, conv_halo_kernel<64, 1>, L.tm_out, L.p);
-    else if (L.cin == 32) e = L.stride == 1 ? cudaLaunchKernelEx(&cfg, conv_halo_kernel<32, 1>, L.tm_out, L.p) : cudaLaunchKernelEx(&cfg, conv_halo_kernel<32, 2>, L.tm_out, L.p);
-    else e = L.stride == 1 ? cudaLaunchKernelEx(&cfg, conv_halo_kernel<16, 1>, L.tm_out, L.p) : cudaLaunchKernelEx(&cfg, conv_halo_kernel<16, 2>, L.tm_out, L.p);
+    const cudaError_t e = L.p.act == 3 ? launch_form<true>(L, cfg) : launch_form<false>(L, cfg);
     return e == cudaSuccess ? 0 : -1;
 }
 

@@ -483,6 +483,7 @@ conv_stem_kernel(const __grid_constant__ CUtensorMap tm_out, const __grid_consta
 
 bool conv_stem_supported(const StemDesc& d) {
     if (d.c1 != C1 || d.c2 != C2 || d.pad_hi2 < 0 || d.pad_hi2 > 1) return false;
+    if (d.act1 > 1 || d.act2 > 1) return false;  // LeakyReLU only (act 2, Mish, runs unfused)
     if (d.act1 && !(d.alpha1 >= 0.f && d.alpha1 <= 1.f)) return false;
     if (d.act2 && !(d.alpha2 >= 0.f && d.alpha2 <= 1.f)) return false;
     if (d.out_pitch % 8 || (reinterpret_cast<uintptr_t>(d.out) & 15) || (reinterpret_cast<uintptr_t>(d.w2) & 15)) return false;

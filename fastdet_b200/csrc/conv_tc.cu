@@ -21,6 +21,7 @@
 // way; strip mode stores rows directly (its rows are scattered over the image).  The production flag combinations have
 // compile-time copies of the epilogue (STRIP / FAST / PLAIN): short-K layers run at the epilogue's instruction count.
 #include "conv_tc.h"
+#include "act.cuh"
 #include "options.h"
 #include "ptx.cuh"
 
@@ -98,7 +99,8 @@ __device__ __forceinline__ float2 bias_act2(uint32_t a0, uint32_t a1, float b0, 
 // FAST: the common production path of the other kernels — bf16 output through 128-byte TMA stores, max(x, alpha x)
 // activation, whole-K tiles — with the same flags fixed at compile time (1x1 layers have K loops of 4-16 K blocks, shorter
 // than one epilogue: they run at the epilogue's speed, which is its instruction count).
-template <int BLOCK_N, bool STRIP = false, bool RES = false, bool FAST = false>
+// MISH: the kernel's activation is Mish (act.cuh) in every copy; the copies without it keep max(x, alpha x) / the select form.
+template <int BLOCK_N, bool STRIP = false, bool RES = false, bool FAST = false, bool MISH = false>
 __device__ __forceinline__ void epilogue_tile(const ConvParams& p, const CUtensorMap* tm_out, uint32_t taddr0,
                                               uint8_t* stage, int& sbuf, long long m_base, int n0, int lane, int half,
                                               uint32_t full_addr, uint32_t aphase, uint32_t empty_addr, long long* t_acc,
@@ -162,7 +164,10 @@ __device__ __forceinline__ void epilogue_tile(const ConvParams& p, const CUtenso
         if (c0 + 32 < c_end) fetch_res(c0 + 32);
         const float* bias = p.bias_c + n0 + c0;  // constant bank, warp-uniform index
         float2 x[16];
-        if (!generic_act) {
+        if constexpr (MISH) {
+#pragma unroll
+            for (int g = 0; g < 16; ++g) x[g] = bias_mish2(acc[2 * g], acc[2 * g + 1], bias[2 * g], bias[2 * g + 1]);
+        } else if (!generic_act) {
 #pragma unroll
             for (int g = 0; g < 16; ++g) x[g] = bias_act2<false>(acc[2 * g], acc[2 * g + 1], bias[2 * g], bias[2 * g + 1], alpha2);
         } else {
@@ -418,7 +423,8 @@ __device__ __forceinline__ void epilogue_tile(const ConvParams& p, const CUtenso
 // memory transposed ([pixel][32 channels] bf16) and re-read so that 4 lanes cover the 64 contiguous bytes this warp
 // owns of one pixel row.
 // PLAIN: compile-time copy for the production case (bf16 slice through TMA stores, no residual, max(x, alpha x)).
-template <bool PLAIN = false>
+// MISH: Mish instead of max(x, alpha x) / the select form, in both copies.
+template <bool PLAIN = false, bool MISH = false>
 __device__ __forceinline__ void epilogue_tile_swapped(const ConvParams& p, const CUtensorMap* tm_out, int& sbuf, uint32_t taddr0,
                                                       float* stage_buf, int ch_warp, long long pix0, int lane, int half,
                                                       uint32_t full_addr, uint32_t aphase, uint32_t empty_addr, long long* t_acc) {
@@ -486,8 +492,10 @@ __device__ __forceinline__ void epilogue_tile_swapped(const ConvParams& p, const
             const uint32_t lane_chunk = static_cast<uint32_t>(lane) >> 3, lane_byte = (static_cast<uint32_t>(lane) & 7u) * 2u;
 #pragma unroll
             for (int q = 0; q < 32; q += 2) {
-                const float2 x = generic_act ? bias_act2<true>(acc[q], acc[q + 1], bias_own, bias_own, alpha2)
-                                             : bias_act2<false>(acc[q], acc[q + 1], bias_own, bias_own, alpha2);
+                float2 x;
+                if constexpr (MISH) x = bias_mish2(acc[q], acc[q + 1], bias_own, bias_own);
+                else x = generic_act ? bias_act2<true>(acc[q], acc[q + 1], bias_own, bias_own, alpha2)
+                                     : bias_act2<false>(acc[q], acc[q + 1], bias_own, bias_own, alpha2);
                 const uint32_t slot = (lane_chunk ^ ((static_cast<uint32_t>(q) >> 1) & 3u)) << 4;  // rows q and q+1 share (q >> 1)
                 *reinterpret_cast<__nv_bfloat16*>(buf + q * 64 + slot + lane_byte) = __float2bfloat16(x.x);
                 *reinterpret_cast<__nv_bfloat16*>(buf + (q + 1) * 64 + slot + lane_byte) = __float2bfloat16(x.y);
@@ -505,7 +513,14 @@ __device__ __forceinline__ void epilogue_tile_swapped(const ConvParams& p, const
         if (PLAIN) continue;
         // channel-major phase: + bias, LeakyReLU; element (pixel q, channel lane) -> stage_buf[q][lane] (fp32: one
         // conflict-free 128-byte row per store instruction)
-        if (!generic_act) {
+        if constexpr (MISH) {
+#pragma unroll
+            for (int q = 0; q < 32; q += 2) {
+                const float2 x = bias_mish2(acc[q], acc[q + 1], bias_own, bias_own);
+                stage_buf[q * 32 + lane] = x.x;
+                stage_buf[(q + 1) * 32 + lane] = x.y;
+            }
+        } else if (!generic_act) {
 #pragma unroll
             for (int q = 0; q < 32; q += 2) {
                 const float2 x = bias_act2<false>(acc[q], acc[q + 1], bias_own, bias_own, alpha2);
@@ -564,7 +579,8 @@ __device__ __forceinline__ void issue_mmas(uint32_t tmem_d, uint64_t adesc, uint
 //              [128r, 128r+128) and stages B rows [128r, 128r+128); the leader (rank 0) issues the MMAs, which
 //              read both CTAs' shared memory.  Per SM and K block this needs 16 KB of A + 16 KB of B instead of
 //              16 + 32 KB, which is what the L2->SM fill latency x shared-memory capacity product can sustain.
-template <int BLOCK_N, bool TWO, bool SWAP = false, bool STRIP = false>
+// MISH: every epilogue copy applies Mish (ConvParams::act 3); a separate instantiation, so the LeakyReLU kernels are unchanged.
+template <int BLOCK_N, bool TWO, bool SWAP = false, bool STRIP = false, bool MISH = false>
 __global__ void __launch_bounds__(NUM_THREADS, 1)
 conv_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB,
                const __grid_constant__ CUtensorMap tmOut, const __grid_constant__ ConvParams p) {
@@ -914,10 +930,10 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
             if (swap) {
                 const int ch_warp = (tile - m_tile * n_tiles_n) * BLOCK_M + quarter * 32;
                 if (p.epi_mode == 0 && !p.residual && p.swap_tma && p.act != 2 && !(kDev && p.debug))
-                    epilogue_tile_swapped<true>(p, &tmOut, sbuf, taddr0, reinterpret_cast<float*>(stage), ch_warp, static_cast<long long>(m_tile) * 256,
+                    epilogue_tile_swapped<true, MISH>(p, &tmOut, sbuf, taddr0, reinterpret_cast<float*>(stage), ch_warp, static_cast<long long>(m_tile) * 256,
                                                 lane, half, full_addr, aphase, empty_addr, prof ? t_acc : nullptr);
                 else
-                    epilogue_tile_swapped<false>(p, &tmOut, sbuf, taddr0, reinterpret_cast<float*>(stage), ch_warp, static_cast<long long>(m_tile) * 256,
+                    epilogue_tile_swapped<false, MISH>(p, &tmOut, sbuf, taddr0, reinterpret_cast<float*>(stage), ch_warp, static_cast<long long>(m_tile) * 256,
                                                  lane, half, full_addr, aphase, empty_addr, prof ? t_acc : nullptr);
                 continue;
             }
@@ -925,20 +941,20 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
             const long long m_base = (strip ? p.strip_qfirst : 0) + static_cast<long long>(m_tile) * TILE_M + cta_rank * BLOCK_M + quarter * 32;
             if constexpr (STRIP) {
                 if (p.residual)
-                    epilogue_tile<BLOCK_N, true, true>(p, &tmOut, taddr0, stage, sbuf, m_base, n0, lane, half, full_addr, aphase, empty_addr,
+                    epilogue_tile<BLOCK_N, true, true, false, MISH>(p, &tmOut, taddr0, stage, sbuf, m_base, n0, lane, half, full_addr, aphase, empty_addr,
                                                        prof ? t_acc : nullptr, tile, part, static_cast<int>(cta_rank) * 4 + quarter);
                 else
-                    epilogue_tile<BLOCK_N, true, false>(p, &tmOut, taddr0, stage, sbuf, m_base, n0, lane, half, full_addr, aphase, empty_addr,
+                    epilogue_tile<BLOCK_N, true, false, false, MISH>(p, &tmOut, taddr0, stage, sbuf, m_base, n0, lane, half, full_addr, aphase, empty_addr,
                                                         prof ? t_acc : nullptr, tile, part, static_cast<int>(cta_rank) * 4 + quarter);
             } else if (BLOCK_N >= 128 && fast_epi) {
                 if (p.residual)
-                    epilogue_tile<BLOCK_N, false, true, true>(p, &tmOut, taddr0, stage, sbuf, m_base, n0, lane, half, full_addr, aphase, empty_addr,
+                    epilogue_tile<BLOCK_N, false, true, true, MISH>(p, &tmOut, taddr0, stage, sbuf, m_base, n0, lane, half, full_addr, aphase, empty_addr,
                                                               prof ? t_acc : nullptr, tile, part, static_cast<int>(cta_rank) * 4 + quarter);
                 else
-                    epilogue_tile<BLOCK_N, false, false, true>(p, &tmOut, taddr0, stage, sbuf, m_base, n0, lane, half, full_addr, aphase, empty_addr,
+                    epilogue_tile<BLOCK_N, false, false, true, MISH>(p, &tmOut, taddr0, stage, sbuf, m_base, n0, lane, half, full_addr, aphase, empty_addr,
                                                                prof ? t_acc : nullptr, tile, part, static_cast<int>(cta_rank) * 4 + quarter);
             } else {
-                epilogue_tile<BLOCK_N>(p, &tmOut, taddr0, stage, sbuf, m_base, n0, lane, half, full_addr, aphase, empty_addr,
+                epilogue_tile<BLOCK_N, false, false, false, MISH>(p, &tmOut, taddr0, stage, sbuf, m_base, n0, lane, half, full_addr, aphase, empty_addr,
                                        prof ? t_acc : nullptr, tile, part, static_cast<int>(cta_rank) * 4 + quarter);
             }
         }
@@ -977,9 +993,9 @@ void set_err(char* err, size_t n, const char* fmt, long long a = 0, long long b 
     if (err && n) snprintf(err, n, fmt, a, b, c);
 }
 
-template <int BN, bool TWO, bool SWAP = false, bool STRIP = false>
+template <int BN, bool TWO, bool SWAP = false, bool STRIP = false, bool MISH = false>
 int set_smem_attr() {
-    return cudaFuncSetAttribute(conv_tc_kernel<BN, TWO, SWAP, STRIP>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_LIMIT) == cudaSuccess
+    return cudaFuncSetAttribute(conv_tc_kernel<BN, TWO, SWAP, STRIP, MISH>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_LIMIT) == cudaSuccess
                ? 0
                : -1;
 }
@@ -1005,7 +1021,10 @@ int conv_tc_init(char* err, size_t errlen) {
     }
     if (set_smem_attr<32, false>() || set_smem_attr<64, false>() || set_smem_attr<128, false>() ||
         set_smem_attr<256, false>() || set_smem_attr<256, true>() || set_smem_attr<256, false, true>() ||
-        set_smem_attr<256, true, false, true>()) {
+        set_smem_attr<256, true, false, true>() || set_smem_attr<32, false, false, false, true>() ||
+        set_smem_attr<64, false, false, false, true>() || set_smem_attr<128, false, false, false, true>() ||
+        set_smem_attr<256, false, false, false, true>() || set_smem_attr<256, true, false, false, true>() ||
+        set_smem_attr<256, false, true, false, true>() || set_smem_attr<256, true, false, true, true>()) {
         set_err(err, errlen, "cudaFuncSetAttribute(MaxDynamicSharedMemorySize) failed: %lld",
                 static_cast<long long>(cudaGetLastError()));
         return -1;
@@ -1100,7 +1119,8 @@ int conv_tc_prepare(const ConvDesc& d, int num_sms, int block_n_hint, ConvLaunch
         // one shared pad column between consecutive image rows and one shared pad row between consecutive images are
         // enough (the right neighbour of a row's last pixel IS the next row's left pad): (W+1)(H+1) positions per image
         const int wp = d.wi + 1, hp = d.hi + 1, rows = 128 + 2 * wp + 2;
-        const bool plain_act = !d.act || (d.alpha >= 0.f && d.alpha <= 1.f);  // the strip kernel compiles the max(x, alpha x) form only
+        // the strip kernel compiles the max(x, alpha x) form and Mish, not the select form
+        const bool plain_act = !d.act || d.act == 2 || (d.alpha >= 0.f && d.alpha <= 1.f);
         const bool legal = two && plain_act && k == 3 && d.stride == 1 && d.pad_lo == 1 && d.pad_hi == 1 && block_k == 64 && !d.out_fp32 &&
                            !d.upsample2x && rows <= 400 && static_cast<long long>(d.n) * wp * hp < (1LL << 30);  // 400 rows: two strip buffers + a 5-stage B ring still fit
         constexpr int STRIP_MIN_W = 12;  // (W+1)(H+1)/(WH) extra rows: 1.04 at 52x52, 1.08 at 26x26, 1.16 at 13x13
@@ -1138,7 +1158,7 @@ int conv_tc_prepare(const ConvDesc& d, int num_sms, int block_n_hint, ConvLaunch
     p.res_v8 = (d.residual && (reinterpret_cast<uintptr_t>(d.residual) & 31) == 0 && d.res_pitch % 16 == 0 && d.cout % 16 == 0) ? 1 : 0;
     if (d.residual && p.epi_mode != 0 && !swap) { set_err(err, errlen, "conv_tc: a residual needs a plain bf16 output"); return -1; }
     p.bias = d.bias;
-    p.act = d.act ? ((d.alpha >= 0.f && d.alpha <= 1.f) ? 1 : 2) : 0;  // 1: max(x, alpha x); 2: select form
+    p.act = d.act == 2 ? 3 : d.act ? ((d.alpha >= 0.f && d.alpha <= 1.f) ? 1 : 2) : 0;  // 1: max(x, alpha x); 2: select form; 3: Mish
     p.alpha = d.alpha;
     p.residual = d.residual;
     p.res_pitch = d.res_pitch;
@@ -1274,6 +1294,22 @@ int conv_tc_prepare(const ConvDesc& d, int num_sms, int block_n_hint, ConvLaunch
     return 0;
 }
 
+// the Mish instantiations of the same forms
+static int launch_mish(const ConvLaunch& L, cudaLaunchConfig_t& cfg) {
+    cudaError_t e;
+    if (L.two_cta && L.p.strip) e = cudaLaunchKernelEx(&cfg, conv_tc_kernel<256, true, false, true, true>, L.tmA, L.tmB, L.tmOut, L.p);
+    else if (L.two_cta) e = cudaLaunchKernelEx(&cfg, conv_tc_kernel<256, true, false, false, true>, L.tmA, L.tmB, L.tmOut, L.p);
+    else if (L.p.swap) e = cudaLaunchKernelEx(&cfg, conv_tc_kernel<256, false, true, false, true>, L.tmA, L.tmB, L.tmOut, L.p);
+    else switch (L.block_n) {
+        case 32: e = cudaLaunchKernelEx(&cfg, conv_tc_kernel<32, false, false, false, true>, L.tmA, L.tmB, L.tmOut, L.p); break;
+        case 64: e = cudaLaunchKernelEx(&cfg, conv_tc_kernel<64, false, false, false, true>, L.tmA, L.tmB, L.tmOut, L.p); break;
+        case 128: e = cudaLaunchKernelEx(&cfg, conv_tc_kernel<128, false, false, false, true>, L.tmA, L.tmB, L.tmOut, L.p); break;
+        case 256: e = cudaLaunchKernelEx(&cfg, conv_tc_kernel<256, false, false, false, true>, L.tmA, L.tmB, L.tmOut, L.p); break;
+        default: return -1;
+    }
+    return e == cudaSuccess ? 0 : -1;
+}
+
 void conv_tc_bind_workspace(ConvLaunch* L, float* ws, int* counters) {
     L->p.ws = ws;
     L->p.counters = counters;
@@ -1302,6 +1338,7 @@ int conv_tc_launch(const ConvLaunch& L, cudaStream_t stream) {
     cfg.attrs = attr;
     cfg.numAttrs = na;
     cudaError_t e;
+    if (L.p.act == 3) return launch_mish(L, cfg);
     if (L.two_cta && L.p.strip) e = cudaLaunchKernelEx(&cfg, conv_tc_kernel<256, true, false, true>, L.tmA, L.tmB, L.tmOut, L.p);
     else if (L.two_cta) e = cudaLaunchKernelEx(&cfg, conv_tc_kernel<256, true>, L.tmA, L.tmB, L.tmOut, L.p);
     else if (L.p.swap) e = cudaLaunchKernelEx(&cfg, conv_tc_kernel<256, false, true>, L.tmA, L.tmB, L.tmOut, L.p);

@@ -23,7 +23,7 @@ struct ConvDesc {
     const __nv_bfloat16* w;  // [cout][ksize*ksize*cin], tap-major then channel
     const float* bias;       // device, [>= round_up(cout, 256)] fp32 (BatchNorm folded in)
     const float* bias_host;  // the same values on the host (they travel in the kernel's parameter block)
-    int act;                 // 0 = linear, 1 = LeakyReLU(alpha)
+    int act;                 // 0 = linear, 1 = LeakyReLU(alpha), 2 = Mish
     float alpha;
     // optional residual (added after the activation, like ONNX Add after LeakyRelu)
     const __nv_bfloat16* residual;
@@ -49,7 +49,7 @@ struct ConvParams {
     int b_resident;    // 1: the N tile's whole filter bank stays in shared memory, the ring carries A only
     int kb_per_stage;  // K blocks per ring stage (one barrier round trip covers all of them)
     const float* bias;
-    int act;
+    int act;  // 0 linear, 1 max(x, alpha x), 2 select form (alpha outside [0, 1]), 3 Mish (the MISH instantiations)
     float alpha;
     const __nv_bfloat16* residual;
     long long res_pitch;

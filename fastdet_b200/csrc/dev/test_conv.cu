@@ -8,6 +8,8 @@
 // A = 2^-23 * (K + 4) * S of the exact value, S = sum |x w| + |b| (+ |res|); a bf16 output adds half a bf16 step at
 // max(|got|, |ref|); the halo kernel's residual form rounds the branch first (+ half a step of the branch); a fused
 // MaxPool(2, 2) takes the largest bound in its window.  Split-K cases are marked "splitK" in the case line.
+// Mish cases (act 2, names starting "mish" / "strip mish" / "halo mish") are held to the Mish form of that model: 1.09 A
+// (max |mish'|) + 6 * 2^-23 * |mish| (the device formula, fastdet_b200/csrc/act.cuh), with one rounding of a residual sum.
 #include <math.h>
 #include <stdio.h>
 #include <stdlib.h>
@@ -46,7 +48,7 @@ static const double kU = ldexp(1.0, -23);  // one fp32 addition, relative to the
 
 struct Case {
     const char* name;
-    int n, h, w, cin, cout, k, stride, pad_lo, pad_hi, act, residual, fp32, upsample, in_pitch_extra, block_n;
+    int n, h, w, cin, cout, k, stride, pad_lo, pad_hi, act, residual, fp32, upsample, in_pitch_extra, block_n;  // act: 1 leaky 0.1, 2 Mish
     int pool;  // 1: MaxPool(2, 2) fused into the epilogue (halo-patch kernel only); omitted = 0
 };
 
@@ -141,7 +143,8 @@ static int run_case(const Case& c, int num_sms) {
     CK(cudaMemcpy(hout.data(), dout, out_bytes, cudaMemcpyDeviceToHost));
 
     // CPU reference: the exact value and S = sum |x w| + |b| (+ |res|), held to the rounding model (see the file header)
-    const bool halo_res = c.block_n == 2048 && c.residual;
+    const bool mish = c.act == 2;
+    const bool halo_res = c.block_n == 2048 && c.residual && !mish;  // (the Mish halo kernel adds the residual in fp32)
     double max_err = 0, max_ref = 0, max_ratio = 0;
     long long bad = 0, first_bad_m = -1;
     int first_bad_n = -1;
@@ -177,10 +180,12 @@ static int run_case(const Case& c, int num_sms) {
                     }
                 }
             double v = acc + bias[co], S = sabs + fabs(bias[co]);
-            if (c.act) v = v > 0 ? v : v * double(0.1f);
+            if (mish) v = v > 30 ? v : v * tanh(log1p(exp(v)));
+            else if (c.act) v = v > 0 ? v : v * double(0.1f);
             const double branch = v;
             if (c.residual) { v += res[m * c.cout + co]; S += fabs(res[m * c.cout + co]); }
-            const double A = kU * (K + 4) * S;
+            double A = kU * (K + 4) * S;
+            if (mish) A = 1.09 * A + 6.0 * kU * fmax(fabs(branch), fabs(v));
             if (c.pool) {  // compared after the loop: maximum over the 2x2 window
                 const size_t pi = ((1ULL * img * oh + oy / 2) * ow + ox / 2) * c.cout + co;
                 if (v > pooled[pi]) pooled[pi] = v;
@@ -376,6 +381,22 @@ int main(int argc, char** argv) {
             {"splitK 3x3 512->1024 13 res", 1, 13, 13, 512, 1024, 3, 1, 1, 1, 1, 1, 0, 0, 0, 0},
             {"splitK 3x3 256->512 26sq",    1, 26, 26, 256, 512, 3, 1, 1, 1, 1, 0, 0, 0, 0, 0},
             {"splitK 2cta 3x3 512->1024",   1, 13, 13, 512, 1024, 3, 1, 1, 1, 1, 1, 0, 0, 0, 512},
+            // Mish (YOLOv4's backbone) in every form: the general, FAST, swapped (both copies), pair, strip, split-K and halo epilogues
+            {"mish 3x3 64->64 s1",          2, 13, 13, 64, 64, 3, 1, 1, 1, 2, 0, 0, 0, 0, 0},
+            {"mish 1x1 512->256 res bn128", 8, 26, 26, 512, 256, 1, 1, 0, 0, 2, 1, 0, 0, 0, 128},
+            {"mish 3x3 128->512 bn256",     2, 13, 13, 128, 512, 3, 1, 1, 1, 2, 0, 0, 0, 0, 256},
+            {"mish swap 3x3 64->128 res",   3, 13, 13, 64, 128, 3, 1, 1, 1, 2, 1, 0, 0, 0, 1024},
+            {"mish swap 1x1 384->128 big",  8, 52, 52, 384, 128, 1, 1, 0, 0, 2, 0, 0, 0, 0, 1024},
+            {"mish 2cta 3x3 64->256 res s2",3, 26, 26, 64, 256, 3, 2, 1, 1, 2, 1, 0, 0, 0, 512},
+            {"mish 2cta 1x1 256->256 up",   2, 13, 13, 256, 256, 1, 1, 0, 0, 2, 0, 0, 1, 64, 512},
+            {"strip mish 3x3 128->256 13 res", 9, 13, 13, 128, 256, 3, 1, 1, 1, 2, 1, 0, 0, 0, 512},
+            {"strip mish 3x3 128->512 2n",  2, 52, 52, 128, 512, 3, 1, 1, 1, 2, 0, 0, 0, 64, 512},
+            {"mish splitK 3x3 512->1024 res", 1, 13, 13, 512, 1024, 3, 1, 1, 1, 2, 1, 0, 0, 0, 0},
+            {"mish splitK 2cta 3x3 512->1024", 1, 13, 13, 512, 1024, 3, 1, 1, 1, 2, 1, 0, 0, 0, 512},
+            {"halo mish 3x3 32->64 s1 res", 2, 72, 76, 32, 64, 3, 1, 1, 1, 2, 1, 0, 0, 0, 2048},
+            {"halo mish 3x3 32->64 s2",     2, 130, 134, 32, 64, 3, 2, 1, 1, 2, 0, 0, 0, 0, 2048},
+            {"halo mish 3x3 64->64 s1 res", 1, 104, 104, 64, 64, 3, 1, 1, 1, 2, 1, 0, 0, 0, 2048},
+            {"halo mish 3x3 32->64 pool",   1, 104, 104, 32, 64, 3, 1, 1, 1, 2, 0, 0, 0, 0, 2048, 1},
         };
         for (const Case& c : cases) fails += run_case(c, sms);
         printf("check: %d failing case(s)\n", fails);

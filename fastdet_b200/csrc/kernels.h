@@ -29,6 +29,14 @@ int launch_conv0_u8(const uint8_t* frames, const float* w, const float* bias, __
 // max-pool over bf16 NHWC slices; cells outside the input take `pad_value` (-inf = ONNX MaxPool padding).
 int launch_maxpool(const __nv_bfloat16* in, int in_pitch, __nv_bfloat16* out, int out_pitch, int n, int hi, int wi,
                    int c, int k, int stride, int pad_lo, int ho, int wo, float pad_value, cudaStream_t s);
+// SPP: the stride-1, symmetrically padded (pad = (k-1)/2, -inf) max-pools of one tensor, k in ks[0..npools), in one launch;
+// pool j's output (same shape as the input) goes to outs[j], all of them rows of out_pitch channels.  One CTA per (frame,
+// 64-channel group) holds the h x w x 64 slab and a row-maximum buffer of the same size in shared memory.
+constexpr int SPP_MAX_POOLS = 4;
+inline bool spp_fits(int h, int w) { return 2LL * h * w * 64 * 2 <= 227 * 1024; }
+int spp_init();  // one-time per device: the kernel's shared-memory opt-in
+int launch_spp(const __nv_bfloat16* in, int in_pitch, int n, int h, int w, int c, int npools, const int* ks,
+               __nv_bfloat16* const* outs, int out_pitch, cudaStream_t s);
 // slice copy, optionally with x2 nearest upsampling (fallback when a Concat/Resize cannot be fused away).
 int launch_copy_slice(const __nv_bfloat16* in, int in_pitch, __nv_bfloat16* out, int out_pitch, int n, int hi,
                       int wi, int c, int upsample2x, cudaStream_t s);

@@ -7,6 +7,8 @@
 #include <algorithm>
 #include <map>
 
+#include "kernels.h"
+
 namespace fd {
 
 uint16_t f32_to_bf16_rn(float f) {
@@ -19,7 +21,7 @@ uint16_t f32_to_bf16_rn(float f) {
 
 namespace {
 
-enum AKind { A_INPUT, A_CONV, A_BN, A_LEAKY, A_ADD, A_MAXPOOL, A_PAD, A_RESIZE, A_CONCAT, A_VIEW };
+enum AKind { A_INPUT, A_CONV, A_BN, A_LEAKY, A_ADD, A_MAXPOOL, A_PAD, A_RESIZE, A_CONCAT, A_VIEW, A_MISH };
 
 struct ANode {
     AKind kind;
@@ -437,6 +439,42 @@ struct Builder {
         return true;
     }
 
+    // Mish written out as Softplus(x) -> Tanh -> Mul(x, tanh) (torch's exporter, symbolic_opset9.mish): the Softplus and
+    // the Tanh become pending chain links, the Mul that closes the chain becomes one A_MISH anode.  Anything else with
+    // Softplus or Tanh in it is refused, naming the node.
+    struct MishLink { int x = -1; std::string node; bool used = false; std::string src; };  // src: a Tanh's Softplus output
+    std::map<std::string, MishLink> softplus, tanh_of;  // by output name
+    std::map<std::string, int> readers;                 // nodes (and graph outputs) that read a tensor
+    // returns true when the node belongs to a Mish chain (then *ok says whether it was accepted)
+    bool mish_link(const OnnxNode& n, int ni, bool* ok) {
+        *ok = true;
+        const std::string& out = n.outputs[0];
+        if (n.op == "Softplus") {
+            const int x = n.inputs.empty() ? -1 : act(n.inputs[0]);
+            if (x < 0) { *ok = fail(n.name + ": Softplus of a tensor that is not an activation"); return true; }
+            softplus[out] = {x, n.name, false};
+            return true;
+        }
+        if (n.op == "Tanh") {
+            auto it = n.inputs.empty() ? softplus.end() : softplus.find(n.inputs[0]);
+            if (it == softplus.end()) { *ok = fail(n.name + ": Tanh is only supported as the tanh(softplus(x)) of Mish"); return true; }
+            it->second.used = true;
+            tanh_of[out] = {it->second.x, n.name, false, n.inputs[0]};
+            return true;
+        }
+        if (n.op != "Mul" || n.inputs.size() != 2) return false;
+        const int t = tanh_of.count(n.inputs[0]) ? 0 : tanh_of.count(n.inputs[1]) ? 1 : -1;
+        if (t < 0) return false;
+        MishLink& tl = tanh_of[n.inputs[t]];
+        tl.used = true;
+        const int x = tl.x;
+        if (act(n.inputs[1 - t]) != x) { *ok = fail(n.name + ": Mul of tanh(softplus(x)) with a tensor other than x is not Mish"); return true; }
+        if (readers[tl.src] != 1) { *ok = fail(softplus[tl.src].node + ": Softplus output of Mish '" + n.name + "' has other readers"); return true; }
+        if (readers[n.inputs[t]] != 1) { *ok = fail(tl.node + ": Tanh output of Mish '" + n.name + "' has other readers"); return true; }
+        add_anode(A_MISH, ni, {x}, an[x].c, an[x].h, an[x].w, out);
+        return true;
+    }
+
     bool walk() {
         for (const auto& kv : g.initializers) consts[kv.first] = kv.second;
         // graph input: the reference feeds {'input': a} (server/detector.py:135)
@@ -454,6 +492,9 @@ bool build_plan(const OnnxGraph& g, int net_w, int net_h, int num_classes, bool 
     if (!B.walk()) return false;
     plan->net_w = net_w; plan->net_h = net_h; plan->num_classes = num_classes;
     const int input_id = B.add_anode(A_INPUT, -1, {}, 3, net_h, net_w, "input");
+    for (const auto& n : g.nodes)
+        for (const auto& nm : n.inputs) ++B.readers[nm];
+    for (const auto& o : g.outputs) ++B.readers[o.name];
 
     // ------------------------------------------------------------------ pass 1: activation graph
     for (size_t ni = 0; ni < g.nodes.size(); ++ni) {
@@ -465,6 +506,19 @@ bool build_plan(const OnnxGraph& g, int net_w, int net_h, int num_classes, bool 
             if (it == n.attrs.end()) return B.fail("Constant node '" + n.name + "' without a tensor value");
             B.consts[out] = it->second.t;
             continue;
+        }
+        {
+            bool ok = true;
+            if (B.mish_link(n, static_cast<int>(ni), &ok)) {
+                if (!ok) return false;
+                continue;
+            }
+            for (const auto& nm : n.inputs) {  // any other reader of a Softplus / Tanh output
+                auto sp = B.softplus.find(nm);
+                if (sp != B.softplus.end()) return B.fail(sp->second.node + ": Softplus is only supported as the softplus of Mish, x * tanh(softplus(x)) (read by '" + n.name + "')");
+                auto th = B.tanh_of.find(nm);
+                if (th != B.tanh_of.end()) return B.fail(th->second.node + ": Tanh is only supported as the tanh(softplus(x)) of Mish, multiplied by x (read by '" + n.name + "')");
+            }
         }
         const int x = n.inputs.empty() ? -1 : B.act(n.inputs[0]);
         if (n.op == "Shape" || x < 0) {
@@ -506,6 +560,9 @@ bool build_plan(const OnnxGraph& g, int net_w, int net_h, int num_classes, bool 
             if (x < 0) return B.fail(n.name + ": activation input is not an activation tensor");
             const int id = B.add_anode(A_LEAKY, static_cast<int>(ni), {x}, B.an[x].c, B.an[x].h, B.an[x].w, out);
             B.an[id].alpha = n.op == "Relu" ? 0.f : n.attr_f("alpha", 0.01f);
+        } else if (n.op == "Mish") {
+            if (x < 0) return B.fail(n.name + ": activation input is not an activation tensor");
+            B.add_anode(A_MISH, static_cast<int>(ni), {x}, B.an[x].c, B.an[x].h, B.an[x].w, out);
         } else if (n.op == "Add") {
             const int y = n.inputs.size() > 1 ? B.act(n.inputs[1]) : -1;
             if (x < 0 || y < 0) return B.fail(n.name + ": Add needs two activation inputs");
@@ -589,6 +646,10 @@ bool build_plan(const OnnxGraph& g, int net_w, int net_h, int num_classes, bool 
             return B.fail("unsupported ONNX operator '" + n.op + "' (node '" + n.name + "')");
         }
     }
+    for (const auto& kv : B.softplus)
+        if (!kv.second.used) return B.fail(kv.second.node + ": Softplus is only supported as the softplus of Mish, x * tanh(softplus(x))");
+    for (const auto& kv : B.tanh_of)
+        if (!kv.second.used) return B.fail(kv.second.node + ": Tanh is only supported as the tanh(softplus(x)) of Mish, multiplied by x");
     std::vector<int> out_anodes;
     for (const auto& o : g.outputs) {
         const int a = B.act(o.name);
@@ -616,7 +677,7 @@ bool build_plan(const OnnxGraph& g, int net_w, int net_h, int num_classes, bool 
             int cur = a, nx;
             owner[a] = id;
             if ((nx = sole_consumer(cur)) >= 0 && an[nx].kind == A_BN) { f.bn = nx; owner[nx] = id; cur = nx; }
-            if ((nx = sole_consumer(cur)) >= 0 && an[nx].kind == A_LEAKY) { f.leaky = nx; owner[nx] = id; cur = nx; }
+            if ((nx = sole_consumer(cur)) >= 0 && (an[nx].kind == A_LEAKY || an[nx].kind == A_MISH)) { f.leaky = nx; owner[nx] = id; cur = nx; }
             if (f.kind == LAYER_CONV && (nx = sole_consumer(cur)) >= 0 && an[nx].kind == A_ADD) {
                 const int other = an[nx].in[0] == cur ? an[nx].in[1] : an[nx].in[0];
                 if (other != cur && other < a) { f.add = nx; f.residual = other; owner[nx] = id; cur = nx; }
@@ -648,6 +709,8 @@ bool build_plan(const OnnxGraph& g, int net_w, int net_h, int num_classes, bool 
         } else if (an[a].kind == A_RESIZE) {
             f.kind = LAYER_COPY; f.resize = a; f.in_anode = an[a].in[0]; f.final_anode = a; f.copy_up = 1;
             owner[a] = id;
+        } else if (an[a].kind == A_MISH) {
+            return B.fail("Mish '" + g.nodes[an[a].node].name + "' cannot be fused into a preceding convolution (it must follow the Conv or its BatchNormalization)");
         } else {
             const char* what = an[a].kind == A_BN ? "BatchNormalization" : an[a].kind == A_LEAKY ? "LeakyRelu" : "Add";
             return B.fail(std::string(what) + " '" + an[a].out_name + "' cannot be fused into a preceding convolution");
@@ -783,8 +846,8 @@ bool build_plan(const OnnxGraph& g, int net_w, int net_h, int num_classes, bool 
             const OnnxTensor& W = *B.cst(n.inputs[1]);
             L.cout = static_cast<int>(W.dims[0]); L.cin = static_cast<int>(W.dims[1]);
             L.ksize = cv.ksize; L.stride = cv.stride; L.pad_lo = cv.pad_lo; L.pad_hi = cv.pad_hi;
-            L.act = f.leaky >= 0 ? 1 : 0;
-            L.alpha = f.leaky >= 0 ? an[f.leaky].alpha : 0.f;
+            L.act = f.leaky < 0 ? 0 : an[f.leaky].kind == A_MISH ? 2 : 1;
+            L.alpha = L.act == 1 ? an[f.leaky].alpha : 0.f;
             L.upsample2x = f.resize >= 0 ? 1 : 0;
             L.pool2 = f.pool >= 0 ? 1 : 0;
             L.out_fp32 = value_of(f.final_anode).fp32 ? 1 : 0;
@@ -855,6 +918,33 @@ bool build_plan(const OnnxGraph& g, int net_w, int net_h, int num_classes, bool 
             // filled below in graph-output order
         }
         plan->layers.push_back(L);
+    }
+    // SPP groups: the stride-1 "same" max-pools (pads (k-1)/2 of -inf, from the MaxPool itself) of one tensor whose outputs
+    // each go only into the same Concat, placed there directly, on maps whose slab fits the kernel's shared memory.  Up to
+    // SPP_MAX_POOLS per launch; layers[i] is the layer of ops[i].
+    {
+        std::map<std::pair<int, int>, std::vector<int>> groups;  // (input value, Concat anode) -> layers
+        for (size_t i = 0; i < ops.size(); ++i) {
+            const Fused& f = ops[i];
+            if (f.kind != LAYER_MAXPOOL || f.pad >= 0) continue;
+            const ANode& p = an[f.pool];
+            const LayerPlan& L = plan->layers[i];
+            if (p.stride != 1 || p.ksize % 2 == 0 || p.pad_lo != p.ksize / 2 || p.pad_hi != p.ksize / 2) continue;
+            if (p.is_output || p.consumers.size() != 1 || an[p.consumers[0]].kind != A_CONCAT) continue;
+            if (L.out.buf != vals[an[p.consumers[0]].value].loc.buf || L.in.buf < 0 || !spp_fits(L.in.h, L.in.w)) continue;
+            groups[{an[f.in_anode].value, p.consumers[0]}].push_back(static_cast<int>(i));
+        }
+        for (const auto& kv : groups) {
+            const std::vector<int>& mem = kv.second;
+            for (size_t s = 0; s + 1 < mem.size(); s += SPP_MAX_POOLS) {
+                const size_t e = std::min(mem.size(), s + SPP_MAX_POOLS);
+                if (e - s < 2) break;
+                for (size_t j = s; j < e; ++j) plan->layers[mem[j]].spp = 1;
+                LayerPlan& last = plan->layers[mem[e - 1]];
+                last.spp = 2;
+                last.spp_members.assign(mem.begin() + s, mem.begin() + e);
+            }
+        }
     }
     for (int a : out_anodes) {
         int found = -1;

@@ -2,9 +2,11 @@
 //
 // The optimisation half of `ort.InferenceSession(...)` (reference server/detector.py:118), rebuilt for this
 // path: Conv -> [BatchNormalization] -> [LeakyRelu] -> [Add] -> [Resize x2] chains collapse into one fused
-// convolution each (BatchNorm folded into fp32 weights/bias before the bf16 rounding), Concat becomes a shared
+// convolution each (BatchNorm folded into fp32 weights/bias before the bf16 rounding; the activation is LeakyRelu / Relu or
+// Mish, written as one Mish node or as Softplus -> Tanh -> Mul), Concat becomes a shared
 // buffer its producers write channel slices of, a channel Slice / Split becomes a view (a location inside its source's
-// buffer, no layer), Pad+MaxPool merge, and every activation gets a bf16 NHWC location.  No device code here; capi.cu turns the plan into buffers, tensor maps and launches.
+// buffer, no layer), Pad+MaxPool merge, the "same" stride-1 max-pools of one tensor that all go into one Concat (an SPP
+// block) run as one launch, and every activation gets a bf16 NHWC location.  No device code here; capi.cu turns the plan into buffers, tensor maps and launches.
 #pragma once
 #include <stdint.h>
 
@@ -31,8 +33,8 @@ struct LayerPlan {
     TensorLoc in, out, res;
     // convolution
     int cin = 0, cout = 0, ksize = 1, stride = 1, pad_lo = 0, pad_hi = 0;
-    int act = 0;  // 0 linear, 1 leaky
-    float alpha = 0.f;
+    int act = 0;  // 0 linear, 1 leaky (alpha), 2 Mish
+    float alpha = 0.f;  // leaky only
     int out_fp32 = 0, upsample2x = 0;
     int pool2 = 0;  // 1: a MaxPool(2, stride 2) that follows the convolution is applied in its epilogue; `out` is the pooled tensor
     size_t w_off = 0;  // LAYER_CONV: element offset into weights_bf16; LAYER_CONV0: into conv0_w
@@ -40,6 +42,11 @@ struct LayerPlan {
     // max-pool (window k, stride s); padding cells hold pad_value (-inf for ONNX MaxPool pads)
     int pool_k = 0, pool_s = 0, pool_pad_lo = 0, pool_pad_hi = 0;
     float pad_value = 0.f;
+    // SPP group (stride-1 max-pools, pad (k-1)/2 with -inf, of one tensor whose outputs all go into one Concat): computed by
+    // one launch (pool.cu launch_spp) at the group's last layer.  1: a member that launches nothing; 2: the last member,
+    // spp_members = every layer of the group in order (itself included).  The members still write their own outputs.
+    int spp = 0;
+    std::vector<int> spp_members;
     double flops = 0.0;  // algorithmic, per frame
 };
 

@@ -3,6 +3,7 @@
 // ONNX Runtime executes at reference server/detector.py:135.  HBM-bound: one 16-byte vector (8 channels)
 // per thread, consecutive threads on consecutive channel groups of consecutive pixels.
 #include <math.h>
+#include <string.h>
 
 #include "kernels.h"
 
@@ -57,6 +58,74 @@ int launch_maxpool(const __nv_bfloat16* in, int in_pitch, __nv_bfloat16* out, in
     const int blocks = static_cast<int>(total / 256 + 1 < 148 * 16 ? total / 256 + 1 : 148 * 16);
     maxpool_kernel<<<blocks, 256, 0, s>>>(in, in_pitch, out, out_pitch, n, hi, wi, c / 8, k, stride, pad_lo, ho, wo,
                                           pad_value);
+    return cudaPeekAtLastError() == cudaSuccess ? 0 : -1;  // (peek: the caller reports the reason)
+}
+
+// SPP (see kernels.h).  A window clipped to the map is the same set of values as the -inf padded one, so every pool is a
+// row maximum over k (slab -> rows buffer) then a column maximum over k (rows buffer -> global): each input element is read
+// from global memory once, each output written once with a 16-byte store.  The result is bit-exact (max is exact).
+struct SppArgs {
+    int k[SPP_MAX_POOLS];
+    __nv_bfloat16* out[SPP_MAX_POOLS];
+    int npools;
+};
+
+__global__ void __launch_bounds__(256)
+spp_kernel(const __nv_bfloat16* __restrict__ in, int in_pitch, int out_pitch, int h, int w, int c, const SppArgs a) {
+    extern __shared__ uint4 spp_smem[];
+    const int hw = h * w;
+    uint4* slab = spp_smem;         // [pixel][8 x 16 bytes]
+    uint4* rows = spp_smem + hw * 8;
+    const int cgroups = (c + 63) / 64;
+    const int f = blockIdx.x / cgroups, c0 = (blockIdx.x - f * cgroups) * 64;
+    const int nq = (c - c0) / 8 < 8 ? (c - c0) / 8 : 8;  // 16-byte channel groups of this CTA
+    const long long pix0 = 1LL * f * hw;
+    for (int i = threadIdx.x; i < hw * 8; i += 256) {
+        const int pix = i >> 3, q = i & 7;
+        if (q < nq) slab[i] = __ldg(reinterpret_cast<const uint4*>(in + (pix0 + pix) * in_pitch + c0 + 8 * q));
+    }
+    __syncthreads();
+#pragma unroll
+    for (int j = 0; j < SPP_MAX_POOLS; ++j) {  // (unrolled: a run-time index into the parameters would copy them to the stack)
+        if (j >= a.npools) break;
+        const int r = a.k[j] >> 1;
+        for (int i = threadIdx.x; i < hw * 8; i += 256) {
+            const int pix = i >> 3, q = i & 7, y = pix / w, x = pix - y * w;
+            if (q >= nq) continue;
+            const int x0 = x - r < 0 ? 0 : x - r, x1 = x + r < w ? x + r : w - 1;
+            uint4 m = slab[(y * w + x0) * 8 + q];
+            for (int xx = x0 + 1; xx <= x1; ++xx) m = max_bf16x8(m, slab[(y * w + xx) * 8 + q]);
+            rows[i] = m;
+        }
+        __syncthreads();
+        __nv_bfloat16* out = a.out[j];
+        for (int i = threadIdx.x; i < hw * 8; i += 256) {
+            const int pix = i >> 3, q = i & 7, y = pix / w, x = pix - y * w;
+            if (q >= nq) continue;
+            const int y0 = y - r < 0 ? 0 : y - r, y1 = y + r < h ? y + r : h - 1;
+            uint4 m = rows[(y0 * w + x) * 8 + q];
+            for (int yy = y0 + 1; yy <= y1; ++yy) m = max_bf16x8(m, rows[(yy * w + x) * 8 + q]);
+            *reinterpret_cast<uint4*>(out + (pix0 + pix) * out_pitch + c0 + 8 * q) = m;
+        }
+        __syncthreads();  // the next pool rewrites the rows buffer
+    }
+}
+
+int spp_init() { return cudaFuncSetAttribute(spp_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024) == cudaSuccess ? 0 : -1; }
+
+int launch_spp(const __nv_bfloat16* in, int in_pitch, int n, int h, int w, int c, int npools, const int* ks,
+               __nv_bfloat16* const* outs, int out_pitch, cudaStream_t s) {
+    if (c % 8 || in_pitch % 8 || out_pitch % 8 || npools < 1 || npools > SPP_MAX_POOLS || !spp_fits(h, w)) return -1;
+    SppArgs a;
+    memset(&a, 0, sizeof(a));
+    a.npools = npools;
+    for (int j = 0; j < npools; ++j) {
+        if (ks[j] < 1 || !(ks[j] & 1)) return -1;
+        a.k[j] = ks[j];
+        a.out[j] = outs[j];
+    }
+    const size_t smem = 2ULL * h * w * 64 * 2;
+    spp_kernel<<<n * ((c + 63) / 64), 256, smem, s>>>(in, in_pitch, out_pitch, h, w, c, a);
     return cudaPeekAtLastError() == cudaSuccess ? 0 : -1;  // (peek: the caller reports the reason)
 }
 

@@ -6,6 +6,7 @@
 //                        NCHW tensor the reference materialises never exists on the serving path.
 #include <stdlib.h>
 
+#include "act.cuh"
 #include "conv_tc.h"
 #include "kernels.h"
 #include "ptx.cuh"
@@ -136,6 +137,8 @@ __device__ __forceinline__ uint32_t c0_max(uint32_t a, uint32_t b) {  // bf16x2 
     return *reinterpret_cast<const uint32_t*>(&r);
 }
 
+// MISH: Mish (act.cuh) instead of LeakyReLU(alpha) when act is set
+template <bool MISH = false>
 __global__ void __launch_bounds__(C0_THREADS)
 conv0_u8_kernel(const uint8_t* __restrict__ frames, const float* __restrict__ wgt, const float* __restrict__ bias,
                 __nv_bfloat16* __restrict__ out, int h, int wd, int cout, int out_pitch, int act, float alpha) {
@@ -198,7 +201,10 @@ conv0_u8_kernel(const uint8_t* __restrict__ frames, const float* __restrict__ wg
                 }
 #pragma unroll
         for (int p = 0; p < 4; ++p) {
-            if (act) {
+            if (MISH) {
+#pragma unroll
+                for (int j = 0; j < 8; ++j) acc[p][j] = mish_f32(acc[p][j]);
+            } else if (act) {
 #pragma unroll
                 for (int j = 0; j < 8; ++j) acc[p][j] = acc[p][j] > 0.f ? acc[p][j] : acc[p][j] * alpha;
             }
@@ -272,7 +278,8 @@ static constexpr int C0W_THREADS = (C0W_EPI_WARPS + 1 + C0W_BUILD_WARPS) * 32, C
 __device__ __forceinline__ int div_magic(int x, unsigned long long m) { return static_cast<int>((static_cast<unsigned long long>(x) * m) >> 40); }
 
 // h, wd: the input frame; the output map is (h / S, wd / S) (stride 2: h and wd even)
-template <int S>
+// MISH: the activation is Mish (act.cuh); act / alpha are not read
+template <int S, bool MISH = false>
 __global__ void __launch_bounds__(C0W_THREADS)
 conv0_ws_kernel(const uint8_t* __restrict__ frames, const float* __restrict__ wgt, const float* __restrict__ bias,
                 const __grid_constant__ CUtensorMap tm_out, int n, int h, int wd, int cout, int act, float alpha,
@@ -515,7 +522,9 @@ conv0_ws_kernel(const uint8_t* __restrict__ frames, const float* __restrict__ wg
 #pragma unroll
             for (int c = 0; c < 16; ++c) {  // two columns per FADD2 / FMUL2
                 float2 x = __fadd2_rn(make_float2(__uint_as_float(acc[2 * c]), __uint_as_float(acc[2 * c + 1])), make_float2(bv[2 * c], bv[2 * c + 1]));
-                if (act != 2) {
+                if constexpr (MISH) {
+                    x = make_float2(mish_f32(x.x), mish_f32(x.y));
+                } else if (act != 2) {
                     const float2 m = __fmul2_rn(x, a2);
                     x.x = fmaxf(x.x, m.x);
                     x.y = fmaxf(x.y, m.y);
@@ -587,16 +596,18 @@ conv0_ws_kernel(const uint8_t* __restrict__ frames, const float* __restrict__ wg
     }
 }
 
-int kernels_init() {
-    return (cudaFuncSetAttribute(conv0_u8_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 100 * 1024) == cudaSuccess &&
-            cudaFuncSetAttribute(conv0_ws_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, C0W_PATCHES * C0Geom<1>::PATCH_BYTES) == cudaSuccess &&
-            cudaFuncSetAttribute(conv0_ws_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, C0W_PATCHES * C0Geom<2>::PATCH_BYTES) == cudaSuccess)
-               ? 0
-               : -1;
+template <bool MISH>
+static bool conv0_smem_attrs() {
+    return cudaFuncSetAttribute(conv0_u8_kernel<MISH>, cudaFuncAttributeMaxDynamicSharedMemorySize, 100 * 1024) == cudaSuccess &&
+           cudaFuncSetAttribute(conv0_ws_kernel<1, MISH>, cudaFuncAttributeMaxDynamicSharedMemorySize, C0W_PATCHES * C0Geom<1>::PATCH_BYTES) == cudaSuccess &&
+           cudaFuncSetAttribute(conv0_ws_kernel<2, MISH>, cudaFuncAttributeMaxDynamicSharedMemorySize, C0W_PATCHES * C0Geom<2>::PATCH_BYTES) == cudaSuccess;
 }
+
+int kernels_init() { return conv0_smem_attrs<false>() && conv0_smem_attrs<true>() ? 0 : -1; }
 
 int launch_conv0_u8(const uint8_t* frames, const float* w, const float* bias, __nv_bfloat16* out, int n, int h,
                     int wd, int cout, int stride, int out_pitch, int act, float alpha, int pool2, cudaStream_t s) {
+    const bool mish = act == 2;
     const int act_mode = act ? ((alpha >= 0.f && alpha <= 1.f) ? 1 : 2) : 0;
     if (stride != 1 && stride != 2) return -1;
     // stride 2: tensor cores only (even input, dense Cout 16 / 32 rows, 2-byte aligned frames for the pair loads)
@@ -619,8 +630,12 @@ int launch_conv0_u8(const uint8_t* frames, const float* w, const float* bias, __
         const int blocks = static_cast<int>(tiles < 148LL ? tiles : 148LL);
         const unsigned long long one40 = 1ULL << 40;
         const unsigned long long mf = (one40 + per_frame - 1) / per_frame, mx = (one40 + tx - 1) / tx;
-        if (stride == 2)
+        if (stride == 2 && mish)
+            conv0_ws_kernel<2, true><<<blocks, C0W_THREADS, C0W_PATCHES * C0Geom<2>::PATCH_BYTES, s>>>(frames, w, bias, tm, n, h, wd, cout, act_mode, alpha, mf, mx, 0);
+        else if (stride == 2)
             conv0_ws_kernel<2><<<blocks, C0W_THREADS, C0W_PATCHES * C0Geom<2>::PATCH_BYTES, s>>>(frames, w, bias, tm, n, h, wd, cout, act_mode, alpha, mf, mx, 0);
+        else if (mish)
+            conv0_ws_kernel<1, true><<<blocks, C0W_THREADS, C0W_PATCHES * C0Geom<1>::PATCH_BYTES, s>>>(frames, w, bias, tm, n, h, wd, cout, act_mode, alpha, mf, mx, pool2);
         else
             conv0_ws_kernel<1><<<blocks, C0W_THREADS, C0W_PATCHES * C0Geom<1>::PATCH_BYTES, s>>>(frames, w, bias, tm, n, h, wd, cout, act_mode, alpha, mf, mx, pool2);
         return cudaPeekAtLastError() == cudaSuccess ? 0 : -1;  // (peek: the caller reports the reason)
@@ -630,7 +645,8 @@ int launch_conv0_u8(const uint8_t* frames, const float* w, const float* bias, __
     const size_t smem = (256 + (C0_TH + 2) * (C0_TW + 2) * 3 + 4 + 27 * cout + cout) * sizeof(float) +
                         static_cast<size_t>(C0_TH) * C0_TW * cout * 2;
     dim3 grid((wd + C0_TW - 1) / C0_TW, (h + C0_TH - 1) / C0_TH, n);
-    conv0_u8_kernel<<<grid, C0_THREADS, smem, s>>>(frames, w, bias, out, h, wd, cout, out_pitch, act, alpha);
+    if (mish) conv0_u8_kernel<true><<<grid, C0_THREADS, smem, s>>>(frames, w, bias, out, h, wd, cout, out_pitch, act, alpha);
+    else conv0_u8_kernel<<<grid, C0_THREADS, smem, s>>>(frames, w, bias, out, h, wd, cout, out_pitch, act, alpha);
     return cudaPeekAtLastError() == cudaSuccess ? 0 : -1;  // (peek: the caller reports the reason)
 }
 

@@ -1,14 +1,16 @@
-"""modelgen.py — synthetic YOLOv3 / YOLOv3-tiny / YOLOv4-tiny ONNX files with random-init weights.
+"""modelgen.py — synthetic YOLOv3 / YOLOv3-tiny / YOLOv4 / YOLOv4-tiny ONNX files with random-init weights.
 
 The reference ships no model files (``*.onnx`` is git-ignored, reference .gitignore:5; README.md:38-48
 names ``yolov3-full.onnx`` / ``yolov3-rsu.onnx`` / ``yolov3-tiny.onnx``), so tests and benchmarks
-generate them.  The topologies are the public Darknet ``yolov3.cfg`` / ``yolov3-tiny.cfg`` / ``yolov4-tiny.cfg``; the graph
+generate them.  The topologies are the public Darknet ``yolov3.cfg`` / ``yolov3-tiny.cfg`` / ``yolov4.cfg`` /
+``yolov4-tiny.cfg``; the graph
 contract is what reference server/detector.py:135-140 requires: one input named ``input`` (f32 NCHW,
 range [0,1]) and 2 or 3 raw head maps ``[N, 3*(5+nc), S/32*k, S/32*k]``, coarsest first.
 
 The file is written with a small hand protobuf encoder (the ``onnx`` package is not installed); the
 exporter variants (BN folded or not, Resize vs Upsample, Pad+MaxPool vs padded MaxPool, initializers
-vs Constant nodes, raw vs typed tensor data, Slice vs Split for YOLOv4-tiny's channel groups) exist so the native
+vs Constant nodes, raw vs typed tensor data, Slice vs Split for YOLOv4-tiny's channel groups, one Mish node vs
+Softplus -> Tanh -> Mul for YOLOv4's activation) exist so the native
 loader is exercised on the forms real exporters emit.
 """
 from __future__ import annotations
@@ -164,6 +166,7 @@ class Layer:
     res_tail: bool = False  # conv that closes a residual branch (its output feeds a shortcut)
     groups: int = 1  # route: keep channel group `group_id` of `groups` equal groups (CSP "route groups")
     group_id: int = 0
+    mish: bool = False  # conv: Mish activation (then leaky is False)
 
 
 def yolov3_layers(num_classes: int) -> List[Layer]:
@@ -267,7 +270,59 @@ def yolov4_tiny_layers(num_classes: int) -> List[Layer]:
     return L
 
 
-ARCHS = {"full": yolov3_layers, "rsu": yolov3_layers, "tiny": yolov3_tiny_layers, "tiny4": yolov4_tiny_layers}
+def yolov4_layers(num_classes: int) -> List[Layer]:
+    """Darknet yolov4.cfg: 162 layers, 110 convs (72 Mish in the CSPDarknet53 backbone, 35 leaky in the neck, 3 linear
+    heads), an SPP block (stride-1 max-pools 5, 9, 13 of one tensor, concatenated), a PAN neck.  The cfg lists the
+    heads finest first; build_onnx emits them coarsest first, as the reference's decoder expects."""
+    L: List[Layer] = []
+    head_c = 3 * (5 + num_classes)
+
+    def conv(f, k, s=1, act="mish", res_tail=False):
+        L.append(Layer("conv", f, k, s, leaky=act == "leaky", mish=act == "mish", res_tail=res_tail))
+
+    def route(*frm):
+        L.append(Layer("route", frm=frm))
+
+    def shortcut():
+        L.append(Layer("shortcut", frm=(-3,)))
+
+    conv(32, 3)                                   # 0
+    conv(64, 3, 2)                                # 1
+    conv(64, 1); route(-2); conv(64, 1)           # 2-4
+    conv(32, 1); conv(64, 3, res_tail=True); shortcut()  # 5-7
+    conv(64, 1); route(-1, -7); conv(64, 1)       # 8-10
+    for c, reps, back in ((128, 2, -10), (256, 8, -28), (512, 8, -28), (1024, 4, -16)):  # ends at 23, 54, 85, 104
+        conv(c, 3, 2)
+        conv(c // 2, 1); route(-2); conv(c // 2, 1)
+        for _ in range(reps):
+            conv(c // 2, 1); conv(c // 2, 3, res_tail=True); shortcut()
+        conv(c // 2, 1); route(-1, back); conv(c, 1)
+    lk = "leaky"
+    conv(512, 1, act=lk); conv(1024, 3, act=lk); conv(512, 1, act=lk)   # 105-107
+    for i, k in enumerate((5, 9, 13)):                                  # SPP, 108-113
+        if i:
+            route(-2 * i)
+        L.append(Layer("maxpool", size=k, stride=1))
+    route(-1, -3, -5, -6)
+    conv(512, 1, act=lk); conv(1024, 3, act=lk); conv(512, 1, act=lk)   # 114-116
+    for c, lateral in ((256, 85), (128, 54)):                           # 117-126, 127-136
+        conv(c, 1, act=lk); L.append(Layer("upsample", stride=2)); route(lateral); conv(c, 1, act=lk); route(-1, -3)
+        for _ in range(2):
+            conv(c, 1, act=lk); conv(2 * c, 3, act=lk)
+        conv(c, 1, act=lk)
+    for c, back in ((128, None), (256, -16), (512, -37)):              # heads at 52, 26, 13 (finest first, as in the cfg)
+        if back is not None:
+            route(-4); conv(c, 3, 2, act=lk); route(-1, back)
+            for _ in range(2):
+                conv(c, 1, act=lk); conv(2 * c, 3, act=lk)
+            conv(c, 1, act=lk)
+        conv(2 * c, 3, act=lk)
+        L.append(Layer("conv", head_c, 1, 1, bn=False, leaky=False))
+        L.append(Layer("yolo"))
+    return L
+
+
+ARCHS = {"full": yolov3_layers, "rsu": yolov3_layers, "tiny": yolov3_tiny_layers, "tiny4": yolov4_tiny_layers, "v4": yolov4_layers}
 
 
 def conv_gflops(arch: str, num_classes: int, size: int) -> float:
@@ -315,11 +370,19 @@ class ExportOptions:
     opset: int = 11
     split_op: str = "Slice"  # route groups: "Slice" (constant starts / ends inputs) | "Split" (sizes as the `split`
     # attribute below opset 13, as an input from 13 on)
+    mish_op: str = "Mish"  # Mish layers: "Mish" (the ONNX op, opset 18) | "softplus" (Softplus -> Tanh -> Mul, as torch's
+    # exporter writes nn.Mish at opsets below 18)
+    mish_as_leaky: bool = False  # the same graph with LeakyRelu(0.1) in place of every Mish (the A/B twin for timing)
 
 
 def _he_sigma(fan_in: int) -> float:
     # variance-preserving for LeakyReLU(0.1): E[f(x)^2] = (1 + 0.01)/2 * var
     return float(np.sqrt(2.0 / (1.01 * fan_in)))
+
+
+def _he_sigma_mish(fan_in: int) -> float:
+    # variance-preserving for Mish: E[mish(x)^2] = 0.452 * var for x ~ N(0, var)
+    return float(np.sqrt(1.0 / (0.452 * fan_in)))
 
 
 def _leaky(x):
@@ -328,7 +391,7 @@ def _leaky(x):
 
 def build_onnx(arch: str, num_classes: int, size: int = 416, seed: int = 0,
                opts: Optional[ExportOptions] = None) -> bytes:
-    """Serialized ModelProto for `arch` in {"tiny", "full", "rsu", "tiny4"} with seeded random weights.
+    """Serialized ModelProto for `arch` in {"tiny", "full", "rsu", "tiny4", "v4"} with seeded random weights.
 
     Weights are the SURVEY §8d recipe — He-normal convs, BatchNorm gamma~U(.8,1.2), beta~N(0,.1),
     mean~N(0,.1), var~U(.8,1.2) — followed by one scalar per layer, fitted on two synthetic frames: each
@@ -375,7 +438,8 @@ def build_onnx(arch: str, num_classes: int, size: int = 416, seed: int = 0,
                 tag = f"conv{n_conv}"
                 fan_in = c * l.size * l.size
                 pad = l.size // 2
-                w = rng.normal(0.0, _he_sigma(fan_in), size=(l.filters, c, l.size, l.size)).astype(np.float32)
+                sigma = _he_sigma_mish(fan_in) if l.mish and not opts.mish_as_leaky else _he_sigma(fan_in)
+                w = rng.normal(0.0, sigma, size=(l.filters, c, l.size, l.size)).astype(np.float32)
                 conv_attrs = dict(dilations=[1, 1], group=1, kernel_shape=[l.size, l.size],
                                   pads=[pad, pad, pad, pad], strides=[l.stride, l.stride])
                 out = f"{tag}_out"
@@ -388,7 +452,8 @@ def build_onnx(arch: str, num_classes: int, size: int = 416, seed: int = 0,
                     inv = 1.0 / np.sqrt(var + np.float32(opts.bn_eps))
                     y = (raw - torch.from_numpy(mean).view(1, -1, 1, 1)) * torch.from_numpy(gamma * inv).view(1, -1, 1, 1) \
                         + torch.from_numpy(beta).view(1, -1, 1, 1)
-                    a = F.leaky_relu(y, 0.1) if l.leaky else y
+                    mish = l.mish and not opts.mish_as_leaky
+                    a = F.mish(y) if mish else F.leaky_relu(y, 0.1) if (l.leaky or l.mish) else y
                     target = 1.0
                     if l.res_tail:
                         target = 0.3 * rms(acts[i - 2])  # the stream this branch is added to (shortcut from -3)
@@ -434,7 +499,17 @@ def build_onnx(arch: str, num_classes: int, size: int = 416, seed: int = 0,
                     add_const(f"{tag}_b", b)
                     nodes.append(node_proto("Conv", [cur, f"{tag}_w", f"{tag}_b"], [out], name=tag,
                                             packed=opts.packed_attrs, **conv_attrs))
-                if l.leaky:
+                if l.mish and not opts.mish_as_leaky:
+                    if opts.mish_op == "Mish":
+                        nodes.append(node_proto("Mish", [out], [f"{tag}_act"], name=tag + "_mish"))
+                    elif opts.mish_op == "softplus":
+                        nodes.append(node_proto("Softplus", [out], [f"{tag}_sp"], name=tag + "_softplus"))
+                        nodes.append(node_proto("Tanh", [f"{tag}_sp"], [f"{tag}_tanh"], name=tag + "_tanh"))
+                        nodes.append(node_proto("Mul", [out, f"{tag}_tanh"], [f"{tag}_act"], name=tag + "_mish"))
+                    else:
+                        raise ValueError(opts.mish_op)
+                    out = f"{tag}_act"
+                elif l.leaky or l.mish:
                     nodes.append(node_proto("LeakyRelu", [out], [f"{tag}_act"], name=tag + "_leaky", alpha=0.1))
                     out = f"{tag}_act"
                 cur, c, s, x = out, l.filters, s // l.stride, a
@@ -491,7 +566,12 @@ def build_onnx(arch: str, num_classes: int, size: int = 416, seed: int = 0,
                 x = x.repeat_interleave(2, dim=2).repeat_interleave(2, dim=3)
             elif l.kind == "maxpool":
                 out = f"pool{i}_out"
-                if l.stride == 1:
+                if l.stride == 1 and l.size % 2:  # SPP: "same" padding of (k-1)/2 on every side
+                    p = l.size // 2
+                    nodes.append(node_proto("MaxPool", [cur], [out], name=f"pool{i}", packed=opts.packed_attrs,
+                                            kernel_shape=[l.size, l.size], pads=[p, p, p, p], strides=[1, 1]))
+                    x = F.max_pool2d(x, l.size, 1, p)
+                elif l.stride == 1:
                     if opts.pool_pad == "pad_node":
                         pads = np.array([0, 0, 0, 0, 0, 0, 1, 1], np.int64)
                         add_const(f"pool{i}_pads", pads)
@@ -519,13 +599,17 @@ def build_onnx(arch: str, num_classes: int, size: int = 416, seed: int = 0,
             spatial.append(s)
             acts.append(x)
 
+    if arch == "v4":
+        outputs.reverse()  # coarsest first: the reference pairs graph output i with ANCHORS[3][i]
     graph = b"".join(_f_bytes(1, n) for n in nodes)
-    graph += _f_str(2, "yolov4-tiny" if arch == "tiny4" else f"yolov3-{arch}")
+    graph += _f_str(2, {"tiny4": "yolov4-tiny", "v4": "yolov4"}.get(arch, f"yolov3-{arch}"))
     graph += b"".join(_f_bytes(5, t) for t in inits)
     graph += _f_bytes(11, value_info("input", (opts.batch, 3, size, size)))
     for name, shape in outputs:
         graph += _f_bytes(12, value_info(name, shape))
     opset = opts.opset if opts.upsample_op == "Resize" else 9
+    if any(l.mish for l in layers) and opts.mish_op == "Mish" and not opts.mish_as_leaky:
+        opset = max(opset, 18)  # (the Mish operator's first opset; Resize and MaxPool keep their meaning there)
     return model_proto(graph, opset)
 
 

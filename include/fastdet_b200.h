@@ -79,7 +79,7 @@ typedef struct fd_info {
 typedef struct fd_layer_desc {
     int32_t kind; /* 0 first conv (u8 in), 1 conv (tcgen05), 2 maxpool, 3 copy/upsample */
     int32_t c, h, w;                /* output tensor, per frame */
-    int32_t cin, ksize, stride, act, has_residual, upsample2x, out_fp32, block_n;
+    int32_t cin, ksize, stride, act, has_residual, upsample2x, out_fp32, block_n;  /* act: 0 linear, 1 LeakyReLU, 2 Mish */
     double flops;                   /* per frame */
     char name[96];                  /* ONNX node name */
     char out_name[96];              /* ONNX tensor name the output corresponds to */
@@ -98,6 +98,8 @@ typedef struct fd_layer_desc {
 #define FD_KERNEL_STEM 8          /* conv_stem_kernel: normalise + first conv + second (stride-2) conv in one kernel; reported for the second */
 #define FD_KERNEL_FUSED_NEXT 9    /* no launch of its own: computed inside the next layer's kernel (FD_KERNEL_STEM / FD_KERNEL_BLOCK) */
 #define FD_KERNEL_BLOCK 10        /* conv_block_kernel: 1x1 + 3x3 + residual of one block in one kernel; reported for the 3x3 */
+#define FD_KERNEL_SPP 11          /* spp_kernel: the stride-1 max-pools of one tensor into one Concat, one launch; reported for the
+                                     group's last pool, the others report FD_KERNEL_FUSED_NEXT (pool.cu) */
 typedef struct fd_layer_exec {
     int32_t kernel;       /* FD_KERNEL_* */
     int32_t bucket;       /* batch-size bucket whose execution state answered (n rounded up) */
